@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (torchrun launches N ranks for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm (numpy oracle port) on host cores
+    python bench.py ... --dump-outputs DIR                   # also writes the last timed step's results as DIR/*.npy
 
 Workload ("step") = BASELINE config 5 IN FULL: F-matrix RANSAC over 4096 synthetic image pairs x 50 000 correspondences x
 8 192 hypotheses (30 % outliers, thr 1.5 px): hypotheses sampled and solved (8-point), every hypothesis scored against
@@ -302,7 +303,9 @@ def run_ours(args) -> None:
     prof = rt.profile(device=local, stream=stream)
     rt.set_option(1, 0, device=local)
     stats = rt.last_stats(device=local, stream=stream)
-    res_dev = sh.unpack(sh.gather(masks=False))                             # the last device-resident step's answer
+    res_dev = sh.unpack(sh.gather(masks=bool(args.dump_outputs)))           # the last device-resident step's answer
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, res_dev)
     ms_e2e, win_e2e = timed(step_host, args.steps)
     # the same step with the passes strictly one after the other on one stream (option 10 = 0): the scorer ALONE on the GPU.
     # In the timed region above the solver of the next pass and the fix-up / selection / masks of the previous one run beside
@@ -434,6 +437,24 @@ def run_ours(args) -> None:
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: str, res: dict) -> None:
+    """Writes what the last timed step returned to its caller as DIR/<name>.npy (float64, the inlier masks float32), so that
+    two builds can be compared output for output on the same seeded inputs.  Under 60 MB in all: the per-pair results of
+    every pair (a sample of 100 000 pairs beyond that) and the masks of 128 pairs (at most 4M entries).  The samples are
+    drawn from a fixed seed, so the same arguments select the same pairs and points."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    P, N = len(res["best_idx"]), len(res["mask"][0])
+    pairs = np.arange(P) if P <= 100_000 else np.sort(rng.choice(P, 100_000, replace=False))
+    rows = np.sort(rng.choice(P, min(P, 128), replace=False))
+    cols = np.arange(N) if len(rows) * N <= 1 << 22 else np.sort(rng.choice(N, (1 << 22) // len(rows), replace=False))
+    out = {"pair_ids": pairs, "best_idx": res["best_idx"][pairs], "best_count": res["best_count"][pairs],
+           "F": res["F"][pairs], "mask_pair_ids": rows, "mask_point_ids": cols}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+    np.save(os.path.join(out_dir, "mask.npy"), np.stack([res["mask"][r][cols] for r in rows]).astype(np.float32))
 
 
 def check_first_pairs(args, rg, rt, philox, synth, sh, res_dev, torch) -> dict:
@@ -1040,7 +1061,10 @@ def main() -> None:
     ap.add_argument("--no-split", action="store_true", help="skip the hypothesis-split legs (configs 3 and 4)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-oracle-check", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup_raised = args.impl == "ours" and args.warmup < 3
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup      # timing rules: W >= 3 (noted in config)
     try:

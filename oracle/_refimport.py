@@ -1,6 +1,6 @@
-"""TEST INFRASTRUCTURE ONLY — imports the *unmodified* reference modules from /root/reference.
+"""TEST INFRASTRUCTURE ONLY — imports the *unmodified* reference modules from the directory named by RG_REFERENCE_DIR.
 
-Only usable in the build container (``/root/reference`` is not present on the GPU box).  Used by
+Only usable where a checkout of the original project is available; point RG_REFERENCE_DIR at it.  Used by
 ``oracle/gen_golden.py`` (fixture generation) and by ``tests/test_oracle_vs_reference.py`` (pins the
 numpy restatements in ``oracle/`` against the real reference code).
 
@@ -14,11 +14,11 @@ import os
 import sys
 import types
 
-REFERENCE_DIR = os.environ.get("RG_REFERENCE_DIR", "/root/reference")
+REFERENCE_DIR = os.environ.get("RG_REFERENCE_DIR", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_DIR, "lab3.py"))
+    return bool(REFERENCE_DIR) and os.path.isfile(os.path.join(REFERENCE_DIR, "lab3.py"))
 
 
 def _stub_matplotlib() -> None:

@@ -1,7 +1,7 @@
 """TEST INFRASTRUCTURE ONLY — generates tests/golden/*.npz by running the UNMODIFIED reference code.
 
-Run in the build container (needs /root/reference):   python -m oracle.gen_golden
-The fixtures travel to the GPU box, where /root/reference does not exist.
+Run with RG_REFERENCE_DIR set to the original project's source tree:   python -m oracle.gen_golden
+Apart from tests/test_oracle_vs_reference.py, the tests read these fixtures and never the original project.
 
 What is recorded
   dino_data.npz      the reference's own input data (BAdino2.mat cameras / 3-D points / clean 2-D tracks, the noisy

@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY — generates tests/golden/ba_golden.npz by running the UNMODIFIED reference bundle adjustment.
 
-Run in the build container (needs /root/reference):   python -m oracle.gen_golden_ba
+Run with RG_REFERENCE_DIR set to the original project's source tree:   python -m oracle.gen_golden_ba
 (kept apart from gen_golden.py, whose gold-standard stage alone runs for several minutes).
 
 The reference's ``Tables()`` constructor loads ``../images/*.ppm`` (fun.getImages, fun.py:59,71 — not in the repository),

@@ -152,6 +152,15 @@ def test_gs_oracle_residuals_and_start_point_match_reference_golden(gs_golden):
         ogs.fmatrix_residuals_gs(g["params0"][:-3], g["in1"], g["in2"])
 
 
+def test_package_host_helpers_match_reference_golden(gs_golden, rg):
+    """The package's lab3 mirror at the reference's own gold-standard start point: lab3.fmatrix_cameras of the RANSAC
+    winner and lab3.fmatrix_residuals_gs, as the reference computed them (oracle/gen_golden.py)."""
+    g = gs_golden
+    C1, _ = rg.lab3.fmatrix_cameras(g["F0"])
+    assert np.allclose(C1.ravel(), g["params0"][:12], rtol=1e-12, atol=1e-15)
+    assert np.allclose(rg.lab3.fmatrix_residuals_gs(g["params0"], g["in1"], g["in2"]), g["resid0"], rtol=1e-12, atol=1e-12)
+
+
 def test_gs_dense_lm_beats_the_reference_stopping_point(gs_golden):
     """The reference's SciPy run stops on ftol at cost 8.288 after 5482 residual evaluations; the LM / Schur iteration
     that the CUDA path implements reaches 5.7407 in ~10 iterations.  F_gold stays within the tolerance of the LM stage."""

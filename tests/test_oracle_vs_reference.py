@@ -1,12 +1,15 @@
 """Pins the oracle restatements and the package's numpy host helpers against the UNMODIFIED reference code, imported
-from /root/reference.  Runs only where the reference tree is mounted (the build container); skipped on the GPU box."""
+from the original project's source tree named by RG_REFERENCE_DIR.  Skipped where that tree is not available; the
+golden vectors under tests/golden/ (tests/test_oracle_golden.py) pin the oracle's F, triangulation, pose and
+resectioning functions without it."""
 import numpy as np
 import pytest
 
 from oracle import _refimport as ri
 from oracle import f_path as orc
 
-pytestmark = pytest.mark.skipif(not ri.reference_available(), reason="/root/reference not mounted")
+pytestmark = pytest.mark.skipif(not ri.reference_available(),
+                                reason="original project not available (set RG_REFERENCE_DIR to its source tree)")
 
 
 @pytest.fixture(scope="module")
