@@ -64,7 +64,9 @@ int rg_host_free(void* p);
  *            evaluations to the FP64 recheck (results do not depend on it); measures the fix-up cost of a less accurate scorer
  * option 10 = pass pipelining of F calls that run in several passes (default 1): the fix-up / selection / mask kernels of
  *            pass k run on a second stream while pass k+1 is solved and scored; 0 = one stream, strictly in order
- *            (results do not depend on it; the caller's stream sees the whole call complete either way) */
+ *            (results do not depend on it; the caller's stream sees the whole call complete either way)
+ * option 11 = test hook: 1 = refinement of PnP poses (rg_pnp_refine_*) always on the multi-CTA path (default: views of
+ *            <= 4096 correspondences run the whole loop in one CTA); same iteration, sums in a different order */
 int rg_set_option(void* ctx, int option, long long value);
 /* summed milliseconds of {prepare, solve, score kernel, fixup + repair, select} over the PASSES since the last read
  * (at most 2048 passes are remembered; *out_calls = passes covered); synchronises `stream` */
@@ -188,6 +190,33 @@ int rg_pnp_minimize_host(void* ctx, void* stream, int m, const double* X, const 
 /* reprojection scoring of H caller-supplied poses (H x 12: R row-major then t) — ransac.py:96-105 */
 int rg_pnp_score_count_host(void* ctx, void* stream, int N, const double* X, const double* y, int H, const double* poses,
                             double thr2, int score_path, int32_t* counts);
+
+/* ---- refinement of PnP poses (DESIGN.md section 4.7) ------------------------------------------------------------ */
+/* The reference's live PnP call is OpenCV's cv.solvePnPRansac (tables.py:141), which ends with solvePnP(ITERATIVE,
+ * useExtrinsicGuess) on the inliers: a Levenberg-Marquardt minimisation of the reprojection error.  The RANSAC above
+ * returns the algebraic DLT pose of pnp.py:132-152; this minimises, per view v over its selected correspondences,
+ *   C_v(R, t) = 1/2 sum_k |W_v (pi(R X_k + t) - y_k)|^2,  pi(p) = (p0/p2, p1/p2),  W_v = K_v[:2, :2] (fx, s; 0, fy) or I
+ * (the principal point cancels; with K the cost is in pixels) over R <- exp([dw]_x) R and t <- t + dt, batched over V
+ * views, no host synchronisation.  Views of <= 4096 correspondences run the whole loop in one CTA (option 11 = 1 forces
+ * the multi-CTA path of larger views); sums in a fixed order, bit-reproducible.
+ *   X (view_off[V], 3), y (view_off[V], 2) C-normalised, view_off HOST int32 CSR table (layout of rg_pnp_ransac_batched_*)
+ *   K : V x 9 row-major on the HOST (NULL = W = I); -2 unless K[1][0] == 0 and the bottom row is (0, 0, 1)
+ *   mask (optional) selects the correspondences of the first round, e.g. the mask of rg_pnp_ransac_batched_dev
+ *   Rt (V x 12, R row-major then t, as rg_pnp_ransac_* write it) is refined IN PLACE
+ *   rounds >= 1: after every round the consensus thr2 >= e at the refined pose (ransac.py:104-105, FP64, C-normalised
+ *   units) is recomputed over all correspondences and the next round refines on it; mask_out (optional) receives the
+ *   last consensus; thr2 is required when rounds > 1 or mask_out is given
+ * Outputs of the last round (optional): cost = C_v at the returned pose; iters; status: 1 = start pose not finite,
+ * 2 = converged (relative decrease <= ftol, actual or predicted), 3 = lambda > 1e12, 4 = max_iter reached, 5 = fewer than
+ * 3 selected correspondences (pose unchanged). */
+int rg_pnp_refine_dev(void* ctx, void* stream, int V, const double* X_dev, const double* y_dev, const int32_t* view_off_host,
+                      const double* K_host, const unsigned char* mask_dev, double* Rt_dev, int max_iter, double ftol,
+                      int rounds, double thr2, unsigned char* mask_out_dev, double* cost_dev, int32_t* iters_dev,
+                      int32_t* status_dev);
+/* the same with host buffers: uploads, calls the above, downloads, synchronises `stream` */
+int rg_pnp_refine_host(void* ctx, void* stream, int V, const double* X, const double* y, const int32_t* view_off,
+                       const double* K, const unsigned char* mask, double* Rt, int max_iter, double ftol, int rounds,
+                       double thr2, unsigned char* mask_out, double* cost, int32_t* iters, int32_t* status);
 
 /* ---- two-view geometry either side of the RANSAC path (SURVEY.md section 8f, rows N1-N3), all FP64 -------------- */
 #define RG_TRI_OPTIMAL 0    /* lab3.triangulate_optimal (lab3.py:382-475): Hartley-Sturm, degree-6 root solve per point */

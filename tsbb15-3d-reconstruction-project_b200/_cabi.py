@@ -73,6 +73,8 @@ SIGNATURES = {
     "rg_camera_resectioning_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rg_gold_standard_host": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
     "rg_gold_standard_dev": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
+    "rg_pnp_refine_host": (_i, [_vp, _vp, _i, _vp, _vp, _pi, _vp, _vp, _vp, _i, _d, _i, _d, _vp, _vp, _vp, _vp]),
+    "rg_pnp_refine_dev": (_i, [_vp, _vp, _i, _vp, _vp, _pi, _vp, _vp, _vp, _i, _d, _i, _d, _vp, _vp, _vp, _vp]),
     "rg_fmatrix_residuals_gs_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rg_bundle_adjust_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _pi, _pi, _i, _i, _d, _vp, _vp, _vp]),
     "rg_bundle_adjust_dev": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _pi, _pi, _i, _i, _d, _vp, _vp, _vp]),

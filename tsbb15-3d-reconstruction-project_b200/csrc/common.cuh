@@ -226,6 +226,10 @@ struct Ctx {
     int opt_ba_cluster = 0;                        // option 3: CTAs in the cluster of the camera-system factorisation (0 = 8)
     int opt_gs_multi = 0;                          // option 5: 1 = gold standard always on the multi-kernel path (no gs_fused)
     int opt_ba_l2 = 0;                             // option 4: 1 = keep the camera system in L2 (ba_solve) even when it fits in DSMEM
+    Buffer pr_ws;                                  // refinement of PnP poses: per-view state, per-block partials, offsets, weights
+    int opt_pr_multi = 0;                          // option 11: 1 = PnP pose refinement always on the multi-CTA path
+    Buffer h_pr_flags;                             // pinned: views still running after every iteration (host entry point)
+    cudaEvent_t pr_iter_ev[2] = {nullptr, nullptr};
     Buffer h_ba_items;                             // pinned: work items of ba_blocks (blocks with a common point x segments)
     Buffer h_ba_flags;                             // pinned: the solver's `done` flag after every iteration (host entry point)
     cudaEvent_t ba_iter_ev[2] = {nullptr, nullptr};

@@ -117,7 +117,7 @@ int rg_shutdown(void* ctx) {
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     for (Buffer* b : {&c->pair_info, &c->pair_frame, &c->state, &c->bbox, &c->pts32, &c->F64, &c->hyp32, &c->flags,
-                      &c->flag_list, &c->gen_idx, &c->stats, &c->best, &c->tie_stats, &c->d_in_a, &c->d_in_b, &c->d_in_c, &c->geom, &c->geom_ws, &c->gs_ws, &c->ba_ws, &c->d_out_a, &c->d_out_b,
+                      &c->flag_list, &c->gen_idx, &c->stats, &c->best, &c->tie_stats, &c->d_in_a, &c->d_in_b, &c->d_in_c, &c->geom, &c->geom_ws, &c->gs_ws, &c->ba_ws, &c->pr_ws, &c->d_out_a, &c->d_out_b,
                       &c->d_out_c, &c->d_out_d, &c->pose64, &c->pose32, &c->X32})
         release(*b);
     for (Buffer* b : {&c->alt.pair_info, &c->alt.pair_frame, &c->alt.state, &c->alt.pts32, &c->alt.F64, &c->alt.hyp32,
@@ -135,8 +135,11 @@ int rg_shutdown(void* ctx) {
     release_pinned(c->h_stats);
     release_pinned(c->h_ba_flags);
     release_pinned(c->h_ba_items);
-    for (int i = 0; i < 2; ++i)
+    release_pinned(c->h_pr_flags);
+    for (int i = 0; i < 2; ++i) {
         if (c->ba_iter_ev[i]) cudaEventDestroy(c->ba_iter_ev[i]);
+        if (c->pr_iter_ev[i]) cudaEventDestroy(c->pr_iter_ev[i]);
+    }
     if (c->prof_ev) {
         for (int i = 0; i < Ctx::kProfRing * Ctx::kProfEvents; ++i) cudaEventDestroy(c->prof_ev[i]);
         delete[] c->prof_ev;
@@ -183,6 +186,8 @@ int rg_device_sm_count(void* ctx) { return ctx ? ((Ctx*)ctx)->sm_count : 0; }
 // option 8: test hook: capacity of the guard-band flag list in records (0 = automatic); a tiny value forces the FP64 recount
 // option 10: 1 (default) = in F calls of several passes the fix-up / selection / mask kernels of pass k run on a second
 //           stream while pass k+1 is solved and scored (two sets of per-pass workspaces); 0 = strictly one after the other
+// option 11: 1 = refinement of PnP poses always on the multi-CTA path (default: views of <= 4096 correspondences run the whole
+//           Levenberg-Marquardt loop in one CTA, one launch per round); test hook comparing the two paths
 // option 9: guard-band safety factor x 1000 (default 1000 = the proven FP32 rounding bound); larger values keep every result
 //           exact and only send more evaluations to the FP64 recheck — used to MEASURE what a less accurate scorer
 //           (tensor-core split-precision accumulation) would cost in fix-up time
@@ -244,6 +249,11 @@ int rg_set_option(void* ctx, int option, long long value) {
     if (option == 10) {
         if (value != 0 && value != 1) { set_error("invalid argument: option 10 (pass pipelining) must be 0 or 1"); return RG_ERR_ARG; }
         c->opt_pipeline = (int)value;
+        return RG_OK;
+    }
+    if (option == 11) {
+        if (value != 0 && value != 1) { set_error("invalid argument: option 11 (PnP refinement path) must be 0 or 1"); return RG_ERR_ARG; }
+        c->opt_pr_multi = (int)value;
         return RG_OK;
     }
     if (option == 8) {

@@ -5,6 +5,7 @@
 #include "pnp_api.cu"
 #include "geom_api.cu"
 #include "gs_api.cu"
+#include "pnp_refine_api.cu"
 #include "ba_api.cu"
 #include "nccl_api.cu"
 #include "p2p_api.cu"

@@ -149,6 +149,63 @@ def pnp_ransac(d_X, d_y, view_off, d_idx, hyp_off, out: PnpOutputs, thr2, n=6, n
     return out
 
 
+def _check_dense(t, name, dtype, tail=(), rows=None):
+    """The kernels index raw device pointers: a tensor must be a contiguous CUDA tensor of the expected dtype and shape
+    (a strided view, e.g. torch.from_numpy of a Fortran-ordered array, would be read in the wrong order)."""
+    torch = _torch()
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == dtype and t.is_contiguous()):
+        raise ValueError(f"{name} must be a contiguous CUDA tensor of dtype {dtype}")
+    if tuple(t.shape[1:]) != tuple(tail) or (rows is not None and t.shape[0] < rows):
+        raise ValueError(f"{name} must have shape (>= {rows}, {', '.join(map(str, tail))})" if tail else
+                         f"{name} must have at least {rows} elements")
+
+
+class PnpRefineOutputs:
+    """Device outputs of pnp_refine: per view cost (float64), iters and status (int32)."""
+
+    def __init__(self, V: int, device=None):
+        torch = _torch()
+        dev = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+        self.cost = torch.empty(max(V, 1), dtype=torch.float64, device=dev)
+        self.iters = torch.empty(max(V, 1), dtype=torch.int32, device=dev)
+        self.status = torch.empty(max(V, 1), dtype=torch.int32, device=dev)
+
+
+def pnp_refine(d_X, d_y, view_off, out: PnpOutputs, d_mask=None, K=None, max_iter=50, ftol=1e-12, rounds=1, thr2=None,
+               mask_out=None, res: PnpRefineOutputs | None = None):
+    """rg_pnp_refine_dev: refines ``out.Rt`` IN PLACE on the current stream (Levenberg-Marquardt on the reprojection
+    error, see runtime.pnp_refine_batched).  ``pnp_ransac(...)`` then ``pnp_refine(..., d_mask=out.mask)`` is the chained
+    form: no host synchronisation between the two.  K: HOST (3, 3) or (V, 3, 3) array (validated before anything is
+    enqueued).  mask_out (uint8 CUDA tensor, may be out.mask) receives the last consensus (needs thr2).  Returns ``res``
+    (allocated when None)."""
+    from . import runtime
+    lib = cabi.load_library()
+    V = len(view_off) - 1
+    if int(rounds) > 1 and thr2 is None:
+        raise ValueError("rounds > 1 needs thr2 (the consensus threshold)")
+    if mask_out is not None and thr2 is None:
+        raise ValueError("mask_out needs thr2 (the consensus threshold)")
+    torch = _torch()
+    n = int(view_off[-1]) if V else 0
+    _check_dense(d_X, "d_X", torch.float64, (3,), n)
+    _check_dense(d_y, "d_y", torch.float64, (2,), n)
+    _check_dense(out.Rt, "out.Rt", torch.float64, (12,), V)
+    if d_mask is not None:
+        _check_dense(d_mask.reshape(-1), "d_mask", torch.uint8, (), n)
+    if mask_out is not None:
+        _check_dense(mask_out.reshape(-1), "mask_out", torch.uint8, (), n)
+    Kt = runtime.pnp_k_table(K, V)
+    if res is None:
+        res = PnpRefineOutputs(V, device=_dev_index(d_X))
+    cabi.check(lib.rg_pnp_refine_dev(
+        _vp(cabi.context(_dev_index(d_X))), _vp(_stream()), V, _vp(d_X.data_ptr()), _vp(d_y.data_ptr()),
+        view_off.ctypes.data_as(_pi32), _vp(cabi.ptr(Kt)), _vp(d_mask.data_ptr()) if d_mask is not None else None,
+        _vp(out.Rt.data_ptr()), int(max_iter), float(ftol), int(rounds), float(thr2) if thr2 is not None else 0.0,
+        _vp(mask_out.data_ptr()) if mask_out is not None else None, _vp(res.cost.data_ptr()), _vp(res.iters.data_ptr()),
+        _vp(res.status.data_ptr())))
+    return res
+
+
 class P2PExchange:
     """The cross-GPU argmax of the hypothesis-split mode as ONE kernel over NVLink peer memory (csrc/p2p_api.cu) instead of
     NCCL collectives.  Collective constructor: every rank of ``group`` builds it at the same point; the 64-byte CUDA IPC

@@ -63,7 +63,7 @@ def _as_pairs(D, name):
     return D
 
 
-def ransac_robust(D_med, D_high, r, thresh, n, sample_idx=None, seed=None):
+def ransac_robust(D_med, D_high, r, thresh, n, sample_idx=None, seed=None, refine=False):
     """RANSAC estimation of the camera pose.
 
     D_med, D_high : (N, 2, 3) correspondences, [:, 0] = C-normalised homogeneous image point, [:, 1] = 3D point
@@ -72,6 +72,9 @@ def ransac_robust(D_med, D_high, r, thresh, n, sample_idx=None, seed=None):
     n             : sample size; n >= 6 uses the DLT pose of pnp.pnp_minimize (6, 7 or 8)
     sample_idx    : optional (r, n) host-drawn indices into D_high (otherwise gen_rnd_indices is called r times; with
                     ``seed`` the global ``random`` module is seeded first)
+    refine        : False (default): the winner's algebraic DLT pose.  True: the winner is refined on its consensus set
+                    (Levenberg-Marquardt on the reprojection error in C-normalised units, runtime.pnp_refine) and C_est
+                    is re-scored at the refined pose
     Returns R_est, t_est, C_est as one-element lists like the reference intends (:109-111): [R], [t],
     [[D_med consensus rows, D_high consensus rows]]; three empty lists if no pose has any D_med consensus."""
     if n == 3:
@@ -100,6 +103,9 @@ def ransac_robust(D_med, D_high, r, thresh, n, sample_idx=None, seed=None):
     res = _rt.pnp_ransac(X, y, sample_idx + n_med, float(thresh), n_sel=n_med, want_mask=True)
     if res["best_idx"] < 0:
         return [], [], []
-    mask = res["mask"].astype(bool)
+    R, t, mask = res["R"], res["t"], res["mask"].astype(bool)
+    if refine:
+        ref = _rt.pnp_refine(X, y, R, t, mask=mask, thr2=float(thresh))
+        R, t, mask = ref["R"], ref["t"], ref["mask"].astype(bool)
     C = [D_med[mask[:n_med]], D_high[mask[n_med:]]]
-    return [res["R"]], [res["t"]], [C]
+    return [R], [t], [C]

@@ -323,6 +323,87 @@ def pnp_minimize(X, y, device=None, stream=0):
     return R, t
 
 
+def pnp_k_table(K, V) -> np.ndarray | None:
+    """K as the (V, 9) host table of rg_pnp_refine_*: None stays None, one (3, 3) is shared by every view."""
+    if K is None:
+        return None
+    K = _f64(K)
+    if K.shape == (3, 3):
+        K = np.broadcast_to(K, (V, 3, 3))
+    if K.shape != (V, 3, 3):
+        raise ValueError("K must be (3, 3) or (V, 3, 3)")
+    if np.any(K[:, 1, 0] != 0.0) or np.any(K[:, 2] != np.array([0.0, 0.0, 1.0])):
+        raise ValueError("K must have K[1, 0] == 0 and bottom row (0, 0, 1)")
+    return np.ascontiguousarray(K.reshape(V, 9))
+
+
+def pnp_refine_batched(X_list, y_list, R, t, masks=None, K=None, max_iter=50, ftol=1e-12, rounds=1, thr2=None,
+                       device=None, stream=0) -> dict:
+    """Levenberg-Marquardt refinement of V PnP poses in ONE library call (rg_pnp_refine_host): per view, the minimum of
+    1/2 sum |W (pi(R X + t) - y)|^2 over the selected correspondences, W = K[:2, :2] (cost in pixels) or I.
+    X_list[v] (N_v, 3), y_list[v] (N_v, 2) C-normalised; R (V, 3, 3), t (V, 3) start poses; masks[v] optional selection;
+    K (3, 3) or (V, 3, 3).  rounds > 1: re-score the consensus thr2 >= e at the refined pose and refine again on it.
+    Returns dict(R, t, cost, iters, status) of the last round, plus the list ``mask`` of last consensus sets when thr2 is
+    given.  status: 1 start pose not finite, 2 converged, 3 lambda > 1e12, 4 max_iter, 5 fewer than 3 points."""
+    V = len(X_list)
+    if len(y_list) != V:
+        raise ValueError("X_list and y_list must have the same length")
+    Xs = [_f64(a).reshape(-1, 3) for a in X_list]
+    ys = [_f64(a).reshape(-1, 2) for a in y_list]
+    view_off = np.zeros(V + 1, dtype=np.int32)
+    for v in range(V):
+        if Xs[v].shape[0] != ys[v].shape[0]:
+            raise ValueError(f"view {v}: X and y must have the same number of rows")
+        view_off[v + 1] = view_off[v] + Xs[v].shape[0]
+    R = _f64(R).reshape(-1, 3, 3)
+    t = _f64(t).reshape(-1, 3)
+    if R.shape[0] != V or t.shape[0] != V:
+        raise ValueError("R must be (V, 3, 3) and t (V, 3)")
+    if int(rounds) < 1:
+        raise ValueError("rounds must be >= 1")
+    if int(rounds) > 1 and thr2 is None:
+        raise ValueError("rounds > 1 needs thr2 (the consensus threshold)")
+    N = int(view_off[-1])
+    X = np.ascontiguousarray(np.concatenate(Xs)) if V else np.zeros((0, 3))
+    y = np.ascontiguousarray(np.concatenate(ys)) if V else np.zeros((0, 2))
+    mask = None
+    if masks is not None:
+        if len(masks) != V or any(len(m) != Xs[v].shape[0] for v, m in enumerate(masks)):
+            raise ValueError("masks must match X_list")
+        mask = np.ascontiguousarray(np.concatenate([np.asarray(m, dtype=bool).astype(np.uint8) for m in masks])) if V else None
+    Kt = pnp_k_table(K, V)
+    Rt = np.ascontiguousarray(np.concatenate([R.reshape(V, 9), t], axis=1))
+    cost = np.full(V, np.nan)
+    iters = np.zeros(V, dtype=np.int32)
+    status = np.zeros(V, dtype=np.int32)
+    mask_out = np.zeros(max(N, 1), dtype=np.uint8) if thr2 is not None else None
+    lib = cabi.load_library()
+    ctx = cabi.context(device)
+    cabi.check(lib.rg_pnp_refine_host(
+        _vp(ctx), _vp(stream), V, _vp(cabi.ptr(X)), _vp(cabi.ptr(y)), view_off.ctypes.data_as(C.POINTER(C.c_int32)),
+        _vp(cabi.ptr(Kt)), _vp(cabi.ptr(mask)), _vp(cabi.ptr(Rt)), int(max_iter), float(ftol), int(rounds),
+        float(thr2) if thr2 is not None else 0.0, _vp(cabi.ptr(mask_out)), _vp(cabi.ptr(cost)), _vp(cabi.ptr(iters)),
+        _vp(cabi.ptr(status))))
+    out = {"R": Rt[:, :9].reshape(V, 3, 3).copy(), "t": Rt[:, 9:].copy(), "cost": cost, "iters": iters, "status": status,
+           "view_off": view_off}
+    if mask_out is not None:
+        out["mask"] = [mask_out[view_off[v]:view_off[v + 1]].copy() for v in range(V)]
+    return out
+
+
+def pnp_refine(X, y, R, t, mask=None, K=None, max_iter=50, ftol=1e-12, rounds=1, thr2=None, device=None, stream=0) -> dict:
+    """pnp_refine_batched for ONE view: X (N, 3), y (N, 2), R (3, 3), t (3,), mask (N,) optional, K (3, 3) optional.
+    Returns dict(R, t, cost, iters, status[, mask])."""
+    r = pnp_refine_batched([X], [y], _f64(R).reshape(1, 3, 3), _f64(t).reshape(1, 3),
+                           masks=None if mask is None else [mask], K=K, max_iter=max_iter, ftol=ftol, rounds=rounds,
+                           thr2=thr2, device=device, stream=stream)
+    out = {"R": r["R"][0], "t": r["t"][0], "cost": float(r["cost"][0]), "iters": int(r["iters"][0]),
+           "status": int(r["status"][0])}
+    if "mask" in r:
+        out["mask"] = r["mask"][0]
+    return out
+
+
 def pnp_score_count(X, y, poses, thr2, score_path=SCORE_FP32_GUARDED, device=None, stream=0):
     lib = cabi.load_library()
     ctx = cabi.context(device)

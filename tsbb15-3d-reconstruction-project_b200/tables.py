@@ -128,13 +128,19 @@ class Tables:
         hit = _rt.match_first_within(coords, np.asarray(y1_hom, dtype=np.float64).reshape(-1, 3), 1e-4)
         return np.where(hit >= 0, obs_idx[np.maximum(hit, 0)], -1)
 
-    def addNewView(self, K, img_index, y1_hom, y2_hom, y1, y2, r=1024, reproj_px=8.0, n=6, seed=0, sample_idx=None):
+    def addNewView(self, K, img_index, y1_hom, y2_hom, y1, y2, r=1024, reproj_px=8.0, n=6, seed=0, sample_idx=None,
+                   refine="algebraic"):
         """Adds the view seen in image ``img_index``: pose from the 2D<->3D correspondences found through the last view
         (PnP-RANSAC), consensus observations appended to the tables.  Returns (A_y1, A_y2): the putative
         correspondences without a 3-D point yet, exactly as the reference does.
 
         r, reproj_px, n, seed / sample_idx : PnP-RANSAC controls (the reference relies on OpenCV's defaults: 100
-        iterations, 8 px reprojection error); reproj_px is converted to C-normalised units with K[0, 0]."""
+        iterations, 8 px reprojection error); reproj_px is converted to C-normalised units with K[0, 0].
+        refine : "algebraic" (default) refits the pose algebraically on the consensus set (runtime.pnp_minimize);
+        "lm" minimises the reprojection error in pixels with K on the consensus set (runtime.pnp_refine), the final
+        stage of OpenCV's solvePnPRansac; the consensus appended is RANSAC's, as solvePnPRansac returns it."""
+        if refine not in ("algebraic", "lm"):
+            raise ValueError("refine must be 'algebraic' or 'lm'")
         y1_hom = np.asarray(y1_hom, dtype=np.float64)
         y2_hom = np.asarray(y2_hom, dtype=np.float64)
         y1 = np.asarray(y1, dtype=np.float64)
@@ -157,7 +163,11 @@ class Tables:
             raise ValueError("addNewView: PnP-RANSAC found no pose with a non-empty consensus set")
         inl = np.flatnonzero(res["mask"])
         R, t = res["R"], res["t"]
-        if inl.size >= 6:                                   # refit on the consensus set (OpenCV refines its winner too)
+        if refine == "lm":
+            # np.triu: K of an RQ factorisation can carry rounding dust below the diagonal
+            ref = _rt.pnp_refine(D_3Dpoints, yn, R, t, mask=res["mask"], K=np.triu(np.asarray(K, dtype=np.float64)))
+            R, t = ref["R"], ref["t"]
+        elif inl.size >= 6:                                 # refit on the consensus set (OpenCV refines its winner too)
             R, t = _rt.pnp_minimize(D_3Dpoints[inl], yn[inl])
         view_index = self.addView(img_index, CameraPose(R, t))
         for yy, x in zip(D_imgcoords_hom[inl], x_i[inl]):
