@@ -99,6 +99,8 @@ def test_shard_range_and_keys(rg):
             assert rs[0][0] == 0 and rs[-1][1] == n
             assert all(rs[i][1] == rs[i + 1][0] for i in range(w - 1))
             assert max(b - a for a, b in rs) - min(b - a for a, b in rs) <= 1
+            assert [par.shard_owner(n, i, w) for i in range(n)] == [r for r, (a, b) in enumerate(rs) for _ in range(a, b)]
+            assert par.shard_owner(n, n, w) == par.shard_owner(n, -1, w) == -1
     assert par.argmax_key(10, 5) > par.argmax_key(10, 6) > par.argmax_key(9, 0)
     assert par.key_decode(par.argmax_key(123, 4567)) == (123, 4567)
 

@@ -25,11 +25,10 @@ _vp = C.c_void_p
 _i = C.c_int
 _d = C.c_double
 _pd = C.POINTER(C.c_double)
-_pi = C.POINTER(C.c_int32)
-_pu8 = C.POINTER(C.c_ubyte)
 _pll = C.POINTER(C.c_longlong)
 
-# name -> (restype, argtypes); mirrors include/rg_b200.h one to one (tests check every symbol is exported)
+# name -> (restype, argtypes); mirrors include/rg_b200.h one to one (tests check every symbol is exported).  Buffers,
+# the int32 offset tables included, are declared void*: ``call`` passes numpy arrays, tensors and addresses through ``ptr``.
 SIGNATURES = {
     "rg_abi_version": (_i, []),
     "rg_last_error": (C.c_char_p, []),
@@ -42,45 +41,45 @@ SIGNATURES = {
     "rg_get_profile": (_i, [_vp, _vp, _pd, C.POINTER(C.c_int)]),
     "rg_microbench_run": (_i, [_pd, _vp]),
     "rg_get_last_stats": (_i, [_vp, _vp, _pll]),
-    "rg_f_ransac_dev": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _pi, _d, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
-    "rg_f_ransac_dev2": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _pi, _d, _i, _i, _i, _i, _i, C.c_ulonglong, _i, _i, _vp, _vp, _vp, _vp, _vp]),
-    "rg_f_ransac_host2": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _pi, _d, _i, _i, _i, _i, C.c_ulonglong, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "rg_sample_indices_dev": (_i, [_vp, _vp, _i, _pi, _pi, _i, C.c_ulonglong, _i, _i, _vp]),
+    "rg_f_ransac_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "rg_f_ransac_dev2": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _i, C.c_ulonglong, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "rg_f_ransac_host2": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, C.c_ulonglong, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "rg_sample_indices_dev": (_i, [_vp, _vp, _i, _vp, _vp, _i, C.c_ulonglong, _i, _i, _vp]),
     "rg_synth_two_view_dev": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _vp, C.c_ulonglong, _d, _d, _d, _d, _vp, _vp]),
-    "rg_f_inlier_mask_dev": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _d, _i, _vp]),
-    "rg_pnp_ransac_batched_dev2": (_i, [_vp, _vp, _i, _vp, _vp, _pi, _pi, _vp, _pi, _i, _d, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "rg_f_inlier_mask_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _d, _i, _vp]),
+    "rg_pnp_ransac_batched_dev2": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "rg_p2p_create": (_i, [_vp, _i, _i, _vp]),
     "rg_p2p_connect": (_i, [_vp, _vp]),
     "rg_p2p_destroy": (_i, [_vp]),
     "rg_p2p_argmax_exchange": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rg_f_last_hypotheses_dev": (_i, [_vp, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp)]),
-    "rg_f_ransac_host": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _pi, _d, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "rg_f_ransac_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rg_f8pt_solve_host": (_i, [_vp, _vp, _i, _vp, _i, _vp, _i, _vp, _vp]),
     "rg_epi_score_count_host": (_i, [_vp, _vp, _i, _vp, _i, _vp, _d, _i, _i, _vp]),
     "rg_fmatrix_residuals_host": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _vp]),
     "rg_fmatrix_stls_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp]),
     "rg_pnp_ransac_host": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _vp, _d, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rg_pnp_ransac_dev": (_i, [_vp, _vp, _i, _i, _vp, _vp, _i, _i, _vp, _d, _i, _vp, _vp, _vp, _vp]),
-    "rg_pnp_ransac_batched_host": (_i, [_vp, _vp, _i, _vp, _vp, _pi, _pi, _vp, _pi, _i, _d, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "rg_pnp_ransac_batched_dev": (_i, [_vp, _vp, _i, _vp, _vp, _pi, _pi, _vp, _pi, _i, _d, _i, _vp, _vp, _vp, _vp]),
+    "rg_pnp_ransac_batched_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "rg_pnp_ransac_batched_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _i, _vp, _vp, _vp, _vp]),
     "rg_pnp_minimize_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rg_pnp_score_count_host": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _d, _i, _vp]),
-    "rg_triangulate_host": (_i, [_vp, _vp, _i, _vp, _vp, _pi, _vp, _vp, _i, _vp]),
-    "rg_triangulate_dev": (_i, [_vp, _vp, _i, _vp, _vp, _pi, _vp, _vp, _i, _vp]),
+    "rg_triangulate_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp]),
+    "rg_triangulate_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _i, _vp]),
     "rg_fmatrix_from_cameras_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp]),
     "rg_relative_pose_host": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
     "rg_relative_pose_dev": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp, _vp]),
     "rg_camera_resectioning_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
-    "rg_gold_standard_host": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
-    "rg_gold_standard_dev": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
-    "rg_pnp_refine_host": (_i, [_vp, _vp, _i, _vp, _vp, _pi, _vp, _vp, _vp, _i, _d, _i, _d, _vp, _vp, _vp, _vp]),
-    "rg_pnp_refine_dev": (_i, [_vp, _vp, _i, _vp, _vp, _pi, _vp, _vp, _vp, _i, _d, _i, _d, _vp, _vp, _vp, _vp]),
+    "rg_gold_standard_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
+    "rg_gold_standard_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
+    "rg_pnp_refine_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _i, _d, _vp, _vp, _vp, _vp]),
+    "rg_pnp_refine_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _i, _d, _vp, _vp, _vp, _vp]),
     "rg_fmatrix_residuals_gs_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
-    "rg_bundle_adjust_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _pi, _pi, _i, _i, _d, _vp, _vp, _vp]),
-    "rg_bundle_adjust_dev": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _pi, _pi, _i, _i, _d, _vp, _vp, _vp]),
-    "rg_ba_residuals_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _pi, _pi, _vp]),
-    "rg_two_view_init_host": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _vp, _vp, _vp, _vp, _vp]),
-    "rg_two_view_init_dev": (_i, [_vp, _vp, _i, _vp, _pi, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "rg_bundle_adjust_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _d, _vp, _vp, _vp]),
+    "rg_bundle_adjust_dev": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _d, _vp, _vp, _vp]),
+    "rg_ba_residuals_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "rg_two_view_init_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "rg_two_view_init_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rg_match_first_within_host": (_i, [_vp, _vp, _i, _i, _vp, _i, _vp, _d, _vp]),
     "rg_argmax_pack_dev": (_i, [_vp, _i, _vp, _vp, _i, _vp]),
     "rg_argmax_allreduce": (_i, [_vp, _vp, _vp, _i]),
@@ -89,6 +88,7 @@ SIGNATURES = {
 }
 
 _lib = None
+_calls: dict = {}                 # name -> (function, one argument converter per argtype), filled by load_library
 _lock = threading.Lock()
 _contexts: dict[int, int] = {}
 
@@ -113,8 +113,21 @@ def load_library() -> C.CDLL:
                 fn = getattr(lib, name)
                 fn.restype = res
                 fn.argtypes = args
+                _calls[name] = (fn, [_CONVERT.get(a, _same) for a in args])
             _lib = lib
     return _lib
+
+
+def call(name: str, *args) -> None:
+    """Calls the library entry point ``name``; raises through ``check`` when it fails.  Each argument is converted for
+    its declared C type: a pointer takes None (NULL), a numpy array, a torch tensor or an int address (see ``ptr``), a
+    number takes a Python or numpy scalar, and any other type (ctypes out-parameters) is passed as given."""
+    if _lib is None:                      # set only after every prototype is declared
+        load_library()
+    fn, conv = _calls[name]
+    if len(args) != len(conv):
+        raise TypeError(f"{name} takes {len(conv)} arguments ({len(args)} given)")
+    check(fn(*[c(a) for c, a in zip(conv, args)]))
 
 
 def check(rc: int) -> None:
@@ -168,18 +181,22 @@ def pinned_empty(shape, dtype, device: int | None = None) -> np.ndarray:
 
 
 def ptr(a) -> int | None:
-    """Raw address of a numpy array / torch tensor / int; None stays NULL."""
+    """Raw address of a numpy array / torch tensor / int / ctypes c_void_p; None stays NULL."""
     if a is None:
         return None
-    if isinstance(a, (int, np.integer)):
-        return int(a)
     if isinstance(a, np.ndarray):
         return a.ctypes.data
+    if isinstance(a, (int, np.integer)):
+        return int(a)
     if hasattr(a, "data_ptr"):
         return int(a.data_ptr())
+    if isinstance(a, C.c_void_p):
+        return a.value
     raise TypeError(f"cannot take the address of {type(a)!r}")
 
 
-def as_i32(a) -> "C.Array":
-    arr = np.ascontiguousarray(a, dtype=np.int32)
-    return arr, arr.ctypes.data_as(_pi)
+def _same(a):
+    return a
+
+
+_CONVERT = {_vp: ptr, _d: float, _i: int, C.c_longlong: int, C.c_ulonglong: int, C.c_size_t: int}

@@ -9,17 +9,18 @@ from . import sampling as _sampling
 from ._cabi import MODE_EPI_MAX, SCORE_FP32_GUARDED, SOLVER_QR, TIE_FIRST
 
 
+def _rows(pairs) -> list:
+    """pairs of (2, N_p) arrays (p1, p2) in the reference layout, or (N_p, 4) arrays -> (N_p, 4) rows (x0, x1, y0, y1)."""
+    return [_rt.pack_pairs(pr[0], pr[1]) if isinstance(pr, (tuple, list)) else
+            np.ascontiguousarray(pr, dtype=np.float64).reshape(-1, 4) for pr in pairs]
+
+
 def f_ransac_pairs(pairs, n_hyp=10000, thr=1.5, seed=0, idx_list=None, host_sampling=False, **kw) -> dict:
     """pairs: list of (p1, p2) with (2, N_p) arrays (reference layout) or of (N_p, 4) arrays.  Unless ``idx_list`` is given,
     the sample index sets are drawn ON THE DEVICE from ``seed`` (Philox; ``philox.sample_indices(N_p, n_hyp, 8, seed, p)``
     replays pair p's samples on the host) — drawing 35 x 10 000 index sets with numpy and uploading their 11 MB cost 88 ms
     and 0.8 ms against 0.5 ms for the whole call.  host_sampling=True restores the host draw (``sampling.fast_batch``)."""
-    pts = []
-    for pr in pairs:
-        if isinstance(pr, (tuple, list)):
-            pts.append(_rt.pack_pairs(pr[0], pr[1]))
-        else:
-            pts.append(np.ascontiguousarray(pr, dtype=np.float64).reshape(-1, 4))
+    pts = _rows(pairs)
     if idx_list is None and not host_sampling:
         return _rt.f_ransac_batched(pts, None, thr=thr, n_hyp=n_hyp, sample_seed=seed, **kw)
     if idx_list is None:
@@ -49,10 +50,4 @@ def two_view_init(pairs, F, K, masks=None, **kw) -> dict:
     from F and K, and the optimally triangulated 3-D point of every (inlier) correspondence in the first camera's frame.
     pairs: list of (p1, p2) with (2, N_p) arrays or of (N_p, 4) arrays; F: (P, 3, 3), e.g. ``f_ransac_pairs(...)["F"]``;
     masks: optional inlier masks (``...["mask"]``)."""
-    pts = []
-    for pr in pairs:
-        if isinstance(pr, (tuple, list)):
-            pts.append(_rt.pack_pairs(pr[0], pr[1]))
-        else:
-            pts.append(np.ascontiguousarray(pr, dtype=np.float64).reshape(-1, 4))
-    return _rt.two_view_init(pts, F, K, masks=masks, **kw)
+    return _rt.two_view_init(_rows(pairs), F, K, masks=masks, **kw)

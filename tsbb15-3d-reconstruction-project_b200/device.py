@@ -6,15 +6,13 @@ decompositions on top of these, ``bench.py`` times them.
 """
 from __future__ import annotations
 
-import ctypes as C
+import contextlib
 
 import numpy as np
 
 from . import _cabi as cabi
 from ._cabi import FLAG_REUSE_POINTS, MODE_EPI_MAX, SCORE_FP32_GUARDED, SOLVER_QR, TIE_FIRST
-
-_vp = C.c_void_p
-_pi32 = C.POINTER(C.c_int32)
+from .runtime import offsets, pnp_k_table  # noqa: F401  (offsets: part of this module's interface)
 
 
 def _torch():
@@ -30,14 +28,16 @@ def _dev_index(t) -> int:
     return int(t.device.index if t.device.index is not None else _torch().cuda.current_device())
 
 
-def offsets(counts) -> np.ndarray:
-    """int32 prefix table [0, c0, c0+c1, ...] (host) of per-pair counts."""
-    counts = np.asarray(counts, dtype=np.int64).ravel()
-    off = np.zeros(counts.size + 1, dtype=np.int64)
-    np.cumsum(counts, out=off[1:])
-    if off[-1] >= 2 ** 31:
-        raise ValueError("batch too large for int32 offsets")
-    return off.astype(np.int32)
+def _cuda_device(device=None):
+    """torch.device of CUDA device ``device`` (default: the current one)."""
+    torch = _torch()
+    return torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+
+
+def _call(name, device: int, *args) -> None:
+    """Entry point ``name`` with the context of CUDA device ``device`` and torch's current stream as its first two
+    arguments."""
+    cabi.call(name, cabi.context(device), _stream(), *args)
 
 
 def synth_two_view(P: int, N: int, first_pair: int = 0, seed_base: int = 1000, cams=None, bbox=None, outlier_frac: float = 0.3,
@@ -47,20 +47,16 @@ def synth_two_view(P: int, N: int, first_pair: int = 0, seed_base: int = 1000, c
     (P, 2) int32 tensor of the camera pairs drawn."""
     torch = _torch()
     from . import synth
-    lib = cabi.load_library()
-    dev = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+    dev = _cuda_device(device)
     cams = np.ascontiguousarray(synth.dino()["Ps"] if cams is None else cams, dtype=np.float64).reshape(-1, 12)
     bbox = np.ascontiguousarray(synth.DINO_BBOX if bbox is None else bbox, dtype=np.float64).reshape(6)
     pts = out if out is not None else torch.empty((P, N, 4), dtype=torch.float64, device=dev)
     cam_pair = torch.empty((P, 2), dtype=torch.int32, device=dev)
-    ctx = cabi.context(dev.index)
     done = 0
     while done < P:                                       # grid.y is limited to 65535 pairs per launch
         n = min(P - done, 32768)
-        cabi.check(lib.rg_synth_two_view_dev(_vp(ctx), _vp(_stream()), n, first_pair + done, N, _vp(cams.ctypes.data),
-                                             cams.shape[0], _vp(bbox.ctypes.data), int(seed_base), float(outlier_frac),
-                                             float(sigma_px), float(image_size[0]), float(image_size[1]),
-                                             _vp(pts[done:].data_ptr()), _vp(cam_pair[done:].data_ptr())))
+        _call("rg_synth_two_view_dev", dev.index, n, first_pair + done, N, cams, cams.shape[0], bbox, seed_base,
+              outlier_frac, sigma_px, image_size[0], image_size[1], pts[done:], cam_pair[done:])
         done += n
     return pts, cam_pair
 
@@ -68,15 +64,12 @@ def synth_two_view(P: int, N: int, first_pair: int = 0, seed_base: int = 1000, c
 def sample_indices(n_points_list, n_hyp, k: int = 8, seed: int = 0, first_pair: int = 0, hyp_first: int = 0, device=None):
     """(sum H, k) int32 CUDA tensor of the index sets a seeded call draws (rg_sample_indices_dev)."""
     torch = _torch()
-    lib = cabi.load_library()
-    dev = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+    dev = _cuda_device(device)
     n_pts = np.ascontiguousarray(n_points_list, dtype=np.int32).ravel()
     P = n_pts.size
     hyp_off = offsets(np.full(P, n_hyp) if np.isscalar(n_hyp) else n_hyp)
     out = torch.empty((int(hyp_off[-1]), k), dtype=torch.int32, device=dev)
-    cabi.check(lib.rg_sample_indices_dev(_vp(cabi.context(dev.index)), _vp(_stream()), P, n_pts.ctypes.data_as(_pi32),
-                                         hyp_off.ctypes.data_as(_pi32), int(k), int(seed), int(first_pair), int(hyp_first),
-                                         _vp(out.data_ptr())))
+    _call("rg_sample_indices_dev", dev.index, P, n_pts, hyp_off, k, seed, first_pair, hyp_first, out)
     return out
 
 
@@ -85,7 +78,7 @@ class FOutputs:
 
     def __init__(self, P: int, n_total: int = 0, device=None, want_mask: bool = False, want_key: bool = False):
         torch = _torch()
-        dev = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+        dev = _cuda_device(device)
         # one contiguous block per pair: [best_idx i32][best_count i32][F 9 x f64] is what the pair-sharded gather ships
         self.best_idx = torch.empty(max(P, 1), dtype=torch.int32, device=dev)
         self.best_count = torch.empty(max(P, 1), dtype=torch.int32, device=dev)
@@ -98,35 +91,24 @@ class FOutputs:
 def f_ransac(d_pts, pair_off, d_idx, hyp_off, out: FOutputs, thr=1.5, mode=MODE_EPI_MAX, tie_mode=TIE_FIRST, solver=SOLVER_QR,
              score_path=SCORE_FP32_GUARDED, flags=0, seed=0, first_pair=0, hyp_first=0):
     """rg_f_ransac_dev2 on CUDA tensors.  d_idx None = samples drawn on the device from ``seed``."""
-    lib = cabi.load_library()
-    P = len(pair_off) - 1
-    ctx = cabi.context(_dev_index(d_pts))
-    cabi.check(lib.rg_f_ransac_dev2(
-        _vp(ctx), _vp(_stream()), P, _vp(d_pts.data_ptr()), pair_off.ctypes.data_as(_pi32),
-        _vp(d_idx.data_ptr()) if d_idx is not None else None, hyp_off.ctypes.data_as(_pi32), float(thr), int(mode),
-        int(tie_mode), int(solver), int(score_path), int(flags), int(seed), int(first_pair), int(hyp_first),
-        _vp(out.best_idx.data_ptr()), _vp(out.best_count.data_ptr()), _vp(out.F.data_ptr()),
-        _vp(out.mask.data_ptr()) if out.mask is not None else None, _vp(out.key.data_ptr()) if out.key is not None else None))
+    _call("rg_f_ransac_dev2", _dev_index(d_pts), len(pair_off) - 1, d_pts, pair_off, d_idx, hyp_off, thr, mode, tie_mode,
+          solver, score_path, flags, seed, first_pair, hyp_first, out.best_idx, out.best_count, out.F, out.mask, out.key)
     return out
 
 
 def f_inlier_mask(d_pts, pair_off, d_F, thr=1.5, mode=MODE_EPI_MAX, out=None):
     """uint8 inlier mask of one F per pair (reference criterion), all on the device."""
     torch = _torch()
-    lib = cabi.load_library()
-    P = len(pair_off) - 1
     if out is None:
         out = torch.empty(max(int(pair_off[-1]), 1), dtype=torch.uint8, device=d_pts.device)
-    cabi.check(lib.rg_f_inlier_mask_dev(_vp(cabi.context(_dev_index(d_pts))), _vp(_stream()), P, _vp(d_pts.data_ptr()),
-                                        pair_off.ctypes.data_as(_pi32), _vp(d_F.data_ptr()), float(thr), int(mode),
-                                        _vp(out.data_ptr())))
+    _call("rg_f_inlier_mask_dev", _dev_index(d_pts), len(pair_off) - 1, d_pts, pair_off, d_F, thr, mode, out)
     return out
 
 
 class PnpOutputs:
     def __init__(self, V: int, n_total: int = 0, device=None, want_mask: bool = False, want_key: bool = False):
         torch = _torch()
-        dev = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+        dev = _cuda_device(device)
         self.best_idx = torch.empty(max(V, 1), dtype=torch.int32, device=dev)
         self.best_count = torch.empty(max(V, 1), dtype=torch.int32, device=dev)
         self.Rt = torch.empty((max(V, 1), 12), dtype=torch.float64, device=dev)
@@ -137,15 +119,9 @@ class PnpOutputs:
 def pnp_ransac(d_X, d_y, view_off, d_idx, hyp_off, out: PnpOutputs, thr2, n=6, n_vote=None, score_path=SCORE_FP32_GUARDED,
                hyp_first=0):
     """rg_pnp_ransac_batched_dev2 on CUDA tensors."""
-    lib = cabi.load_library()
-    V = len(view_off) - 1
     vote = None if n_vote is None else np.ascontiguousarray(n_vote, dtype=np.int32)
-    cabi.check(lib.rg_pnp_ransac_batched_dev2(
-        _vp(cabi.context(_dev_index(d_X))), _vp(_stream()), V, _vp(d_X.data_ptr()), _vp(d_y.data_ptr()),
-        view_off.ctypes.data_as(_pi32), vote.ctypes.data_as(_pi32) if vote is not None else None, _vp(d_idx.data_ptr()),
-        hyp_off.ctypes.data_as(_pi32), int(n), float(thr2), int(score_path), int(hyp_first), _vp(out.best_idx.data_ptr()),
-        _vp(out.best_count.data_ptr()), _vp(out.Rt.data_ptr()), _vp(out.mask.data_ptr()) if out.mask is not None else None,
-        _vp(out.key.data_ptr()) if out.key is not None else None))
+    _call("rg_pnp_ransac_batched_dev2", _dev_index(d_X), len(view_off) - 1, d_X, d_y, view_off, vote, d_idx, hyp_off, n,
+          thr2, score_path, hyp_first, out.best_idx, out.best_count, out.Rt, out.mask, out.key)
     return out
 
 
@@ -165,7 +141,7 @@ class PnpRefineOutputs:
 
     def __init__(self, V: int, device=None):
         torch = _torch()
-        dev = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+        dev = _cuda_device(device)
         self.cost = torch.empty(max(V, 1), dtype=torch.float64, device=dev)
         self.iters = torch.empty(max(V, 1), dtype=torch.int32, device=dev)
         self.status = torch.empty(max(V, 1), dtype=torch.int32, device=dev)
@@ -178,8 +154,6 @@ def pnp_refine(d_X, d_y, view_off, out: PnpOutputs, d_mask=None, K=None, max_ite
     form: no host synchronisation between the two.  K: HOST (3, 3) or (V, 3, 3) array (validated before anything is
     enqueued).  mask_out (uint8 CUDA tensor, may be out.mask) receives the last consensus (needs thr2).  Returns ``res``
     (allocated when None)."""
-    from . import runtime
-    lib = cabi.load_library()
     V = len(view_off) - 1
     if int(rounds) > 1 and thr2 is None:
         raise ValueError("rounds > 1 needs thr2 (the consensus threshold)")
@@ -194,15 +168,11 @@ def pnp_refine(d_X, d_y, view_off, out: PnpOutputs, d_mask=None, K=None, max_ite
         _check_dense(d_mask.reshape(-1), "d_mask", torch.uint8, (), n)
     if mask_out is not None:
         _check_dense(mask_out.reshape(-1), "mask_out", torch.uint8, (), n)
-    Kt = runtime.pnp_k_table(K, V)
+    Kt = pnp_k_table(K, V)
     if res is None:
         res = PnpRefineOutputs(V, device=_dev_index(d_X))
-    cabi.check(lib.rg_pnp_refine_dev(
-        _vp(cabi.context(_dev_index(d_X))), _vp(_stream()), V, _vp(d_X.data_ptr()), _vp(d_y.data_ptr()),
-        view_off.ctypes.data_as(_pi32), _vp(cabi.ptr(Kt)), _vp(d_mask.data_ptr()) if d_mask is not None else None,
-        _vp(out.Rt.data_ptr()), int(max_iter), float(ftol), int(rounds), float(thr2) if thr2 is not None else 0.0,
-        _vp(mask_out.data_ptr()) if mask_out is not None else None, _vp(res.cost.data_ptr()), _vp(res.iters.data_ptr()),
-        _vp(res.status.data_ptr())))
+    _call("rg_pnp_refine_dev", _dev_index(d_X), V, d_X, d_y, view_off, Kt, d_mask, out.Rt, max_iter, ftol, rounds,
+          0.0 if thr2 is None else thr2, mask_out, res.cost, res.iters, res.status)
     return res
 
 
@@ -214,27 +184,26 @@ class P2PExchange:
     def __init__(self, group=None, device=None):
         torch = _torch()
         import torch.distributed as dist
-        self.lib = cabi.load_library()
-        self.dev = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+        self.dev = _cuda_device(device)
         self.ctx = cabi.context(self.dev.index)
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         # every step below is followed by a collective that ALL ranks reach even when a local CUDA call failed, so that a
         # rank whose IPC mapping is refused (containers without shared IPC namespaces) makes everybody raise, not hang
-        h = (C.c_char * 64)()
+        h = np.zeros(64, dtype=np.uint8)
         err = None
         try:
-            cabi.check(self.lib.rg_p2p_create(_vp(self.ctx), self.rank, self.world, h))
+            cabi.call("rg_p2p_create", self.ctx, self.rank, self.world, h)
         except Exception as e:           # noqa: BLE001 - reported to every rank below
             err = repr(e)
-        mine = (err, bytes(h.raw))
+        mine = (err, h.tobytes())
         got = [mine]
         if self.world > 1:
             got = [None] * self.world
             dist.all_gather_object(got, mine, group=group)
         if err is None and all(g[0] is None for g in got):
             try:
-                cabi.check(self.lib.rg_p2p_connect(_vp(self.ctx), b"".join(g[1] for g in got)))
+                cabi.call("rg_p2p_connect", self.ctx, np.frombuffer(b"".join(g[1] for g in got), dtype=np.uint8))
             except Exception as e:       # noqa: BLE001
                 err = repr(e)
         errs = [err]
@@ -243,7 +212,7 @@ class P2PExchange:
             dist.all_gather_object(errs, err, group=group)          # also the barrier: every peer mapped every buffer
         bad = [(r, e) for r, e in enumerate(errs) if e is not None] + [(r, g[0]) for r, g in enumerate(got) if g[0] is not None]
         if bad:
-            self.lib.rg_p2p_destroy(_vp(self.ctx))
+            self.close()
             raise cabi.RGError(f"peer-memory exchange unavailable (rank {bad[0][0]}: {bad[0][1]})")
         self.status = torch.zeros(1, dtype=torch.int32, device=self.dev)
 
@@ -251,10 +220,8 @@ class P2PExchange:
         """key (P,) int64, payload (P, npay) float64 -> winner's global index / count / payload on every rank (async)."""
         P = key.numel()
         npay = payload.shape[1] if payload is not None else 0
-        cabi.check(self.lib.rg_p2p_argmax_exchange(
-            _vp(self.ctx), _vp(_stream()), P, _vp(key.data_ptr()), _vp(payload.data_ptr()) if npay else None, npay,
-            _vp(best_idx.data_ptr()), _vp(best_count.data_ptr()), _vp(payload_out.data_ptr()) if npay else None,
-            _vp(self.status.data_ptr())))
+        cabi.call("rg_p2p_argmax_exchange", self.ctx, _stream(), P, key, payload if npay else None, npay, best_idx,
+                  best_count, payload_out if npay else None, self.status)
 
     def check(self):
         s = int(self.status.item())
@@ -262,4 +229,7 @@ class P2PExchange:
             raise cabi.RGError(f"p2p argmax exchange: rank {s - 1} did not arrive (timeout)")
 
     def close(self):
-        self.lib.rg_p2p_destroy(_vp(self.ctx))
+        """Unmaps the peers' buffers.  Best effort (a failure is not raised): it also runs on the constructor's error
+        path, where the error to report is the one that made the exchange unavailable."""
+        with contextlib.suppress(cabi.RGError, ValueError):
+            cabi.call("rg_p2p_destroy", self.ctx)

@@ -16,6 +16,7 @@ from __future__ import annotations
 
 import numpy as np
 
+from . import _cabi as cabi
 from . import runtime as _rt
 
 
@@ -24,6 +25,15 @@ def shard_range(n_units: int, rank: int, world: int) -> tuple[int, int]:
     base, extra = divmod(n_units, world)
     lo = rank * base + min(rank, extra)
     return lo, lo + base + (1 if rank < extra else 0)
+
+
+def shard_owner(n_units: int, index: int, world: int) -> int:
+    """The rank whose ``shard_range`` block holds unit ``index``; -1 when none does."""
+    for r in range(world):
+        lo, hi = shard_range(n_units, r, world)
+        if lo <= index < hi:
+            return r
+    return -1
 
 
 def argmax_key(count: int, index: int) -> int:
@@ -98,21 +108,31 @@ class NcclComm:
 def argmax_allreduce_c(best_idx, best_count, index_offset, comm: NcclComm, stream=0):
     """(best_idx, best_count) of this rank's hypothesis block -> global winner, entirely through the C ABI on the device:
     rg_argmax_pack_dev -> rg_argmax_allreduce (ONE ncclAllReduce(max) of 8 bytes per pair) -> rg_argmax_unpack_dev."""
-    import ctypes as C
     import torch
-    from . import _cabi as cabi
-    lib = cabi.load_library()
-    vp = C.c_void_p
     bi = torch.as_tensor(np.atleast_1d(np.asarray(best_idx, dtype=np.int32))).cuda()
     bc = torch.as_tensor(np.atleast_1d(np.asarray(best_count, dtype=np.int32))).cuda()
     P = bi.numel()
     key = torch.empty(P, dtype=torch.int64, device=bi.device)
     st = stream or torch.cuda.current_stream().cuda_stream
-    cabi.check(lib.rg_argmax_pack_dev(vp(st), P, vp(bi.data_ptr()), vp(bc.data_ptr()), int(index_offset), vp(key.data_ptr())))
-    cabi.check(lib.rg_argmax_allreduce(comm.handle, vp(st), vp(key.data_ptr()), P))
-    cabi.check(lib.rg_argmax_unpack_dev(vp(st), P, vp(key.data_ptr()), vp(bi.data_ptr()), vp(bc.data_ptr())))
+    cabi.call("rg_argmax_pack_dev", st, P, bi, bc, index_offset, key)
+    cabi.call("rg_argmax_allreduce", comm.handle, st, key, P)
+    cabi.call("rg_argmax_unpack_dev", st, P, key, bi, bc)
     torch.cuda.current_stream().synchronize()
     return bi.cpu().numpy(), bc.cpu().numpy()
+
+
+def _gather_blocks(block: np.ndarray, sizes, group=None) -> np.ndarray:
+    """Rank r passes its block of ``sizes[r]`` rows; every rank receives the blocks of all ranks, concatenated in rank
+    order.  One all_gather of fixed-size buffers, padded to the largest block."""
+    import torch
+    rank, world = _world(group)
+    block = torch.from_numpy(np.ascontiguousarray(block))
+    buf = torch.zeros((max(1, int(max(sizes))),) + tuple(block.shape[1:]), dtype=block.dtype)
+    buf[:block.shape[0]] = block
+    buf = buf.to(_device_for_collectives(group))
+    gathered = [torch.empty_like(buf) for _ in range(world)]
+    _dist().all_gather(gathered, buf, group=group)
+    return np.concatenate([g[:n].cpu().numpy() for g, n in zip(gathered, sizes)])
 
 
 def f_ransac_pairs_sharded(pts_list, idx_list, thr=1.5, group=None, gather=True, gather_mask=False, compute=None,
@@ -136,58 +156,58 @@ def f_ransac_pairs_sharded(pts_list, idx_list, thr=1.5, group=None, gather=True,
         out_local["mask"] = list(local["mask"])
     if not gather or world == 1:
         return out_local
+    starts = [shard_range(P, r, world)[0] for r in range(world)] + [P]          # the ranks' first pairs
+    # one float64 row per pair: [best_idx, best_count, F(9)]
+    rows = _gather_blocks(np.column_stack([out_local["best_idx"], out_local["best_count"],
+                                           out_local["F"].reshape(hi - lo, 9)]), np.diff(starts), group)
+    out = {"range": (lo, hi), "best_idx": rows[:, 0].astype(np.int32), "best_count": rows[:, 1].astype(np.int32),
+           "F": rows[:, 2:].reshape(P, 3, 3)}
+    if gather_mask:
+        off = _rt.offsets([np.asarray(p).reshape(-1, 4).shape[0] for p in pts_list])     # of the pairs' masks
+        mine = np.concatenate([np.zeros(0, np.uint8)] + [np.asarray(m, dtype=np.uint8) for m in out_local["mask"]])
+        out["mask"] = _rt._split(_gather_blocks(mine, np.diff(off[starts]), group), off)
+    return out
+
+
+def _split_winner(best_idx: int, best_count: int, lo: int, payload: np.ndarray, mask, H: int, group=None,
+                  reduced_key: int | None = None):
+    """The winner of ONE RANSAC whose H hypotheses are split over the ranks: this rank's winner is hypothesis ``lo +
+    best_idx`` (-1: none); one max-all-reduce of the ranks' ``argmax_key``, unless ``reduced_key`` already holds its
+    result, picks the global winner, and its owner broadcasts its float64 ``payload`` (the model) and its inlier
+    ``mask`` (as bytes).  Returns (best_idx, best_count, payload, mask, owner); (-1, 0, NaN, zeros, -1) when no rank
+    has a winner."""
+    rank, world = _world(group)
+    key = argmax_key(best_count, lo + best_idx) if best_idx >= 0 else 0
+    if world == 1:
+        cnt, gi = key_decode(key) if key else (0, -1)
+        return gi, cnt, payload, mask, 0
     import torch
     dist = _dist()
     dev = _device_for_collectives(group)
-    # fixed-size payload per pair: [best_idx, best_count, F(9)] as float64 -> one all_gather of padded blocks
-    per = (P + world - 1) // world
-    buf = torch.full((per, 11), float("nan"), dtype=torch.float64)
-    n_loc = hi - lo
-    if n_loc:
-        buf[:n_loc, 0] = torch.from_numpy(out_local["best_idx"].astype(np.float64))
-        buf[:n_loc, 1] = torch.from_numpy(out_local["best_count"].astype(np.float64))
-        buf[:n_loc, 2:] = torch.from_numpy(out_local["F"].reshape(n_loc, 9))
-    buf = buf.to(dev)
-    gathered = [torch.empty_like(buf) for _ in range(world)]
-    dist.all_gather(gathered, buf, group=group)
-    best_idx = np.full(P, -1, dtype=np.int32)
-    best_count = np.zeros(P, dtype=np.int32)
-    F = np.full((P, 3, 3), np.nan)
-    for r in range(world):
-        a, b = shard_range(P, r, world)
-        if b > a:
-            blk = gathered[r][:b - a].cpu().numpy()
-            best_idx[a:b] = blk[:, 0].astype(np.int32)
-            best_count[a:b] = blk[:, 1].astype(np.int32)
-            F[a:b] = blk[:, 2:].reshape(-1, 3, 3)
-    out = {"range": (lo, hi), "best_idx": best_idx, "best_count": best_count, "F": F}
-    if gather_mask:
-        sizes = [int(np.asarray(p).reshape(-1, 4).shape[0]) for p in pts_list]
-        shard_bytes = [sum(sizes[slice(*shard_range(P, r, world))]) for r in range(world)]
-        mbuf = torch.zeros(max(max(shard_bytes), 1), dtype=torch.uint8)
-        if n_loc:
-            mine = np.concatenate([np.asarray(m, dtype=np.uint8) for m in out_local["mask"]]) if shard_bytes[rank] else np.zeros(0, np.uint8)
-            mbuf[:mine.size] = torch.from_numpy(mine)
-        mbuf = mbuf.to(dev)
-        mg = [torch.empty_like(mbuf) for _ in range(world)]
-        dist.all_gather(mg, mbuf, group=group)
-        masks = []
-        for r in range(world):
-            a, b = shard_range(P, r, world)
-            flat = mg[r].cpu().numpy()
-            o = 0
-            for p in range(a, b):
-                masks.append(flat[o:o + sizes[p]].copy())
-                o += sizes[p]
-        out["mask"] = masks
-    return out
+    if reduced_key is None:
+        k = torch.tensor([key], dtype=torch.int64, device=dev)
+        dist.all_reduce(k, op=dist.ReduceOp.MAX, group=group)
+        reduced_key = int(k.item())
+    if reduced_key == 0:
+        return -1, 0, np.full(payload.size, np.nan), np.zeros(len(mask), np.uint8), -1
+    cnt, gi = key_decode(reduced_key)
+    owner = shard_owner(H, gi, world)
+    src = dist.get_global_rank(group, owner) if group is not None else owner
+    pw = torch.zeros(payload.size, dtype=torch.float64)
+    mw = torch.zeros(len(mask), dtype=torch.uint8)
+    if rank == owner:
+        pw = torch.from_numpy(np.ascontiguousarray(payload, dtype=np.float64))
+        mw = torch.from_numpy(np.ascontiguousarray(np.asarray(mask, dtype=np.uint8)))
+    pw, mw = pw.to(dev), mw.to(dev)
+    dist.broadcast(pw, src=src, group=group)
+    dist.broadcast(mw, src=src, group=group)
+    return gi, cnt, pw.cpu().numpy(), mw.cpu().numpy(), owner
 
 
 def f_ransac_split_hypotheses(pts, idx, thr=1.5, group=None, compute=None, nccl_comm: NcclComm | None = None, **kw) -> dict:
     """One pair, hypotheses split across ranks, one max-all-reduce of an int64 key (first-maximum selection).
     nccl_comm: reduce through the library's own C entry point ``rg_argmax_allreduce`` on that communicator instead of
     ``torch.distributed.all_reduce`` (same key, same result)."""
-    import torch
     rank, world = _world(group)
     idx = np.ascontiguousarray(idx, dtype=np.int32)
     H = idx.shape[0]
@@ -205,34 +225,14 @@ def f_ransac_split_hypotheses(pts, idx, thr=1.5, group=None, compute=None, nccl_
     else:                                            # H < world: this rank holds no hypothesis
         local = {"best_idx": np.array([-1], np.int32), "best_count": np.array([0], np.int32),
                  "F": np.full((1, 3, 3), np.nan), "mask": [np.zeros(n, np.uint8)]}
-    li = int(local["best_idx"][0])
-    key = argmax_key(int(local["best_count"][0]), lo + li) if li >= 0 else 0
-    if world == 1:
-        cnt, gi = key_decode(key) if key else (0, -1)
-        return {"best_idx": gi, "best_count": cnt, "F": local["F"][0], "mask": local["mask"][0], "owner": 0}
-    dist = _dist()
-    dev = _device_for_collectives(group)
-    if nccl_comm is not None:
+    reduced = None
+    if nccl_comm is not None and world > 1:
         gi_a, cnt_a = argmax_allreduce_c(local["best_idx"][:1], local["best_count"][:1], lo, nccl_comm)
-        gkey = argmax_key(int(cnt_a[0]), int(gi_a[0])) if gi_a[0] >= 0 else 0
-    else:
-        k = torch.tensor([key], dtype=torch.int64, device=dev)
-        dist.all_reduce(k, op=dist.ReduceOp.MAX, group=group)
-        gkey = int(k.item())
-    if gkey == 0:
-        return {"best_idx": -1, "best_count": 0, "F": np.full((3, 3), np.nan), "mask": np.zeros(n, np.uint8), "owner": -1}
-    cnt, gi = key_decode(gkey)
-    owner = next(r for r in range(world) if shard_range(H, r, world)[0] <= gi < shard_range(H, r, world)[1])
-    src = dist.get_global_rank(group, owner) if group is not None else owner
-    Fw = torch.zeros(9, dtype=torch.float64)
-    mw = torch.zeros(n, dtype=torch.uint8)                       # the mask travels as bytes, not as float64
-    if rank == owner:
-        Fw = torch.from_numpy(np.ascontiguousarray(np.asarray(local["F"][0], dtype=np.float64).reshape(9)))
-        mw = torch.from_numpy(np.ascontiguousarray(np.asarray(local["mask"][0], dtype=np.uint8)))
-    Fw, mw = Fw.to(dev), mw.to(dev)
-    dist.broadcast(Fw, src=src, group=group)
-    dist.broadcast(mw, src=src, group=group)
-    return {"best_idx": gi, "best_count": cnt, "F": Fw.cpu().numpy().reshape(3, 3), "mask": mw.cpu().numpy(), "owner": owner}
+        reduced = argmax_key(int(cnt_a[0]), int(gi_a[0])) if gi_a[0] >= 0 else 0
+    gi, cnt, F, mask, owner = _split_winner(int(local["best_idx"][0]), int(local["best_count"][0]), lo,
+                                            np.asarray(local["F"][0], dtype=np.float64).reshape(9), local["mask"][0], H,
+                                            group, reduced)
+    return {"best_idx": gi, "best_count": cnt, "F": F.reshape(3, 3), "mask": mask, "owner": owner}
 
 
 def pnp_ransac_split_hypotheses(X, y, idx, thr2, group=None, compute=None, **kw) -> dict:
@@ -240,7 +240,6 @@ def pnp_ransac_split_hypotheses(X, y, idx, thr2, group=None, compute=None, **kw)
     all N correspondences and scores its slice of the (H, n) samples; the same 8-byte max-all-reduce on
     ``(count << 32) | ~index`` as the F path picks the winner (first maximum, ransac.py:108); its owner broadcasts
     R, t and the consensus mask."""
-    import torch
     rank, world = _world(group)
     idx = np.ascontiguousarray(idx, dtype=np.int32)
     H = idx.shape[0]
@@ -254,34 +253,10 @@ def pnp_ransac_split_hypotheses(X, y, idx, thr2, group=None, compute=None, **kw)
     else:
         local = {"best_idx": -1, "best_count": 0, "R": np.full((3, 3), np.nan), "t": np.full(3, np.nan),
                  "mask": np.zeros(n, np.uint8)}
-    li = int(local["best_idx"])
-    key = argmax_key(int(local["best_count"]), lo + li) if li >= 0 else 0
-    if world == 1:
-        cnt, gi = key_decode(key) if key else (0, -1)
-        return {"best_idx": gi, "best_count": cnt, "R": local["R"], "t": local["t"], "mask": local["mask"], "owner": 0}
-    dist = _dist()
-    dev = _device_for_collectives(group)
-    k = torch.tensor([key], dtype=torch.int64, device=dev)
-    dist.all_reduce(k, op=dist.ReduceOp.MAX, group=group)
-    gkey = int(k.item())
-    if gkey == 0:
-        return {"best_idx": -1, "best_count": 0, "R": np.full((3, 3), np.nan), "t": np.full(3, np.nan),
-                "mask": np.zeros(n, np.uint8), "owner": -1}
-    cnt, gi = key_decode(gkey)
-    owner = next(r for r in range(world) if shard_range(H, r, world)[0] <= gi < shard_range(H, r, world)[1])
-    src = dist.get_global_rank(group, owner) if group is not None else owner
-    Rt = torch.zeros(12, dtype=torch.float64)
-    mw = torch.zeros(n, dtype=torch.uint8)
-    if rank == owner:
-        Rt[:9] = torch.from_numpy(np.asarray(local["R"], dtype=np.float64).reshape(9))
-        Rt[9:] = torch.from_numpy(np.asarray(local["t"], dtype=np.float64).reshape(3))
-        mw = torch.from_numpy(np.ascontiguousarray(np.asarray(local["mask"], dtype=np.uint8)))
-    Rt, mw = Rt.to(dev), mw.to(dev)
-    dist.broadcast(Rt, src=src, group=group)
-    dist.broadcast(mw, src=src, group=group)
-    Rt = Rt.cpu().numpy()
-    return {"best_idx": gi, "best_count": cnt, "R": Rt[:9].reshape(3, 3), "t": Rt[9:].copy(), "mask": mw.cpu().numpy(),
-            "owner": owner}
+    Rt = np.concatenate([np.ravel(local["R"]), np.ravel(local["t"])]).astype(np.float64)
+    gi, cnt, Rt, mask, owner = _split_winner(int(local["best_idx"]), int(local["best_count"]), lo, Rt, local["mask"], H,
+                                             group)
+    return {"best_idx": gi, "best_count": cnt, "R": Rt[:9].reshape(3, 3), "t": Rt[9:].copy(), "mask": mask, "owner": owner}
 
 
 def pnp_ransac_views_sharded(X_list, y_list, idx_list, thr2, group=None, compute=None, **kw) -> dict:
@@ -300,33 +275,12 @@ def pnp_ransac_views_sharded(X_list, y_list, idx_list, thr2, group=None, compute
            "R": np.asarray(local["R"]), "t": np.asarray(local["t"])}
     if world == 1:
         return out
-    import torch
-    dist = _dist()
-    dev = _device_for_collectives(group)
-    per = (V + world - 1) // world
-    buf = torch.full((per, 14), float("nan"), dtype=torch.float64)
-    n_loc = hi - lo
-    if n_loc:
-        buf[:n_loc, 0] = torch.from_numpy(out["best_idx"].astype(np.float64))
-        buf[:n_loc, 1] = torch.from_numpy(out["best_count"].astype(np.float64))
-        buf[:n_loc, 2:11] = torch.from_numpy(out["R"].reshape(n_loc, 9))
-        buf[:n_loc, 11:] = torch.from_numpy(out["t"].reshape(n_loc, 3))
-    buf = buf.to(dev)
-    gathered = [torch.empty_like(buf) for _ in range(world)]
-    dist.all_gather(gathered, buf, group=group)
-    best_idx = np.full(V, -1, dtype=np.int32)
-    best_count = np.zeros(V, dtype=np.int32)
-    R = np.full((V, 3, 3), np.nan)
-    t = np.full((V, 3), np.nan)
-    for r in range(world):
-        a, b = shard_range(V, r, world)
-        if b > a:
-            blk = gathered[r][:b - a].cpu().numpy()
-            best_idx[a:b] = blk[:, 0].astype(np.int32)
-            best_count[a:b] = blk[:, 1].astype(np.int32)
-            R[a:b] = blk[:, 2:11].reshape(-1, 3, 3)
-            t[a:b] = blk[:, 11:]
-    return {"range": (lo, hi), "best_idx": best_idx, "best_count": best_count, "R": R, "t": t}
+    starts = [shard_range(V, r, world)[0] for r in range(world)] + [V]          # the ranks' first views
+    # one float64 row per view: [best_idx, best_count, R(9), t(3)]
+    rows = _gather_blocks(np.column_stack([out["best_idx"], out["best_count"], out["R"].reshape(hi - lo, 9),
+                                           out["t"].reshape(hi - lo, 3)]), np.diff(starts), group)
+    return {"range": (lo, hi), "best_idx": rows[:, 0].astype(np.int32), "best_count": rows[:, 1].astype(np.int32),
+            "R": rows[:, 2:11].reshape(V, 3, 3), "t": rows[:, 11:].copy()}
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -351,7 +305,7 @@ class PairShardedRansac:
         self.lo, self.hi = shard_range(self.P_total, self.rank, self.world)
         self.P = self.hi - self.lo
         self.per = (self.P_total + self.world - 1) // self.world          # padded shard size of the gathers
-        self.dev = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+        self.dev = dv._cuda_device(device)
         self.pair_off = dv.offsets(np.full(self.P, self.N))
         self.hyp_off = dv.offsets(np.full(self.P, self.H))
         # results of the local shard as ONE block [F: per x 72 B][idx: per x 4 B][count: per x 4 B] -> one all-gather
@@ -401,18 +355,10 @@ class PairShardedRansac:
     def run_host(self, thr=1.5, sample_seed: int = 0, mode=0, tie_mode=0, solver=0, score_path=0, h_idx=None):
         """rg_f_ransac_host2 on the local shard (synchronous: returns when the shard's results are in host memory), then the
         all-gather of the 80-byte results of all ranks (H2D of the local block, NCCL, D2H of everything)."""
-        import ctypes as C
-        from . import _cabi as cabi
-        lib = cabi.load_library()
-        pi32 = C.POINTER(C.c_int32)
-        st = self.dv._stream()
         if self.P:
-            cabi.check(lib.rg_f_ransac_host2(
-                _vp(cabi.context(self.dev.index)), _vp(st), self.P, _vp(self.h_pts.data_ptr()), self.pair_off.ctypes.data_as(pi32),
-                _vp(h_idx.data_ptr()) if h_idx is not None else None, self.hyp_off.ctypes.data_as(pi32), float(thr), int(mode),
-                int(tie_mode), int(solver), int(score_path), int(sample_seed), int(self.lo), _vp(self.h_best_idx.data_ptr()),
-                _vp(self.h_best_count.data_ptr()), _vp(self.h_F.data_ptr()),
-                _vp(self.h_mask.data_ptr()) if self.h_mask is not None else None, None, None, None))
+            self.dv._call("rg_f_ransac_host2", self.dev.index, self.P, self.h_pts, self.pair_off, h_idx, self.hyp_off, thr,
+                          mode, tie_mode, solver, score_path, sample_seed, self.lo, self.h_best_idx, self.h_best_count,
+                          self.h_F, self.h_mask, None, None, None)
         if self.world == 1:
             return self.h_block
         self.block.copy_(self.h_block, non_blocking=True)
@@ -507,25 +453,21 @@ class SplitHypothesesF:
             self.out.key.zero_()
             self.out.F.fill_(float("nan"))
         if self.exchange == "none":
-            lib = cabi_lib()
-            _check(lib.rg_argmax_unpack_dev(_vp(dv._stream()), 1, _vp(self.out.key.data_ptr()), _vp(self.g_idx.data_ptr()),
-                                            _vp(self.g_cnt.data_ptr())))
+            cabi.call("rg_argmax_unpack_dev", dv._stream(), 1, self.out.key, self.g_idx, self.g_cnt)
             self.g_F.copy_(self.out.F)
         elif self.exchange == "p2p":
             self.p2p.argmax(self.out.key, self.out.F, self.g_idx, self.g_cnt, self.g_F)
         else:
-            lib = cabi_lib()
             dist = _dist()
             if self.nccl_comm is not None:
                 gkey = self.out.key.clone()
-                _check(lib.rg_argmax_allreduce(self.nccl_comm.handle, _vp(dv._stream()), _vp(gkey.data_ptr()), 1))
+                cabi.call("rg_argmax_allreduce", self.nccl_comm.handle, dv._stream(), gkey, 1)
             else:
                 gkey = self.out.key.clone()
                 dist.all_reduce(gkey, op=dist.ReduceOp.MAX, group=self.group)
             # payload: the owner is the rank whose block holds the winning global index; everybody else contributes zeros
             # to a 72-byte sum
-            _check(lib.rg_argmax_unpack_dev(_vp(dv._stream()), 1, _vp(gkey.data_ptr()), _vp(self.g_idx.data_ptr()),
-                                            _vp(self.g_cnt.data_ptr())))
+            cabi.call("rg_argmax_unpack_dev", dv._stream(), 1, gkey, self.g_idx, self.g_cnt)
             own = ((self.g_idx >= self.lo) & (self.g_idx < self.hi)).to(torch.float64)
             self.g_F.copy_(torch.nan_to_num(self.out.F) * own)
             dist.all_reduce(self.g_F, op=dist.ReduceOp.SUM, group=self.group)
@@ -558,7 +500,7 @@ class SplitHypothesesF:
         if self.p2p is not None:
             self.p2p.check()
         gi, gc = int(self.g_idx.item()), int(self.g_cnt.item())
-        owner = next((r for r in range(self.world) if shard_range(self.H, r, self.world)[0] <= gi < shard_range(self.H, r, self.world)[1]), -1)
+        owner = shard_owner(self.H, gi, self.world)
         return {"best_idx": gi, "best_count": gc, "F": self.g_F.cpu().numpy().reshape(3, 3), "mask": self.mask.cpu().numpy(),
                 "owner": owner}
 
@@ -602,14 +544,12 @@ class SplitHypothesesPnp:
         if self.exchange == "p2p":
             self.p2p.argmax(self.out.key, self.out.Rt, self.g_idx, self.g_cnt, self.g_Rt)
         else:
-            lib = cabi_lib()
             gkey = self.out.key
             if self.exchange == "nccl":
                 dist = _dist()
                 gkey = self.out.key.clone()
                 dist.all_reduce(gkey, op=dist.ReduceOp.MAX, group=self.group)
-            _check(lib.rg_argmax_unpack_dev(_vp(dv._stream()), 1, _vp(gkey.data_ptr()), _vp(self.g_idx.data_ptr()),
-                                            _vp(self.g_cnt.data_ptr())))
+            cabi.call("rg_argmax_unpack_dev", dv._stream(), 1, gkey, self.g_idx, self.g_cnt)
             if self.exchange == "nccl":
                 own = ((self.g_idx >= self.lo) & (self.g_idx < self.hi)).to(torch.float64)
                 self.g_Rt.copy_(torch.nan_to_num(self.out.Rt) * own)
@@ -624,18 +564,3 @@ class SplitHypothesesPnp:
         Rt = self.g_Rt.cpu().numpy().reshape(12)
         return {"best_idx": int(self.g_idx.item()), "best_count": int(self.g_cnt.item()), "R": Rt[:9].reshape(3, 3),
                 "t": Rt[9:].copy()}
-
-
-def cabi_lib():
-    from . import _cabi as cabi
-    return cabi.load_library()
-
-
-def _check(rc):
-    from . import _cabi as cabi
-    cabi.check(rc)
-
-
-def _vp(x):
-    import ctypes as C
-    return C.c_void_p(x)
