@@ -66,7 +66,13 @@ int rg_host_free(void* p);
  *            pass k run on a second stream while pass k+1 is solved and scored; 0 = one stream, strictly in order
  *            (results do not depend on it; the caller's stream sees the whole call complete either way)
  * option 11 = test hook: 1 = refinement of PnP poses (rg_pnp_refine_*) always on the multi-CTA path (default: views of
- *            <= 4096 correspondences run the whole loop in one CTA); same iteration, sums in a different order */
+ *            <= 4096 correspondences run the whole loop in one CTA); same iteration, sums in a different order
+ * option 12 = bounded sweep of F calls (default 1): rg_f_ransac_host / _host2 with counts == NULL and rg_f_ransac_dev2
+ *            with RG_FLAG_BOUNDED score every hypothesis on a prefix of each pair, finish the K best prefix counts, and
+ *            score in full only the pairs where another hypothesis could still reach the maximum (DESIGN.md section 4);
+ *            winners, counts, F and masks are those of the full sweep; 0 = every hypothesis against every correspondence
+ * option 13 = prefix share rho of the bounded sweep in thousandths, [1, 1000] (default 450); results do not depend on it
+ * option 14 = candidates K per pair of the bounded sweep, [1, 65536] (default 512); results do not depend on it */
 int rg_set_option(void* ctx, int option, long long value);
 /* summed milliseconds of {prepare, solve, score kernel, fixup + repair, select} over the PASSES since the last read
  * (at most 2048 passes are remembered; *out_calls = passes covered); synchronises `stream` */
@@ -100,9 +106,12 @@ int rg_f_ransac_dev(void* ctx, void* stream, int P, const double* pts64_dev, con
  *                     skip the bounding-box / FP32-copy kernels (hypothesis-split mode scores many hypothesis sets
  *                     against one pair);
  *   hyp_index_base  : hypothesis-split mode (SURVEY 8e item 2): this rank holds hypotheses [base, base + H_p) of every pair;
+ *   flags & RG_FLAG_BOUNDED : run the bounded sweep when option 12 is on (the results are the same; afterwards
+ *                     rg_f_last_hypotheses_dev returns no counts, since hypotheses that cannot win keep a prefix count);
  *   key_dev (P, optional) : the cross-GPU argmax key of every pair, (count << 32) | (0xFFFFFFFF - global hypothesis
  *                     index), 0 if no hypothesis of this rank has an inlier (fun.py:320-323: first maximum wins). */
 #define RG_FLAG_REUSE_POINTS 1
+#define RG_FLAG_BOUNDED 2
 int rg_f_ransac_dev2(void* ctx, void* stream, int P, const double* pts64_dev, const int32_t* pair_off_host,
                      const int32_t* idx_dev /* may be NULL */, const int32_t* hyp_off_host, double thr, int mode,
                      int tie_mode, int solver, int score_path, int flags, unsigned long long sample_seed, int first_pair_id,
@@ -124,10 +133,15 @@ int rg_f_inlier_mask_dev(void* ctx, void* stream, int P, const double* pts64_dev
  * after rg_f_ransac_host they cover only its last sub-batch — use that function's counts / F_all / flags outputs):
  * counts (hyp_off[P] int32), F_all (hyp_off[P] x 9 doubles), flags (bit0: rank-deficient sample, bit1: non-finite F,
  * bit2: a sample index outside [0, N) of the pair — the solver clamps it; rg_f_ransac_host then returns -2 and
- * rg_get_last_stats reports the number of such hypotheses in out8[4]) */
+ * rg_get_last_stats reports the number of such hypotheses in out8[4]).  *counts_dev is NULL after a bounded sweep. */
 int rg_f_last_hypotheses_dev(void* ctx, const int32_t** counts_dev, const double** F_all_dev,
                              const unsigned char** flags_dev);
-/* Same with host buffers; counts / F_all / flags / mask are optional (NULL = not copied back).  The batch is uploaded pass
+/* what the last F call executed: out4 = {hypothesis x correspondence evaluations, hypotheses not scored in full (proved
+ * unable to reach their pair's maximum), pairs that fell back to scoring every hypothesis in full, K (0: full sweep)}.
+ * Synchronises `stream`. */
+int rg_f_last_bounded_stats(void* ctx, void* stream, long long* out4);
+/* Same with host buffers; counts / F_all / flags / mask are optional (NULL = not copied back; counts == NULL runs the
+ * bounded sweep when option 12 is on).  The batch is uploaded pass
  * by pass on a second stream, so the copy of pass k+1 overlaps the scoring of pass k (page-locked buffers needed for the
  * overlap; pageable ones are still correct). */
 int rg_f_ransac_host(void* ctx, void* stream, int P, const double* pts64, const int32_t* pair_off, const int32_t* idx,

@@ -8,7 +8,7 @@ from . import _cabi, runtime, sampling  # noqa: F401
 from ._cabi import (MODE_EPI_MAX, MODE_SAMPSON, RGError, SCORE_FP32_GUARDED, SCORE_FP64, SOLVER_JACOBI, SOLVER_QR,  # noqa: F401
                     TIE_FIRST, TIE_REFERENCE, TRI_LINEAR, TRI_OPTIMAL)
 
-from ._cabi import FLAG_REUSE_POINTS  # noqa: F401
+from ._cabi import FLAG_BOUNDED, FLAG_REUSE_POINTS  # noqa: F401
 
 __all__ = ["runtime", "sampling", "lab3", "fun", "ransac", "pnp", "tables", "help_classes", "correspondences", "batched",
            "parallel", "synth", "philox", "device"]

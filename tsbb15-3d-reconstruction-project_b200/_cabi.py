@@ -20,6 +20,7 @@ SOLVER_QR, SOLVER_JACOBI = 0, 1
 SCORE_FP32_GUARDED, SCORE_FP64 = 0, 1
 TRI_OPTIMAL, TRI_LINEAR = 0, 1
 FLAG_REUSE_POINTS = 1
+FLAG_BOUNDED = 2
 
 _vp = C.c_void_p
 _i = C.c_int
@@ -53,6 +54,7 @@ SIGNATURES = {
     "rg_p2p_destroy": (_i, [_vp]),
     "rg_p2p_argmax_exchange": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rg_f_last_hypotheses_dev": (_i, [_vp, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp)]),
+    "rg_f_last_bounded_stats": (_i, [_vp, _vp, _pll]),
     "rg_f_ransac_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rg_f8pt_solve_host": (_i, [_vp, _vp, _i, _vp, _i, _vp, _i, _vp, _vp]),
     "rg_epi_score_count_host": (_i, [_vp, _vp, _i, _vp, _i, _vp, _d, _i, _i, _vp]),

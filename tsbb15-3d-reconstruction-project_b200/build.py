@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "librg_b200.so")
 SOURCES = ["librg_b200.cu"]
-HEADERS = ["ctx.cu", "f_api.cu", "pnp_api.cu", "geom_api.cu", "geom_kernels.cuh", "gs_api.cu", "gs_kernels.cuh", "ba_api.cu", "ba_kernels.cuh", "nccl_api.cu", "p2p_api.cu", "philox.cuh", "microbench.cu", "common.cuh", "score_core.cuh", "f_kernels.cuh", "jacobi.cuh", "pnp_kernels.cuh", "pnp_refine_api.cu", "pnp_refine_kernels.cuh", "tall.cuh", "plan.cuh"]
+HEADERS = ["ctx.cu", "f_api.cu", "pnp_api.cu", "geom_api.cu", "geom_kernels.cuh", "gs_api.cu", "gs_kernels.cuh", "ba_api.cu", "ba_kernels.cuh", "nccl_api.cu", "p2p_api.cu", "philox.cuh", "microbench.cu", "common.cuh", "score_core.cuh", "f_kernels.cuh", "jacobi.cuh", "pnp_kernels.cuh", "pnp_refine_api.cu", "pnp_refine_kernels.cuh", "tall.cuh", "plan.cuh", "bounded.cuh"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared", "-Xptxas", "-v", "-ldl"]
 

@@ -1,0 +1,195 @@
+// Bounded sweep of the F path: score every hypothesis on a prefix of each pair's correspondences, finish only the best
+// prefix scores, and prove that no other hypothesis can reach the pair's maximum.
+//
+// Per pass, after the head (memset, prepare, solve):
+//   prefix stage     score_packed over every hypothesis x groups [0, gA) (the main table's window) + fix-up: counts[h] = c_A(h),
+//                    the exact count over the first k = min(n, gA * kSub) correspondences
+//   bnd_select       per pair the K hypotheses with the largest (c_A, -index), gathered into compact Hyp32 records + map
+//   candidate stage  score_packed over the compact records x groups [gA, G) + fix-up (map: compact -> global index):
+//                    sfx_c[j] = exact count of candidate j over the other n - k correspondences
+//   bnd_check        L = max_j c_A + sfx_c over the candidates.  A non-candidate's full count is at most c_A(h) + (n - k); if
+//                    that is below L it can never be the maximum nor tie with it.  Pairs where some non-candidate has
+//                    c_A(h) + (n - k) >= L are marked; the others get the candidates' full counts written into counts.
+//   bnd_fb_plan      the fallback table: the marked pairs' items over [gA, G) for EVERY hypothesis (usually none)
+//   fallback stage   score_packed with the item count read from the device + fix-up into sfx_f; bnd_merge adds sfx_f to the
+//                    marked pairs' counts, which are then full counts for every hypothesis of those pairs.
+// In an unmarked pair a hypothesis that was not fully scored keeps c_A(h) <= full(h) < L <= max, so argmax_counts' first
+// maximum, the tie replay over the hypotheses with count == max and the winner's mask are those of a full sweep.
+#pragma once
+#include "score_core.cuh"
+
+namespace rg {
+
+// one 256-thread block fits beside the four resident scorer blocks of an SM (bnd_select runs beside the next pass's scorer)
+constexpr int kSelectThreads = 256;
+
+// exclusive prefix of `v` over the block (in thread order) and the block total; every thread calls it
+__device__ __forceinline__ int block_excl_scan(int v, int* s_warp, int& total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    int incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += t;
+    }
+    __syncthreads();
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    int before = 0;
+    total = 0;
+    for (int w = 0; w < nw; ++w) {
+        const int t = s_warp[w];
+        if (w < warp) before += t;
+        total += t;
+    }
+    return before + incl - v;
+}
+
+// One CTA per pair: the candidates are the min(K, H) hypotheses with the largest (c_A, -index), stored in index order.
+// sel[p] = {T, last, n_sel, 0}: a hypothesis is a candidate iff c_A > T or (c_A == T and index <= last); T = -1 when every
+// hypothesis is one.
+__global__ void __launch_bounds__(kSelectThreads) bnd_select(const int* __restrict__ counts, const PairInfo* __restrict__ pi,
+                                                              const PairInfo* __restrict__ pc, const Hyp32* __restrict__ hyp32,
+                                                              Hyp32* __restrict__ hypc, int* __restrict__ map,
+                                                              int4* __restrict__ sel) {
+    __shared__ int hist[256];
+    __shared__ int s_warp[32];
+    __shared__ int s_bin, s_k, s_last;
+    const int p = blockIdx.x;
+    const PairInfo info = pi[p];
+    const int Kp = pc[p].H, cbase = pc[p].hyp_off;
+    const int* cnt = counts + info.hyp_off;
+    int T = -1, need = 0;
+    if (Kp < info.H) {
+        // radix select of the Kp-th largest count, 8 bits at a time from the top
+        unsigned prefix = 0u, mask = 0u;
+        int k = Kp;
+        for (int shift = 24; shift >= 0; shift -= 8) {
+            for (int b = threadIdx.x; b < 256; b += blockDim.x) hist[b] = 0;
+            __syncthreads();
+            for (int h = threadIdx.x; h < info.H; h += blockDim.x) {
+                const unsigned v = (unsigned)cnt[h];
+                if ((v & mask) == prefix) atomicAdd(&hist[(v >> shift) & 255u], 1);
+            }
+            __syncthreads();
+            if (threadIdx.x == 0) {
+                int cum = 0, b = 255;
+                for (; b > 0 && cum + hist[b] < k; --b) cum += hist[b];
+                s_bin = b;
+                s_k = k - cum;
+            }
+            __syncthreads();
+            prefix |= (unsigned)s_bin << shift;
+            mask |= 255u << shift;
+            k = s_k;
+            __syncthreads();
+        }
+        T = (int)prefix;
+        need = k;                      // candidates among the hypotheses with c_A == T (the first `need` in index order)
+    }
+    if (threadIdx.x == 0) s_last = -1;
+    int taken = 0, ties = 0;
+    for (int base = 0; base < info.H; base += blockDim.x) {
+        const int h = base + threadIdx.x;
+        const int v = h < info.H ? cnt[h] : -2;
+        const bool eq = v == T;
+        int tot_eq = 0, tot_sel = 0;
+        const int eq_before = block_excl_scan(eq ? 1 : 0, s_warp, tot_eq);
+        const bool is_sel = h < info.H && (v > T || (eq && ties + eq_before < need));
+        const int pos = taken + block_excl_scan(is_sel ? 1 : 0, s_warp, tot_sel);
+        if (is_sel) {
+            RG_ASSERT(pos < Kp);
+            hypc[cbase + pos] = hyp32[info.hyp_off + h];
+            map[cbase + pos] = info.hyp_off + h;
+            if (eq) atomicMax(&s_last, h);
+        }
+        taken += tot_sel;
+        ties += tot_eq;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        RG_ASSERT(taken == Kp);
+        sel[p] = make_int4(T, s_last, taken, 0);
+    }
+}
+
+__device__ __forceinline__ int block_reduce_max(int v, int* s) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v = max(v, __shfl_xor_sync(0xffffffffu, v, o));
+    __syncthreads();
+    if ((threadIdx.x & 31) == 0) s[threadIdx.x >> 5] = v;
+    __syncthreads();
+    int r = s[0];
+    for (int w = 1; w < (int)(blockDim.x >> 5); ++w) r = max(r, s[w]);
+    return r;
+}
+
+// One CTA per pair, after the candidate stage's fix-up.  stats: [0] fallback evaluations, [1] hypotheses not fully scored,
+// [2] pairs that fell back.
+__global__ void __launch_bounds__(256) bnd_check(int* __restrict__ counts, const int* __restrict__ sfx_c,
+                                                  const int* __restrict__ map, const PairInfo* __restrict__ pi,
+                                                  const PairInfo* __restrict__ pc, const int4* __restrict__ sel,
+                                                  int* __restrict__ mark, unsigned long long* __restrict__ stats) {
+    __shared__ int s_red[8];
+    const int p = blockIdx.x;
+    const PairInfo info = pi[p];
+    const int Kp = pc[p].H, cbase = pc[p].hyp_off;
+    const int4 sl = sel[p];
+    const int rest = info.n - min(info.n, info.g_end * kSub);     // correspondences outside the prefix
+    int L = 0;
+    for (int j = threadIdx.x; j < Kp; j += blockDim.x) L = max(L, counts[map[cbase + j]] + sfx_c[cbase + j]);
+    L = block_reduce_max(L, s_red);
+    // escapees: non-candidates whose bound reaches L (>=: a tie with the maximum must be scored too)
+    int esc = 0;
+    for (int h = threadIdx.x; h < info.H; h += blockDim.x) {
+        const int v = counts[info.hyp_off + h];
+        const bool cand = v > sl.x || (v == sl.x && h <= sl.y);
+        esc |= (!cand && (long long)v + rest >= (long long)L) ? 1 : 0;
+    }
+    esc = block_reduce_max(esc, s_red);
+    if (esc) {
+        if (threadIdx.x == 0) {
+            mark[p] = 1;
+            atomicAdd(&stats[0], (unsigned long long)info.H * (unsigned long long)rest);
+            atomicAdd(&stats[2], 1ull);
+        }
+        return;
+    }
+    for (int j = threadIdx.x; j < Kp; j += blockDim.x) counts[map[cbase + j]] += sfx_c[cbase + j];
+    if (threadIdx.x == 0 && info.H > Kp) atomicAdd(&stats[1], (unsigned long long)(info.H - Kp));
+}
+
+// One CTA: the live fallback table = the template with the items of unmarked pairs removed; *n_items = their total.
+__global__ void __launch_bounds__(kSelectThreads) bnd_fb_plan(const PairInfo* __restrict__ pf, const int* __restrict__ mark,
+                                                               int P, PairInfo* __restrict__ fb, int* __restrict__ n_items) {
+    __shared__ int s_warp[32];
+    int run = 0;
+    for (int base = 0; base < P; base += blockDim.x) {
+        const int p = base + threadIdx.x;
+        int items = 0;
+        PairInfo o;
+        if (p < P) {
+            o = pf[p];
+            if (mark[p] && o.groups_per_split > 0) items = (o.H + kHypPerBlock - 1) / kHypPerBlock * o.nsplit;
+        }
+        int tot = 0;
+        const int before = block_excl_scan(items, s_warp, tot);
+        if (p < P) {
+            o.item_off = run + before;
+            fb[p] = o;
+        }
+        run += tot;
+    }
+    if (threadIdx.x == 0) *n_items = run;
+}
+
+// One CTA per pair: marked pairs add the fallback's suffix counts to the prefix counts
+__global__ void __launch_bounds__(256) bnd_merge(int* __restrict__ counts, const int* __restrict__ sfx_f,
+                                                  const PairInfo* __restrict__ pi, const int* __restrict__ mark) {
+    const int p = blockIdx.x;
+    if (!mark[p]) return;
+    const PairInfo info = pi[p];
+    for (int h = threadIdx.x; h < info.H; h += blockDim.x) counts[info.hyp_off + h] += sfx_f[info.hyp_off + h];
+}
+
+}  // namespace rg

@@ -155,9 +155,11 @@ struct PairInfo {
     int n_all;                 // PnP: all correspondences of the view (n = those that vote, n <= n_all); F path: n_all == n
     int hyp_first;             // index of the pair's first hypothesis inside the pair's full hypothesis set (hypothesis-split
                                // mode: this rank holds hypotheses [hyp_first, hyp_first + H) of the pair); 0 otherwise
-    int pad0;
+    int g_base, g_end;         // window of kSub-point groups the scorer's items cover (absolute groups of the pair; a full
+                               // sweep has [0, n_pad / kSub), the bounded sweep scores a prefix and a suffix, bounded.cuh)
+    int pad0, pad1, pad2;
 };
-static_assert(sizeof(PairInfo) == 48, "PairInfo layout");
+static_assert(sizeof(PairInfo) == 64, "PairInfo layout");
 
 // Frame of the FP32 scorer, computed on the device from the pair's bounding box (f_normalise):
 // x~ = (x - c1)/thr, y~ = (y - c2)/thr  => threshold is exactly 1, |x~|,|y~| <= B.  Kept apart from PairInfo so that a
@@ -174,7 +176,13 @@ struct FPlan {
     long long Ntot = 0, Htot = 0, N32tot = 0;
     int n_items = 0;
     int maxN = 0, maxH = 0;
-    double evals = 0.0;                  // sum_p n_p * H_p
+    double evals = 0.0;                  // sum_p n_p * H_p (bounded sweep: of the prefix stage)
+    // bounded sweep (bounded.cuh): three tables per pass, [prefix stage | candidate suffix stage | fallback template]
+    bool bounded = false;
+    int K = 0;                           // candidates per pair
+    long long Ctot = 0;                  // candidates of the pass (sum_p min(K, H_p))
+    int n_items_c = 0, n_items_f = 0;    // scorer items of the candidate stage / of the fallback with every pair marked
+    double evals_c = 0.0, evals_f = 0.0; // their evaluations (real correspondences)
 };
 
 struct Ctx {
@@ -182,6 +190,7 @@ struct Ctx {
     int sm_count = 0;
     // device workspaces (grow-only)
     Buffer pair_info, pair_frame, state, pts32, F64, hyp32, flags, flag_list, stats, best, tie_stats, bbox;
+    Buffer bnd;                                    // bounded sweep: candidate records, compact -> global map, selection, fallback table
     // `state` = everything one cudaMemsetAsync clears per pass: [bbox keys][counts][work counter, list size][ovf bytes]
     int* counts_ptr = nullptr;                     // inside `state` (valid after f_state_layout of the current pass)
     unsigned char* ovf_ptr = nullptr;
@@ -189,12 +198,15 @@ struct Ctx {
     // Pass pipelining (F calls of several passes): the caller's stream runs the scorers back to back; the solver ("head") of
     // pass k+1 and the fix-up / selection / mask kernels ("tail") of pass k-1 run on a second stream BESIDE the scorer of pass k
     // — they are latency bound (23 % issue active) and one of their blocks fits next to the scorer's four on every SM.  The
-    // per-pass workspaces exist twice; ws_swap() exchanges the named buffers with this second set, so all the code keeps
-    // using c->F64, c->state, ... for "the set of the pass being queued".
-    struct PassSet { Buffer pair_info, pair_frame, state, pts32, F64, hyp32, flags, flag_list, best, tie_stats; } alt;
+    // per-pass workspaces exist two or three times (the bounded sweep keeps a pass alive across the next pass's prefix
+    // stage); ws_use() moves the named buffers into spare[ws_slot] and those of the wanted set out of spare[slot], so all the
+    // code keeps using c->F64, c->state, ... for "the set of the pass being queued".  spare[ws_slot] is always empty.
+    struct PassSet { Buffer pair_info, pair_frame, state, pts32, F64, hyp32, flags, flag_list, best, tie_stats, bnd; } spare[3];
     cudaStream_t tail_stream = nullptr;
-    cudaEvent_t head_done[2] = {nullptr, nullptr};      // recorded on the side stream after the solver of the pass in set i
-    cudaEvent_t score_done[2] = {nullptr, nullptr};     // recorded on the caller's stream after the scorer of the pass in set i
+    cudaEvent_t head_done[3] = {nullptr, nullptr, nullptr};   // recorded on the side stream after the solver of the pass in set i
+    cudaEvent_t score_done[3] = {nullptr, nullptr, nullptr};  // recorded on the caller's stream after the scorer of the pass in set i
+    cudaEvent_t cand_done[3] = {nullptr, nullptr, nullptr};   // bounded sweep: side stream, candidates of the pass in set i chosen
+    cudaEvent_t sweep_done[3] = {nullptr, nullptr, nullptr};  // bounded sweep: caller's stream, last scorer of the pass in set i
     cudaEvent_t tail_done[2] = {nullptr, nullptr};      // [0]: recorded on the side stream behind the last tail kernel of a run
     cudaEvent_t pipe_gate = nullptr;                    // recorded on the caller's stream before the side stream starts a run
     bool tail_pending[2] = {false, false};              // tail_done[i] was recorded and nobody has waited for it yet
@@ -212,6 +224,12 @@ struct Ctx {
     long long opt_list_cap = 0;                    // option 8 (test hook): capacity of the guard-band flag list in records (0 = automatic)
     double opt_band_scale = 1.0;                   // option 9: guard-band safety factor (>= 1)
     long long opt_pass_evals = 0;                  // option 6: evaluations per pass of a large batch (0 = default)
+    int opt_bounded = 1;                           // option 12: F calls without per-hypothesis counts run the bounded sweep
+    int opt_rho_milli = 450;                       // option 13: prefix share rho of the bounded sweep, in thousandths
+    int opt_bounded_k = 512;                       // option 14: candidates per pair of the bounded sweep
+    bool last_bounded = false;                     // the last F call ran the bounded sweep (its counts are not full counts)
+    long long bnd_host_evals = 0;                  // evaluations of its prefix and candidate stages (known on the host)
+    Buffer bnd_stats;                              // device: [0] fallback evaluations, [1] hypotheses not fully scored, [2] fallback pairs
     // peer-to-peer argmax exchange (hypothesis-split mode over NVLink), see p2p_api.cu
     void* p2p_local = nullptr; size_t p2p_bytes = 0; int p2p_rank = 0, p2p_world = 0; unsigned p2p_seq = 0;
     void* p2p_peer[16] = {nullptr};
@@ -256,7 +274,8 @@ struct Ctx {
     int opt_profile = 0;
     static constexpr int kProfPhases = 5;          // prepare, solve, score kernel, fixup+repair, select
     static constexpr int kProfScoreStart = 6;      // extra boundary: the scorer's own start (pipelined passes: the solver ended long before)
-    static constexpr int kProfEvents = 7;          // boundaries 0..5 + the scorer start
+    static constexpr int kProfSweep = 7;           // bounded sweep: boundaries 7/8 around the candidate stage's scorer, 9/10 the fallback's
+    static constexpr int kProfEvents = 11;         // boundaries 0..5 + the scorer start + the two later scorer launches
     static constexpr int kProfRing = 2048;         // passes remembered between two reads (20 steps of a tapered 64-pass sweep)
     cudaEvent_t* prof_ev = nullptr;                // kProfRing * kProfEvents events
     int prof_cur = -1;                             // pass opened by the last prof_mark(.., 0) (sequential callers)

@@ -118,16 +118,20 @@ int rg_shutdown(void* ctx) {
     cudaDeviceSynchronize();
     for (Buffer* b : {&c->pair_info, &c->pair_frame, &c->state, &c->bbox, &c->pts32, &c->F64, &c->hyp32, &c->flags,
                       &c->flag_list, &c->gen_idx, &c->stats, &c->best, &c->tie_stats, &c->d_in_a, &c->d_in_b, &c->d_in_c, &c->geom, &c->geom_ws, &c->gs_ws, &c->ba_ws, &c->pr_ws, &c->d_out_a, &c->d_out_b,
-                      &c->d_out_c, &c->d_out_d, &c->pose64, &c->pose32, &c->X32})
+                      &c->d_out_c, &c->d_out_d, &c->pose64, &c->pose32, &c->X32, &c->bnd, &c->bnd_stats})
         release(*b);
-    for (Buffer* b : {&c->alt.pair_info, &c->alt.pair_frame, &c->alt.state, &c->alt.pts32, &c->alt.F64, &c->alt.hyp32,
-                      &c->alt.flags, &c->alt.flag_list, &c->alt.best, &c->alt.tie_stats})
-        release(*b);
-    for (int i = 0; i < 2; ++i) {
+    for (Ctx::PassSet& o : c->spare)
+        for (Buffer* b : {&o.pair_info, &o.pair_frame, &o.state, &o.pts32, &o.F64, &o.hyp32, &o.flags, &o.flag_list, &o.best,
+                          &o.tie_stats, &o.bnd})
+            release(*b);
+    for (int i = 0; i < 3; ++i) {
         if (c->head_done[i]) cudaEventDestroy(c->head_done[i]);
         if (c->score_done[i]) cudaEventDestroy(c->score_done[i]);
-        if (c->tail_done[i]) cudaEventDestroy(c->tail_done[i]);
+        if (c->cand_done[i]) cudaEventDestroy(c->cand_done[i]);
+        if (c->sweep_done[i]) cudaEventDestroy(c->sweep_done[i]);
     }
+    for (int i = 0; i < 2; ++i)
+        if (c->tail_done[i]) cudaEventDestroy(c->tail_done[i]);
     if (c->pipe_gate) cudaEventDestroy(c->pipe_gate);
     if (c->tail_stream) cudaStreamDestroy(c->tail_stream);
     release_pinned(c->h_stage[0]);
@@ -188,6 +192,11 @@ int rg_device_sm_count(void* ctx) { return ctx ? ((Ctx*)ctx)->sm_count : 0; }
 //           stream while pass k+1 is solved and scored (two sets of per-pass workspaces); 0 = strictly one after the other
 // option 11: 1 = refinement of PnP poses always on the multi-CTA path (default: views of <= 4096 correspondences run the whole
 //           Levenberg-Marquardt loop in one CTA, one launch per round); test hook comparing the two paths
+// option 12: 1 (default) = F calls that want no per-hypothesis counts run the bounded sweep (bounded.cuh: hypotheses that
+//           provably cannot reach their pair's maximum are not scored in full; results are those of the full sweep);
+//           0 = every hypothesis against every correspondence
+// option 13: prefix share rho of the bounded sweep in thousandths, in [1, 1000] (default 450)
+// option 14: candidates per pair of the bounded sweep, in [1, 65536] (default 512)
 // option 9: guard-band safety factor x 1000 (default 1000 = the proven FP32 rounding bound); larger values keep every result
 //           exact and only send more evaluations to the FP64 recheck — used to MEASURE what a less accurate scorer
 //           (tensor-core split-precision accumulation) would cost in fix-up time
@@ -256,6 +265,21 @@ int rg_set_option(void* ctx, int option, long long value) {
         c->opt_pr_multi = (int)value;
         return RG_OK;
     }
+    if (option == 12) {
+        if (value != 0 && value != 1) { set_error("invalid argument: option 12 (bounded sweep) must be 0 or 1"); return RG_ERR_ARG; }
+        c->opt_bounded = (int)value;
+        return RG_OK;
+    }
+    if (option == 13) {
+        if (value < 1 || value > 1000) { set_error("invalid argument: option 13 (prefix share x 1000) must be in [1, 1000]"); return RG_ERR_ARG; }
+        c->opt_rho_milli = (int)value;
+        return RG_OK;
+    }
+    if (option == 14) {
+        if (value < 1 || value > 65536) { set_error("invalid argument: option 14 (candidates per pair) must be in [1, 65536]"); return RG_ERR_ARG; }
+        c->opt_bounded_k = (int)value;
+        return RG_OK;
+    }
     if (option == 8) {
         if (value < 0 || value > 1000000000ll) { set_error("invalid argument: option 8 (flag list capacity) must be in [0, 1e9]"); return RG_ERR_ARG; }
         c->opt_list_cap = value;
@@ -267,6 +291,8 @@ int rg_set_option(void* ctx, int option, long long value) {
 
 // Phase times of the calls made since profiling was switched on / last read (option 1): out_ms[0..4] = summed
 // milliseconds of {prepare, solve, score kernel, fixup + repair, select}, *out_calls = number of calls covered.
+// A pass of the bounded sweep has three scorer launches: its score phase is their sum; its fixup phase runs from the end of
+// the prefix stage to the chosen candidates, and its select phase from there to the end of its tail.
 // Synchronises the stream; resets the ring.
 int rg_get_profile(void* ctx, void* stream, double* out_ms5, int* out_calls) {
     RG_CHECK_ARG(ctx != nullptr && out_ms5 != nullptr && out_calls != nullptr, "null argument");
@@ -285,6 +311,12 @@ int rg_get_profile(void* ctx, void* stream, double* out_ms5, int* out_calls) {
             float ms = 0.f;
             RG_CUDA(cudaEventElapsedTime(&ms, (k == 2 && own_start) ? e[Ctx::kProfScoreStart] : e[k], e[k + 1]));
             out_ms5[k] += ms;
+        }
+        for (int b = Ctx::kProfSweep; b + 1 < Ctx::kProfEvents; b += 2) {   // the bounded sweep's later scorer launches
+            if (((c->prof_masks[call] >> b) & 3u) != 3u) continue;
+            float ms = 0.f;
+            RG_CUDA(cudaEventElapsedTime(&ms, e[b], e[b + 1]));
+            out_ms5[2] += ms;
         }
         ++complete;
     }

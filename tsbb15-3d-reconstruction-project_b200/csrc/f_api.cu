@@ -4,9 +4,11 @@
 //   memset(state) -> [f_bbox -> f_normalise] -> f8_solve (draws its own samples when idx is NULL) -> score_packed -> fixup_list -> argmax_counts
 //   -> [f_tie_stats -> f_tie_resolve] -> f_mask
 // over a contiguous block of pairs whose workspaces (hypotheses, FP32 points, flag list) stay bounded; BASELINE config 5
-// (4096 pairs x 50 000 x 8 192) runs as 64 passes of 64 pairs.  The per-pass PairInfo table is planned on the host into
+// (4096 pairs x 50 000 x 8 192) runs as 64 passes of 64 pairs.  A call that wants no per-hypothesis counts runs the bounded
+// sweep instead of score_packed -> fixup_list (bounded.cuh): prefix stage, candidates, candidate suffix stage, check, fallback.  The per-pass PairInfo table is planned on the host into
 // double-buffered pinned staging, so the host plans pass k+1 while pass k runs.
 #include "f_kernels.cuh"
+#include "bounded.cuh"
 #include "jacobi.cuh"
 #include "philox.cuh"
 #include "plan.cuh"
@@ -15,7 +17,7 @@
 
 namespace rg {
 
-enum : int { FLAG_REUSE_POINTS = 1 };
+enum : int { FLAG_REUSE_POINTS = 1, FLAG_BOUNDED = 2 };
 
 constexpr double kDefaultPassEvals = 2.7e10;        // 64 pairs of the config-5 shape
 constexpr long long kMaxPassHyp = 1ll << 22;        // hypotheses per pass (F64 workspace 288 MB)
@@ -23,16 +25,26 @@ constexpr long long kMaxPassHyp = 1ll << 22;        // hypotheses per pass (F64 
 struct ScoreState {
     unsigned* bbox; int* counts; int* work; unsigned* list_n; unsigned char* ovf;
     size_t off_counts, bytes;
+    // bounded sweep (Ctot >= 0): work counters / list sizes of the candidate (c) and fallback (f) stages, the fallback's
+    // item count, suffix counts, marks of the pairs that fell back, overflow marks
+    int *c_work, *f_work, *f_items, *sfx_c, *sfx_f, *mark;
+    unsigned *c_list_n, *f_list_n;
+    unsigned char *ovf_c, *ovf_f;
 };
 
-// [bbox keys: P x words][counts: H][work counter][list size][pad][ovf: H bytes] — one cudaMemsetAsync clears a pass's state
-int score_state_layout(Ctx* c, int P, long long Htot, int bbox_words, ScoreState& s) {
+// [bbox keys: P x words][counts: H][work counter][list size][pad][ovf: H bytes]
+//   + bounded sweep: [8 counters][sfx_c: C][sfx_f: H][mark: P][ovf_c: C bytes][ovf_f: H bytes]
+// — one cudaMemsetAsync clears a pass's state
+int score_state_layout(Ctx* c, int P, long long Htot, int bbox_words, ScoreState& s, long long Ctot = -1) {
     const size_t H = (size_t)std::max<long long>(Htot, 1);
     const size_t bbox_bytes = (((size_t)std::max(P, 1) * bbox_words * 4) + 15) / 16 * 16;
     const size_t cnt_bytes = ((H + 2) * 4 + 15) / 16 * 16;
     const size_t ovf_bytes = (H + 15) / 16 * 16;
+    const size_t C = (size_t)std::max<long long>(Ctot, 1);
+    const size_t bnd_ints = Ctot >= 0 ? ((8 + C + H + (size_t)std::max(P, 1)) * 4 + 15) / 16 * 16 : 0;
+    const size_t bnd_ovf = Ctot >= 0 ? (C + H + 15) / 16 * 16 : 0;
     s.off_counts = bbox_bytes;
-    s.bytes = bbox_bytes + cnt_bytes + ovf_bytes;
+    s.bytes = bbox_bytes + cnt_bytes + ovf_bytes + bnd_ints + bnd_ovf;
     int rc = ensure(c->state, s.bytes);
     if (rc) return rc;
     char* base = (char*)c->state.ptr;
@@ -41,8 +53,27 @@ int score_state_layout(Ctx* c, int P, long long Htot, int bbox_words, ScoreState
     s.work = s.counts + H;
     s.list_n = (unsigned*)(s.counts + H + 1);
     s.ovf = (unsigned char*)(base + bbox_bytes + cnt_bytes);
+    if (Ctot >= 0) {
+        int* b = (int*)(base + bbox_bytes + cnt_bytes + ovf_bytes);
+        s.c_work = b; s.c_list_n = (unsigned*)(b + 1); s.f_work = b + 2; s.f_list_n = (unsigned*)(b + 3); s.f_items = b + 4;
+        s.sfx_c = b + 8; s.sfx_f = s.sfx_c + C; s.mark = s.sfx_f + H;
+        s.ovf_c = (unsigned char*)(base + bbox_bytes + cnt_bytes + ovf_bytes + bnd_ints);
+        s.ovf_f = s.ovf_c + C;
+    }
     c->counts_ptr = s.counts;
     c->ovf_ptr = s.ovf;
+    return RG_OK;
+}
+
+// per-set workspace of the bounded sweep: [compact Hyp32 records: C][map: C][sel: P int4][live fallback table: P]
+struct BndWs { Hyp32* hypc; int* map; int4* sel; PairInfo* fb; };
+static int bnd_workspace(Ctx* c, const FPlan& plan, BndWs& w) {
+    const size_t C = (size_t)std::max<long long>(plan.Ctot, 1), P = (size_t)std::max(plan.P, 1);
+    const size_t o_map = C * sizeof(Hyp32), o_sel = o_map + (C * 4 + 63) / 64 * 64, o_fb = o_sel + P * sizeof(int4);
+    int rc = ensure(c->bnd, o_fb + P * sizeof(PairInfo));
+    if (rc) return rc;
+    char* b = (char*)c->bnd.ptr;
+    w.hypc = (Hyp32*)b; w.map = (int*)(b + o_map); w.sel = (int4*)(b + o_sel); w.fb = (PairInfo*)(b + o_fb);
     return RG_OK;
 }
 
@@ -72,20 +103,28 @@ struct FCall {
     double thr = 1.5;
     int mode = MODE_EPI_MAX, tie_mode = TIE_FIRST, solver = SOLVER_QR, score_path = SCORE_FP32_GUARDED, flags = 0;
     unsigned long long sample_seed = 0; int first_pair = 0; int hyp_first = 0;
+    bool bounded = false;          // bounded sweep (bounded.cuh): the per-hypothesis counts are not all full counts
     int* best_idx = nullptr; int* best_count = nullptr; double* best_F = nullptr; unsigned char* mask = nullptr;
     unsigned long long* keys = nullptr;
 };
 
-// ---- pass pipelining (Ctx::alt, common.cuh; the driver is f_run_piped below) ----
-// Single-pass calls never swap: their launch chain stays on the caller's stream in the current set (capturable in a CUDA graph,
-// RG_FLAG_REUSE_POINTS finds its prepared points).
-static void ws_swap(Ctx* c) {
-    std::swap(c->pair_info, c->alt.pair_info);   std::swap(c->pair_frame, c->alt.pair_frame);
-    std::swap(c->state, c->alt.state);           std::swap(c->pts32, c->alt.pts32);
-    std::swap(c->F64, c->alt.F64);               std::swap(c->hyp32, c->alt.hyp32);
-    std::swap(c->flags, c->alt.flags);           std::swap(c->flag_list, c->alt.flag_list);
-    std::swap(c->best, c->alt.best);             std::swap(c->tie_stats, c->alt.tie_stats);
-    c->ws_slot ^= 1;
+// ---- pass pipelining (Ctx::spare, common.cuh; the drivers are f_run_piped / f_run_piped_bounded below) ----
+// Single-pass calls never switch: their launch chain stays on the caller's stream in the current set (capturable in a CUDA
+// graph, RG_FLAG_REUSE_POINTS finds its prepared points).
+static void ws_exchange(Ctx* c, Ctx::PassSet& o) {
+    std::swap(c->pair_info, o.pair_info);   std::swap(c->pair_frame, o.pair_frame);
+    std::swap(c->state, o.state);           std::swap(c->pts32, o.pts32);
+    std::swap(c->F64, o.F64);               std::swap(c->hyp32, o.hyp32);
+    std::swap(c->flags, o.flags);           std::swap(c->flag_list, o.flag_list);
+    std::swap(c->best, o.best);             std::swap(c->tie_stats, o.tie_stats);
+    std::swap(c->bnd, o.bnd);
+}
+
+static void ws_use(Ctx* c, int slot) {
+    if (c->ws_slot == slot) return;
+    ws_exchange(c, c->spare[c->ws_slot]);        // park the current set (its spare entry was empty) ...
+    ws_exchange(c, c->spare[slot]);              // ... and take the wanted one out of its entry
+    c->ws_slot = slot;
     c->plan_valid = false;                       // the cached PairInfo table lives in the set that just left
     c->prep_pts = nullptr;                       // ... and so do the prepared points
 }
@@ -108,6 +147,8 @@ static int tail_carveout(Ctx* c, bool want_max) {
     RG_CUDA(cudaFuncSetAttribute(f_tie_resolve, cudaFuncAttributePreferredSharedMemoryCarveout, v));
     RG_CUDA(cudaFuncSetAttribute(f8_solve_qr<MODE_EPI_MAX>, cudaFuncAttributePreferredSharedMemoryCarveout, v));
     RG_CUDA(cudaFuncSetAttribute(f8_solve_qr<MODE_SAMPSON>, cudaFuncAttributePreferredSharedMemoryCarveout, v));
+    for (const void* f : {(const void*)bnd_select, (const void*)bnd_check, (const void*)bnd_fb_plan, (const void*)bnd_merge})
+        RG_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, v));
     c->tail_carve_max = (int)want_max;
     return RG_OK;
 }
@@ -119,11 +160,14 @@ static int pipe_setup(Ctx* c) {
         RG_CUDA(cudaDeviceGetStreamPriorityRange(&lo_p, &hi_p));
         RG_CUDA(cudaStreamCreateWithPriority(&c->tail_stream, cudaStreamNonBlocking, low ? lo_p : 0));
     }
-    for (int i = 0; i < 2; ++i) {
+    for (int i = 0; i < 3; ++i) {
         if (!c->head_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->head_done[i], cudaEventDisableTiming));
         if (!c->score_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->score_done[i], cudaEventDisableTiming));
-        if (!c->tail_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->tail_done[i], cudaEventDisableTiming));
+        if (!c->cand_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->cand_done[i], cudaEventDisableTiming));
+        if (!c->sweep_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->sweep_done[i], cudaEventDisableTiming));
     }
+    for (int i = 0; i < 2; ++i)
+        if (!c->tail_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->tail_done[i], cudaEventDisableTiming));
     if (!c->pipe_gate) RG_CUDA(cudaEventCreateWithFlags(&c->pipe_gate, cudaEventDisableTiming));
     return RG_OK;
 }
@@ -205,6 +249,8 @@ struct PassCtl {
     FPlan plan;
     ScoreState s;
     FlagList fl{nullptr, nullptr, 0u, nullptr};
+    FlagList flc{nullptr, nullptr, 0u, nullptr}, flf{nullptr, nullptr, 0u, nullptr};   // bounded sweep: candidate / fallback stage
+    BndWs bw{};
     bool scored = false;                  // the packed scorer ran: its flag list wants the fix-up
     int slot = 0;                         // workspace set of the pass (Ctx::alt)
     int prof_call = -1;                   // ring index of the pass's phase events (option 1)
@@ -226,8 +272,13 @@ static int f_score_only(Ctx* c, cudaStream_t st, PassCtl& k) {
     if (k.a.score_path == SCORE_FP32_GUARDED) {
         int bps = 1, rc = score_blocks_per_sm<EpiPolicy<MODE>>(&bps);
         if (rc) return rc;
-        k.fl = flag_list_for(c, k.s, plan.evals, &rc);
+        // (the later stages of a bounded pass reuse the records once the previous stage's fix-up has read them)
+        k.fl = flag_list_for(c, k.s, std::max(plan.evals, plan.evals_f), &rc);
         if (rc) return rc;
+        if (plan.bounded) {
+            k.flc = FlagList{k.fl.rec, k.s.c_list_n, k.fl.cap, k.s.ovf_c};
+            k.flf = FlagList{k.fl.rec, k.s.f_list_n, k.fl.cap, k.s.ovf_f};
+        }
         constexpr size_t smem = score_smem_bytes<EpiPolicy<MODE>>();
         const int grid = std::min(plan.n_items, c->sm_count * bps);
         score_packed<EpiPolicy<MODE>><<<grid, kScoreThreads, smem, st>>>((const float4*)c->pts32.ptr, (const Hyp32*)c->hyp32.ptr,
@@ -245,20 +296,84 @@ static int f_score_only(Ctx* c, cudaStream_t st, PassCtl& k) {
 
 // beside_scorer: the kernel will run NEXT TO the following pass's scorer (4 blocks x 128 threads x 96 registers per SM leave
 // room for exactly one 256-thread, 64-register block): a grid of one block per SM runs beside the scorer instead of ahead of it
+// stage: what the fix-up corrects — STAGE_MAIN the pass's scorer (full sweep, or the bounded sweep's prefix stage), STAGE_CAND
+// the candidate suffix stage (compact records, counts in sfx_c), STAGE_FALLBACK the fallback stage (counts in sfx_f)
+enum : int { STAGE_MAIN = 0, STAGE_CAND = 1, STAGE_FALLBACK = 2 };
 template <int MODE>
-static int f_fixup_launch(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) {
+static int f_fixup_launch(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer, int stage = STAGE_MAIN) {
     if (!k.scored) return RG_OK;
     const FPlan& plan = k.plan;
-    typename EpiFix<MODE>::Params fp{(const float4*)c->pts32.ptr, (const double4*)k.a.pts64, (const Hyp32*)c->hyp32.ptr,
-                                     (const double*)c->F64.ptr, (const PairInfo*)c->pair_info.ptr,
-                                     (const PairFrame*)c->pair_frame.ptr, plan.P};
-    int fgrid = fixup_grid(c, plan.evals);
+    const PairInfo* pi = (const PairInfo*)c->pair_info.ptr;
+    const Hyp32* hyp = (const Hyp32*)c->hyp32.ptr;
+    const int* map = nullptr;
+    FlagList fl = k.fl;
+    long long H = plan.Htot;
+    int* counts = k.s.counts;
+    double evals = plan.evals;
+    if (stage == STAGE_CAND) {
+        pi += plan.P; hyp = k.bw.hypc; map = k.bw.map; fl = k.flc; H = plan.Ctot; counts = k.s.sfx_c; evals = plan.evals_c;
+    } else if (stage == STAGE_FALLBACK) {
+        pi = k.bw.fb; fl = k.flf; counts = k.s.sfx_f; evals = plan.evals_f;
+    }
+    typename EpiFix<MODE>::Params fp{(const float4*)c->pts32.ptr, (const double4*)k.a.pts64, hyp, (const double*)c->F64.ptr,
+                                     pi, (const PairFrame*)c->pair_frame.ptr, plan.P, map};
+    int fgrid = fixup_grid(c, evals);
     if (beside_scorer) {
         static const int forced = [] { const char* e = getenv("RG_TAIL_GRID"); return e ? atoi(e) : 0; }();   // experiment hook
         fgrid = std::min(fgrid, forced > 0 ? forced : c->sm_count);
     }
-    fixup_list<EpiFix<MODE>><<<fgrid, 256, 0, ts>>>(fp, k.fl, (int)plan.Htot, k.s.counts, (unsigned long long*)c->stats.ptr);
+    fixup_list<EpiFix<MODE>><<<fgrid, 256, 0, ts>>>(fp, fl, (int)H, counts, (unsigned long long*)c->stats.ptr);
     c->last_stats[7] += 1;
+    RG_CUDA(cudaGetLastError());
+    return RG_OK;
+}
+
+// bounded sweep, after the prefix stage: its fix-up (exact prefix counts c_A) and the choice of the candidates
+template <int MODE>
+static int f_bnd_cands(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) {
+    if (k.scored) {
+        int rc = f_fixup_launch<MODE>(c, ts, k, beside_scorer);
+        if (rc) return rc;
+        const PairInfo* pi = (const PairInfo*)c->pair_info.ptr;
+        bnd_select<<<k.plan.P, kSelectThreads, 0, ts>>>(k.s.counts, pi, pi + k.plan.P, (const Hyp32*)c->hyp32.ptr, k.bw.hypc,
+                                                        k.bw.map, k.bw.sel);
+        c->last_stats[7] += 1;
+        RG_CUDA(cudaGetLastError());
+    }
+    prof_mark_at(c, ts, k.prof_call, 4);
+    return RG_OK;
+}
+
+// bounded sweep, after the candidates: candidate suffix stage + its fix-up, check, fallback stage (queued at full grid, its
+// item count comes from bnd_fb_plan: normally zero).  The fallback's fix-up and merge belong to the tail.
+template <int MODE>
+static int f_bnd_sweep(Ctx* c, cudaStream_t st, PassCtl& k) {
+    if (!k.scored) return RG_OK;
+    const FPlan& plan = k.plan;
+    const PairInfo* pi = (const PairInfo*)c->pair_info.ptr;
+    int bps = 1, rc = score_blocks_per_sm<EpiPolicy<MODE>>(&bps);
+    if (rc) return rc;
+    constexpr size_t smem = score_smem_bytes<EpiPolicy<MODE>>();
+    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep);
+    if (plan.n_items_c > 0) {
+        score_packed<EpiPolicy<MODE>><<<std::min(plan.n_items_c, c->sm_count * bps), kScoreThreads, smem, st>>>(
+            (const float4*)c->pts32.ptr, k.bw.hypc, pi + plan.P, plan.P, plan.n_items_c, k.s.sfx_c, k.flc, k.s.c_work);
+        c->last_stats[7] += 1;
+    }
+    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 1);
+    if (plan.n_items_c > 0 && (rc = f_fixup_launch<MODE>(c, st, k, false, STAGE_CAND))) return rc;
+    bnd_check<<<plan.P, 256, 0, st>>>(k.s.counts, k.s.sfx_c, k.bw.map, pi, pi + plan.P, k.bw.sel, k.s.mark,
+                                      (unsigned long long*)c->bnd_stats.ptr);
+    bnd_fb_plan<<<1, kSelectThreads, 0, st>>>(pi + 2 * (size_t)plan.P, k.s.mark, plan.P, k.bw.fb, k.s.f_items);
+    c->last_stats[7] += 2;
+    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 2);
+    if (plan.n_items_f > 0) {
+        score_packed<EpiPolicy<MODE>><<<std::min(plan.n_items_f, c->sm_count * bps), kScoreThreads, smem, st>>>(
+            (const float4*)c->pts32.ptr, (const Hyp32*)c->hyp32.ptr, k.bw.fb, plan.P, plan.n_items_f, k.s.sfx_f, k.flf,
+            k.s.f_work, k.s.f_items);
+        c->last_stats[7] += 1;
+    }
+    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 3);
     RG_CUDA(cudaGetLastError());
     return RG_OK;
 }
@@ -315,15 +430,19 @@ static int f_pass_head(Ctx* c, cudaStream_t hs, PassCtl& k) {
     FPlan& plan = k.plan;
     int bps = 1, rc = score_blocks_per_sm<EpiPolicy<MODE_EPI_MAX>>(&bps);
     if (rc) return rc;
-    if ((rc = f_plan(c, hs, a.P, a.pair_off, a.hyp_off, plan, bps, nullptr, a.hyp_first))) return rc;
+    if ((rc = f_plan(c, hs, a.P, a.pair_off, a.hyp_off, plan, bps, nullptr, a.hyp_first, a.bounded ? c->opt_bounded_k : 0,
+                     c->opt_rho_milli)))
+        return rc;
     for (int p = 0; p < a.P; ++p) {
         const int n = a.pair_off[p + 1] - a.pair_off[p], H = a.hyp_off[p + 1] - a.hyp_off[p];
         RG_CHECK_ARG(H == 0 || n >= 8, "a pair with hypotheses needs at least 8 correspondences");
     }
     const bool seeded = a.idx == nullptr && plan.Htot > 0;
     if ((rc = f_workspace(c, plan, seeded))) return rc;
-    if ((rc = score_state_layout(c, a.P, plan.Htot, 8, k.s))) return rc;
+    if ((rc = score_state_layout(c, a.P, plan.Htot, 8, k.s, a.bounded ? plan.Ctot : -1))) return rc;
+    if (a.bounded && (rc = bnd_workspace(c, plan, k.bw))) return rc;
     if (a.P == 0) return RG_OK;
+    c->bnd_host_evals += (long long)(plan.evals + plan.evals_c);
     const ScoreState& s = k.s;
 
     bool reuse = (a.flags & FLAG_REUSE_POINTS) != 0;
@@ -361,13 +480,30 @@ static int f_pass_score(Ctx* c, cudaStream_t st, PassCtl& k) {
     return rc;
 }
 
+static int f_pass_cands(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) {
+    if (k.a.P == 0) return RG_OK;
+    return (k.a.mode == MODE_SAMPSON) ? f_bnd_cands<MODE_SAMPSON>(c, ts, k, beside_scorer)
+                                      : f_bnd_cands<MODE_EPI_MAX>(c, ts, k, beside_scorer);
+}
+
+static int f_pass_sweep(Ctx* c, cudaStream_t st, PassCtl& k) {
+    if (k.a.P == 0) return RG_OK;
+    return (k.a.mode == MODE_SAMPSON) ? f_bnd_sweep<MODE_SAMPSON>(c, st, k) : f_bnd_sweep<MODE_EPI_MAX>(c, st, k);
+}
+
 static int f_pass_tail(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) {
     if (k.a.P == 0) return RG_OK;
     const FCall& a = k.a;
-    int rc = (a.mode == MODE_SAMPSON) ? f_fixup_launch<MODE_SAMPSON>(c, ts, k, beside_scorer)
-                                      : f_fixup_launch<MODE_EPI_MAX>(c, ts, k, beside_scorer);
+    const int stage = a.bounded ? STAGE_FALLBACK : STAGE_MAIN;
+    int rc = (a.mode == MODE_SAMPSON) ? f_fixup_launch<MODE_SAMPSON>(c, ts, k, beside_scorer, stage)
+                                      : f_fixup_launch<MODE_EPI_MAX>(c, ts, k, beside_scorer, stage);
     if (rc) return rc;
-    prof_mark_at(c, ts, k.prof_call, 4);
+    if (a.bounded && k.scored) {
+        bnd_merge<<<k.plan.P, 256, 0, ts>>>(k.s.counts, k.s.sfx_f, (const PairInfo*)c->pair_info.ptr, k.s.mark);
+        c->last_stats[7] += 1;
+        RG_CUDA(cudaGetLastError());
+    }
+    if (!a.bounded) prof_mark_at(c, ts, k.prof_call, 4);
     if ((rc = f_select_launch(c, ts, k.plan, k.s, a.pts64, a.thr, a.mode, a.tie_mode, a.mask, a.best_F, a.best_idx, a.best_count,
                               a.keys)))
         return rc;
@@ -384,11 +520,8 @@ static int f_pass(Ctx* c, cudaStream_t st, const FCall& a) {
     if (c->tail_carve_max > 0 && (rc = tail_carveout(c, false))) return rc;
     if ((rc = f_pass_head(c, st, k))) return rc;
     if ((rc = f_pass_score(c, st, k))) return rc;
+    if (a.bounded && ((rc = f_pass_cands(c, st, k, false)) || (rc = f_pass_sweep(c, st, k)))) return rc;
     return f_pass_tail(c, st, k, false);
-}
-
-static void ws_use(Ctx* c, int slot) {
-    if (c->ws_slot != slot) ws_swap(c);
 }
 
 // Several passes, software-pipelined over two streams and two workspace sets:
@@ -450,6 +583,87 @@ static int f_run_piped(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs, bool
     return RG_OK;
 }
 
+// The bounded sweep's passes, over two streams and THREE workspace sets (pass k lives until its tail, which follows the
+// prefix stage of pass k+1 and its own candidate stage):
+//
+//   caller's stream :  S1(0)          S1(1)  S3+FB(0)          S1(2)  S3+FB(1)          S1(3) ...  S3+FB(n-1)
+//   side stream     :  head(0) head(1)  cands(0) head(2)  cands(1) tail(0) head(3)  cands(2) tail(1) head(4) ...  tail(n-1)
+//
+// S1 = prefix stage, cands = its fix-up + bnd_select, S3+FB = candidate stage, its fix-up, bnd_check, bnd_fb_plan and the
+// fallback stage, tail = fallback fix-up, bnd_merge, selection, masks.  The caller's stream only waits between S3 and FB for
+// the candidate stage's fix-up and the check (two small launches); everything else on the side stream runs beside a scorer.
+// head(k+3) reuses pass k's set and is queued behind tail(k) on the side stream.
+static int f_run_piped_bounded(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs, bool join) {
+    const int n = (int)jobs.size();
+    if (n == 0) return RG_OK;
+    int rc;
+    if ((rc = pipe_setup(c))) return rc;
+    if ((rc = tail_carveout(c, true))) return rc;
+    cudaStream_t side = c->tail_stream;
+    auto fail = [&](int code) {                       // leave nothing in flight behind an error return
+        cudaStreamSynchronize(st);
+        cudaStreamSynchronize(side);
+        c->tail_pending[0] = c->tail_pending[1] = false;
+        return code;
+    };
+    if ((rc = pipe_join(c, st))) return rc;
+    RG_CUDA(cudaEventRecord(c->pipe_gate, st));
+    RG_CUDA(cudaStreamWaitEvent(side, c->pipe_gate, 0));
+    for (int k = 0; k < n; ++k) jobs[k].slot = (c->ws_slot + 1 + k) % 3;
+    auto head = [&](int k) -> int {
+        ws_use(c, jobs[k].slot);
+        if (jobs[k].ready) RG_CUDA(cudaStreamWaitEvent(side, jobs[k].ready, 0));
+        int r = f_pass_head(c, side, jobs[k]);
+        if (r) return r;
+        RG_CUDA(cudaEventRecord(c->head_done[jobs[k].slot], side));
+        return RG_OK;
+    };
+    auto sweep = [&](int k) -> int {                  // caller's stream
+        PassCtl& j = jobs[k];
+        RG_CUDA(cudaStreamWaitEvent(st, c->cand_done[j.slot], 0));
+        ws_use(c, j.slot);
+        int r = f_pass_sweep(c, st, j);
+        if (r) return r;
+        RG_CUDA(cudaEventRecord(c->sweep_done[j.slot], st));
+        return RG_OK;
+    };
+    auto tail = [&](int k, bool beside) -> int {      // side stream
+        PassCtl& j = jobs[k];
+        RG_CUDA(cudaStreamWaitEvent(side, c->sweep_done[j.slot], 0));
+        ws_use(c, j.slot);
+        int r = f_pass_tail(c, side, j, beside);
+        if (r) return r;
+        if (j.done) RG_CUDA(cudaEventRecord(j.done, side));
+        if (j.done && j.out_stream && j.out_bytes) {
+            RG_CUDA(cudaStreamWaitEvent(j.out_stream, j.done, 0));
+            RG_CUDA(cudaMemcpyAsync(j.out_dst, j.out_src, j.out_bytes, cudaMemcpyDeviceToHost, j.out_stream));
+        }
+        return RG_OK;
+    };
+    if ((rc = head(0))) return fail(rc);
+    if (n > 1 && (rc = head(1))) return fail(rc);
+    for (int k = 0; k < n; ++k) {
+        PassCtl& j = jobs[k];
+        RG_CUDA(cudaStreamWaitEvent(st, c->head_done[j.slot], 0));
+        ws_use(c, j.slot);
+        if ((rc = f_pass_score(c, st, j))) return fail(rc);
+        RG_CUDA(cudaEventRecord(c->score_done[j.slot], st));
+        if (k > 0 && (rc = sweep(k - 1))) return fail(rc);
+        RG_CUDA(cudaStreamWaitEvent(side, c->score_done[j.slot], 0));
+        ws_use(c, j.slot);
+        if ((rc = f_pass_cands(c, side, j, k + 1 < n))) return fail(rc);
+        RG_CUDA(cudaEventRecord(c->cand_done[j.slot], side));
+        if (k > 0 && (rc = tail(k - 1, true))) return fail(rc);
+        if (k + 2 < n && (rc = head(k + 2))) return fail(rc);
+    }
+    if ((rc = sweep(n - 1))) return fail(rc);
+    if ((rc = tail(n - 1, false))) return fail(rc);
+    RG_CUDA(cudaEventRecord(c->tail_done[0], side));
+    c->tail_pending[0] = true;
+    if (join) return pipe_join(c, st);
+    return RG_OK;
+}
+
 static int f_check_call(const FCall& a) {
     RG_CHECK_ARG(a.P >= 0 && a.pair_off && a.hyp_off, "bad pair table");
     RG_CHECK_ARG(a.thr > 0.0 && std::isfinite(a.thr), "thr must be positive and finite");
@@ -457,7 +671,7 @@ static int f_check_call(const FCall& a) {
     RG_CHECK_ARG(a.tie_mode == TIE_FIRST || a.tie_mode == TIE_REFERENCE, "unknown tie mode");
     RG_CHECK_ARG(a.solver == SOLVER_QR || a.solver == SOLVER_JACOBI, "unknown solver");
     RG_CHECK_ARG(a.score_path == SCORE_FP32_GUARDED || a.score_path == SCORE_FP64, "unknown scoring path");
-    RG_CHECK_ARG((a.flags & ~FLAG_REUSE_POINTS) == 0, "unknown flag bits");
+    RG_CHECK_ARG((a.flags & ~(FLAG_REUSE_POINTS | FLAG_BOUNDED)) == 0, "unknown flag bits");
     RG_CHECK_ARG(a.hyp_first >= 0 && a.first_pair >= 0, "negative index base");
     if (a.P > 0) {
         RG_CHECK_ARG(a.pair_off[0] == 0 && a.hyp_off[0] == 0, "offset arrays must start at 0");
@@ -508,15 +722,30 @@ static FCall f_sub_call(const FCall& a, int p0, int p1, std::vector<int>& po, st
 // full pipeline on device pointers; asynchronous with respect to the host except for the PairInfo staging.  A call of several
 // passes is pipelined (f_run_piped, option 10); the caller's stream has joined every tail when this returns, i.e. it keeps
 // the stream semantics of a plain sequence of launches.
-static int f_ransac_dev(Ctx* c, cudaStream_t st, const FCall& a) {
-    int rc = f_check_call(a);
+// statistics of rg_f_last_bounded_stats: cleared at the start of a call (not between the sub-batches of a host call)
+static int bnd_stats_reset(Ctx* c, cudaStream_t st, bool bounded) {
+    int rc = ensure(c->bnd_stats, sizeof(unsigned long long) * 4);
     if (rc) return rc;
+    RG_CUDA(cudaMemsetAsync(c->bnd_stats.ptr, 0, sizeof(unsigned long long) * 4, st));
+    c->bnd_host_evals = 0;
+    c->last_bounded = bounded;
+    return RG_OK;
+}
+
+static int f_ransac_dev(Ctx* c, cudaStream_t st, const FCall& a_in) {
+    int rc = f_check_call(a_in);
+    if (rc) return rc;
+    FCall a = a_in;
+    a.bounded = a.bounded && a.score_path == SCORE_FP32_GUARDED;      // (the FP64 path always scores everything)
     RG_CUDA(cudaSetDevice(c->device));
     c->last_stats[7] = 0;
     c->last_passes = 0;
     if ((rc = ensure(c->stats, sizeof(unsigned long long) * 8))) return rc;
     if ((rc = ensure_pinned(c->h_stats, sizeof(unsigned long long) * 8))) return rc;
-    if (!c->accumulate_stats) RG_CUDA(cudaMemsetAsync(c->stats.ptr, 0, sizeof(unsigned long long) * 8, st));
+    if (!c->accumulate_stats) {
+        RG_CUDA(cudaMemsetAsync(c->stats.ptr, 0, sizeof(unsigned long long) * 8, st));
+        if ((rc = bnd_stats_reset(c, st, a.bounded))) return rc;
+    }
     if (a.P == 0) return RG_OK;
     std::vector<int> bounds, po, ho;
     f_pass_bounds(c, a, bounds);
@@ -528,7 +757,7 @@ static int f_ransac_dev(Ctx* c, cudaStream_t st, const FCall& a) {
         //  987.1 -> 988.6 ms; profiles/r02_taper.txt)
         std::vector<PassCtl> jobs(n_pass);
         for (int k = 0; k < n_pass; ++k) jobs[k].a = f_sub_call(a, bounds[k], bounds[k + 1], jobs[k].po, jobs[k].ho);
-        if ((rc = f_run_piped(c, st, jobs, true))) return rc;
+        if ((rc = a.bounded ? f_run_piped_bounded(c, st, jobs, true) : f_run_piped(c, st, jobs, true))) return rc;
     } else {
         for (int k = 0; k < n_pass; ++k) {
             if (n_pass == 1) {
@@ -560,6 +789,7 @@ int rg_f_ransac_dev2(void* ctx, void* stream, int P, const double* pts64_dev, co
     a.P = P; a.pts64 = pts64_dev; a.pair_off = pair_off_host; a.idx = idx_dev; a.hyp_off = hyp_off_host;
     a.thr = thr; a.mode = mode; a.tie_mode = tie_mode; a.solver = solver; a.score_path = score_path; a.flags = flags;
     a.sample_seed = sample_seed; a.first_pair = first_pair_id; a.hyp_first = hyp_index_base;
+    a.bounded = (flags & FLAG_BOUNDED) != 0 && ((Ctx*)ctx)->opt_bounded != 0;
     a.best_idx = best_idx_dev; a.best_count = best_count_dev; a.best_F = best_F_dev; a.mask = mask_dev; a.keys = key_dev;
     return f_ransac_dev((Ctx*)ctx, (cudaStream_t)stream, a);
 }
@@ -658,12 +888,13 @@ int rg_f_inlier_mask_dev(void* ctx, void* stream, int P, const double* pts64_dev
 }
 
 // device pointers to the per-hypothesis results of the LAST call on this context (valid until the next call; a call that
-// ran in several passes only keeps its last pass, and is refused here)
+// ran in several passes only keeps its last pass, and is refused here).  After a bounded sweep *counts_dev is NULL: the
+// hypotheses it proved unable to win hold prefix counts only.
 int rg_f_last_hypotheses_dev(void* ctx, const int** counts_dev, const double** F_all_dev, const unsigned char** flags_dev) {
     RG_CHECK_ARG(ctx != nullptr, "ctx is null");
     Ctx* c = (Ctx*)ctx;
     RG_CHECK_ARG(c->last_passes <= 1, "the last call ran in several passes: per-hypothesis results are not retained");
-    if (counts_dev) *counts_dev = (const int*)c->counts_ptr;
+    if (counts_dev) *counts_dev = c->last_bounded ? nullptr : (const int*)c->counts_ptr;
     if (F_all_dev) *F_all_dev = (const double*)c->F64.ptr;
     if (flags_dev) *flags_dev = (const unsigned char*)c->flags.ptr;
     return RG_OK;
@@ -688,6 +919,23 @@ int rg_get_last_stats(void* ctx, void* stream, long long* out8) {
     return RG_OK;
 }
 
+// out[0] hypothesis x correspondence evaluations the last F call executed, [1] hypotheses it did not score in full (proved
+// unable to reach their pair's maximum), [2] pairs whose bound failed and that were scored in full, [3] candidates per pair
+// (0: the call ran the full sweep).  Synchronises the stream.
+int rg_f_last_bounded_stats(void* ctx, void* stream, long long* out4) {
+    RG_CHECK_ARG(ctx != nullptr && out4 != nullptr, "null argument");
+    Ctx* c = (Ctx*)ctx;
+    RG_CUDA(cudaSetDevice(c->device));
+    RG_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
+    unsigned long long d[4] = {0, 0, 0, 0};
+    if (c->bnd_stats.ptr) RG_CUDA(cudaMemcpy(d, c->bnd_stats.ptr, sizeof(d), cudaMemcpyDeviceToHost));
+    out4[0] = c->bnd_host_evals + (long long)d[0];
+    out4[1] = (long long)d[1];
+    out4[2] = (long long)d[2];
+    out4[3] = c->last_bounded ? c->opt_bounded_k : 0;
+    return RG_OK;
+}
+
 // Host-buffer entry point.  The pairs are processed in passes (f_pass_bounds; a batch that fits one pass is still cut in two
 // when that hides a worthwhile part of the upload: the first sub-batch is the smallest whose scoring time covers the upload
 // of the rest, both estimated with the rates MEASURED on this context by earlier calls).  All uploads are queued on a second
@@ -705,6 +953,7 @@ int rg_f_ransac_host2(void* ctx, void* stream, int P, const double* pts64, const
     FCall a;
     a.P = P; a.pair_off = pair_off; a.hyp_off = hyp_off; a.thr = thr; a.mode = mode; a.tie_mode = tie_mode;
     a.solver = solver; a.score_path = score_path; a.sample_seed = sample_seed; a.first_pair = first_pair_id;
+    a.bounded = counts == nullptr && c->opt_bounded != 0 && score_path == SCORE_FP32_GUARDED;
     int rc = f_check_call(a);
     if (rc) return rc;
     RG_CUDA(cudaSetDevice(c->device));
@@ -843,7 +1092,8 @@ int rg_f_ransac_host2(void* ctx, void* stream, int P, const double* pts64, const
         if ((rc = ensure(c->stats, sizeof(unsigned long long) * 8))) return rc;
         if ((rc = ensure_pinned(c->h_stats, sizeof(unsigned long long) * 8))) return rc;
         RG_CUDA(cudaMemsetAsync(c->stats.ptr, 0, sizeof(unsigned long long) * 8, st));
-        rc = f_run_piped(c, st, jobs, false);
+        if ((rc = bnd_stats_reset(c, st, a.bounded))) return rc;
+        rc = a.bounded ? f_run_piped_bounded(c, st, jobs, false) : f_run_piped(c, st, jobs, false);
         launches = c->last_stats[7];
     }
     for (int k = 0; k < S && rc == RG_OK && !piped; ++k) {

@@ -708,6 +708,7 @@ struct EpiFix {
     struct Params {
         const float4* pts32; const double4* pts64; const Hyp32* hyp32; const double* F64; const PairInfo* pi;
         const PairFrame* fr; int P;
+        const int* map = nullptr;      // bounded sweep, candidate stage: compact hypothesis index -> index into F64
     };
     __device__ static __forceinline__ int pair_of(const Params& p, int h) {
         int lo = 0, hi = p.P;
@@ -739,7 +740,8 @@ struct EpiFix {
     __device__ static __forceinline__ int exact(const Params& p, int h, int i, int pair) {
         const PairInfo& info = p.pi[pair];
         const double4 v = p.pts64[info.pt_off + i];
-        return epi_inlier64(p.F64 + (size_t)h * 9, v.x, v.y, v.z, v.w, p.fr[pair].thr, MODE);
+        const size_t g = p.map != nullptr ? (size_t)p.map[h] : (size_t)h;
+        return epi_inlier64(p.F64 + g * 9, v.x, v.y, v.z, v.w, p.fr[pair].thr, MODE);
     }
 };
 

@@ -6,7 +6,7 @@
 namespace rg {
 
 struct ScoreState;                                   // f_api.cu (same translation unit)
-int score_state_layout(Ctx* c, int P, long long Htot, int bbox_words, ScoreState& s);
+int score_state_layout(Ctx* c, int P, long long Htot, int bbox_words, ScoreState& s, long long Ctot);
 FlagList flag_list_for(Ctx* c, const ScoreState& s, double evals, int* rc_out);
 int fixup_grid(const Ctx* c, double evals);
 

@@ -47,7 +47,7 @@ __device__ __forceinline__ float2 ffma2_sbs(float s, float2 b, float c) {       
 
 struct ScoreItem {
     int pair, h_base, H_end;        // hypotheses [h_base, min(h_base + kHypPerBlock, H_end)) (global indices)
-    int g0, g1;                     // kSub-point groups [g0, g1) of the pair
+    int g0, g1;                     // kSub-point groups [g0, g1) of the pair (inside its window [g_base, g_end))
 };
 
 __device__ __forceinline__ ScoreItem decode_item(const PairInfo* __restrict__ pi, int P, int item) {
@@ -62,9 +62,8 @@ __device__ __forceinline__ ScoreItem decode_item(const PairInfo* __restrict__ pi
     it.pair = lo;
     it.h_base = info.hyp_off + hb * kHypPerBlock;
     it.H_end = info.hyp_off + info.H;
-    const int ngroups = info.n_pad / kSub;
-    it.g0 = min(sp * info.groups_per_split, ngroups);
-    it.g1 = min(it.g0 + info.groups_per_split, ngroups);
+    it.g0 = min(info.g_base + sp * info.groups_per_split, info.g_end);
+    it.g1 = min(it.g0 + info.groups_per_split, info.g_end);
     RG_ASSERT(it.g0 < it.g1 && it.h_base < it.H_end && it.h_base >= info.hyp_off);
     return it;
 }
@@ -137,14 +136,15 @@ constexpr size_t score_smem_bytes() { return kStages * sizeof(ScoreStage<Pol>) +
 // persistent block: first item blockIdx.x, then items claimed from a global counter (dynamic: with static round-robin a
 // batch whose item count is not a multiple of the grid leaves most SMs idle during the last round); every item = kHypPerBlock
 // hypotheses x a contiguous range of kSub-point groups of one pair.  Host guarantees every item has >= 1 group and >= 1
-// hypothesis; *work_counter is 0 at launch.
+// hypothesis; *work_counter is 0 at launch.  n_items_dev (optional): the item count is read from the device instead (a stage
+// whose size is decided on the device — the bounded sweep's fallback — is queued at full grid and usually has no items).
 // Points and (at the first chunk of an item) hypothesis records arrive by 1-D bulk TMA on one mbarrier per stage;
 // the next chunk / next item is always in flight while the current one is being scored.
 template <class Pol>
 __global__ void __launch_bounds__(kScoreThreads, kScoreBlocksPerSM)
 score_packed(const float4* __restrict__ pts32, const typename Pol::Rec* __restrict__ hyp32,
              const PairInfo* __restrict__ pi, int P, int n_items, int* __restrict__ counts,
-             FlagList flist, int* __restrict__ work_counter) {
+             FlagList flist, int* __restrict__ work_counter, const int* __restrict__ n_items_dev = nullptr) {
     __shared__ int s_next;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     ScoreStage<Pol>* st = reinterpret_cast<ScoreStage<Pol>*>(smem_raw);
@@ -155,6 +155,7 @@ score_packed(const float4* __restrict__ pts32, const typename Pol::Rec* __restri
 
     const int tid = threadIdx.x;
     int item = blockIdx.x;
+    if (n_items_dev != nullptr) n_items = *n_items_dev;
     if (item >= n_items) return;
     if (tid == 0) {
         mbar_init(&full[0], 1);
@@ -273,7 +274,8 @@ score_packed(const float4* __restrict__ pts32, const typename Pol::Rec* __restri
 //            op sequence) -> band mask + FP32 decisions;
 //   level 2  queue the band evaluations; one lane per evaluation applies the reference formula in FP64 and corrects
 //            counts[h] by (exact decision - FP32 decision).
-// Hypotheses marked in flist.ovf (list overflow) are recounted over all their correspondences in FP64 first.
+// Hypotheses marked in flist.ovf (list overflow) are recounted in FP64 first, over the correspondences of the pair's scored
+// window [g_base, g_end) (the whole pair in a full sweep): counts[h] then holds the exact count over that window.
 // stats: [0] flagged groups, [1] band evaluations, [2] changed decisions, [3] hypotheses recounted after a list overflow.
 //   Fix::pair_of(params, h)                                       pair / view of a global hypothesis index
 //   Fix::n_points(params, aux)                                    voting correspondences of that pair / view
@@ -298,8 +300,9 @@ __global__ void __launch_bounds__(256) fixup_list(typename Fix::Params prm, Flag
             if (!flist.ovf[h]) continue;               // uniform per block
             const int aux = Fix::pair_of(prm, h);
             const int n = Fix::n_points(prm, aux);
+            const int i1 = min(n, prm.pi[aux].g_end * kSub);
             int c = 0;
-            for (int i = threadIdx.x; i < n; i += blockDim.x) c += Fix::exact(prm, h, i, aux);
+            for (int i = min(n, prm.pi[aux].g_base * kSub) + (int)threadIdx.x; i < i1; i += blockDim.x) c += Fix::exact(prm, h, i, aux);
             c = __reduce_add_sync(full, c);
             __syncthreads();
             if (lane == 0) s_red[warp] = c;

@@ -11,7 +11,7 @@ import contextlib
 import numpy as np
 
 from . import _cabi as cabi
-from ._cabi import FLAG_REUSE_POINTS, MODE_EPI_MAX, SCORE_FP32_GUARDED, SOLVER_QR, TIE_FIRST
+from ._cabi import FLAG_BOUNDED, FLAG_REUSE_POINTS, MODE_EPI_MAX, SCORE_FP32_GUARDED, SOLVER_QR, TIE_FIRST
 from .runtime import offsets, pnp_k_table  # noqa: F401  (offsets: part of this module's interface)
 
 
@@ -89,8 +89,10 @@ class FOutputs:
 
 
 def f_ransac(d_pts, pair_off, d_idx, hyp_off, out: FOutputs, thr=1.5, mode=MODE_EPI_MAX, tie_mode=TIE_FIRST, solver=SOLVER_QR,
-             score_path=SCORE_FP32_GUARDED, flags=0, seed=0, first_pair=0, hyp_first=0):
-    """rg_f_ransac_dev2 on CUDA tensors.  d_idx None = samples drawn on the device from ``seed``."""
+             score_path=SCORE_FP32_GUARDED, flags=FLAG_BOUNDED, seed=0, first_pair=0, hyp_first=0):
+    """rg_f_ransac_dev2 on CUDA tensors.  d_idx None = samples drawn on the device from ``seed``.  The default flags ask for
+    the bounded sweep (option 12 decides whether it runs): the results are those of the full sweep, only the per-hypothesis
+    counts behind ``rg_f_last_hypotheses_dev`` are not kept."""
     _call("rg_f_ransac_dev2", _dev_index(d_pts), len(pair_off) - 1, d_pts, pair_off, d_idx, hyp_off, thr, mode, tie_mode,
           solver, score_path, flags, seed, first_pair, hyp_first, out.best_idx, out.best_count, out.F, out.mask, out.key)
     return out

@@ -154,6 +154,13 @@ def profile(device=None, stream=0) -> dict:
             "select_ms": out[4]}
 
 
+def bounded_stats(device=None, stream=0) -> dict:
+    """What the last F call executed: see rg_f_last_bounded_stats (K = 0: it ran the full sweep)."""
+    out = (C.c_longlong * 4)()
+    _call("rg_f_last_bounded_stats", device, stream, out)
+    return {"evals": out[0], "not_fully_scored": out[1], "fallback_pairs": out[2], "K": out[3]}
+
+
 def last_stats(device=None, stream=0) -> dict:
     out = (C.c_longlong * 8)()
     _call("rg_get_last_stats", device, stream, out)
