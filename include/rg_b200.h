@@ -34,6 +34,8 @@ extern "C" {
 #define RG_SOLVER_JACOBI 1  /* register-resident one-sided Jacobi SVD, one hypothesis per 16-lane group */
 #define RG_SCORE_FP32_GUARDED 0 /* FP32 fma.rn.f32x2 scorer + rigorous guard band re-evaluated in FP64 (exact counts) */
 #define RG_SCORE_FP64 1         /* every evaluation in FP64 with the reference formula */
+#define RG_SCORE_FP32_BOUND 2   /* rg_epi_score_count_host only: the bounded sweep's bound-only prefix scorer, whose counts
+                                   are upper bounds of the exact counts (option 15) */
 
 /* ---- context -------------------------------------------------------------------------------------------------- */
 int rg_abi_version(void);
@@ -72,7 +74,11 @@ int rg_host_free(void* p);
  *            score in full only the pairs where another hypothesis could still reach the maximum (DESIGN.md section 4);
  *            winners, counts, F and masks are those of the full sweep; 0 = every hypothesis against every correspondence
  * option 13 = prefix share rho of the bounded sweep in thousandths, [1, 1000] (default 450); results do not depend on it
- * option 14 = candidates K per pair of the bounded sweep, [1, 65536] (default 512); results do not depend on it */
+ * option 14 = candidates K per pair of the bounded sweep, [1, 65536] (default 512); results do not depend on it
+ * option 15 = prefix stage of the bounded sweep: 1 (default) = bound-only FP32 scorer (counts r^2 < T, an upper bound on
+ *            every hypothesis's prefix count, with no guard-band fix-up; the K candidates are then scored over the whole
+ *            pair), 0 = guarded scorer + FP64 fix-up (exact prefix counts; the candidates are scored on the rest of the
+ *            pair); results do not depend on it (DESIGN.md section 4) */
 int rg_set_option(void* ctx, int option, long long value);
 /* summed milliseconds of {prepare, solve, score kernel, fixup + repair, select} over the PASSES since the last read
  * (at most 2048 passes are remembered; *out_calls = passes covered); synchronises `stream` */
@@ -140,6 +146,10 @@ int rg_f_last_hypotheses_dev(void* ctx, const int32_t** counts_dev, const double
  * unable to reach their pair's maximum), pairs that fell back to scoring every hypothesis in full, K (0: full sweep)}.
  * Synchronises `stream`. */
 int rg_f_last_bounded_stats(void* ctx, void* stream, long long* out4);
+/* the evaluations of the last F call split by scorer: out2 = {bound-only prefix stages (option 15 = 1), guarded scorer
+ * (exact prefix, candidate and fallback stages, or the full sweep)}; out2[0] + out2[1] = out4[0] above.
+ * Synchronises `stream`. */
+int rg_f_last_bounded_evals(void* ctx, void* stream, long long* out2);
 /* Same with host buffers; counts / F_all / flags / mask are optional (NULL = not copied back; counts == NULL runs the
  * bounded sweep when option 12 is on).  The batch is uploaded pass
  * by pass on a second stream, so the copy of pass k+1 overlaps the scoring of pass k (page-locked buffers needed for the
@@ -160,7 +170,8 @@ int rg_f_ransac_host2(void* ctx, void* stream, int P, const double* pts64, const
  * 8-point solve of H samples — lab3.fmatrix_stls on 8 points (lab3.py:269-329) */
 int rg_f8pt_solve_host(void* ctx, void* stream, int N, const double* pts64, int H, const int32_t* idx, int solver,
                        double* F_all, unsigned char* flags /* may be NULL */);
-/* inlier counts of H caller-supplied F over N correspondences — fmatrix_residuals + threshold (fun.py:315-317) */
+/* inlier counts of H caller-supplied F over N correspondences — fmatrix_residuals + threshold (fun.py:315-317);
+ * score_path RG_SCORE_FP32_BOUND returns the bound-only scorer's upper bounds of those counts instead */
 int rg_epi_score_count_host(void* ctx, void* stream, int N, const double* pts64, int H, const double* F_all, double thr,
                             int mode, int score_path, int32_t* counts);
 /* lab3.fmatrix_residuals (lab3.py:188-227): x, y are (2, N) row-major, out is (2, N) signed distances */

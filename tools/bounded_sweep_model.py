@@ -27,9 +27,10 @@ def prefix_points(n: int, rho: float) -> int:
 
 
 def bounded_rule(pre: np.ndarray, full: np.ndarray, rest: int, K: int) -> dict:
-    """The rule bnd_select / bnd_check apply to one pair.  pre: exact prefix counts, full: exact full counts, rest: points
-    outside the prefix.  Returns the candidate mask, the escapees, whether the pair falls back, and the counts the tail
-    sees (full counts where they were computed, prefix counts elsewhere)."""
+    """The rule bnd_select / bnd_check apply to one pair.  pre: prefix counts — exact, or upper bounds of the exact ones
+    (the bound-only prefix stage, option 15) — full: exact full counts, rest: points outside the prefix.  Returns the
+    candidate mask, the escapees, whether the pair falls back, and the counts the tail sees (full counts where they were
+    computed, prefix counts elsewhere)."""
     H = len(pre)
     order = np.lexsort((np.arange(H), -pre))           # (prefix count desc, index asc)
     cand = np.zeros(H, bool)

@@ -17,7 +17,7 @@ LIB_PATH = os.environ.get("RG_LIB", os.path.join(_HERE, "librg_b200.so"))   # RG
 MODE_EPI_MAX, MODE_SAMPSON = 0, 1
 TIE_FIRST, TIE_REFERENCE = 0, 1
 SOLVER_QR, SOLVER_JACOBI = 0, 1
-SCORE_FP32_GUARDED, SCORE_FP64 = 0, 1
+SCORE_FP32_GUARDED, SCORE_FP64, SCORE_FP32_BOUND = 0, 1, 2
 TRI_OPTIMAL, TRI_LINEAR = 0, 1
 FLAG_REUSE_POINTS = 1
 FLAG_BOUNDED = 2
@@ -55,6 +55,7 @@ SIGNATURES = {
     "rg_p2p_argmax_exchange": (_i, [_vp, _vp, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rg_f_last_hypotheses_dev": (_i, [_vp, C.POINTER(_vp), C.POINTER(_vp), C.POINTER(_vp)]),
     "rg_f_last_bounded_stats": (_i, [_vp, _vp, _pll]),
+    "rg_f_last_bounded_evals": (_i, [_vp, _vp, _pll]),
     "rg_f_ransac_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _d, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rg_f8pt_solve_host": (_i, [_vp, _vp, _i, _vp, _i, _vp, _i, _vp, _vp]),
     "rg_epi_score_count_host": (_i, [_vp, _vp, _i, _vp, _i, _vp, _d, _i, _i, _vp]),

@@ -2,19 +2,23 @@
 // prefix scores, and prove that no other hypothesis can reach the pair's maximum.
 //
 // Per pass, after the head (memset, prepare, solve):
-//   prefix stage     score_packed over every hypothesis x groups [0, gA) (the main table's window) + fix-up: counts[h] = c_A(h),
-//                    the exact count over the first k = min(n, gA * kSub) correspondences
-//   bnd_select       per pair the K hypotheses with the largest (c_A, -index), gathered into compact Hyp32 records + map
-//   candidate stage  score_packed over the compact records x groups [gA, G) + fix-up (map: compact -> global index):
-//                    sfx_c[j] = exact count of candidate j over the other n - k correspondences
-//   bnd_check        L = max_j c_A + sfx_c over the candidates.  A non-candidate's full count is at most c_A(h) + (n - k); if
+//   prefix stage     every hypothesis x groups [0, gA) (the main table's window): counts[h] = c^(h) >= c_A(h), where c_A is
+//                    the exact count over the first k = min(n, gA * kSub) correspondences.  Option 15 = 1 (default):
+//                    score_packed<EpiBoundPolicy>, an upper bound with no fix-up; option 15 = 0: score_packed<EpiPolicy> +
+//                    fix-up, c^ = c_A exactly.
+//   bnd_select       per pair the K hypotheses with the largest (c^, -index), gathered into compact Hyp32 records + map
+//   candidate stage  score_packed over the compact records + fix-up (map: compact -> global index), over [gA, G) after an
+//                    exact prefix (sfx_c[j] = exact count over the other n - k correspondences) or over [0, G) after a
+//                    bound-only prefix (sfx_c[j] = exact full count)
+//   bnd_check        L = the candidates' largest full count.  A non-candidate's full count is at most c^(h) + (n - k); if
 //                    that is below L it can never be the maximum nor tie with it.  Pairs where some non-candidate has
-//                    c_A(h) + (n - k) >= L are marked; the others get the candidates' full counts written into counts.
-//   bnd_fb_plan      the fallback table: the marked pairs' items over [gA, G) for EVERY hypothesis (usually none)
+//                    c^(h) + (n - k) >= L are marked; the others get the candidates' full counts written into counts.
+//   bnd_fb_plan      the fallback table: the marked pairs' items over the candidates' window for EVERY hypothesis (usually none)
 //   fallback stage   score_packed with the item count read from the device + fix-up into sfx_f; bnd_merge adds sfx_f to the
-//                    marked pairs' counts, which are then full counts for every hypothesis of those pairs.
-// In an unmarked pair a hypothesis that was not fully scored keeps c_A(h) <= full(h) < L <= max, so argmax_counts' first
-// maximum, the tie replay over the hypotheses with count == max and the winner's mask are those of a full sweep.
+//                    marked pairs' prefix counts (or writes it, after a bound-only prefix): full counts for every hypothesis.
+// In an unmarked pair a hypothesis that was not fully scored keeps c^(h) < L <= max and has full(h) <= c^(h) + (n - k) < L,
+// so argmax_counts' first maximum, the tie replay over the hypotheses with count == max and the winner's mask are those of
+// a full sweep.
 #pragma once
 #include "score_core.cuh"
 
@@ -125,11 +129,13 @@ __device__ __forceinline__ int block_reduce_max(int v, int* s) {
 }
 
 // One CTA per pair, after the candidate stage's fix-up.  stats: [0] fallback evaluations, [1] hypotheses not fully scored,
-// [2] pairs that fell back.
+// [2] pairs that fell back.  exact_prefix: counts hold exact prefix counts and sfx_c suffix counts; otherwise counts hold
+// upper bounds of the prefix counts and sfx_c full counts.
 __global__ void __launch_bounds__(256) bnd_check(int* __restrict__ counts, const int* __restrict__ sfx_c,
                                                   const int* __restrict__ map, const PairInfo* __restrict__ pi,
                                                   const PairInfo* __restrict__ pc, const int4* __restrict__ sel,
-                                                  int* __restrict__ mark, unsigned long long* __restrict__ stats) {
+                                                  int* __restrict__ mark, unsigned long long* __restrict__ stats,
+                                                  bool exact_prefix) {
     __shared__ int s_red[8];
     const int p = blockIdx.x;
     const PairInfo info = pi[p];
@@ -137,7 +143,8 @@ __global__ void __launch_bounds__(256) bnd_check(int* __restrict__ counts, const
     const int4 sl = sel[p];
     const int rest = info.n - min(info.n, info.g_end * kSub);     // correspondences outside the prefix
     int L = 0;
-    for (int j = threadIdx.x; j < Kp; j += blockDim.x) L = max(L, counts[map[cbase + j]] + sfx_c[cbase + j]);
+    for (int j = threadIdx.x; j < Kp; j += blockDim.x)
+        L = max(L, (exact_prefix ? counts[map[cbase + j]] : 0) + sfx_c[cbase + j]);
     L = block_reduce_max(L, s_red);
     // escapees: non-candidates whose bound reaches L (>=: a tie with the maximum must be scored too)
     int esc = 0;
@@ -150,12 +157,13 @@ __global__ void __launch_bounds__(256) bnd_check(int* __restrict__ counts, const
     if (esc) {
         if (threadIdx.x == 0) {
             mark[p] = 1;
-            atomicAdd(&stats[0], (unsigned long long)info.H * (unsigned long long)rest);
+            atomicAdd(&stats[0], (unsigned long long)info.H * (unsigned long long)(exact_prefix ? rest : info.n));
             atomicAdd(&stats[2], 1ull);
         }
         return;
     }
-    for (int j = threadIdx.x; j < Kp; j += blockDim.x) counts[map[cbase + j]] += sfx_c[cbase + j];
+    for (int j = threadIdx.x; j < Kp; j += blockDim.x)
+        counts[map[cbase + j]] = (exact_prefix ? counts[map[cbase + j]] : 0) + sfx_c[cbase + j];
     if (threadIdx.x == 0 && info.H > Kp) atomicAdd(&stats[1], (unsigned long long)(info.H - Kp));
 }
 
@@ -183,13 +191,16 @@ __global__ void __launch_bounds__(kSelectThreads) bnd_fb_plan(const PairInfo* __
     if (threadIdx.x == 0) *n_items = run;
 }
 
-// One CTA per pair: marked pairs add the fallback's suffix counts to the prefix counts
+// One CTA per pair: marked pairs add the fallback's suffix counts to the exact prefix counts, or take the fallback's full
+// counts after a bound-only prefix
 __global__ void __launch_bounds__(256) bnd_merge(int* __restrict__ counts, const int* __restrict__ sfx_f,
-                                                  const PairInfo* __restrict__ pi, const int* __restrict__ mark) {
+                                                  const PairInfo* __restrict__ pi, const int* __restrict__ mark,
+                                                  bool exact_prefix) {
     const int p = blockIdx.x;
     if (!mark[p]) return;
     const PairInfo info = pi[p];
-    for (int h = threadIdx.x; h < info.H; h += blockDim.x) counts[info.hyp_off + h] += sfx_f[info.hyp_off + h];
+    for (int h = threadIdx.x; h < info.H; h += blockDim.x)
+        counts[info.hyp_off + h] = (exact_prefix ? counts[info.hyp_off + h] : 0) + sfx_f[info.hyp_off + h];
 }
 
 }  // namespace rg

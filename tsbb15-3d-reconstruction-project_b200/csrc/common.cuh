@@ -53,7 +53,7 @@ void set_error(const char* fmt, ...);
 enum : int { MODE_EPI_MAX = 0, MODE_SAMPSON = 1 };
 enum : int { TIE_FIRST = 0, TIE_REFERENCE = 1 };
 enum : int { SOLVER_QR = 0, SOLVER_JACOBI = 1 };
-enum : int { SCORE_FP32_GUARDED = 0, SCORE_FP64 = 1 };
+enum : int { SCORE_FP32_GUARDED = 0, SCORE_FP64 = 1, SCORE_FP32_BOUND = 2 };
 
 // ---------------------------------------------------------------------------------------------
 // device-side records
@@ -61,12 +61,13 @@ enum : int { SCORE_FP32_GUARDED = 0, SCORE_FP64 = 1 };
 // Per hypothesis, FP32 scorer input: F~ = M1^T F M2 scaled to unit weighted abs-sum (f), the image-2 line normal
 // l2 = (F~^T x~)[:2] ROTATED by the per-hypothesis angle that removes the x0 term of its second component
 // (g = c, d, e, a, b:  l2x' = c x0 + d x1 + e,  l2y' = a x1 + b;  |l2'|^2 = |l2|^2, one FMA fewer per evaluation), and the
-// rigorous rounding-error band G (see DESIGN.md "guard band").  64 bytes, 16-byte aligned.
+// rigorous rounding-error band G (see DESIGN.md "guard band") and the constant T of the bound-only prefix scorer
+// (r^2 < T holds for every reference inlier, DESIGN.md section 4.2).  64 bytes, 16-byte aligned.
 struct __align__(16) Hyp32 {
     float f[9];
     float g[5];
     float G;
-    float pad0;
+    float T;
 };
 static_assert(sizeof(Hyp32) == 64, "Hyp32 layout");
 
@@ -177,8 +178,9 @@ struct FPlan {
     int n_items = 0;
     int maxN = 0, maxH = 0;
     double evals = 0.0;                  // sum_p n_p * H_p (bounded sweep: of the prefix stage)
-    // bounded sweep (bounded.cuh): three tables per pass, [prefix stage | candidate suffix stage | fallback template]
+    // bounded sweep (bounded.cuh): three tables per pass, [prefix stage | candidate stage | fallback template]
     bool bounded = false;
+    bool bound_prefix = false;           // the prefix stage counts an upper bound (EpiBoundPolicy); later stages cover [0, G)
     int K = 0;                           // candidates per pair
     long long Ctot = 0;                  // candidates of the pass (sum_p min(K, H_p))
     int n_items_c = 0, n_items_f = 0;    // scorer items of the candidate stage / of the fallback with every pair marked
@@ -227,8 +229,10 @@ struct Ctx {
     int opt_bounded = 1;                           // option 12: F calls without per-hypothesis counts run the bounded sweep
     int opt_rho_milli = 450;                       // option 13: prefix share rho of the bounded sweep, in thousandths
     int opt_bounded_k = 512;                       // option 14: candidates per pair of the bounded sweep
+    int opt_bound_prefix = 1;                      // option 15: 1 = bound-only prefix stage, 0 = exact (guarded + fix-up) prefix
     bool last_bounded = false;                     // the last F call ran the bounded sweep (its counts are not full counts)
-    long long bnd_host_evals = 0;                  // evaluations of its prefix and candidate stages (known on the host)
+    long long bnd_host_evals = 0;                  // guarded-scorer evaluations of its prefix and candidate stages (known on the host)
+    long long bnd_bound_evals = 0;                 // evaluations of its bound-only prefix stages (option 15 = 1)
     Buffer bnd_stats;                              // device: [0] fallback evaluations, [1] hypotheses not fully scored, [2] fallback pairs
     // peer-to-peer argmax exchange (hypothesis-split mode over NVLink), see p2p_api.cu
     void* p2p_local = nullptr; size_t p2p_bytes = 0; int p2p_rank = 0, p2p_world = 0; unsigned p2p_seq = 0;

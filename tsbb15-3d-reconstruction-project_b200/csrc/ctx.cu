@@ -197,6 +197,8 @@ int rg_device_sm_count(void* ctx) { return ctx ? ((Ctx*)ctx)->sm_count : 0; }
 //           0 = every hypothesis against every correspondence
 // option 13: prefix share rho of the bounded sweep in thousandths, in [1, 1000] (default 450)
 // option 14: candidates per pair of the bounded sweep, in [1, 65536] (default 512)
+// option 15: prefix stage of the bounded sweep: 1 (default) = bound-only scorer (upper-bound counts, no fix-up; the
+//           candidates are then scored over the whole pair), 0 = guarded scorer + fix-up (exact prefix counts)
 // option 9: guard-band safety factor x 1000 (default 1000 = the proven FP32 rounding bound); larger values keep every result
 //           exact and only send more evaluations to the FP64 recheck — used to MEASURE what a less accurate scorer
 //           (tensor-core split-precision accumulation) would cost in fix-up time
@@ -278,6 +280,11 @@ int rg_set_option(void* ctx, int option, long long value) {
     if (option == 14) {
         if (value < 1 || value > 65536) { set_error("invalid argument: option 14 (candidates per pair) must be in [1, 65536]"); return RG_ERR_ARG; }
         c->opt_bounded_k = (int)value;
+        return RG_OK;
+    }
+    if (option == 15) {
+        if (value != 0 && value != 1) { set_error("invalid argument: option 15 (bound-only prefix stage) must be 0 or 1"); return RG_ERR_ARG; }
+        c->opt_bound_prefix = (int)value;
         return RG_OK;
     }
     if (option == 8) {

@@ -5,7 +5,8 @@
 //   -> [f_tie_stats -> f_tie_resolve] -> f_mask
 // over a contiguous block of pairs whose workspaces (hypotheses, FP32 points, flag list) stay bounded; BASELINE config 5
 // (4096 pairs x 50 000 x 8 192) runs as 64 passes of 64 pairs.  A call that wants no per-hypothesis counts runs the bounded
-// sweep instead of score_packed -> fixup_list (bounded.cuh): prefix stage, candidates, candidate suffix stage, check, fallback.  The per-pass PairInfo table is planned on the host into
+// sweep instead of score_packed -> fixup_list (bounded.cuh): bound-only prefix stage, candidates, candidate stage, check,
+// fallback.  The per-pass PairInfo table is planned on the host into
 // double-buffered pinned staging, so the host plans pass k+1 while pass k runs.
 #include "f_kernels.cuh"
 #include "bounded.cuh"
@@ -268,8 +269,8 @@ static int f_score_only(Ctx* c, cudaStream_t st, PassCtl& k) {
     const FPlan& plan = k.plan;
     const PairInfo* pi = (const PairInfo*)c->pair_info.ptr;
     k.scored = false;
-    if (plan.Htot == 0 || plan.Ntot == 0 || (k.a.score_path == SCORE_FP32_GUARDED && plan.n_items == 0)) return RG_OK;
-    if (k.a.score_path == SCORE_FP32_GUARDED) {
+    if (plan.Htot == 0 || plan.Ntot == 0 || (k.a.score_path != SCORE_FP64 && plan.n_items == 0)) return RG_OK;
+    if (k.a.score_path != SCORE_FP64) {
         int bps = 1, rc = score_blocks_per_sm<EpiPolicy<MODE>>(&bps);
         if (rc) return rc;
         // (the later stages of a bounded pass reuse the records once the previous stage's fix-up has read them)
@@ -279,10 +280,18 @@ static int f_score_only(Ctx* c, cudaStream_t st, PassCtl& k) {
             k.flc = FlagList{k.fl.rec, k.s.c_list_n, k.fl.cap, k.s.ovf_c};
             k.flf = FlagList{k.fl.rec, k.s.f_list_n, k.fl.cap, k.s.ovf_f};
         }
-        constexpr size_t smem = score_smem_bytes<EpiPolicy<MODE>>();
-        const int grid = std::min(plan.n_items, c->sm_count * bps);
-        score_packed<EpiPolicy<MODE>><<<grid, kScoreThreads, smem, st>>>((const float4*)c->pts32.ptr, (const Hyp32*)c->hyp32.ptr,
-                                                                        pi, plan.P, plan.n_items, k.s.counts, k.fl, k.s.work);
+        if (plan.bound_prefix || k.a.score_path == SCORE_FP32_BOUND) {      // upper-bound counts: no flags, no fix-up
+            static_assert(score_smem_bytes<EpiBoundPolicy>() == score_smem_bytes<EpiPolicy<MODE>>(), "same stage ring");
+            if ((rc = score_blocks_per_sm<EpiBoundPolicy>(&bps))) return rc;
+            score_packed<EpiBoundPolicy><<<std::min(plan.n_items, c->sm_count * bps), kScoreThreads,
+                                           score_smem_bytes<EpiBoundPolicy>(), st>>>(
+                (const float4*)c->pts32.ptr, (const Hyp32*)c->hyp32.ptr, pi, plan.P, plan.n_items, k.s.counts, k.fl, k.s.work);
+        } else {
+            constexpr size_t smem = score_smem_bytes<EpiPolicy<MODE>>();
+            const int grid = std::min(plan.n_items, c->sm_count * bps);
+            score_packed<EpiPolicy<MODE>><<<grid, kScoreThreads, smem, st>>>((const float4*)c->pts32.ptr, (const Hyp32*)c->hyp32.ptr,
+                                                                            pi, plan.P, plan.n_items, k.s.counts, k.fl, k.s.work);
+        }
         k.scored = true;
     } else {
         const int zs = std::max(1, std::min(64, ceil_div(plan.maxN, 2048)));
@@ -296,8 +305,8 @@ static int f_score_only(Ctx* c, cudaStream_t st, PassCtl& k) {
 
 // beside_scorer: the kernel will run NEXT TO the following pass's scorer (4 blocks x 128 threads x 96 registers per SM leave
 // room for exactly one 256-thread, 64-register block): a grid of one block per SM runs beside the scorer instead of ahead of it
-// stage: what the fix-up corrects — STAGE_MAIN the pass's scorer (full sweep, or the bounded sweep's prefix stage), STAGE_CAND
-// the candidate suffix stage (compact records, counts in sfx_c), STAGE_FALLBACK the fallback stage (counts in sfx_f)
+// stage: what the fix-up corrects — STAGE_MAIN the pass's scorer (full sweep, or the bounded sweep's exact prefix stage),
+// STAGE_CAND the candidate stage (compact records, counts in sfx_c), STAGE_FALLBACK the fallback stage (counts in sfx_f)
 enum : int { STAGE_MAIN = 0, STAGE_CAND = 1, STAGE_FALLBACK = 2 };
 template <int MODE>
 static int f_fixup_launch(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer, int stage = STAGE_MAIN) {
@@ -328,11 +337,11 @@ static int f_fixup_launch(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_score
     return RG_OK;
 }
 
-// bounded sweep, after the prefix stage: its fix-up (exact prefix counts c_A) and the choice of the candidates
+// bounded sweep, after the prefix stage: its fix-up (exact prefix only: counts c_A) and the choice of the candidates
 template <int MODE>
 static int f_bnd_cands(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) {
     if (k.scored) {
-        int rc = f_fixup_launch<MODE>(c, ts, k, beside_scorer);
+        int rc = k.plan.bound_prefix ? RG_OK : f_fixup_launch<MODE>(c, ts, k, beside_scorer);
         if (rc) return rc;
         const PairInfo* pi = (const PairInfo*)c->pair_info.ptr;
         bnd_select<<<k.plan.P, kSelectThreads, 0, ts>>>(k.s.counts, pi, pi + k.plan.P, (const Hyp32*)c->hyp32.ptr, k.bw.hypc,
@@ -344,7 +353,7 @@ static int f_bnd_cands(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) 
     return RG_OK;
 }
 
-// bounded sweep, after the candidates: candidate suffix stage + its fix-up, check, fallback stage (queued at full grid, its
+// bounded sweep, after the candidates: candidate stage + its fix-up, check, fallback stage (queued at full grid, its
 // item count comes from bnd_fb_plan: normally zero).  The fallback's fix-up and merge belong to the tail.
 template <int MODE>
 static int f_bnd_sweep(Ctx* c, cudaStream_t st, PassCtl& k) {
@@ -363,7 +372,7 @@ static int f_bnd_sweep(Ctx* c, cudaStream_t st, PassCtl& k) {
     prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 1);
     if (plan.n_items_c > 0 && (rc = f_fixup_launch<MODE>(c, st, k, false, STAGE_CAND))) return rc;
     bnd_check<<<plan.P, 256, 0, st>>>(k.s.counts, k.s.sfx_c, k.bw.map, pi, pi + plan.P, k.bw.sel, k.s.mark,
-                                      (unsigned long long*)c->bnd_stats.ptr);
+                                      (unsigned long long*)c->bnd_stats.ptr, !plan.bound_prefix);
     bnd_fb_plan<<<1, kSelectThreads, 0, st>>>(pi + 2 * (size_t)plan.P, k.s.mark, plan.P, k.bw.fb, k.s.f_items);
     c->last_stats[7] += 2;
     prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 2);
@@ -378,7 +387,7 @@ static int f_bnd_sweep(Ctx* c, cudaStream_t st, PassCtl& k) {
     return RG_OK;
 }
 
-// scorer + fix-up on one stream (stage entry point rg_epi_score_count_host)
+// scorer + fix-up on one stream (stage entry point rg_epi_score_count_host; SCORE_FP32_BOUND: the bound-only scorer alone)
 template <int MODE>
 static int f_score_launch(Ctx* c, cudaStream_t st, const FPlan& plan, const ScoreState& s, const double* pts64, double thr,
                           int score_path) {
@@ -388,7 +397,7 @@ static int f_score_launch(Ctx* c, cudaStream_t st, const FPlan& plan, const Scor
     int rc = f_score_only<MODE>(c, st, k);
     if (rc) return rc;
     prof_mark(c, st, 3);
-    return f_fixup_launch<MODE>(c, st, k, false);
+    return score_path == SCORE_FP32_BOUND ? RG_OK : f_fixup_launch<MODE>(c, st, k, false);
 }
 
 static int f_select_launch(Ctx* c, cudaStream_t st, const FPlan& plan, const ScoreState& s, const double* pts64, double thr,
@@ -431,7 +440,7 @@ static int f_pass_head(Ctx* c, cudaStream_t hs, PassCtl& k) {
     int bps = 1, rc = score_blocks_per_sm<EpiPolicy<MODE_EPI_MAX>>(&bps);
     if (rc) return rc;
     if ((rc = f_plan(c, hs, a.P, a.pair_off, a.hyp_off, plan, bps, nullptr, a.hyp_first, a.bounded ? c->opt_bounded_k : 0,
-                     c->opt_rho_milli)))
+                     c->opt_rho_milli, a.bounded && c->opt_bound_prefix != 0)))
         return rc;
     for (int p = 0; p < a.P; ++p) {
         const int n = a.pair_off[p + 1] - a.pair_off[p], H = a.hyp_off[p + 1] - a.hyp_off[p];
@@ -442,7 +451,12 @@ static int f_pass_head(Ctx* c, cudaStream_t hs, PassCtl& k) {
     if ((rc = score_state_layout(c, a.P, plan.Htot, 8, k.s, a.bounded ? plan.Ctot : -1))) return rc;
     if (a.bounded && (rc = bnd_workspace(c, plan, k.bw))) return rc;
     if (a.P == 0) return RG_OK;
-    c->bnd_host_evals += (long long)(plan.evals + plan.evals_c);
+    if (plan.bound_prefix) {
+        c->bnd_bound_evals += (long long)plan.evals;
+        c->bnd_host_evals += (long long)plan.evals_c;
+    } else {
+        c->bnd_host_evals += (long long)(plan.evals + plan.evals_c);
+    }
     const ScoreState& s = k.s;
 
     bool reuse = (a.flags & FLAG_REUSE_POINTS) != 0;
@@ -499,7 +513,8 @@ static int f_pass_tail(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) 
                                       : f_fixup_launch<MODE_EPI_MAX>(c, ts, k, beside_scorer, stage);
     if (rc) return rc;
     if (a.bounded && k.scored) {
-        bnd_merge<<<k.plan.P, 256, 0, ts>>>(k.s.counts, k.s.sfx_f, (const PairInfo*)c->pair_info.ptr, k.s.mark);
+        bnd_merge<<<k.plan.P, 256, 0, ts>>>(k.s.counts, k.s.sfx_f, (const PairInfo*)c->pair_info.ptr, k.s.mark,
+                                            !k.plan.bound_prefix);
         c->last_stats[7] += 1;
         RG_CUDA(cudaGetLastError());
     }
@@ -728,6 +743,7 @@ static int bnd_stats_reset(Ctx* c, cudaStream_t st, bool bounded) {
     if (rc) return rc;
     RG_CUDA(cudaMemsetAsync(c->bnd_stats.ptr, 0, sizeof(unsigned long long) * 4, st));
     c->bnd_host_evals = 0;
+    c->bnd_bound_evals = 0;
     c->last_bounded = bounded;
     return RG_OK;
 }
@@ -929,10 +945,23 @@ int rg_f_last_bounded_stats(void* ctx, void* stream, long long* out4) {
     RG_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
     unsigned long long d[4] = {0, 0, 0, 0};
     if (c->bnd_stats.ptr) RG_CUDA(cudaMemcpy(d, c->bnd_stats.ptr, sizeof(d), cudaMemcpyDeviceToHost));
-    out4[0] = c->bnd_host_evals + (long long)d[0];
+    out4[0] = c->bnd_bound_evals + c->bnd_host_evals + (long long)d[0];
     out4[1] = (long long)d[1];
     out4[2] = (long long)d[2];
     out4[3] = c->last_bounded ? c->opt_bounded_k : 0;
+    return RG_OK;
+}
+
+// out[0] evaluations of the last F call's bound-only prefix stages (upper-bound counts), [1] evaluations of its guarded
+// scorer (exact prefix, candidate and fallback stages, or the full sweep); their sum is out4[0] of rg_f_last_bounded_stats.
+// Synchronises the stream.
+int rg_f_last_bounded_evals(void* ctx, void* stream, long long* out2) {
+    RG_CHECK_ARG(ctx != nullptr && out2 != nullptr, "null argument");
+    long long s[4];
+    int rc = rg_f_last_bounded_stats(ctx, stream, s);
+    if (rc) return rc;
+    out2[0] = ((Ctx*)ctx)->bnd_bound_evals;
+    out2[1] = s[0] - out2[0];
     return RG_OK;
 }
 
@@ -1192,7 +1221,8 @@ int rg_epi_score_count_host(void* ctx, void* stream, int N, const double* pts64,
     RG_CHECK_ARG(N >= 0 && H >= 0 && counts, "bad sizes / null output");
     RG_CHECK_ARG(thr > 0.0 && std::isfinite(thr), "thr must be positive and finite");
     RG_CHECK_ARG(mode == MODE_EPI_MAX || mode == MODE_SAMPSON, "unknown scoring mode");
-    RG_CHECK_ARG(score_path == SCORE_FP32_GUARDED || score_path == SCORE_FP64, "unknown scoring path");
+    RG_CHECK_ARG(score_path == SCORE_FP32_GUARDED || score_path == SCORE_FP64 || score_path == SCORE_FP32_BOUND,
+                 "unknown scoring path");
     Ctx* c = (Ctx*)ctx;
     cudaStream_t st = (cudaStream_t)stream;
     RG_CUDA(cudaSetDevice(c->device));

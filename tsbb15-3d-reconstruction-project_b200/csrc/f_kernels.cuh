@@ -214,7 +214,7 @@ __device__ __forceinline__ void make_hyp32(const double* __restrict__ F, const P
         for (int k = 0; k < 9; ++k) h.f[k] = qnan;
 #pragma unroll
         for (int k = 0; k < 5; ++k) h.g[k] = qnan;
-        h.G = 0.f; h.pad0 = 0.f;
+        h.G = 0.f; h.T = 0.f;
         *out = h;
         return;
     }
@@ -255,7 +255,10 @@ __device__ __forceinline__ void make_hyp32(const double* __restrict__ F, const P
     // the bound assumes no FP32 underflow: with an extreme threshold / point spread (s1, s2 ~ 1/B^2 near the denormal
     // range) every evaluation of this hypothesis is sent to the FP64 recheck instead
     if (!(Mb > 1e-28) || !(B < 1e12)) h.G = INFINITY;
-    h.pad0 = 0.f;
+    // bound-only prefix scorer (EpiBoundPolicy): a reference inlier has q^ <= G (the band above) and m^ <= Mb (1 + eps)^14
+    // + 2^-146 (coefficients rounded, |x~|, |y~| <= B, subnormal results included), so r^2 < T (DESIGN.md section 4.2).
+    // G = inf gives T = inf: every evaluation counts and the pair falls back to the full sweep.
+    h.T = __double2float_ru((1.0 + 0x1p-16) * Mb + (1.0 + 0x1p-20) * (double)h.G + 0x1p-126);
     *out = h;
 }
 
@@ -622,6 +625,7 @@ template <int MODE>
 struct EpiPolicy {
     typedef Hyp32 Rec;
     typedef Hyp2 Regs;
+    static constexpr bool kBoundOnly = false;
     static constexpr int kVec4PerPair = 2;      // [x0a x0b x1a x1b] [y0a y0b y1a y1b]
     static constexpr int kChunkPts = RG_EPI_CHUNK;   // 16 KB of points per stage by default
 
@@ -698,6 +702,69 @@ struct EpiPolicy {
             cnt[k] += __float_as_uint(q.x) >> 31;
             cnt[k] += __float_as_uint(q.y) >> 31;
             minabs[k] = fminf(minabs[k], fminf(fabsf(q.x), fabsf(q.y)));
+        }
+    }
+};
+
+// Bound-only policy of the bounded sweep's prefix stage: counts r^2 < T (Hyp32::T), an upper bound on the exact count
+// (every reference inlier passes, DESIGN.md section 4.2).  r is computed with EpiPolicy's op sequence, so it is bit-identical
+// to the guarded scorer's; no image-2 normal, no norms, no guard band, no fix-up.  MODE only selects T (make_hyp32).
+struct HypBound {
+    float f[9];
+    float nT;            // -T
+};
+
+struct EpiBoundPolicy {
+    typedef Hyp32 Rec;
+    typedef HypBound Regs;
+    static constexpr bool kBoundOnly = true;
+    static constexpr int kVec4PerPair = 2;
+    static constexpr int kChunkPts = RG_EPI_CHUNK;
+
+    __device__ static __forceinline__ void load(const Hyp32* __restrict__ sh, int slot, bool valid, HypBound& out, float& G) {
+        G = 0.f;
+        if (valid) {
+            const float4* p = reinterpret_cast<const float4*>(sh + slot);
+            const float4 a = p[0], b = p[1], c = p[2], d = p[3];
+            const float f[9] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x};
+#pragma unroll
+            for (int k = 0; k < 9; ++k) out.f[k] = f[k];
+            out.nT = -d.w;
+        } else {                          // NaN r: q is a positive NaN and never counts
+            const float qnan = __int_as_float(0x7FFFFFFF);
+#pragma unroll
+            for (int k = 0; k < 9; ++k) out.f[k] = qnan;
+            out.nT = 0.f;
+        }
+    }
+
+    template <int K>
+    __device__ static __forceinline__ void evalN(const HypBound (&H)[K], const float4* __restrict__ pr, unsigned (&cnt)[K]) {
+        const float4 X = pr[0], Y = pr[1];
+        const float2 x0 = make_float2(X.x, X.y), x1 = make_float2(X.z, X.w);
+        const float2 y0 = make_float2(Y.x, Y.y), y1 = make_float2(Y.z, Y.w);
+        float2 l1x[K], l1y[K], l1z[K], r[K];
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            l1x[k] = ffma2_sbs(H[k].f[1], y1, H[k].f[2]);
+            l1y[k] = ffma2_sbs(H[k].f[4], y1, H[k].f[5]);
+            l1z[k] = ffma2_sbs(H[k].f[7], y1, H[k].f[8]);
+        }
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            l1x[k] = ffma2_sbc(H[k].f[0], y0, l1x[k]);
+            l1y[k] = ffma2_sbc(H[k].f[3], y0, l1y[k]);
+            l1z[k] = ffma2_sbc(H[k].f[6], y0, l1z[k]);
+        }
+#pragma unroll
+        for (int k = 0; k < K; ++k) r[k] = __ffma2_rn(l1y[k], x1, l1z[k]);
+#pragma unroll
+        for (int k = 0; k < K; ++k) r[k] = __ffma2_rn(l1x[k], x0, r[k]);
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const float2 q = __ffma2_rn(r[k], r[k], make_float2(H[k].nT, H[k].nT));     // sign bit set <=> r^2 < T
+            cnt[k] += __float_as_uint(q.x) >> 31;
+            cnt[k] += __float_as_uint(q.y) >> 31;
         }
     }
 };

@@ -114,10 +114,11 @@ inline int bounded_prefix_groups(int G, int rho_milli) {
 
 // bounded_k > 0: the bounded sweep's three tables (bounded.cuh) go into pair_info as [prefix stage | candidate stage |
 // fallback template], P entries each; the prefix stage is also the pass's main table (solver, selection, masks).
+// bound_prefix: the prefix stage counts an upper bound only, so the candidate and fallback stages cover the whole pair.
 inline int f_plan(Ctx* c, cudaStream_t st, int P, const int* pair_off, const int* hyp_off, FPlan& plan, int blocks_per_sm,
                   const int* n_vote = nullptr /* PnP: per-view number of voting correspondences (<= view size) */,
                   int hyp_first = 0 /* hypothesis-split mode: global index of this rank's first hypothesis */,
-                  int bounded_k = 0, int rho_milli = 0) {
+                  int bounded_k = 0, int rho_milli = 0, bool bound_prefix = false) {
     RG_CHECK_ARG(P >= 0 && P <= 65535, "number of pairs must be in [0, 65535]");
     RG_CHECK_ARG(pair_off != nullptr && hyp_off != nullptr, "offset arrays are null");
     RG_CHECK_ARG(pair_off[0] == 0 && hyp_off[0] == 0, "offset arrays must start at 0");
@@ -135,7 +136,7 @@ inline int f_plan(Ctx* c, cudaStream_t st, int P, const int* pair_off, const int
     for (int p = 0; p <= P; ++p) { mix((unsigned)pair_off[p]); mix((unsigned)hyp_off[p]); }
     if (n_vote) for (int p = 0; p < P; ++p) mix((unsigned)n_vote[p]);
     mix((unsigned)hyp_first); mix((unsigned)blocks_per_sm); mix(n_vote ? 1u : 0u); mix((unsigned)P);
-    mix((unsigned)bounded_k); mix((unsigned)rho_milli);
+    mix((unsigned)bounded_k); mix((unsigned)rho_milli); mix(bound_prefix ? 1u : 0u);
     if (c->plan_valid && c->plan_hash == hsh && c->plan_cached.P == P && c->pair_info.ptr == c->plan_table) {
         plan = c->plan_cached;
         return RG_OK;
@@ -175,10 +176,12 @@ inline int f_plan(Ctx* c, cudaStream_t st, int P, const int* pair_off, const int
     plan.N32tot = off32;
     if (bounded_k > 0) {
         // prefix stage: every hypothesis over groups [0, gA); candidate stage: min(K, H) compact records per pair over
-        // [gA, G); fallback template: every hypothesis over [gA, G) (bnd_fb_plan keeps the marked pairs' items)
+        // [gA, G) ([0, G) after a bound-only prefix); fallback template: every hypothesis over the same window as the
+        // candidates (bnd_fb_plan keeps the marked pairs' items)
         PairInfo* pc = pi + P;
         PairInfo* pf = pi + 2 * (size_t)P;
         plan.bounded = true;
+        plan.bound_prefix = bound_prefix;
         plan.K = bounded_k;
         plan.evals = 0.0;
         long long coff = 0;
@@ -188,14 +191,15 @@ inline int f_plan(Ctx* c, cudaStream_t st, int P, const int* pair_off, const int
             const int kA = std::min(o.n, gA * kSub);              // real correspondences of the prefix
             o.g_end = gA;
             pf[p] = o;
-            pf[p].g_base = gA; pf[p].g_end = G;
+            pf[p].g_base = bound_prefix ? 0 : gA; pf[p].g_end = G;
             pc[p] = pf[p];
             pc[p].hyp_off = (int)coff;
             pc[p].H = std::min(o.H, bounded_k);
             coff += pc[p].H;
+            const int rest = bound_prefix ? o.n : o.n - kA;          // real correspondences of the later stages' window
             plan.evals += (double)kA * (double)o.H;
-            plan.evals_c += (double)(o.n - kA) * (double)pc[p].H;
-            plan.evals_f += (double)(o.n - kA) * (double)o.H;
+            plan.evals_c += (double)rest * (double)pc[p].H;
+            plan.evals_f += (double)rest * (double)o.H;
         }
         plan.Ctot = coff;
         const long long nc = plan_items(c, pc, P, blocks_per_sm), nf = plan_items(c, pf, P, blocks_per_sm);

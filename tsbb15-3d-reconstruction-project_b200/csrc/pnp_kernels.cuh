@@ -651,6 +651,7 @@ struct Pose2 { float p[12]; };
 struct PnpPolicy {
     typedef Pose32 Rec;
     typedef Pose2 Regs;
+    static constexpr bool kBoundOnly = false;
     static constexpr int kVec4PerPair = 3;
     static constexpr int kChunkPts = 512;       // 12 KB of points per stage (two flag words)
 

@@ -121,6 +121,8 @@ __device__ __forceinline__ void flag_append(const FlagList& L, unsigned fl, int 
 // Policy requirements:
 //   typedef Rec;                       hypothesis record in global/shared memory (sizeof % 16 == 0)
 //   typedef Regs;                      hypothesis in registers
+//   static constexpr bool kBoundOnly;  true: evalN(H, pair, cnt) counts an upper bound and the guard-band bookkeeping
+//                                      (min|q|, flags, list appends) is compiled out; the counts need no fix-up
 //   static constexpr int kVec4PerPair; float4 per packed point pair
 //   static constexpr int kChunkPts;    points per shared-memory stage
 //   static void load(const Rec* sh, int slot, bool valid, Regs&, float& G);
@@ -229,31 +231,36 @@ score_packed(const float4* __restrict__ pts32, const typename Pol::Rec* __restri
                     Pol::load(st[stage].hyp, k * kScoreThreads + tid, hid[k] < cur.H_end, Hy[k], G[k]);
             }
             const float4* sp = st[stage].pts;
-            // chunk = whole flag words (32 flag groups of kSub points each), except the last word of an item
-            const int ngr = npts / kSub;
-            const int gfirst = cur.g0 + done / kSub;
-            for (int wq = 0; wq * 32 < ngr; ++wq) {
-                const int ng = min(32, ngr - wq * 32);
-                unsigned flag[kHypPerThread];
-#pragma unroll
-                for (int k = 0; k < kHypPerThread; ++k) flag[k] = 0u;
-                const float4* wp = sp + wq * 32 * (kSub / 2) * kV;
-                for (int g = 0; g < ng; ++g) {
-                    float ma[kHypPerThread];
-#pragma unroll
-                    for (int k = 0; k < kHypPerThread; ++k) ma[k] = INFINITY;
-                    const float4* gp = wp + g * (kSub / 2) * kV;
+            if constexpr (Pol::kBoundOnly) {           // upper-bound counts only: no min|q|, no flags, no list
 #pragma unroll kPairUnroll
-                    for (int j = 0; j < kSub / 2; ++j) Pol::template evalN<kHypPerThread>(Hy, gp + j * kV, cnt, ma);
-                    const unsigned bit = 1u << g;             // uniform: the shift stays in the uniform datapath
+                for (int j = 0; j < npts / 2; ++j) Pol::template evalN<kHypPerThread>(Hy, sp + j * kV, cnt);
+            } else {
+                // chunk = whole flag words (32 flag groups of kSub points each), except the last word of an item
+                const int ngr = npts / kSub;
+                const int gfirst = cur.g0 + done / kSub;
+                for (int wq = 0; wq * 32 < ngr; ++wq) {
+                    const int ng = min(32, ngr - wq * 32);
+                    unsigned flag[kHypPerThread];
 #pragma unroll
-                    for (int k = 0; k < kHypPerThread; ++k)   // (NaN: no flag) FSETP + predicated LOP3; plain C++ compiles to FSETP + SEL + SHF + LOP3
-                        asm("{\n.reg .pred p;\nsetp.le.f32 p, %1, %2;\n@p or.b32 %0, %0, %3;\n}"
-                            : "+r"(flag[k]) : "f"(ma[k]), "f"(G[k]), "r"(bit));
+                    for (int k = 0; k < kHypPerThread; ++k) flag[k] = 0u;
+                    const float4* wp = sp + wq * 32 * (kSub / 2) * kV;
+                    for (int g = 0; g < ng; ++g) {
+                        float ma[kHypPerThread];
+#pragma unroll
+                        for (int k = 0; k < kHypPerThread; ++k) ma[k] = INFINITY;
+                        const float4* gp = wp + g * (kSub / 2) * kV;
+#pragma unroll kPairUnroll
+                        for (int j = 0; j < kSub / 2; ++j) Pol::template evalN<kHypPerThread>(Hy, gp + j * kV, cnt, ma);
+                        const unsigned bit = 1u << g;             // uniform: the shift stays in the uniform datapath
+#pragma unroll
+                        for (int k = 0; k < kHypPerThread; ++k)   // (NaN: no flag) FSETP + predicated LOP3; plain C++ compiles to FSETP + SEL + SHF + LOP3
+                            asm("{\n.reg .pred p;\nsetp.le.f32 p, %1, %2;\n@p or.b32 %0, %0, %3;\n}"
+                                : "+r"(flag[k]) : "f"(ma[k]), "f"(G[k]), "r"(bit));
+                    }
+#pragma unroll
+                    for (int k = 0; k < kHypPerThread; ++k)
+                        flag_append(flist, hid[k] < cur.H_end ? flag[k] : 0u, hid[k], gfirst + wq * 32);
                 }
-#pragma unroll
-                for (int k = 0; k < kHypPerThread; ++k)
-                    flag_append(flist, hid[k] < cur.H_end ? flag[k] : 0u, hid[k], gfirst + wq * 32);
             }
             __syncthreads();          // everyone is done with this stage before it is refilled
             stage ^= 1;

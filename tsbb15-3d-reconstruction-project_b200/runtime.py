@@ -155,10 +155,14 @@ def profile(device=None, stream=0) -> dict:
 
 
 def bounded_stats(device=None, stream=0) -> dict:
-    """What the last F call executed: see rg_f_last_bounded_stats (K = 0: it ran the full sweep)."""
+    """What the last F call executed: see rg_f_last_bounded_stats (K = 0: it ran the full sweep).  ``evals`` splits into
+    ``bound_evals`` (bound-only prefix stages) and ``guarded_evals`` (rg_f_last_bounded_evals)."""
     out = (C.c_longlong * 4)()
     _call("rg_f_last_bounded_stats", device, stream, out)
-    return {"evals": out[0], "not_fully_scored": out[1], "fallback_pairs": out[2], "K": out[3]}
+    split = (C.c_longlong * 2)()
+    _call("rg_f_last_bounded_evals", device, stream, split)
+    return {"evals": out[0], "not_fully_scored": out[1], "fallback_pairs": out[2], "K": out[3],
+            "bound_evals": split[0], "guarded_evals": split[1]}
 
 
 def last_stats(device=None, stream=0) -> dict:
