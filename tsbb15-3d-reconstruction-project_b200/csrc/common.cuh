@@ -196,7 +196,6 @@ struct Ctx {
     // `state` = everything one cudaMemsetAsync clears per pass: [bbox keys][counts][work counter, list size][ovf bytes]
     int* counts_ptr = nullptr;                     // inside `state` (valid after f_state_layout of the current pass)
     unsigned char* ovf_ptr = nullptr;
-    Buffer gen_idx;                                // device-drawn sample indices of the current pass (seeded calls)
     // Pass pipelining (F calls of several passes): the caller's stream runs the scorers back to back; the solver ("head") of
     // pass k+1 and the fix-up / selection / mask kernels ("tail") of pass k-1 run on a second stream BESIDE the scorer of pass k
     // — they are latency bound (23 % issue active) and one of their blocks fits next to the scorer's four on every SM.  The
@@ -209,9 +208,8 @@ struct Ctx {
     cudaEvent_t score_done[3] = {nullptr, nullptr, nullptr};  // recorded on the caller's stream after the scorer of the pass in set i
     cudaEvent_t cand_done[3] = {nullptr, nullptr, nullptr};   // bounded sweep: side stream, candidates of the pass in set i chosen
     cudaEvent_t sweep_done[3] = {nullptr, nullptr, nullptr};  // bounded sweep: caller's stream, last scorer of the pass in set i
-    cudaEvent_t tail_done[2] = {nullptr, nullptr};      // [0]: recorded on the side stream behind the last tail kernel of a run
+    cudaEvent_t tail_done = nullptr;                    // recorded on the side stream behind the last tail kernel of a run
     cudaEvent_t pipe_gate = nullptr;                    // recorded on the caller's stream before the side stream starts a run
-    bool tail_pending[2] = {false, false};              // tail_done[i] was recorded and nobody has waited for it yet
     int tail_carve_max = -1;                            // shared-memory carve-out preference of the tail kernels: -1 never set, 0 default, 1 max
     int ws_slot = 0;                                    // which set is the current one
     int opt_pipeline = 1;                               // option 10: 0 = passes strictly one after the other on one stream
@@ -272,7 +270,6 @@ struct Ctx {
     cudaEvent_t d2h_done = nullptr;
     cudaEvent_t copy_gate = nullptr;               // recorded on the caller's stream before the first upload
     int opt_host_slices = 0;                       // option 2: 0 = automatic, n >= 1 = force n sub-batches
-    bool accumulate_stats = false;                 // sub-batches after the first add to the call's statistics
     long long last_stats[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     // optional phase profiling (option 1): CUDA events on the launching stream around the phases of every call
     int opt_profile = 0;

@@ -117,7 +117,7 @@ int rg_shutdown(void* ctx) {
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     for (Buffer* b : {&c->pair_info, &c->pair_frame, &c->state, &c->bbox, &c->pts32, &c->F64, &c->hyp32, &c->flags,
-                      &c->flag_list, &c->gen_idx, &c->stats, &c->best, &c->tie_stats, &c->d_in_a, &c->d_in_b, &c->d_in_c, &c->geom, &c->geom_ws, &c->gs_ws, &c->ba_ws, &c->pr_ws, &c->d_out_a, &c->d_out_b,
+                      &c->flag_list, &c->stats, &c->best, &c->tie_stats, &c->d_in_a, &c->d_in_b, &c->d_in_c, &c->geom, &c->geom_ws, &c->gs_ws, &c->ba_ws, &c->pr_ws, &c->d_out_a, &c->d_out_b,
                       &c->d_out_c, &c->d_out_d, &c->pose64, &c->pose32, &c->X32, &c->bnd, &c->bnd_stats})
         release(*b);
     for (Ctx::PassSet& o : c->spare)
@@ -130,8 +130,7 @@ int rg_shutdown(void* ctx) {
         if (c->cand_done[i]) cudaEventDestroy(c->cand_done[i]);
         if (c->sweep_done[i]) cudaEventDestroy(c->sweep_done[i]);
     }
-    for (int i = 0; i < 2; ++i)
-        if (c->tail_done[i]) cudaEventDestroy(c->tail_done[i]);
+    if (c->tail_done) cudaEventDestroy(c->tail_done);
     if (c->pipe_gate) cudaEventDestroy(c->pipe_gate);
     if (c->tail_stream) cudaStreamDestroy(c->tail_stream);
     release_pinned(c->h_stage[0]);

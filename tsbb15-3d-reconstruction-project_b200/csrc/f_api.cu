@@ -109,7 +109,7 @@ struct FCall {
     unsigned long long* keys = nullptr;
 };
 
-// ---- pass pipelining (Ctx::spare, common.cuh; the drivers are f_run_piped / f_run_piped_bounded below) ----
+// ---- pass pipelining (Ctx::spare, common.cuh; the schedules are in f_run_piped below) ----
 // Single-pass calls never switch: their launch chain stays on the caller's stream in the current set (capturable in a CUDA
 // graph, RG_FLAG_REUSE_POINTS finds its prepared points).
 static void ws_exchange(Ctx* c, Ctx::PassSet& o) {
@@ -167,19 +167,8 @@ static int pipe_setup(Ctx* c) {
         if (!c->cand_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->cand_done[i], cudaEventDisableTiming));
         if (!c->sweep_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->sweep_done[i], cudaEventDisableTiming));
     }
-    for (int i = 0; i < 2; ++i)
-        if (!c->tail_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->tail_done[i], cudaEventDisableTiming));
+    if (!c->tail_done) RG_CUDA(cudaEventCreateWithFlags(&c->tail_done, cudaEventDisableTiming));
     if (!c->pipe_gate) RG_CUDA(cudaEventCreateWithFlags(&c->pipe_gate, cudaEventDisableTiming));
-    return RG_OK;
-}
-
-// the caller's stream waits for every tail still in flight (end of a call, or before anything reads a pass's results)
-static int pipe_join(Ctx* c, cudaStream_t st) {
-    for (int i = 0; i < 2; ++i)
-        if (c->tail_pending[i]) {
-            RG_CUDA(cudaStreamWaitEvent(st, c->tail_done[i], 0));
-            c->tail_pending[i] = false;
-        }
     return RG_OK;
 }
 
@@ -189,7 +178,7 @@ static unsigned long long hash_offsets(const int* off, int n) {
     return h;
 }
 
-static int f_workspace(Ctx* c, const FPlan& plan, bool seeded) {
+static int f_workspace(Ctx* c, const FPlan& plan) {
     int rc;
     const size_t H = (size_t)std::max<long long>(plan.Htot, 1);
     if ((rc = ensure(c->F64, sizeof(double) * 9 * H))) return rc;
@@ -200,7 +189,6 @@ static int f_workspace(Ctx* c, const FPlan& plan, bool seeded) {
     if ((rc = ensure(c->tie_stats, sizeof(double2) * H))) return rc;
     if ((rc = ensure(c->pair_frame, sizeof(PairFrame) * (size_t)std::max(plan.P, 1)))) return rc;
     if ((rc = ensure_pinned(c->h_stats, sizeof(unsigned long long) * 8))) return rc;
-    (void)seeded;
     return RG_OK;
 }
 
@@ -253,14 +241,18 @@ struct PassCtl {
     FlagList flc{nullptr, nullptr, 0u, nullptr}, flf{nullptr, nullptr, 0u, nullptr};   // bounded sweep: candidate / fallback stage
     BndWs bw{};
     bool scored = false;                  // the packed scorer ran: its flag list wants the fix-up
-    int slot = 0;                         // workspace set of the pass (Ctx::alt)
+    int slot = 0;                         // workspace set of the pass (Ctx::spare; pipelined runs only)
     int prof_call = -1;                   // ring index of the pass's phase events (option 1)
-    cudaEvent_t ready = nullptr;          // optional: the pass's inputs have arrived (host entry point)
+    cudaEvent_t ready = nullptr;          // optional: the pass's inputs have arrived; the stream that runs its head waits for it
     cudaEvent_t done = nullptr;           // optional: recorded behind the pass's last tail kernel
     // optional: a copy queued on out_stream behind `done` as soon as the pass's tail is queued (host entry point: the pass's
     // inlier masks travel back while later passes are scored; queued after all passes instead, a 64-pass call had its host
     // thread stuck in the driver's launch queue and every mask download ended up behind the last scorer)
     cudaStream_t out_stream = nullptr; void* out_dst = nullptr; const void* out_src = nullptr; size_t out_bytes = 0;
+    // optional: host destinations of the pass's per-hypothesis counts / F / flags, copied behind its tail (they live in the
+    // pass's workspace set, which the next pass reuses: a call that wants them runs its passes one after the other)
+    int* out_counts = nullptr; double* out_F_all = nullptr; unsigned char* out_flags = nullptr;
+    bool wants_hypotheses() const { return out_counts || out_F_all || out_flags; }
 };
 
 // counts / work counter / flag list are already cleared by the pass's memset
@@ -446,11 +438,9 @@ static int f_pass_head(Ctx* c, cudaStream_t hs, PassCtl& k) {
         const int n = a.pair_off[p + 1] - a.pair_off[p], H = a.hyp_off[p + 1] - a.hyp_off[p];
         RG_CHECK_ARG(H == 0 || n >= 8, "a pair with hypotheses needs at least 8 correspondences");
     }
-    const bool seeded = a.idx == nullptr && plan.Htot > 0;
-    if ((rc = f_workspace(c, plan, seeded))) return rc;
+    if ((rc = f_workspace(c, plan))) return rc;
     if ((rc = score_state_layout(c, a.P, plan.Htot, 8, k.s, a.bounded ? plan.Ctot : -1))) return rc;
     if (a.bounded && (rc = bnd_workspace(c, plan, k.bw))) return rc;
-    if (a.P == 0) return RG_OK;
     if (plan.bound_prefix) {
         c->bnd_bound_evals += (long long)plan.evals;
         c->bnd_host_evals += (long long)plan.evals_c;
@@ -487,7 +477,6 @@ static int f_pass_head(Ctx* c, cudaStream_t hs, PassCtl& k) {
 }
 
 static int f_pass_score(Ctx* c, cudaStream_t st, PassCtl& k) {
-    if (k.a.P == 0) return RG_OK;
     prof_mark_at(c, st, k.prof_call, Ctx::kProfScoreStart);
     const int rc = (k.a.mode == MODE_SAMPSON) ? f_score_only<MODE_SAMPSON>(c, st, k) : f_score_only<MODE_EPI_MAX>(c, st, k);
     prof_mark_at(c, st, k.prof_call, 3);
@@ -495,18 +484,15 @@ static int f_pass_score(Ctx* c, cudaStream_t st, PassCtl& k) {
 }
 
 static int f_pass_cands(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) {
-    if (k.a.P == 0) return RG_OK;
     return (k.a.mode == MODE_SAMPSON) ? f_bnd_cands<MODE_SAMPSON>(c, ts, k, beside_scorer)
                                       : f_bnd_cands<MODE_EPI_MAX>(c, ts, k, beside_scorer);
 }
 
 static int f_pass_sweep(Ctx* c, cudaStream_t st, PassCtl& k) {
-    if (k.a.P == 0) return RG_OK;
     return (k.a.mode == MODE_SAMPSON) ? f_bnd_sweep<MODE_SAMPSON>(c, st, k) : f_bnd_sweep<MODE_EPI_MAX>(c, st, k);
 }
 
 static int f_pass_tail(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) {
-    if (k.a.P == 0) return RG_OK;
     const FCall& a = k.a;
     const int stage = a.bounded ? STAGE_FALLBACK : STAGE_MAIN;
     int rc = (a.mode == MODE_SAMPSON) ? f_fixup_launch<MODE_SAMPSON>(c, ts, k, beside_scorer, stage)
@@ -526,156 +512,123 @@ static int f_pass_tail(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) 
     return RG_OK;
 }
 
-// one pass on device pointers, everything on the caller's stream in the current workspace set; offsets are relative to the pass
-static int f_pass(Ctx* c, cudaStream_t st, const FCall& a) {
-    PassCtl k;
-    k.a = a;
-    k.slot = c->ws_slot;
-    int rc;
-    if (c->tail_carve_max > 0 && (rc = tail_carveout(c, false))) return rc;
-    if ((rc = f_pass_head(c, st, k))) return rc;
-    if ((rc = f_pass_score(c, st, k))) return rc;
-    if (a.bounded && ((rc = f_pass_cands(c, st, k, false)) || (rc = f_pass_sweep(c, st, k)))) return rc;
-    return f_pass_tail(c, st, k, false);
+// the pass's downloads, queued on stream ts behind its tail: per-hypothesis results, then `done` and the copy behind it
+static int f_pass_downloads(Ctx* c, cudaStream_t ts, const PassCtl& k) {
+    const size_t H = (size_t)k.plan.Htot;
+    if (k.out_counts && H) RG_CUDA(cudaMemcpyAsync(k.out_counts, c->counts_ptr, sizeof(int) * H, cudaMemcpyDeviceToHost, ts));
+    if (k.out_F_all && H) RG_CUDA(cudaMemcpyAsync(k.out_F_all, c->F64.ptr, sizeof(double) * 9 * H, cudaMemcpyDeviceToHost, ts));
+    if (k.out_flags && H) RG_CUDA(cudaMemcpyAsync(k.out_flags, c->flags.ptr, H, cudaMemcpyDeviceToHost, ts));
+    if (!k.done) return RG_OK;
+    RG_CUDA(cudaEventRecord(k.done, ts));
+    if (k.out_stream && k.out_bytes) {
+        RG_CUDA(cudaStreamWaitEvent(k.out_stream, k.done, 0));
+        RG_CUDA(cudaMemcpyAsync(k.out_dst, k.out_src, k.out_bytes, cudaMemcpyDeviceToHost, k.out_stream));
+    }
+    return RG_OK;
 }
 
-// Several passes, software-pipelined over two streams and two workspace sets:
+// passes one after the other, everything on the caller's stream in the current workspace set
+static int f_run_serial(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs) {
+    int rc;
+    if (c->tail_carve_max > 0 && (rc = tail_carveout(c, false))) return rc;
+    for (PassCtl& k : jobs) {
+        if (k.ready) RG_CUDA(cudaStreamWaitEvent(st, k.ready, 0));
+        if ((rc = f_pass_head(c, st, k)) || (rc = f_pass_score(c, st, k))) return rc;
+        if (k.a.bounded && ((rc = f_pass_cands(c, st, k, false)) || (rc = f_pass_sweep(c, st, k)))) return rc;
+        if ((rc = f_pass_tail(c, st, k, false)) || (rc = f_pass_downloads(c, st, k))) return rc;
+    }
+    return RG_OK;
+}
+
+// Several passes, software-pipelined over the caller's stream and a side stream.  The full sweep uses two workspace sets:
 //
 //   caller's stream :            score(0)            score(1)            score(2)         ...      join
 //   side stream     :  head(0)   head(1)   tail(0)   head(2)   tail(1)   head(3)   tail(2) ...
 //
 // The caller's stream runs the scorers back to back; the side stream's kernels run BESIDE them: the tail of pass k and the head
 // of pass k+2 need the same workspace set, which the side stream's own order serialises.  head(k+1) is queued before tail(k)
-// (tail(k) has to wait for score(k), head(k+1) has not).  jobs[k].ready / .done tie in the host entry point's uploads and mask
-// downloads.  join: the caller's stream waits for the last tail before this returns (otherwise pipe_join() does it later).
-static int f_run_piped(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs, bool join) {
-    const int n = (int)jobs.size();
-    if (n == 0) return RG_OK;
-    int rc;
-    if ((rc = pipe_setup(c))) return rc;
-    if ((rc = tail_carveout(c, true))) return rc;
-    cudaStream_t side = c->tail_stream;
-    auto fail = [&](int code) {                       // leave nothing in flight behind an error return
-        cudaStreamSynchronize(st);
-        cudaStreamSynchronize(side);
-        c->tail_pending[0] = c->tail_pending[1] = false;
-        return code;
-    };
-    if ((rc = pipe_join(c, st))) return rc;           // (a previous unjoined run on this context)
-    RG_CUDA(cudaEventRecord(c->pipe_gate, st));       // the side stream may not overtake what the caller queued before the call
-    RG_CUDA(cudaStreamWaitEvent(side, c->pipe_gate, 0));
-    const int base = c->ws_slot ^ 1;
-    for (int k = 0; k < n; ++k) jobs[k].slot = (base + k) & 1;
-    auto head = [&](int k) -> int {
-        ws_use(c, jobs[k].slot);
-        if (jobs[k].ready) RG_CUDA(cudaStreamWaitEvent(side, jobs[k].ready, 0));
-        int r = f_pass_head(c, side, jobs[k]);
-        if (r) return r;
-        RG_CUDA(cudaEventRecord(c->head_done[jobs[k].slot], side));
-        return RG_OK;
-    };
-    if ((rc = head(0))) return fail(rc);
-    for (int k = 0; k < n; ++k) {
-        PassCtl& j = jobs[k];
-        RG_CUDA(cudaStreamWaitEvent(st, c->head_done[j.slot], 0));
-        ws_use(c, j.slot);
-        if ((rc = f_pass_score(c, st, j))) return fail(rc);
-        RG_CUDA(cudaEventRecord(c->score_done[j.slot], st));
-        if (k + 1 < n && (rc = head(k + 1))) return fail(rc);
-        RG_CUDA(cudaStreamWaitEvent(side, c->score_done[j.slot], 0));
-        ws_use(c, j.slot);
-        if ((rc = f_pass_tail(c, side, j, k + 1 < n))) return fail(rc);
-        if (j.done) RG_CUDA(cudaEventRecord(j.done, side));
-        if (j.done && j.out_stream && j.out_bytes) {
-            RG_CUDA(cudaStreamWaitEvent(j.out_stream, j.done, 0));
-            RG_CUDA(cudaMemcpyAsync(j.out_dst, j.out_src, j.out_bytes, cudaMemcpyDeviceToHost, j.out_stream));
-        }
-    }
-    RG_CUDA(cudaEventRecord(c->tail_done[0], side));
-    c->tail_pending[0] = true;
-    // (the current set is the last pass's: counts_ptr / F64 / flags of rg_f_last_hypotheses_dev and the prepared points)
-    if (join) return pipe_join(c, st);
-    return RG_OK;
-}
-
-// The bounded sweep's passes, over two streams and THREE workspace sets (pass k lives until its tail, which follows the
-// prefix stage of pass k+1 and its own candidate stage):
+// (tail(k) has to wait for score(k), head(k+1) has not).
 //
-//   caller's stream :  S1(0)          S1(1)  S3+FB(0)          S1(2)  S3+FB(1)          S1(3) ...  S3+FB(n-1)
+// The bounded sweep uses THREE workspace sets (pass k lives until its tail, which follows the prefix stage of pass k+1 and its
+// own candidate stage):
+//
+//   caller's stream :  S1(0)          S1(1)  S3+FB(0)          S1(2)  S3+FB(1)          S1(3) ...  S3+FB(n-1)        join
 //   side stream     :  head(0) head(1)  cands(0) head(2)  cands(1) tail(0) head(3)  cands(2) tail(1) head(4) ...  tail(n-1)
 //
 // S1 = prefix stage, cands = its fix-up + bnd_select, S3+FB = candidate stage, its fix-up, bnd_check, bnd_fb_plan and the
 // fallback stage, tail = fallback fix-up, bnd_merge, selection, masks.  The caller's stream only waits between S3 and FB for
 // the candidate stage's fix-up and the check (two small launches); everything else on the side stream runs beside a scorer.
 // head(k+3) reuses pass k's set and is queued behind tail(k) on the side stream.
-static int f_run_piped_bounded(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs, bool join) {
+//
+// Either way the caller's stream ends behind the last tail (join), and the current set is the last pass's (counts_ptr / F64 /
+// flags of rg_f_last_hypotheses_dev and the prepared points).
+static int f_run_piped(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs) {
     const int n = (int)jobs.size();
-    if (n == 0) return RG_OK;
+    const bool bounded = jobs[0].a.bounded;
     int rc;
-    if ((rc = pipe_setup(c))) return rc;
-    if ((rc = tail_carveout(c, true))) return rc;
+    if ((rc = pipe_setup(c)) || (rc = tail_carveout(c, true))) return rc;
     cudaStream_t side = c->tail_stream;
-    auto fail = [&](int code) {                       // leave nothing in flight behind an error return
-        cudaStreamSynchronize(st);
-        cudaStreamSynchronize(side);
-        c->tail_pending[0] = c->tail_pending[1] = false;
-        return code;
-    };
-    if ((rc = pipe_join(c, st))) return rc;
-    RG_CUDA(cudaEventRecord(c->pipe_gate, st));
+    RG_CUDA(cudaEventRecord(c->pipe_gate, st));       // the side stream may not overtake what the caller queued before the call
     RG_CUDA(cudaStreamWaitEvent(side, c->pipe_gate, 0));
-    for (int k = 0; k < n; ++k) jobs[k].slot = (c->ws_slot + 1 + k) % 3;
-    auto head = [&](int k) -> int {
-        ws_use(c, jobs[k].slot);
-        if (jobs[k].ready) RG_CUDA(cudaStreamWaitEvent(side, jobs[k].ready, 0));
-        int r = f_pass_head(c, side, jobs[k]);
-        if (r) return r;
-        RG_CUDA(cudaEventRecord(c->head_done[jobs[k].slot], side));
-        return RG_OK;
-    };
-    auto sweep = [&](int k) -> int {                  // caller's stream
+    for (int k = 0; k < n; ++k) jobs[k].slot = (c->ws_slot + 1 + k) % (bounded ? 3 : 2);
+    auto head = [&](int k) -> int {                   // side stream
         PassCtl& j = jobs[k];
-        RG_CUDA(cudaStreamWaitEvent(st, c->cand_done[j.slot], 0));
         ws_use(c, j.slot);
-        int r = f_pass_sweep(c, st, j);
+        if (j.ready) RG_CUDA(cudaStreamWaitEvent(side, j.ready, 0));
+        int r = f_pass_head(c, side, j);
         if (r) return r;
-        RG_CUDA(cudaEventRecord(c->sweep_done[j.slot], st));
+        RG_CUDA(cudaEventRecord(c->head_done[j.slot], side));
         return RG_OK;
     };
-    auto tail = [&](int k, bool beside) -> int {      // side stream
-        PassCtl& j = jobs[k];
-        RG_CUDA(cudaStreamWaitEvent(side, c->sweep_done[j.slot], 0));
-        ws_use(c, j.slot);
-        int r = f_pass_tail(c, side, j, beside);
-        if (r) return r;
-        if (j.done) RG_CUDA(cudaEventRecord(j.done, side));
-        if (j.done && j.out_stream && j.out_bytes) {
-            RG_CUDA(cudaStreamWaitEvent(j.out_stream, j.done, 0));
-            RG_CUDA(cudaMemcpyAsync(j.out_dst, j.out_src, j.out_bytes, cudaMemcpyDeviceToHost, j.out_stream));
-        }
-        return RG_OK;
-    };
-    if ((rc = head(0))) return fail(rc);
-    if (n > 1 && (rc = head(1))) return fail(rc);
-    for (int k = 0; k < n; ++k) {
+    auto score = [&](int k) -> int {                  // caller's stream
         PassCtl& j = jobs[k];
         RG_CUDA(cudaStreamWaitEvent(st, c->head_done[j.slot], 0));
         ws_use(c, j.slot);
-        if ((rc = f_pass_score(c, st, j))) return fail(rc);
+        int r = f_pass_score(c, st, j);
+        if (r) return r;
         RG_CUDA(cudaEventRecord(c->score_done[j.slot], st));
-        if (k > 0 && (rc = sweep(k - 1))) return fail(rc);
-        RG_CUDA(cudaStreamWaitEvent(side, c->score_done[j.slot], 0));
+        return RG_OK;
+    };
+    auto tail = [&](int k, cudaEvent_t gate, bool beside) -> int {      // side stream, behind `gate` of the caller's stream
+        PassCtl& j = jobs[k];
+        RG_CUDA(cudaStreamWaitEvent(side, gate, 0));
         ws_use(c, j.slot);
-        if ((rc = f_pass_cands(c, side, j, k + 1 < n))) return fail(rc);
-        RG_CUDA(cudaEventRecord(c->cand_done[j.slot], side));
-        if (k > 0 && (rc = tail(k - 1, true))) return fail(rc);
-        if (k + 2 < n && (rc = head(k + 2))) return fail(rc);
+        int r = f_pass_tail(c, side, j, beside);
+        return r ? r : f_pass_downloads(c, side, j);
+    };
+    if ((rc = head(0))) return rc;
+    if (!bounded) {
+        for (int k = 0; k < n; ++k) {
+            if ((rc = score(k))) return rc;
+            if (k + 1 < n && (rc = head(k + 1))) return rc;
+            if ((rc = tail(k, c->score_done[jobs[k].slot], k + 1 < n))) return rc;
+        }
+    } else {
+        auto sweep = [&](int k) -> int {              // caller's stream
+            PassCtl& j = jobs[k];
+            RG_CUDA(cudaStreamWaitEvent(st, c->cand_done[j.slot], 0));
+            ws_use(c, j.slot);
+            int r = f_pass_sweep(c, st, j);
+            if (r) return r;
+            RG_CUDA(cudaEventRecord(c->sweep_done[j.slot], st));
+            return RG_OK;
+        };
+        if (n > 1 && (rc = head(1))) return rc;
+        for (int k = 0; k < n; ++k) {
+            PassCtl& j = jobs[k];
+            if ((rc = score(k))) return rc;
+            if (k > 0 && (rc = sweep(k - 1))) return rc;
+            RG_CUDA(cudaStreamWaitEvent(side, c->score_done[j.slot], 0));
+            ws_use(c, j.slot);
+            if ((rc = f_pass_cands(c, side, j, k + 1 < n))) return rc;
+            RG_CUDA(cudaEventRecord(c->cand_done[j.slot], side));
+            if (k > 0 && (rc = tail(k - 1, c->sweep_done[jobs[k - 1].slot], true))) return rc;
+            if (k + 2 < n && (rc = head(k + 2))) return rc;
+        }
+        if ((rc = sweep(n - 1)) || (rc = tail(n - 1, c->sweep_done[jobs[n - 1].slot], false))) return rc;
     }
-    if ((rc = sweep(n - 1))) return fail(rc);
-    if ((rc = tail(n - 1, false))) return fail(rc);
-    RG_CUDA(cudaEventRecord(c->tail_done[0], side));
-    c->tail_pending[0] = true;
-    if (join) return pipe_join(c, st);
+    RG_CUDA(cudaEventRecord(c->tail_done, side));
+    RG_CUDA(cudaStreamWaitEvent(st, c->tail_done, 0));
     return RG_OK;
 }
 
@@ -697,6 +650,10 @@ static int f_check_call(const FCall& a) {
     return RG_OK;
 }
 
+static double pair_evals(const FCall& a, int p) {
+    return (double)(a.pair_off[p + 1] - a.pair_off[p]) * (double)(a.hyp_off[p + 1] - a.hyp_off[p]);
+}
+
 // pass boundaries: contiguous blocks of pairs with bounded evaluations / hypotheses (every pass holds at least one pair)
 static void f_pass_bounds(const Ctx* c, const FCall& a, std::vector<int>& bounds) {
     const double budget = c->opt_pass_evals > 0 ? (double)c->opt_pass_evals : kDefaultPassEvals;
@@ -705,7 +662,7 @@ static void f_pass_bounds(const Ctx* c, const FCall& a, std::vector<int>& bounds
     double ev = 0.0;
     long long hy = 0;
     for (int p = 0; p < a.P; ++p) {
-        const double e = (double)(a.pair_off[p + 1] - a.pair_off[p]) * (double)(a.hyp_off[p + 1] - a.hyp_off[p]);
+        const double e = pair_evals(a, p);
         const long long h = a.hyp_off[p + 1] - a.hyp_off[p];
         if (p > bounds.back() && (ev + e > budget || hy + h > kMaxPassHyp || p - bounds.back() >= 32768)) {
             bounds.push_back(p);
@@ -714,6 +671,62 @@ static void f_pass_bounds(const Ctx* c, const FCall& a, std::vector<int>& bounds
         ev += e; hy += h;
     }
     bounds.push_back(a.P);
+}
+
+// Sub-batches of the host entry point: the passes of f_pass_bounds, the first of them cut further when that hides a
+// worthwhile part of the upload.  The scoring and upload times are estimated with the rates MEASURED on this context by
+// earlier calls.  Every sub-batch is a sub-range of a pass of f_pass_bounds, and therefore one pass itself (its limits are
+// monotone).  A plan may hold empty sub-batches.
+static void f_host_batches(const Ctx* c, const FCall& a, double evals, double bytes_per_hyp, std::vector<int>& bounds) {
+    const int P = a.P;
+    f_pass_bounds(c, a, bounds);
+    const double r_ev = c->rate_evals_per_s > 0.0 ? c->rate_evals_per_s : 1.5e12;       // until measured: round-1 figures
+    const double r_up = c->rate_h2d_bytes_per_s > 0.0 ? c->rate_h2d_bytes_per_s : 5.0e10;
+    // how many extra passes are affordable: each costs ~0.1 ms of small kernels; spend at most 1 % of the call on them
+    const int levels = (int)std::min(5.0, std::floor(0.01 * (evals / r_ev) / 1.0e-4));
+    if (levels >= 2 && c->opt_host_slices == 0 && !c->opt_profile) {
+        // Large batch: nothing hides the upload of the FIRST pass (102 MB for 64 config-5 pairs: 2 ms at 55 GB/s, 17 ms
+        // when eight ranks share the host link), so the first pass is cut into sub-passes of doubling size — 1/2^levels of
+        // it first — each of which covers the upload of the next one.
+        const int p_end = bounds[1];
+        double first_evals = 0.0;
+        for (int p = 0; p < p_end; ++p) first_evals += pair_evals(a, p);
+        std::vector<int> nb;
+        nb.push_back(0);
+        double target = first_evals / (double)(1 << levels), acc = 0.0;
+        for (int p = 0; p < p_end; ++p) {
+            acc += pair_evals(a, p);
+            if (acc >= target && p + 1 < p_end) {
+                nb.push_back(p + 1);
+                acc = 0.0;
+                target *= 2.0;
+            }
+        }
+        for (size_t k = 1; k < bounds.size(); ++k) nb.push_back(bounds[k]);
+        bounds.swap(nb);
+    } else if (bounds.size() == 2 && P >= 2 && !c->opt_profile && c->opt_host_slices != 1) {
+        // a batch that fits one pass: the first sub-batch is the smallest whose scoring time covers the upload of the rest
+        int first = 1;
+        double score_s = 0.0;
+        auto rest_bytes = [&](int f) {
+            return 32.0 * (double)(a.pair_off[P] - a.pair_off[f]) + bytes_per_hyp * (double)(a.hyp_off[P] - a.hyp_off[f]);
+        };
+        for (first = 1; first < P; ++first) {
+            score_s += pair_evals(a, first - 1) / r_ev;
+            if (score_s >= rest_bytes(first) / r_up) break;
+        }
+        first = std::max(1, std::min(first, std::max(1, P / 2)));
+        double sc = 0.0;
+        for (int q = 0; q < first; ++q) sc += pair_evals(a, q) / r_ev;
+        const double hidden_s = std::min(sc, rest_bytes(first) / r_up);
+        int S = c->opt_host_slices > 0 ? c->opt_host_slices : (hidden_s > 1.5e-4 ? 2 : 1);     // a pass costs ~0.1 ms of small kernels
+        S = std::max(1, std::min(S, P));
+        if (S > 1) {
+            bounds.clear();
+            bounds.push_back(0);
+            for (int k = 1; k <= S; ++k) bounds.push_back(first + (int)((long long)(P - first) * (k - 1) / (S - 1)));
+        }
+    }
 }
 
 // sub-call of pairs [p0, p1) with offsets rebased to the pass
@@ -734,18 +747,45 @@ static FCall f_sub_call(const FCall& a, int p0, int p1, std::vector<int>& po, st
     return s;
 }
 
-// full pipeline on device pointers; asynchronous with respect to the host except for the PairInfo staging.  A call of several
-// passes is pipelined (f_run_piped, option 10); the caller's stream has joined every tail when this returns, i.e. it keeps
-// the stream semantics of a plain sequence of launches.
-// statistics of rg_f_last_bounded_stats: cleared at the start of a call (not between the sub-batches of a host call)
-static int bnd_stats_reset(Ctx* c, cudaStream_t st, bool bounded) {
-    int rc = ensure(c->bnd_stats, sizeof(unsigned long long) * 4);
-    if (rc) return rc;
-    RG_CUDA(cudaMemsetAsync(c->bnd_stats.ptr, 0, sizeof(unsigned long long) * 4, st));
-    c->bnd_host_evals = 0;
-    c->bnd_bound_evals = 0;
-    c->last_bounded = bounded;
-    return RG_OK;
+// Runs the passes of one F call (one job per pass, from f_sub_call) and owns the call's statistics (rg_get_last_stats,
+// rg_f_last_bounded_stats).  Several passes are pipelined (f_run_piped, option 10) unless a pass wants its per-hypothesis
+// results; otherwise they run one after the other on the caller's stream, so a single-pass call never swaps sets or
+// streams: it stays capturable in a CUDA graph and RG_FLAG_REUSE_POINTS finds its prepared points.  Asynchronous with
+// respect to the host except for the PairInfo staging; the caller's stream ends behind every pass, i.e. the call keeps the
+// stream semantics of a plain sequence of launches.
+// (Cutting the first / last pass into 1/8 .. 1/2 pieces to shorten the exposed head and tail was tried: the smaller passes
+// cost the scorer as much as they save — 512-pair sweep 126.96 -> 127.32 ms resident, full sweep end to end 987.1 -> 988.6
+// ms; profiles/r02_taper.txt.)
+static int f_run_passes(Ctx* c, cudaStream_t st, bool bounded, std::vector<PassCtl>& jobs) {
+    c->last_passes = (int)jobs.size();                // (the empty sub-batches of a host call count, and run nothing)
+    jobs.erase(std::remove_if(jobs.begin(), jobs.end(), [](const PassCtl& j) { return j.a.P == 0; }), jobs.end());
+    const bool piped = jobs.size() > 1 && c->opt_pipeline &&
+                       std::none_of(jobs.begin(), jobs.end(), [](const PassCtl& j) { return j.wants_hypotheses(); });
+    const size_t stats_bytes = sizeof(unsigned long long) * 8, bnd_bytes = sizeof(unsigned long long) * 4;
+    const int rc = [&]() -> int {
+        int r;
+        if ((r = ensure(c->stats, stats_bytes)) || (r = ensure_pinned(c->h_stats, stats_bytes)) ||
+            (r = ensure(c->bnd_stats, bnd_bytes)))
+            return r;
+        RG_CUDA(cudaMemsetAsync(c->stats.ptr, 0, stats_bytes, st));
+        RG_CUDA(cudaMemsetAsync(c->bnd_stats.ptr, 0, bnd_bytes, st));
+        c->bnd_host_evals = 0;
+        c->bnd_bound_evals = 0;
+        c->last_bounded = bounded;
+        c->last_stats[7] = 0;
+        if ((r = piped ? f_run_piped(c, st, jobs) : f_run_serial(c, st, jobs))) return r;
+        RG_CUDA(cudaMemcpyAsync(c->h_stats.ptr, c->stats.ptr, stats_bytes, cudaMemcpyDeviceToHost, st));
+        return RG_OK;
+    }();
+    if (rc) {                                         // leave nothing in flight behind an error return
+        cudaStreamSynchronize(st);
+        if (piped && c->tail_stream) cudaStreamSynchronize(c->tail_stream);
+        for (const PassCtl& j : jobs) {
+            if (j.ready) cudaEventSynchronize(j.ready);       // (the host entry point's uploads)
+            if (j.out_stream) cudaStreamSynchronize(j.out_stream);
+        }
+    }
+    return rc;
 }
 
 static int f_ransac_dev(Ctx* c, cudaStream_t st, const FCall& a_in) {
@@ -754,39 +794,13 @@ static int f_ransac_dev(Ctx* c, cudaStream_t st, const FCall& a_in) {
     FCall a = a_in;
     a.bounded = a.bounded && a.score_path == SCORE_FP32_GUARDED;      // (the FP64 path always scores everything)
     RG_CUDA(cudaSetDevice(c->device));
-    c->last_stats[7] = 0;
-    c->last_passes = 0;
-    if ((rc = ensure(c->stats, sizeof(unsigned long long) * 8))) return rc;
-    if ((rc = ensure_pinned(c->h_stats, sizeof(unsigned long long) * 8))) return rc;
-    if (!c->accumulate_stats) {
-        RG_CUDA(cudaMemsetAsync(c->stats.ptr, 0, sizeof(unsigned long long) * 8, st));
-        if ((rc = bnd_stats_reset(c, st, a.bounded))) return rc;
-    }
-    if (a.P == 0) return RG_OK;
-    std::vector<int> bounds, po, ho;
+    std::vector<int> bounds;
     f_pass_bounds(c, a, bounds);
-    const int n_pass = (int)bounds.size() - 1;
-    RG_CHECK_ARG(n_pass == 1 || !(a.flags & FLAG_REUSE_POINTS), "RG_FLAG_REUSE_POINTS needs a call that fits one pass");
-    if (n_pass > 1 && c->opt_pipeline) {
-        // (cutting the first / last pass into 1/8 .. 1/2 pieces to shorten the exposed head and tail was tried: the smaller
-        //  passes cost the scorer as much as they save — 512-pair sweep 126.96 -> 127.32 ms resident, full sweep end to end
-        //  987.1 -> 988.6 ms; profiles/r02_taper.txt)
-        std::vector<PassCtl> jobs(n_pass);
-        for (int k = 0; k < n_pass; ++k) jobs[k].a = f_sub_call(a, bounds[k], bounds[k + 1], jobs[k].po, jobs[k].ho);
-        if ((rc = a.bounded ? f_run_piped_bounded(c, st, jobs, true) : f_run_piped(c, st, jobs, true))) return rc;
-    } else {
-        for (int k = 0; k < n_pass; ++k) {
-            if (n_pass == 1) {
-                if ((rc = f_pass(c, st, a))) return rc;
-            } else {
-                FCall s = f_sub_call(a, bounds[k], bounds[k + 1], po, ho);
-                if ((rc = f_pass(c, st, s))) return rc;
-            }
-        }
-    }
-    c->last_passes = (int)bounds.size() - 1;
-    RG_CUDA(cudaMemcpyAsync(c->h_stats.ptr, c->stats.ptr, sizeof(unsigned long long) * 8, cudaMemcpyDeviceToHost, st));
-    return RG_OK;
+    const int n_pass = a.P > 0 ? (int)bounds.size() - 1 : 0;
+    RG_CHECK_ARG(n_pass <= 1 || !(a.flags & FLAG_REUSE_POINTS), "RG_FLAG_REUSE_POINTS needs a call that fits one pass");
+    std::vector<PassCtl> jobs(n_pass);
+    for (int k = 0; k < n_pass; ++k) jobs[k].a = f_sub_call(a, bounds[k], bounds[k + 1], jobs[k].po, jobs[k].ho);
+    return f_run_passes(c, st, a.bounded, jobs);
 }
 
 }  // namespace rg
@@ -965,12 +979,11 @@ int rg_f_last_bounded_evals(void* ctx, void* stream, long long* out2) {
     return RG_OK;
 }
 
-// Host-buffer entry point.  The pairs are processed in passes (f_pass_bounds; a batch that fits one pass is still cut in two
-// when that hides a worthwhile part of the upload: the first sub-batch is the smallest whose scoring time covers the upload
-// of the rest, both estimated with the rates MEASURED on this context by earlier calls).  All uploads are queued on a second
-// stream (one event per pass), the kernels of pass k wait only for their own inputs, so the upload of pass k+1 overlaps
-// the scoring of pass k (needs pinned host buffers to actually overlap; pageable ones are still correct).  Results are
-// identical to a single batch: pairs are independent.  idx == NULL: samples drawn on the device from sample_seed.
+// Host-buffer entry point.  The pairs are processed in sub-batches of one pass each (f_host_batches).  All uploads are
+// queued on a second stream (one event per sub-batch), the kernels of sub-batch k wait only for their own inputs, so the
+// upload of sub-batch k+1 overlaps the scoring of sub-batch k (needs pinned host buffers to actually overlap; pageable ones
+// are still correct).  Results are identical to a single batch: pairs are independent.  idx == NULL: samples drawn on the
+// device from sample_seed.
 int rg_f_ransac_host2(void* ctx, void* stream, int P, const double* pts64, const int* pair_off, const int* idx,
                       const int* hyp_off, double thr, int mode, int tie_mode, int solver, int score_path,
                       unsigned long long sample_seed, int first_pair_id, int* best_idx, int* best_count, double* best_F,
@@ -996,58 +1009,11 @@ int rg_f_ransac_host2(void* ctx, void* stream, int P, const double* pts64, const
     if ((rc = ensure(c->d_out_b, sizeof(double) * 9 * (size_t)P))) return rc;
     if (mask && (rc = ensure(c->d_out_c, std::max<size_t>(Ntot, 1)))) return rc;
 
-    std::vector<int> bounds;
-    f_pass_bounds(c, a, bounds);
-    const double r_ev = c->rate_evals_per_s > 0.0 ? c->rate_evals_per_s : 1.5e12;       // until measured: round-1 figures
-    const double r_up = c->rate_h2d_bytes_per_s > 0.0 ? c->rate_h2d_bytes_per_s : 5.0e10;
     const double bytes_per_hyp = seeded ? 0.0 : 32.0;
-    double total_evals = 0.0;
-    for (int p = 0; p < P; ++p) total_evals += (double)(pair_off[p + 1] - pair_off[p]) * (double)(hyp_off[p + 1] - hyp_off[p]);
-    // how many extra passes are affordable: each costs ~0.1 ms of small kernels; spend at most 1 % of the call on them
-    const int levels = (int)std::min(5.0, std::floor(0.01 * (total_evals / r_ev) / 1.0e-4));
-    if (levels >= 2 && c->opt_host_slices == 0 && !c->opt_profile) {
-        // Large batch: nothing hides the upload of the FIRST pass (102 MB for 64 config-5 pairs: 2 ms at 55 GB/s, 17 ms
-        // when eight ranks share the host link), so the first pass is cut into sub-passes of doubling size — 1/2^levels of
-        // it first — each of which covers the upload of the next one.
-        const int p_end = bounds[1];
-        double first_evals = 0.0;
-        for (int p = 0; p < p_end; ++p) first_evals += (double)(pair_off[p + 1] - pair_off[p]) * (double)(hyp_off[p + 1] - hyp_off[p]);
-        std::vector<int> nb;
-        nb.push_back(0);
-        double target = first_evals / (double)(1 << levels), acc = 0.0;
-        for (int p = 0; p < p_end; ++p) {
-            acc += (double)(pair_off[p + 1] - pair_off[p]) * (double)(hyp_off[p + 1] - hyp_off[p]);
-            if (acc >= target && p + 1 < p_end) {
-                nb.push_back(p + 1);
-                acc = 0.0;
-                target *= 2.0;
-            }
-        }
-        for (size_t k = 1; k < bounds.size(); ++k) nb.push_back(bounds[k]);
-        bounds.swap(nb);
-    } else if (bounds.size() == 2 && P >= 2 && !c->opt_profile && c->opt_host_slices != 1) {
-        int first = 1;
-        double score_s = 0.0;
-        auto rest_bytes = [&](int f) {
-            return 32.0 * (double)(pair_off[P] - pair_off[f]) + bytes_per_hyp * (double)(hyp_off[P] - hyp_off[f]);
-        };
-        for (first = 1; first < P; ++first) {
-            score_s += (double)(pair_off[first] - pair_off[first - 1]) * (double)(hyp_off[first] - hyp_off[first - 1]) / r_ev;
-            if (score_s >= rest_bytes(first) / r_up) break;
-        }
-        first = std::max(1, std::min(first, std::max(1, P / 2)));
-        double sc = 0.0;
-        for (int q = 0; q < first; ++q)
-            sc += (double)(pair_off[q + 1] - pair_off[q]) * (double)(hyp_off[q + 1] - hyp_off[q]) / r_ev;
-        const double hidden_s = std::min(sc, rest_bytes(first) / r_up);
-        int S = c->opt_host_slices > 0 ? c->opt_host_slices : (hidden_s > 1.5e-4 ? 2 : 1);     // a pass costs ~0.1 ms of small kernels
-        S = std::max(1, std::min(S, P));
-        if (S > 1) {
-            bounds.clear();
-            bounds.push_back(0);
-            for (int k = 1; k <= S; ++k) bounds.push_back(first + (int)((long long)(P - first) * (k - 1) / (S - 1)));
-        }
-    }
+    double evals = 0.0;
+    for (int p = 0; p < P; ++p) evals += pair_evals(a, p);
+    std::vector<int> bounds;
+    f_host_batches(c, a, evals, bytes_per_hyp, bounds);
     const int S = (int)bounds.size() - 1;
     if (!c->copy_stream) RG_CUDA(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
     if (!c->copy_gate) RG_CUDA(cudaEventCreateWithFlags(&c->copy_gate, cudaEventDisableTiming));
@@ -1061,9 +1027,6 @@ int rg_f_ransac_host2(void* ctx, void* stream, int P, const double* pts64, const
     // the inlier masks of pass k travel back on a third stream while pass k+1 is scored (205 MB for the config-5 sweep:
     // 3.7 ms at the end of the call otherwise)
     const bool stream_masks = mask != nullptr && S > 1;
-    // sub-batches pipelined with each other over two streams unless per-hypothesis results are copied out after every
-    // sub-batch (which needs that sub-batch finished anyway)
-    const bool piped = S > 1 && c->opt_pipeline && !(counts || F_all || flags);
     if (stream_masks) {
         if (!c->d2h_stream) RG_CUDA(cudaStreamCreateWithFlags(&c->d2h_stream, cudaStreamNonBlocking));
         if (!c->d2h_done) RG_CUDA(cudaEventCreateWithFlags(&c->d2h_done, cudaEventDisableTiming));
@@ -1096,82 +1059,24 @@ int rg_f_ransac_host2(void* ctx, void* stream, int P, const double* pts64, const
     a.pts64 = d_pts; a.idx = d_ix;
     a.best_idx = d_idx; a.best_count = d_cnt; a.best_F = (double*)c->d_out_b.ptr;
     a.mask = mask ? (unsigned char*)c->d_out_c.ptr : nullptr;
-    std::vector<int> po, ho;
-    rc = RG_OK;
-    long long launches = 0;
-    if (piped) {
-        // every sub-batch is one pass (the bounds come from f_pass_bounds and were only refined); the passes are pipelined
-        // over two streams (f_run_piped): heads wait for their own upload, mask downloads hang on the tails
-        std::vector<PassCtl> jobs;
-        jobs.reserve(S);
-        for (int k = 0; k < S; ++k) {
-            if (bounds[k + 1] == bounds[k]) continue;
-            jobs.emplace_back();
-            PassCtl& j = jobs.back();
-            j.a = f_sub_call(a, bounds[k], bounds[k + 1], j.po, j.ho);
-            j.ready = c->pass_ready[k];
-            if (stream_masks) {
-                const size_t n0 = (size_t)pair_off[bounds[k]], n1 = (size_t)pair_off[bounds[k + 1]];
-                j.done = c->pass_done[k];
-                j.out_stream = c->d2h_stream;
-                j.out_dst = mask + n0; j.out_src = (const unsigned char*)c->d_out_c.ptr + n0; j.out_bytes = n1 - n0;
-            }
-        }
-        c->last_stats[7] = 0;
-        if ((rc = ensure(c->stats, sizeof(unsigned long long) * 8))) return rc;
-        if ((rc = ensure_pinned(c->h_stats, sizeof(unsigned long long) * 8))) return rc;
-        RG_CUDA(cudaMemsetAsync(c->stats.ptr, 0, sizeof(unsigned long long) * 8, st));
-        if ((rc = bnd_stats_reset(c, st, a.bounded))) return rc;
-        rc = a.bounded ? f_run_piped_bounded(c, st, jobs, false) : f_run_piped(c, st, jobs, false);
-        launches = c->last_stats[7];
-    }
-    for (int k = 0; k < S && rc == RG_OK && !piped; ++k) {
+    // one job per sub-batch: its head waits for its own upload, its mask download hangs on its tail
+    std::vector<PassCtl> jobs(S);
+    for (int k = 0; k < S; ++k) {
+        PassCtl& j = jobs[k];
         const int p0 = bounds[k], p1 = bounds[k + 1];
-        if (p1 == p0) continue;
-        const size_t h0 = (size_t)hyp_off[p0];
-        if (S > 1) RG_CUDA(cudaStreamWaitEvent(st, c->pass_ready[k], 0));
-        c->accumulate_stats = k > 0;
-        if (S == 1) {
-            rc = f_ransac_dev(c, st, a);
-        } else {
-            FCall s = f_sub_call(a, p0, p1, po, ho);
-            rc = f_ransac_dev(c, st, s);
-        }
-        c->accumulate_stats = false;
-        launches += c->last_stats[7];
-        if (rc) break;
-        // per-hypothesis results live in per-pass workspaces: fetch them before the next pass overwrites them
-        const size_t Hk = (size_t)hyp_off[p1] - h0;
-        if ((counts || F_all || flags) && c->last_passes > 1) {
-            set_error("invalid argument: per-hypothesis outputs need sub-batches that fit one pass");
-            rc = RG_ERR_ARG;
-            break;
-        }
-        if (counts && Hk) RG_CUDA(cudaMemcpyAsync(counts + h0, c->counts_ptr, sizeof(int) * Hk, cudaMemcpyDeviceToHost, st));
-        if (F_all && Hk) RG_CUDA(cudaMemcpyAsync(F_all + 9 * h0, c->F64.ptr, sizeof(double) * 9 * Hk, cudaMemcpyDeviceToHost, st));
-        if (flags && Hk) RG_CUDA(cudaMemcpyAsync(flags + h0, c->flags.ptr, Hk, cudaMemcpyDeviceToHost, st));
+        const size_t n0 = (size_t)pair_off[p0], h0 = (size_t)hyp_off[p0];
+        j.a = f_sub_call(a, p0, p1, j.po, j.ho);
+        if (S > 1) j.ready = c->pass_ready[k];
         if (stream_masks) {
-            const size_t n0 = (size_t)pair_off[p0], n1 = (size_t)pair_off[p1];
-            RG_CUDA(cudaEventRecord(c->pass_done[k], st));
-            RG_CUDA(cudaStreamWaitEvent(c->d2h_stream, c->pass_done[k], 0));
-            if (n1 > n0)
-                RG_CUDA(cudaMemcpyAsync(mask + n0, (unsigned char*)c->d_out_c.ptr + n0, n1 - n0, cudaMemcpyDeviceToHost, c->d2h_stream));
+            j.done = c->pass_done[k];
+            j.out_stream = c->d2h_stream;
+            j.out_dst = mask + n0; j.out_src = a.mask + n0; j.out_bytes = (size_t)pair_off[p1] - n0;
         }
+        if (counts) j.out_counts = counts + h0;
+        if (F_all) j.out_F_all = F_all + 9 * h0;
+        if (flags) j.out_flags = flags + h0;
     }
-    c->last_stats[7] = launches;
-    c->last_passes = S;
-    if (rc) {
-        cudaStreamSynchronize(st);
-        if (S > 1) cudaStreamSynchronize(cs);
-        if (c->tail_stream) cudaStreamSynchronize(c->tail_stream);
-        c->tail_pending[0] = c->tail_pending[1] = false;
-        if (stream_masks) cudaStreamSynchronize(c->d2h_stream);
-        return rc;
-    }
-    if (piped) {                                      // join the last tail, then the statistics are final
-        if ((rc = pipe_join(c, st))) return rc;
-        RG_CUDA(cudaMemcpyAsync(c->h_stats.ptr, c->stats.ptr, sizeof(unsigned long long) * 8, cudaMemcpyDeviceToHost, st));
-    }
+    if ((rc = f_run_passes(c, st, a.bounded, jobs))) return rc;
     if (stream_masks) {                               // the caller's stream also waits for the mask downloads
         RG_CUDA(cudaEventRecord(c->d2h_done, c->d2h_stream));
         RG_CUDA(cudaStreamWaitEvent(st, c->d2h_done, 0));
@@ -1185,8 +1090,6 @@ int rg_f_ransac_host2(void* ctx, void* stream, int P, const double* pts64, const
     {   // measured rates for the next call's sub-batch model (exponential average; uploads of < 1 MB say nothing)
         float ms_up = 0.f, ms_run = 0.f;
         const double up_bytes = 32.0 * (double)Ntot + bytes_per_hyp * (double)Htot;
-        double evals = 0.0;
-        for (int p = 0; p < P; ++p) evals += (double)(pair_off[p + 1] - pair_off[p]) * (double)(hyp_off[p + 1] - hyp_off[p]);
         if (cudaEventElapsedTime(&ms_up, c->rate_ev[0], c->rate_ev[1]) == cudaSuccess && ms_up > 0.f && up_bytes > 1e6) {
             const double r = up_bytes / (ms_up * 1e-3);
             c->rate_h2d_bytes_per_s = c->rate_h2d_bytes_per_s > 0.0 ? 0.75 * c->rate_h2d_bytes_per_s + 0.25 * r : r;
@@ -1232,7 +1135,7 @@ int rg_epi_score_count_host(void* ctx, void* stream, int N, const double* pts64,
     int bps = 1, rc = score_blocks_per_sm<EpiPolicy<MODE_EPI_MAX>>(&bps);
     if (rc) return rc;
     if ((rc = f_plan(c, st, 1, pair_off, hyp_off, plan, bps))) return rc;
-    if ((rc = f_workspace(c, plan, false))) return rc;
+    if ((rc = f_workspace(c, plan))) return rc;
     ScoreState s;
     if ((rc = score_state_layout(c, 1, H, 8, s))) return rc;
     if ((rc = ensure(c->d_in_a, sizeof(double) * 4 * std::max<size_t>((size_t)N, 1)))) return rc;
@@ -1276,7 +1179,7 @@ int rg_f8pt_solve_host(void* ctx, void* stream, int N, const double* pts64, int 
     int bps = 1, rc = score_blocks_per_sm<EpiPolicy<MODE_EPI_MAX>>(&bps);
     if (rc) return rc;
     if ((rc = f_plan(c, st, 1, pair_off, hyp_off, plan, bps))) return rc;
-    if ((rc = f_workspace(c, plan, false))) return rc;
+    if ((rc = f_workspace(c, plan))) return rc;
     ScoreState s;
     if ((rc = score_state_layout(c, 1, H, 8, s))) return rc;
     if ((rc = ensure(c->d_in_a, sizeof(double) * 4 * (size_t)N))) return rc;
