@@ -78,7 +78,11 @@ int rg_host_free(void* p);
  * option 15 = prefix stage of the bounded sweep: 1 (default) = bound-only FP32 scorer (counts r^2 < T, an upper bound on
  *            every hypothesis's prefix count, with no guard-band fix-up; the K candidates are then scored over the whole
  *            pair), 0 = guarded scorer + FP64 fix-up (exact prefix counts; the candidates are scored on the rest of the
- *            pair); results do not depend on it (DESIGN.md section 4) */
+ *            pair); results do not depend on it (DESIGN.md section 4)
+ * option 16 = share rho0 of the bound-only prefix's first stage in thousandths, [1, 1000] (default 380): every hypothesis
+ *            is scored on the first rho0 of its pair, the candidates are chosen there, and only the hypotheses that
+ *            share cannot yet rule out are extended to rho; rho0 >= rho (or option 15 = 0) is a one-stage prefix;
+ *            results do not depend on it */
 int rg_set_option(void* ctx, int option, long long value);
 /* summed milliseconds of {prepare, solve, score kernel, fixup + repair, select} over the PASSES since the last read
  * (at most 2048 passes are remembered; *out_calls = passes covered); synchronises `stream` */
@@ -146,7 +150,8 @@ int rg_f_last_hypotheses_dev(void* ctx, const int32_t** counts_dev, const double
  * unable to reach their pair's maximum), pairs that fell back to scoring every hypothesis in full, K (0: full sweep)}.
  * Synchronises `stream`. */
 int rg_f_last_bounded_stats(void* ctx, void* stream, long long* out4);
-/* the evaluations of the last F call split by scorer: out2 = {bound-only prefix stages (option 15 = 1), guarded scorer
+/* the evaluations of the last F call split by scorer: out2 = {bound-only prefix stages (option 15 = 1; both stages of
+ * option 16, the second counted on the device), guarded scorer
  * (exact prefix, candidate and fallback stages, or the full sweep)}; out2[0] + out2[1] = out4[0] above.
  * Synchronises `stream`. */
 int rg_f_last_bounded_evals(void* ctx, void* stream, long long* out2);

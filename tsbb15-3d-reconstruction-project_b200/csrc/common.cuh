@@ -177,13 +177,16 @@ struct FPlan {
     long long Ntot = 0, Htot = 0, N32tot = 0;
     int n_items = 0;
     int maxN = 0, maxH = 0;
-    double evals = 0.0;                  // sum_p n_p * H_p (bounded sweep: of the prefix stage)
-    // bounded sweep (bounded.cuh): three tables per pass, [prefix stage | candidate stage | fallback template]
+    double evals = 0.0;                  // sum_p n_p * H_p (bounded sweep: of prefix stage A)
+    // bounded sweep (bounded.cuh): four tables per pass, [prefix stage A | candidate stage | fallback template |
+    // stage-B template]
     bool bounded = false;
     bool bound_prefix = false;           // the prefix stage counts an upper bound (EpiBoundPolicy); later stages cover [0, G)
     int K = 0;                           // candidates per pair
     long long Ctot = 0;                  // candidates of the pass (sum_p min(K, H_p))
+    long long Btot = 0;                  // room for stage B's records (sum_p H_p - min(K, H_p))
     int n_items_c = 0, n_items_f = 0;    // scorer items of the candidate stage / of the fallback with every pair marked
+    int n_items_b = 0;                   // scorer items of stage B with every non-candidate live (0: one-step prefix)
     double evals_c = 0.0, evals_f = 0.0; // their evaluations (real correspondences)
 };
 
@@ -228,10 +231,12 @@ struct Ctx {
     int opt_rho_milli = 450;                       // option 13: prefix share rho of the bounded sweep, in thousandths
     int opt_bounded_k = 512;                       // option 14: candidates per pair of the bounded sweep
     int opt_bound_prefix = 1;                      // option 15: 1 = bound-only prefix stage, 0 = exact (guarded + fix-up) prefix
+    int opt_rho0_milli = 380;                      // option 16: share rho0 of the bound-only prefix stage A, in thousandths
     bool last_bounded = false;                     // the last F call ran the bounded sweep (its counts are not full counts)
     long long bnd_host_evals = 0;                  // guarded-scorer evaluations of its prefix and candidate stages (known on the host)
-    long long bnd_bound_evals = 0;                 // evaluations of its bound-only prefix stages (option 15 = 1)
-    Buffer bnd_stats;                              // device: [0] fallback evaluations, [1] hypotheses not fully scored, [2] fallback pairs
+    long long bnd_bound_evals = 0;                 // evaluations of its bound-only prefix stages A (option 15 = 1)
+    Buffer bnd_stats;                              // device: [0] fallback evaluations, [1] hypotheses not fully scored, [2] fallback pairs,
+                                                   // [3] evaluations of the bound-only prefix stages B
     // peer-to-peer argmax exchange (hypothesis-split mode over NVLink), see p2p_api.cu
     void* p2p_local = nullptr; size_t p2p_bytes = 0; int p2p_rank = 0, p2p_world = 0; unsigned p2p_seq = 0;
     void* p2p_peer[16] = {nullptr};
@@ -275,8 +280,9 @@ struct Ctx {
     int opt_profile = 0;
     static constexpr int kProfPhases = 5;          // prepare, solve, score kernel, fixup+repair, select
     static constexpr int kProfScoreStart = 6;      // extra boundary: the scorer's own start (pipelined passes: the solver ended long before)
-    static constexpr int kProfSweep = 7;           // bounded sweep: boundaries 7/8 around the candidate stage's scorer, 9/10 the fallback's
-    static constexpr int kProfEvents = 11;         // boundaries 0..5 + the scorer start + the two later scorer launches
+    static constexpr int kProfSweep = 7;           // bounded sweep: boundaries 7/8 around the candidate stage's scorer, 9/10 stage B's,
+                                                   // 11/12 the fallback's
+    static constexpr int kProfEvents = 13;         // boundaries 0..5 + the scorer start + the three later scorer launches
     static constexpr int kProfRing = 2048;         // passes remembered between two reads (20 steps of a tapered 64-pass sweep)
     cudaEvent_t* prof_ev = nullptr;                // kProfRing * kProfEvents events
     int prof_cur = -1;                             // pass opened by the last prof_mark(.., 0) (sequential callers)

@@ -286,6 +286,11 @@ int rg_set_option(void* ctx, int option, long long value) {
         c->opt_bound_prefix = (int)value;
         return RG_OK;
     }
+    if (option == 16) {
+        if (value < 1 || value > 1000) { set_error("invalid argument: option 16 (stage-A prefix share x 1000) must be in [1, 1000]"); return RG_ERR_ARG; }
+        c->opt_rho0_milli = (int)value;
+        return RG_OK;
+    }
     if (option == 8) {
         if (value < 0 || value > 1000000000ll) { set_error("invalid argument: option 8 (flag list capacity) must be in [0, 1e9]"); return RG_ERR_ARG; }
         c->opt_list_cap = value;
@@ -297,8 +302,8 @@ int rg_set_option(void* ctx, int option, long long value) {
 
 // Phase times of the calls made since profiling was switched on / last read (option 1): out_ms[0..4] = summed
 // milliseconds of {prepare, solve, score kernel, fixup + repair, select}, *out_calls = number of calls covered.
-// A pass of the bounded sweep has three scorer launches: its score phase is their sum; its fixup phase runs from the end of
-// the prefix stage to the chosen candidates, and its select phase from there to the end of its tail.
+// A pass of the bounded sweep has three or four scorer launches: its score phase is their sum; its fixup phase runs from the
+// end of prefix stage A to the chosen candidates, and its select phase from there to the end of its tail.
 // Synchronises the stream; resets the ring.
 int rg_get_profile(void* ctx, void* stream, double* out_ms5, int* out_calls) {
     RG_CHECK_ARG(ctx != nullptr && out_ms5 != nullptr && out_calls != nullptr, "null argument");

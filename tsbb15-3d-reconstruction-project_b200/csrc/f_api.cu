@@ -5,9 +5,9 @@
 //   -> [f_tie_stats -> f_tie_resolve] -> f_mask
 // over a contiguous block of pairs whose workspaces (hypotheses, FP32 points, flag list) stay bounded; BASELINE config 5
 // (4096 pairs x 50 000 x 8 192) runs as 64 passes of 64 pairs.  A call that wants no per-hypothesis counts runs the bounded
-// sweep instead of score_packed -> fixup_list (bounded.cuh): bound-only prefix stage, candidates, candidate stage, check,
-// fallback.  The per-pass PairInfo table is planned on the host into
-// double-buffered pinned staging, so the host plans pass k+1 while pass k runs.
+// sweep instead of score_packed -> fixup_list (bounded.cuh): bound-only prefix stage A, candidates, candidate stage,
+// extension of the prefix for the hypotheses still alive (stage B), check, fallback.  The per-pass PairInfo table is
+// planned on the host into double-buffered pinned staging, so the host plans pass k+1 while pass k runs.
 #include "f_kernels.cuh"
 #include "bounded.cuh"
 #include "jacobi.cuh"
@@ -27,22 +27,26 @@ struct ScoreState {
     unsigned* bbox; int* counts; int* work; unsigned* list_n; unsigned char* ovf;
     size_t off_counts, bytes;
     // bounded sweep (Ctot >= 0): work counters / list sizes of the candidate (c) and fallback (f) stages, the fallback's
-    // item count, suffix counts, marks of the pairs that fell back, overflow marks
+    // item count, suffix counts, marks of the pairs that fell back, overflow marks; stage B's work counter, item count,
+    // counts (compact, as its records) and |S| per pair
     int *c_work, *f_work, *f_items, *sfx_c, *sfx_f, *mark;
+    int *b_work, *b_items, *cnt_b, *n_s;
     unsigned *c_list_n, *f_list_n;
     unsigned char *ovf_c, *ovf_f;
 };
 
 // [bbox keys: P x words][counts: H][work counter][list size][pad][ovf: H bytes]
-//   + bounded sweep: [8 counters][sfx_c: C][sfx_f: H][mark: P][ovf_c: C bytes][ovf_f: H bytes]
+//   + bounded sweep: [8 counters][sfx_c: C][sfx_f: H][mark: P][cnt_b: B][n_s: P][ovf_c: C bytes][ovf_f: H bytes]
 // — one cudaMemsetAsync clears a pass's state
-int score_state_layout(Ctx* c, int P, long long Htot, int bbox_words, ScoreState& s, long long Ctot = -1) {
+int score_state_layout(Ctx* c, int P, long long Htot, int bbox_words, ScoreState& s, long long Ctot = -1,
+                       long long Btot = 0) {
     const size_t H = (size_t)std::max<long long>(Htot, 1);
     const size_t bbox_bytes = (((size_t)std::max(P, 1) * bbox_words * 4) + 15) / 16 * 16;
     const size_t cnt_bytes = ((H + 2) * 4 + 15) / 16 * 16;
     const size_t ovf_bytes = (H + 15) / 16 * 16;
     const size_t C = (size_t)std::max<long long>(Ctot, 1);
-    const size_t bnd_ints = Ctot >= 0 ? ((8 + C + H + (size_t)std::max(P, 1)) * 4 + 15) / 16 * 16 : 0;
+    const size_t B = (size_t)std::max<long long>(Btot, 1), P1 = (size_t)std::max(P, 1);
+    const size_t bnd_ints = Ctot >= 0 ? ((8 + C + H + P1 + B + P1) * 4 + 15) / 16 * 16 : 0;
     const size_t bnd_ovf = Ctot >= 0 ? (C + H + 15) / 16 * 16 : 0;
     s.off_counts = bbox_bytes;
     s.bytes = bbox_bytes + cnt_bytes + ovf_bytes + bnd_ints + bnd_ovf;
@@ -57,7 +61,8 @@ int score_state_layout(Ctx* c, int P, long long Htot, int bbox_words, ScoreState
     if (Ctot >= 0) {
         int* b = (int*)(base + bbox_bytes + cnt_bytes + ovf_bytes);
         s.c_work = b; s.c_list_n = (unsigned*)(b + 1); s.f_work = b + 2; s.f_list_n = (unsigned*)(b + 3); s.f_items = b + 4;
-        s.sfx_c = b + 8; s.sfx_f = s.sfx_c + C; s.mark = s.sfx_f + H;
+        s.b_work = b + 5; s.b_items = b + 6;
+        s.sfx_c = b + 8; s.sfx_f = s.sfx_c + C; s.mark = s.sfx_f + H; s.cnt_b = s.mark + P1; s.n_s = s.cnt_b + B;
         s.ovf_c = (unsigned char*)(base + bbox_bytes + cnt_bytes + ovf_bytes + bnd_ints);
         s.ovf_f = s.ovf_c + C;
     }
@@ -67,14 +72,19 @@ int score_state_layout(Ctx* c, int P, long long Htot, int bbox_words, ScoreState
 }
 
 // per-set workspace of the bounded sweep: [compact Hyp32 records: C][map: C][sel: P int4][live fallback table: P]
-struct BndWs { Hyp32* hypc; int* map; int4* sel; PairInfo* fb; };
+//   [stage B's compact Hyp32 records: B][its map: B][live stage-B table: P]
+struct BndWs { Hyp32* hypc; int* map; int4* sel; PairInfo* fb; Hyp32* hypb; int* mapb; PairInfo* bt; };
 static int bnd_workspace(Ctx* c, const FPlan& plan, BndWs& w) {
     const size_t C = (size_t)std::max<long long>(plan.Ctot, 1), P = (size_t)std::max(plan.P, 1);
+    const size_t B = (size_t)std::max<long long>(plan.Btot, 1);
     const size_t o_map = C * sizeof(Hyp32), o_sel = o_map + (C * 4 + 63) / 64 * 64, o_fb = o_sel + P * sizeof(int4);
-    int rc = ensure(c->bnd, o_fb + P * sizeof(PairInfo));
+    const size_t o_hypb = o_fb + P * sizeof(PairInfo), o_mapb = o_hypb + B * sizeof(Hyp32);
+    const size_t o_bt = o_mapb + (B * 4 + 63) / 64 * 64;
+    int rc = ensure(c->bnd, o_bt + P * sizeof(PairInfo));
     if (rc) return rc;
     char* b = (char*)c->bnd.ptr;
     w.hypc = (Hyp32*)b; w.map = (int*)(b + o_map); w.sel = (int4*)(b + o_sel); w.fb = (PairInfo*)(b + o_fb);
+    w.hypb = (Hyp32*)(b + o_hypb); w.mapb = (int*)(b + o_mapb); w.bt = (PairInfo*)(b + o_bt);
     return RG_OK;
 }
 
@@ -148,7 +158,8 @@ static int tail_carveout(Ctx* c, bool want_max) {
     RG_CUDA(cudaFuncSetAttribute(f_tie_resolve, cudaFuncAttributePreferredSharedMemoryCarveout, v));
     RG_CUDA(cudaFuncSetAttribute(f8_solve_qr<MODE_EPI_MAX>, cudaFuncAttributePreferredSharedMemoryCarveout, v));
     RG_CUDA(cudaFuncSetAttribute(f8_solve_qr<MODE_SAMPSON>, cudaFuncAttributePreferredSharedMemoryCarveout, v));
-    for (const void* f : {(const void*)bnd_select, (const void*)bnd_check, (const void*)bnd_fb_plan, (const void*)bnd_merge})
+    for (const void* f : {(const void*)bnd_select, (const void*)bnd_extend, (const void*)bnd_check, (const void*)bnd_live_plan,
+                          (const void*)bnd_merge})
         RG_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, v));
     c->tail_carve_max = (int)want_max;
     return RG_OK;
@@ -345,36 +356,52 @@ static int f_bnd_cands(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) 
     return RG_OK;
 }
 
-// bounded sweep, after the candidates: candidate stage + its fix-up, check, fallback stage (queued at full grid, its
-// item count comes from bnd_fb_plan: normally zero).  The fallback's fix-up and merge belong to the tail.
+// bounded sweep, after the candidates: candidate stage + its fix-up, extension (bnd_extend, stage B), check, fallback
+// stage.  Stage B and the fallback are queued at full grid with their item counts read from the device (bnd_live_plan;
+// the fallback normally has none).  The fallback's fix-up and merge belong to the tail.
 template <int MODE>
 static int f_bnd_sweep(Ctx* c, cudaStream_t st, PassCtl& k) {
     if (!k.scored) return RG_OK;
     const FPlan& plan = k.plan;
     const PairInfo* pi = (const PairInfo*)c->pair_info.ptr;
-    int bps = 1, rc = score_blocks_per_sm<EpiPolicy<MODE>>(&bps);
-    if (rc) return rc;
+    const PairInfo *pc = pi + plan.P, *pf = pi + 2 * (size_t)plan.P, *pb = pi + 3 * (size_t)plan.P;
+    unsigned long long* bstats = (unsigned long long*)c->bnd_stats.ptr;
+    int bps = 1, bps_b = 1, rc = score_blocks_per_sm<EpiPolicy<MODE>>(&bps);
+    if (rc || (rc = score_blocks_per_sm<EpiBoundPolicy>(&bps_b))) return rc;
     constexpr size_t smem = score_smem_bytes<EpiPolicy<MODE>>();
     prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep);
     if (plan.n_items_c > 0) {
         score_packed<EpiPolicy<MODE>><<<std::min(plan.n_items_c, c->sm_count * bps), kScoreThreads, smem, st>>>(
-            (const float4*)c->pts32.ptr, k.bw.hypc, pi + plan.P, plan.P, plan.n_items_c, k.s.sfx_c, k.flc, k.s.c_work);
+            (const float4*)c->pts32.ptr, k.bw.hypc, pc, plan.P, plan.n_items_c, k.s.sfx_c, k.flc, k.s.c_work);
         c->last_stats[7] += 1;
     }
     prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 1);
     if (plan.n_items_c > 0 && (rc = f_fixup_launch<MODE>(c, st, k, false, STAGE_CAND))) return rc;
-    bnd_check<<<plan.P, 256, 0, st>>>(k.s.counts, k.s.sfx_c, k.bw.map, pi, pi + plan.P, k.bw.sel, k.s.mark,
-                                      (unsigned long long*)c->bnd_stats.ptr, !plan.bound_prefix);
-    bnd_fb_plan<<<1, kSelectThreads, 0, st>>>(pi + 2 * (size_t)plan.P, k.s.mark, plan.P, k.bw.fb, k.s.f_items);
+    bnd_extend<<<plan.P, 256, 0, st>>>(k.s.counts, k.s.sfx_c, k.bw.map, pi, pc, pb, (const Hyp32*)c->hyp32.ptr, k.bw.sel,
+                                       k.bw.hypb, k.bw.mapb, k.s.n_s, k.s.mark, bstats,
+                                       !plan.bound_prefix);
+    c->last_stats[7] += 1;
+    if (plan.n_items_b > 0) {
+        bnd_live_plan<<<1, kSelectThreads, 0, st>>>(pb, k.s.n_s, plan.P, k.bw.bt, k.s.b_items);
+        prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 2);
+        score_packed<EpiBoundPolicy><<<std::min(plan.n_items_b, c->sm_count * bps_b), kScoreThreads,
+                                       score_smem_bytes<EpiBoundPolicy>(), st>>>(
+            (const float4*)c->pts32.ptr, k.bw.hypb, k.bw.bt, plan.P, plan.n_items_b, k.s.cnt_b, k.fl, k.s.b_work, k.s.b_items);
+        prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 3);
+        c->last_stats[7] += 2;
+    }
+    bnd_check<<<plan.P, 256, 0, st>>>(k.s.counts, k.s.sfx_c, k.bw.map, k.s.cnt_b, k.bw.mapb, k.s.n_s, pi, pc, pb, k.bw.sel,
+                                      k.s.mark, bstats, !plan.bound_prefix);
+    bnd_live_plan<<<1, kSelectThreads, 0, st>>>(pf, k.s.mark, plan.P, k.bw.fb, k.s.f_items);
     c->last_stats[7] += 2;
-    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 2);
+    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 4);
     if (plan.n_items_f > 0) {
         score_packed<EpiPolicy<MODE>><<<std::min(plan.n_items_f, c->sm_count * bps), kScoreThreads, smem, st>>>(
             (const float4*)c->pts32.ptr, (const Hyp32*)c->hyp32.ptr, k.bw.fb, plan.P, plan.n_items_f, k.s.sfx_f, k.flf,
             k.s.f_work, k.s.f_items);
         c->last_stats[7] += 1;
     }
-    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 3);
+    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 5);
     RG_CUDA(cudaGetLastError());
     return RG_OK;
 }
@@ -432,14 +459,14 @@ static int f_pass_head(Ctx* c, cudaStream_t hs, PassCtl& k) {
     int bps = 1, rc = score_blocks_per_sm<EpiPolicy<MODE_EPI_MAX>>(&bps);
     if (rc) return rc;
     if ((rc = f_plan(c, hs, a.P, a.pair_off, a.hyp_off, plan, bps, nullptr, a.hyp_first, a.bounded ? c->opt_bounded_k : 0,
-                     c->opt_rho_milli, a.bounded && c->opt_bound_prefix != 0)))
+                     c->opt_rho_milli, a.bounded && c->opt_bound_prefix != 0, c->opt_rho0_milli)))
         return rc;
     for (int p = 0; p < a.P; ++p) {
         const int n = a.pair_off[p + 1] - a.pair_off[p], H = a.hyp_off[p + 1] - a.hyp_off[p];
         RG_CHECK_ARG(H == 0 || n >= 8, "a pair with hypotheses needs at least 8 correspondences");
     }
     if ((rc = f_workspace(c, plan))) return rc;
-    if ((rc = score_state_layout(c, a.P, plan.Htot, 8, k.s, a.bounded ? plan.Ctot : -1))) return rc;
+    if ((rc = score_state_layout(c, a.P, plan.Htot, 8, k.s, a.bounded ? plan.Ctot : -1, plan.Btot))) return rc;
     if (a.bounded && (rc = bnd_workspace(c, plan, k.bw))) return rc;
     if (plan.bound_prefix) {
         c->bnd_bound_evals += (long long)plan.evals;
@@ -555,9 +582,11 @@ static int f_run_serial(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs) {
 //   caller's stream :  S1(0)          S1(1)  S3+FB(0)          S1(2)  S3+FB(1)          S1(3) ...  S3+FB(n-1)        join
 //   side stream     :  head(0) head(1)  cands(0) head(2)  cands(1) tail(0) head(3)  cands(2) tail(1) head(4) ...  tail(n-1)
 //
-// S1 = prefix stage, cands = its fix-up + bnd_select, S3+FB = candidate stage, its fix-up, bnd_check, bnd_fb_plan and the
-// fallback stage, tail = fallback fix-up, bnd_merge, selection, masks.  The caller's stream only waits between S3 and FB for
-// the candidate stage's fix-up and the check (two small launches); everything else on the side stream runs beside a scorer.
+// S1 = prefix stage A, cands = its fix-up + bnd_select, S3+FB = candidate stage, its fix-up, bnd_extend, bnd_live_plan,
+// prefix stage B, bnd_check, bnd_live_plan and the fallback stage, tail = fallback fix-up, bnd_merge, selection, masks.
+// The caller's stream only waits between S3 and FB for the candidate stage's fix-up, bnd_extend, the two table kernels
+// and bnd_check (small one-CTA-per-pair launches; stage B itself is a short full-grid scorer of a few hundred hypotheses
+// per pair); everything else on the side stream runs beside a scorer.
 // head(k+3) reuses pass k's set and is queued behind tail(k) on the side stream.
 //
 // Either way the caller's stream ends behind the last tail (join), and the current set is the last pass's (counts_ptr / F64 /
@@ -952,30 +981,37 @@ int rg_get_last_stats(void* ctx, void* stream, long long* out8) {
 // out[0] hypothesis x correspondence evaluations the last F call executed, [1] hypotheses it did not score in full (proved
 // unable to reach their pair's maximum), [2] pairs whose bound failed and that were scored in full, [3] candidates per pair
 // (0: the call ran the full sweep).  Synchronises the stream.
+static int bnd_stats_read(Ctx* c, void* stream, unsigned long long (&d)[4]) {
+    RG_CUDA(cudaSetDevice(c->device));
+    RG_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
+    if (c->bnd_stats.ptr) RG_CUDA(cudaMemcpy(d, c->bnd_stats.ptr, sizeof(d), cudaMemcpyDeviceToHost));
+    return RG_OK;
+}
+
 int rg_f_last_bounded_stats(void* ctx, void* stream, long long* out4) {
     RG_CHECK_ARG(ctx != nullptr && out4 != nullptr, "null argument");
     Ctx* c = (Ctx*)ctx;
-    RG_CUDA(cudaSetDevice(c->device));
-    RG_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
     unsigned long long d[4] = {0, 0, 0, 0};
-    if (c->bnd_stats.ptr) RG_CUDA(cudaMemcpy(d, c->bnd_stats.ptr, sizeof(d), cudaMemcpyDeviceToHost));
-    out4[0] = c->bnd_bound_evals + c->bnd_host_evals + (long long)d[0];
+    int rc = bnd_stats_read(c, stream, d);
+    if (rc) return rc;
+    out4[0] = c->bnd_bound_evals + (long long)d[3] + c->bnd_host_evals + (long long)d[0];
     out4[1] = (long long)d[1];
     out4[2] = (long long)d[2];
     out4[3] = c->last_bounded ? c->opt_bounded_k : 0;
     return RG_OK;
 }
 
-// out[0] evaluations of the last F call's bound-only prefix stages (upper-bound counts), [1] evaluations of its guarded
-// scorer (exact prefix, candidate and fallback stages, or the full sweep); their sum is out4[0] of rg_f_last_bounded_stats.
-// Synchronises the stream.
+// out[0] evaluations of the last F call's bound-only prefix stages A and B (upper-bound counts; stage B's depend on the
+// data and are counted on the device), [1] evaluations of its guarded scorer (exact prefix, candidate and fallback stages,
+// or the full sweep); their sum is out4[0] of rg_f_last_bounded_stats.  Synchronises the stream.
 int rg_f_last_bounded_evals(void* ctx, void* stream, long long* out2) {
     RG_CHECK_ARG(ctx != nullptr && out2 != nullptr, "null argument");
-    long long s[4];
-    int rc = rg_f_last_bounded_stats(ctx, stream, s);
+    Ctx* c = (Ctx*)ctx;
+    unsigned long long d[4] = {0, 0, 0, 0};
+    int rc = bnd_stats_read(c, stream, d);
     if (rc) return rc;
-    out2[0] = ((Ctx*)ctx)->bnd_bound_evals;
-    out2[1] = s[0] - out2[0];
+    out2[0] = c->bnd_bound_evals + (long long)d[3];
+    out2[1] = c->bnd_host_evals + (long long)d[0];
     return RG_OK;
 }
 

@@ -112,13 +112,14 @@ inline int bounded_prefix_groups(int G, int rho_milli) {
     return (int)std::min<long long>(G, (g + 31) / 32 * 32);
 }
 
-// bounded_k > 0: the bounded sweep's three tables (bounded.cuh) go into pair_info as [prefix stage | candidate stage |
-// fallback template], P entries each; the prefix stage is also the pass's main table (solver, selection, masks).
-// bound_prefix: the prefix stage counts an upper bound only, so the candidate and fallback stages cover the whole pair.
+// bounded_k > 0: the bounded sweep's four tables (bounded.cuh) go into pair_info as [prefix stage A | candidate stage |
+// fallback template | stage-B template], P entries each; stage A's table is also the pass's main table (solver, selection,
+// masks).  bound_prefix: the prefix stages count an upper bound only, so the candidate and fallback stages cover the whole
+// pair, and stage A stops at rho0 (rho0_milli) when that is shorter than rho; stage B covers the rest of the prefix.
 inline int f_plan(Ctx* c, cudaStream_t st, int P, const int* pair_off, const int* hyp_off, FPlan& plan, int blocks_per_sm,
                   const int* n_vote = nullptr /* PnP: per-view number of voting correspondences (<= view size) */,
                   int hyp_first = 0 /* hypothesis-split mode: global index of this rank's first hypothesis */,
-                  int bounded_k = 0, int rho_milli = 0, bool bound_prefix = false) {
+                  int bounded_k = 0, int rho_milli = 0, bool bound_prefix = false, int rho0_milli = 0) {
     RG_CHECK_ARG(P >= 0 && P <= 65535, "number of pairs must be in [0, 65535]");
     RG_CHECK_ARG(pair_off != nullptr && hyp_off != nullptr, "offset arrays are null");
     RG_CHECK_ARG(pair_off[0] == 0 && hyp_off[0] == 0, "offset arrays must start at 0");
@@ -136,13 +137,13 @@ inline int f_plan(Ctx* c, cudaStream_t st, int P, const int* pair_off, const int
     for (int p = 0; p <= P; ++p) { mix((unsigned)pair_off[p]); mix((unsigned)hyp_off[p]); }
     if (n_vote) for (int p = 0; p < P; ++p) mix((unsigned)n_vote[p]);
     mix((unsigned)hyp_first); mix((unsigned)blocks_per_sm); mix(n_vote ? 1u : 0u); mix((unsigned)P);
-    mix((unsigned)bounded_k); mix((unsigned)rho_milli); mix(bound_prefix ? 1u : 0u);
+    mix((unsigned)bounded_k); mix((unsigned)rho_milli); mix(bound_prefix ? 1u : 0u); mix((unsigned)rho0_milli);
     if (c->plan_valid && c->plan_hash == hsh && c->plan_cached.P == P && c->pair_info.ptr == c->plan_table) {
         plan = c->plan_cached;
         return RG_OK;
     }
     c->plan_valid = false;
-    const int n_tables = bounded_k > 0 ? 3 : 1;
+    const int n_tables = bounded_k > 0 ? 4 : 1;
     const int turn = c->stage_turn;       // double-buffered staging: planning pass k+1 does not wait for pass k's kernels
     c->stage_turn ^= 1;
     int rc = ensure_pinned(c->h_stage[turn], sizeof(PairInfo) * (size_t)P * n_tables);
@@ -175,19 +176,22 @@ inline int f_plan(Ctx* c, cudaStream_t st, int P, const int* pair_off, const int
     plan.Htot = hyp_off[P];
     plan.N32tot = off32;
     if (bounded_k > 0) {
-        // prefix stage: every hypothesis over groups [0, gA); candidate stage: min(K, H) compact records per pair over
+        // prefix stage A: every hypothesis over groups [0, gA0); candidate stage: min(K, H) compact records per pair over
         // [gA, G) ([0, G) after a bound-only prefix); fallback template: every hypothesis over the same window as the
-        // candidates (bnd_fb_plan keeps the marked pairs' items)
+        // candidates (bnd_live_plan keeps the marked pairs' items); stage-B template: room for the H - min(K, H)
+        // non-candidates over [gA0, gA) (bnd_live_plan keeps the items of those bnd_extend gathered)
         PairInfo* pc = pi + P;
         PairInfo* pf = pi + 2 * (size_t)P;
+        PairInfo* pb = pi + 3 * (size_t)P;
         plan.bounded = true;
         plan.bound_prefix = bound_prefix;
         plan.K = bounded_k;
         plan.evals = 0.0;
-        long long coff = 0;
+        long long coff = 0, boff = 0;
         for (int p = 0; p < P; ++p) {
             PairInfo& o = pi[p];
             const int G = o.g_end, gA = bounded_prefix_groups(G, rho_milli);
+            const int gA0 = bound_prefix ? std::min(gA, bounded_prefix_groups(G, rho0_milli)) : gA;
             const int kA = std::min(o.n, gA * kSub);              // real correspondences of the prefix
             o.g_end = gA;
             pf[p] = o;
@@ -196,16 +200,25 @@ inline int f_plan(Ctx* c, cudaStream_t st, int P, const int* pair_off, const int
             pc[p].hyp_off = (int)coff;
             pc[p].H = std::min(o.H, bounded_k);
             coff += pc[p].H;
+            pb[p] = o;
+            pb[p].g_base = gA0;
+            pb[p].hyp_off = (int)boff;
+            pb[p].H = o.H - pc[p].H;
+            boff += pb[p].H;
+            o.g_end = gA0;
             const int rest = bound_prefix ? o.n : o.n - kA;          // real correspondences of the later stages' window
-            plan.evals += (double)kA * (double)o.H;
+            plan.evals += (double)std::min(o.n, gA0 * kSub) * (double)o.H;
             plan.evals_c += (double)rest * (double)pc[p].H;
             plan.evals_f += (double)rest * (double)o.H;
         }
         plan.Ctot = coff;
-        const long long nc = plan_items(c, pc, P, blocks_per_sm), nf = plan_items(c, pf, P, blocks_per_sm);
-        RG_CHECK_ARG(nc >= 0 && nf >= 0, "too many scorer work items");
+        plan.Btot = boff;
+        const long long nc = plan_items(c, pc, P, blocks_per_sm), nf = plan_items(c, pf, P, blocks_per_sm),
+                        nb = plan_items(c, pb, P, blocks_per_sm);
+        RG_CHECK_ARG(nc >= 0 && nf >= 0 && nb >= 0, "too many scorer work items");
         plan.n_items_c = (int)nc;
         plan.n_items_f = (int)nf;
+        plan.n_items_b = (int)nb;
     }
     const long long n_items = plan_items(c, pi, P, blocks_per_sm);
     RG_CHECK_ARG(n_items >= 0, "too many scorer work items");

@@ -156,7 +156,8 @@ def profile(device=None, stream=0) -> dict:
 
 def bounded_stats(device=None, stream=0) -> dict:
     """What the last F call executed: see rg_f_last_bounded_stats (K = 0: it ran the full sweep).  ``evals`` splits into
-    ``bound_evals`` (bound-only prefix stages) and ``guarded_evals`` (rg_f_last_bounded_evals)."""
+    ``bound_evals`` (bound-only prefix stages: stage A over the first rho0 = option 16 of every pair, and stage B, the
+    survivors over the rest of the prefix) and ``guarded_evals`` (rg_f_last_bounded_evals)."""
     out = (C.c_longlong * 4)()
     _call("rg_f_last_bounded_stats", device, stream, out)
     split = (C.c_longlong * 2)()
