@@ -326,6 +326,29 @@ int rg_bundle_adjust_host(void* ctx, void* stream, int n_views, int n_points, in
 int rg_bundle_adjust_dev(void* ctx, void* stream, int n_views, int n_points, int n_obs, double* cams_dev, double* pts_dev,
                          const double* uv_dev, const int32_t* cam_idx_host, const int32_t* pt_idx_host, int n_fixed, int max_iter,
                          double ftol, double* cost_dev, int32_t* iters_dev, int32_t* status_dev);
+/* The same with a robust loss: the `loss` and `f_scale` of the reference's least_squares call (tables.py:317), with
+ * SciPy's definitions (scipy/optimize/_lsq/least_squares.py).  Every scalar residual f of EpsilonBA gets z = (f / C)^2,
+ * C = f_scale > 0, and the cost is 0.5 * sum C^2 rho(z) (SciPy's sol.cost) with
+ *   RG_LOSS_LINEAR   rho = z                                  (the entry points above; f_scale has no effect)
+ *   RG_LOSS_SOFT_L1  rho = 2 (sqrt(1 + z) - 1)
+ *   RG_LOSS_HUBER    rho = z for z <= 1, 2 sqrt(z) - 1 above
+ *   RG_LOSS_CAUCHY   rho = log(1 + z)
+ *   RG_LOSS_ARCTAN   rho = arctan(z)
+ * uv is C-normalised, so a scale of s pixels is f_scale = s / K[0][0].  The linearisation is iteratively reweighted least
+ * squares (each residual row and its Jacobian row weighted by sqrt(rho'(z))), not SciPy's second-order-corrected scaling
+ * (DESIGN.md section 4.6).  An unknown loss, or an f_scale that is not finite and > 0, is an invalid argument (-2).
+ * RG_LOSS_LINEAR gives results bit-identical to rg_bundle_adjust_host / _dev. */
+#define RG_LOSS_LINEAR 0
+#define RG_LOSS_SOFT_L1 1
+#define RG_LOSS_HUBER 2
+#define RG_LOSS_CAUCHY 3
+#define RG_LOSS_ARCTAN 4
+int rg_bundle_adjust_host2(void* ctx, void* stream, int n_views, int n_points, int n_obs, double* cams, double* pts,
+                           const double* uv, const int32_t* cam_idx, const int32_t* pt_idx, int n_fixed, int max_iter, double ftol,
+                           int loss, double f_scale, double* cost, int32_t* iters, int32_t* status);
+int rg_bundle_adjust_dev2(void* ctx, void* stream, int n_views, int n_points, int n_obs, double* cams_dev, double* pts_dev,
+                          const double* uv_dev, const int32_t* cam_idx_host, const int32_t* pt_idx_host, int n_fixed, int max_iter,
+                          double ftol, int loss, double f_scale, double* cost_dev, int32_t* iters_dev, int32_t* status_dev);
 /* EpsilonBA(x0, u, v, table) (tables.py:266-296): x = [all camera matrices raveled (n_views x 12), all points (n_points x 3)]
  * (tables.py:315, fun.reshapeToCamera3DPoints2 fun.py:282-289); out (2 * n_obs) = interleaved u / v residuals */
 int rg_ba_residuals_host(void* ctx, void* stream, int n_views, int n_points, int n_obs, const double* x, const double* u,

@@ -21,6 +21,7 @@ SCORE_FP32_GUARDED, SCORE_FP64, SCORE_FP32_BOUND = 0, 1, 2
 TRI_OPTIMAL, TRI_LINEAR = 0, 1
 FLAG_REUSE_POINTS = 1
 FLAG_BOUNDED = 2
+LOSS_LINEAR, LOSS_SOFT_L1, LOSS_HUBER, LOSS_CAUCHY, LOSS_ARCTAN = 0, 1, 2, 3, 4
 
 _vp = C.c_void_p
 _i = C.c_int
@@ -80,6 +81,8 @@ SIGNATURES = {
     "rg_fmatrix_residuals_gs_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rg_bundle_adjust_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _d, _vp, _vp, _vp]),
     "rg_bundle_adjust_dev": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _d, _vp, _vp, _vp]),
+    "rg_bundle_adjust_host2": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _d, _i, _d, _vp, _vp, _vp]),
+    "rg_bundle_adjust_dev2": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _d, _i, _d, _vp, _vp, _vp]),
     "rg_ba_residuals_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rg_two_view_init_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "rg_two_view_init_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

@@ -16,15 +16,42 @@ __global__ void __launch_bounds__(256) ba_gather_uv(const double* __restrict__ u
 
 static inline char* align16(char* w) { return (char*)(((uintptr_t)w + 15) & ~(uintptr_t)15); }
 
+// the kernels that depend on the loss (ba_points, ba_trial: rho and its weights; ba_blocks: the record layout)
+struct BaLossKernels {
+    decltype(&ba_points<LOSS_LINEAR>) points;
+    decltype(&ba_trial<LOSS_LINEAR>) trial;
+    decltype(&ba_blocks<false>) blocks;
+};
+
+template <int L>
+static BaLossKernels ba_loss_kernels() { return {ba_points<L>, ba_trial<L>, ba_blocks<L != LOSS_LINEAR>}; }
+
+static bool ba_loss_kernels(int loss, BaLossKernels& k) {
+    switch (loss) {
+        case LOSS_LINEAR: k = ba_loss_kernels<LOSS_LINEAR>(); return true;
+        case LOSS_SOFT_L1: k = ba_loss_kernels<LOSS_SOFT_L1>(); return true;
+        case LOSS_HUBER: k = ba_loss_kernels<LOSS_HUBER>(); return true;
+        case LOSS_CAUCHY: k = ba_loss_kernels<LOSS_CAUCHY>(); return true;
+        case LOSS_ARCTAN: k = ba_loss_kernels<LOSS_ARCTAN>(); return true;
+        default: return false;
+    }
+}
+
 // cams_dev (nC x 12) and pts_dev (nP x 3) are refined in place; uv_dev (nO x 2) in the caller's observation order;
-// cam_idx / pt_idx are HOST arrays (table bookkeeping lives on the host in the reference too).
+// cam_idx / pt_idx are HOST arrays (table bookkeeping lives on the host in the reference too).  loss (LOSS_*) and
+// f_scale = C: every residual component f contributes C^2 rho((f / C)^2) to twice the cost.
 static int bundle_adjust_dev(Ctx* c, cudaStream_t st, int nC, int nP, int nO, double* cams, double* pts, const double* uv,
-                             const int* cam_idx, const int* pt_idx, int n_fixed, int max_iter, double ftol, double* cost,
-                             int* iters, int* status, bool host_paced) {
+                             const int* cam_idx, const int* pt_idx, int n_fixed, int max_iter, double ftol, int loss,
+                             double f_scale, double* cost, int* iters, int* status, bool host_paced) {
     RG_CHECK_ARG(nC >= 0 && nP >= 0 && nO >= 0, "negative size");
     RG_CHECK_ARG(n_fixed >= 0, "n_fixed must be >= 0");
     RG_CHECK_ARG(max_iter >= 0 && max_iter <= 10000, "max_iter must be in [0, 10000]");
     RG_CHECK_ARG(ftol >= 0.0 && std::isfinite(ftol), "ftol must be finite and >= 0");
+    BaLossKernels kern;
+    RG_CHECK_ARG(ba_loss_kernels(loss, kern), "loss must be one of RG_LOSS_LINEAR .. RG_LOSS_ARCTAN");
+    const double ic = 1.0 / f_scale, c2 = f_scale * f_scale;
+    RG_CHECK_ARG(std::isfinite(f_scale) && f_scale > 0.0 && std::isfinite(ic) && std::isfinite(c2) && c2 > 0.0,
+                 "f_scale must be finite and > 0 (with a finite, non-zero square)");
     RG_CHECK_ARG(nO == 0 || (cam_idx && pt_idx && uv), "null observation table");
     RG_CHECK_ARG((nC == 0 || cams) && (nP == 0 || pts), "null parameter buffers");
     const int nF = std::max(0, nC - n_fixed);
@@ -199,11 +226,12 @@ static int bundle_adjust_dev(Ctx* c, cudaStream_t st, int nC, int nP, int nO, do
             RG_CUDA(cudaEventSynchronize(c->ba_iter_ev[it & 1]));          // iteration it - 2 has finished
             if (h_flags[it - 2]) break;
         }
-        ba_points<<<nparts, kBaPointThreads, 0, st>>>(bs, cams, pts, Xtrial, uvS, d_ocam, d_pt_off, nP, pblk, cost_part, bad_part, obs2_part, lin);
+        kern.points<<<nparts, kBaPointThreads, 0, st>>>(bs, cams, pts, Xtrial, uvS, d_ocam, d_pt_off, nP, pblk, cost_part, bad_part,
+                                                          obs2_part, lin, ic, c2);
         if (nF > 0) {
             if (sparse_blocks) RG_CUDA(cudaMemsetAsync(S, 0, sizeof(double) * s_elems, st));   // blocks without a common point
-            ba_blocks<<<(unsigned)n_items, kBaBlockThreads, 0, st>>>(bs, d_items, part, pts, lin, d_ocam, d_opt, d_pt_off, d_cam_off,
-                                                                    d_cam_obs, pblk, n_fixed, nF, S);
+            kern.blocks<<<(unsigned)n_items, kBaBlockThreads, 0, st>>>(bs, d_items, part, pts, lin, d_ocam, d_opt, d_pt_off, d_cam_off,
+                                                                      d_cam_obs, pblk, n_fixed, nF, S);
             if (any_split) {
                 ba_blocks_reduce<<<(unsigned)n_blocks, kBaBlockThreads, 0, st>>>(bs, d_items, d_first, (int)n_blocks, part, nF, S);
                 ++launches;
@@ -213,7 +241,8 @@ static int bundle_adjust_dev(Ctx* c, cudaStream_t st, int nC, int nP, int nO, do
         } else {
             ba_solve_none<<<1, 1, 0, st>>>(bs);
         }
-        ba_trial<<<nparts, kBaPointThreads, 0, st>>>(bs, cams, dC, pts, Xtrial, uvS, d_ocam, d_pt_off, nP, pblk, lin, trial_part);
+        kern.trial<<<nparts, kBaPointThreads, 0, st>>>(bs, cams, dC, pts, Xtrial, uvS, d_ocam, d_pt_off, nP, pblk, lin, trial_part,
+                                                         ic, c2);
         ba_accept<<<1, 256, 0, st>>>(bs, cams, dC, nC, cost_part, trial_part, bad_part, obs2_part, nparts, ftol, max_iter);
         launches += nF > 0 ? 5 : 4;
         if (h_flags) {
@@ -222,7 +251,8 @@ static int bundle_adjust_dev(Ctx* c, cudaStream_t st, int nC, int nP, int nO, do
         }
     }
     if (max_iter == 0) {
-        ba_points<<<nparts, kBaPointThreads, 0, st>>>(bs, cams, pts, Xtrial, uvS, d_ocam, d_pt_off, nP, pblk, cost_part, bad_part, obs2_part, lin);
+        kern.points<<<nparts, kBaPointThreads, 0, st>>>(bs, cams, pts, Xtrial, uvS, d_ocam, d_pt_off, nP, pblk, cost_part, bad_part,
+                                                          obs2_part, lin, ic, c2);
         ba_cost_only<<<1, 1, 0, st>>>(bs, cost_part, nparts);
         launches += 2;
     }
@@ -240,17 +270,24 @@ using namespace rg;
 
 extern "C" {
 
+int rg_bundle_adjust_dev2(void* ctx, void* stream, int n_views, int n_points, int n_obs, double* cams_dev, double* pts_dev,
+                          const double* uv_dev, const int32_t* cam_idx_host, const int32_t* pt_idx_host, int n_fixed, int max_iter,
+                          double ftol, int loss, double f_scale, double* cost_dev, int32_t* iters_dev, int32_t* status_dev) {
+    RG_CHECK_ARG(ctx != nullptr, "ctx is null");
+    return bundle_adjust_dev((Ctx*)ctx, (cudaStream_t)stream, n_views, n_points, n_obs, cams_dev, pts_dev, uv_dev, cam_idx_host,
+                             pt_idx_host, n_fixed, max_iter, ftol, loss, f_scale, cost_dev, iters_dev, status_dev, false);
+}
+
 int rg_bundle_adjust_dev(void* ctx, void* stream, int n_views, int n_points, int n_obs, double* cams_dev, double* pts_dev,
                          const double* uv_dev, const int32_t* cam_idx_host, const int32_t* pt_idx_host, int n_fixed, int max_iter,
                          double ftol, double* cost_dev, int32_t* iters_dev, int32_t* status_dev) {
-    RG_CHECK_ARG(ctx != nullptr, "ctx is null");
-    return bundle_adjust_dev((Ctx*)ctx, (cudaStream_t)stream, n_views, n_points, n_obs, cams_dev, pts_dev, uv_dev, cam_idx_host,
-                             pt_idx_host, n_fixed, max_iter, ftol, cost_dev, iters_dev, status_dev, false);
+    return rg_bundle_adjust_dev2(ctx, stream, n_views, n_points, n_obs, cams_dev, pts_dev, uv_dev, cam_idx_host, pt_idx_host,
+                                 n_fixed, max_iter, ftol, LOSS_LINEAR, 1.0, cost_dev, iters_dev, status_dev);
 }
 
-int rg_bundle_adjust_host(void* ctx, void* stream, int n_views, int n_points, int n_obs, double* cams, double* pts,
-                          const double* uv, const int32_t* cam_idx, const int32_t* pt_idx, int n_fixed, int max_iter, double ftol,
-                          double* cost, int32_t* iters, int32_t* status) {
+int rg_bundle_adjust_host2(void* ctx, void* stream, int n_views, int n_points, int n_obs, double* cams, double* pts,
+                           const double* uv, const int32_t* cam_idx, const int32_t* pt_idx, int n_fixed, int max_iter, double ftol,
+                           int loss, double f_scale, double* cost, int32_t* iters, int32_t* status) {
     RG_CHECK_ARG(ctx != nullptr, "ctx is null");
     RG_CHECK_ARG(n_views >= 0 && n_points >= 0 && n_obs >= 0, "negative size");
     RG_CHECK_ARG((n_views == 0 || cams) && (n_points == 0 || pts) && (n_obs == 0 || uv), "null buffers");
@@ -268,8 +305,8 @@ int rg_bundle_adjust_host(void* ctx, void* stream, int n_views, int n_points, in
     if (nc) RG_CUDA(cudaMemcpyAsync(dcam, cams, sizeof(double) * 12 * nc, cudaMemcpyHostToDevice, st));
     if (np) RG_CUDA(cudaMemcpyAsync(dpts, pts, sizeof(double) * 3 * np, cudaMemcpyHostToDevice, st));
     if (no) RG_CUDA(cudaMemcpyAsync(duv, uv, sizeof(double) * 2 * no, cudaMemcpyHostToDevice, st));
-    rc = bundle_adjust_dev(c, st, n_views, n_points, n_obs, dcam, dpts, duv, cam_idx, pt_idx, n_fixed, max_iter, ftol, dcost, dit,
-                           dit + 1, true);
+    rc = bundle_adjust_dev(c, st, n_views, n_points, n_obs, dcam, dpts, duv, cam_idx, pt_idx, n_fixed, max_iter, ftol, loss, f_scale,
+                           dcost, dit, dit + 1, true);
     if (rc) return rc;
     if (nc) RG_CUDA(cudaMemcpyAsync(cams, dcam, sizeof(double) * 12 * nc, cudaMemcpyDeviceToHost, st));
     if (np) RG_CUDA(cudaMemcpyAsync(pts, dpts, sizeof(double) * 3 * np, cudaMemcpyDeviceToHost, st));
@@ -278,6 +315,13 @@ int rg_bundle_adjust_host(void* ctx, void* stream, int n_views, int n_points, in
     if (status) RG_CUDA(cudaMemcpyAsync(status, dit + 1, sizeof(int), cudaMemcpyDeviceToHost, st));
     RG_CUDA(cudaStreamSynchronize(st));
     return RG_OK;
+}
+
+int rg_bundle_adjust_host(void* ctx, void* stream, int n_views, int n_points, int n_obs, double* cams, double* pts,
+                          const double* uv, const int32_t* cam_idx, const int32_t* pt_idx, int n_fixed, int max_iter, double ftol,
+                          double* cost, int32_t* iters, int32_t* status) {
+    return rg_bundle_adjust_host2(ctx, stream, n_views, n_points, n_obs, cams, pts, uv, cam_idx, pt_idx, n_fixed, max_iter, ftol,
+                                  LOSS_LINEAR, 1.0, cost, iters, status);
 }
 
 #ifdef RG_BA_PROF

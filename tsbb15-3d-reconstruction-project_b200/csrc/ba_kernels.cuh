@@ -13,6 +13,13 @@
 //   J_c^T J_c = M (x) Xh Xh^T      J_c^T J_p = T (x) Xh      V_j = sum_o Q^T Q      g_j = sum_o Q^T r
 // so the block (k, l) of the reduced system is   [k == l] sum_o M_o (x) XX  -  sum_{o in k, o' in l, same point}
 // (T_o V_j'^-1 T_o'^T) (x) Xh Xh^T : a 3x3 matrix per pair of observations, expanded by the 4x4 outer product.
+//
+// Robust losses (the loss / f_scale of SciPy's least_squares): every scalar residual f contributes C^2 rho((f / C)^2) to
+// twice the cost.  The linearisation is IRLS: the residual row and the Jacobian row of each component are weighted by
+// w = rho'(z), i.e. every product above gets W = diag(w0, w1) between its two factors (M = P2^T W P2, T = P2^T W Q,
+// V_j = sum Q^T W Q, g_j = sum Q^T W r); the gradient is exact, the normal matrix the weighted Gauss-Newton one.  M then
+// has M11 != M00, and the linearisation record stores w0, w1 in place of the third entry of P2^T W r (rebuilt from the
+// first two: -(u a0 + v a1)).  The loss is a template parameter; the linear instantiation is the unweighted code.
 #pragma once
 #include <cooperative_groups.h>
 #include "gs_kernels.cuh"
@@ -25,9 +32,11 @@ constexpr int kBaPointThreads = 128;
 constexpr int kBaPointLanes = 8;          // lanes that share one point in ba_points / ba_trial (one observation of the track each)
 constexpr int kBaBlockThreads = 192;      // chunk of observations per pass; threads 0..143 own the 12x12 entries
 constexpr int kBaRec = 17;                // doubles per staged observation: A (9) | X (3) | z (3) | M00, M22
+constexpr int kBaRecW = 18;               // the same for a robust loss: A (9) | X (3) | z (3) | M00, M11, M22
 constexpr int kBaSegChunks = 2;            // chunks of kBaBlockThreads observations per work item of ba_blocks
 constexpr int kBaPart = 168;              // doubles per partial block: 144 entries | 12 rhs | 12 diagonal damping sums
 constexpr int kBaLin = 16;                // doubles per observation written by ba_points: T (9) | iy^2, u, v | P2^T r (3) | pad
+                                          // robust loss: T (9) | iy^2, u, v | (P2^T W r)[0..1] | w0, w1
 constexpr int kBaSolveThreads = 512;
 constexpr int kBaSolveFixed = 192;        // doubles at the start of ba_solve*'s dynamic shared memory: Ld (144) | Li (16) | scratch (32)
 constexpr int kBaMaxFree = 170;           // free views: the 12 x (n + 1) Cholesky panel must fit in shared memory
@@ -65,6 +74,34 @@ __device__ __forceinline__ void ba_obs(const double* __restrict__ C, const doubl
     g.ok = isfinite(g.r0) && isfinite(g.r1) && isfinite(g.iy);
 }
 
+// rho(z) and w = rho'(z) of SciPy's losses (scipy/optimize/_lsq/least_squares.py) at z = (f / C)^2
+template <int kLoss>
+__device__ __forceinline__ void ba_rho(const double z, double& rho, double& w) {
+    if constexpr (kLoss == LOSS_SOFT_L1) {
+        const double s = sqrt(1.0 + z);
+        rho = 2.0 * (s - 1.0); w = 1.0 / s;
+    } else if constexpr (kLoss == LOSS_HUBER) {
+        if (z <= 1.0) { rho = z; w = 1.0; }
+        else { const double s = sqrt(z); rho = 2.0 * s - 1.0; w = 1.0 / s; }
+    } else if constexpr (kLoss == LOSS_CAUCHY) {
+        rho = log1p(z); w = 1.0 / (1.0 + z);
+    } else if constexpr (kLoss == LOSS_ARCTAN) {
+        rho = atan(z); w = 1.0 / fma(z, z, 1.0);
+    } else {
+        rho = z; w = 1.0;
+    }
+}
+
+// C^2 (rho(z0) + rho(z1)) of one observation, with the weights; ic = 1 / C, c2 = C^2
+template <int kLoss>
+__device__ __forceinline__ double ba_robust(const BaObs& g, const double ic, const double c2, double& w0, double& w1) {
+    const double s0 = g.r0 * ic, s1 = g.r1 * ic;
+    double p0, p1;
+    ba_rho<kLoss>(s0 * s0, p0, w0);
+    ba_rho<kLoss>(s1 * s1, p1, w1);
+    return c2 * (p0 + p1);
+}
+
 // T = P2^T Q with P2 = [[iy, 0, -u iy], [0, iy, -v iy]]
 __device__ __forceinline__ void ba_T(const BaObs& g, double (&T)[3][3]) {
     const double p02 = -g.u * g.iy, p12 = -g.v * g.iy;
@@ -94,12 +131,14 @@ __device__ __forceinline__ double ba_block_sum(double v, double* sh) {
 // e_j = V'^-1 g_j, cost partials
 // observations are stored sorted by point: the track of point j is [pt_off[j], pt_off[j+1])
 // ------------------------------------------------------------------------------------------------
+template <int kLoss>
 __global__ void __launch_bounds__(kBaPointThreads) ba_points(BaState* __restrict__ st, const double* __restrict__ cams,
                                                              double* __restrict__ X, const double* __restrict__ Xtrial,
                                                              const double2* __restrict__ uv, const int* __restrict__ ocam,
                                                              const int* __restrict__ pt_off, int nP, double* __restrict__ pblk,
                                                              double* __restrict__ cost_part, int* __restrict__ bad_part,
-                                                             double* __restrict__ obs2_part, double* __restrict__ lin) {
+                                                             double* __restrict__ obs2_part, double* __restrict__ lin,
+                                                             double ic, double c2) {
     __shared__ double sh[kBaPointThreads / 32];
     if (st->done) return;
     const double lambda = st->lambda;
@@ -134,6 +173,31 @@ __global__ void __launch_bounds__(kBaPointThreads) ba_points(BaState* __restrict
                 ++bad;
                 const double4 z4 = make_double4(0.0, 0.0, 0.0, 0.0);
                 lo[0] = z4; lo[1] = z4; lo[2] = z4; lo[3] = z4;
+                continue;
+            }
+            if constexpr (kLoss != LOSS_LINEAR) {
+                double w0, w1;
+                cost += ba_robust<kLoss>(b, ic, c2, w0, w1);
+                const double a0 = w0 * b.r0, a1 = w1 * b.r1;               // W r
+                double T[3][3];
+                ba_T(b, T);
+#pragma unroll
+                for (int c = 0; c < 3; ++c) {                               // P2^T W Q = P2^T W P2 C[:, :3]
+                    T[0][c] *= w0;
+                    T[1][c] *= w1;
+                    T[2][c] = -(b.u * T[0][c] + b.v * T[1][c]);
+                }
+                lo[0] = make_double4(T[0][0], T[0][1], T[0][2], T[1][0]);
+                lo[1] = make_double4(T[1][1], T[1][2], T[2][0], T[2][1]);
+                lo[2] = make_double4(T[2][2], b.iy * b.iy, b.u, b.v);
+                lo[3] = make_double4(b.iy * a0, b.iy * a1, w0, w1);
+#pragma unroll
+                for (int a = 0; a < 3; ++a) {
+#pragma unroll
+                    for (int c = a; c < 3; ++c) V[sym3(a, c)] += w0 * b.Q[0][a] * b.Q[0][c] + w1 * b.Q[1][a] * b.Q[1][c];
+                    g[a] += b.Q[0][a] * a0 + b.Q[1][a] * a1;
+                }
+                obs2 += m.x * m.x + m.y * m.y;
                 continue;
             }
             {
@@ -194,8 +258,9 @@ __global__ void __launch_bounds__(kBaPointThreads) ba_points(BaState* __restrict
 // observation's linearisation (written by ba_points), looks through the point's track for observations in view l,
 // stages A = [k == l] M - T V'^-1 T'^T and Xh in shared memory (ordered ballot compaction); then thread (r, c) adds
 // A[a][a2] Xh[b] Xh[b2] over the chunk.  Row n of the matrix (leading dimension n + 1) receives the right-hand side,
-// so that the factorisation performs the forward substitution as it goes.
+// so that the factorisation performs the forward substitution as it goes.  kW: the record of a robust loss (weights w0, w1).
 // ------------------------------------------------------------------------------------------------
+template <bool kW>
 __global__ void __launch_bounds__(kBaBlockThreads, 3) ba_blocks(const BaState* __restrict__ st, const int4* __restrict__ items,
                                                                 double* __restrict__ part,
                                                                 const double* __restrict__ X, const double* __restrict__ lin,
@@ -206,7 +271,8 @@ __global__ void __launch_bounds__(kBaBlockThreads, 3) ba_blocks(const BaState* _
     if (st->done) return;
     const int4 item = items[blockIdx.x];                    // (kf, lf, segment, segments of this block)
     const int kf = item.x, lf = item.y;
-    __shared__ double rec[kBaBlockThreads * kBaRec];
+    constexpr int kRec = kW ? kBaRecW : kBaRec;
+    __shared__ double rec[kBaBlockThreads * kRec];
     __shared__ int wcount[kBaBlockThreads / 32 + 1];
     const int k = n_fixed + kf, l = n_fixed + lf;
     const bool diag = kf == lf;
@@ -221,7 +287,7 @@ __global__ void __launch_bounds__(kBaBlockThreads, 3) ba_blocks(const BaState* _
     for (int base = lo; base < hi; base += kBaBlockThreads) {
         const int oi = base + tid;
         bool valid = false;
-        double A[9], Xh[3], z[3], m00 = 0.0, m22 = 0.0;
+        double A[9], Xh[3], z[3], m00 = 0.0, m11 = 0.0, m22 = 0.0;
         if (oi < hi) {
             const int o = cam_obs[oi], j = opt[o];
             const int t0 = pt_off[j], t1 = pt_off[j + 1];
@@ -242,14 +308,23 @@ __global__ void __launch_bounds__(kBaBlockThreads, 3) ba_blocks(const BaState* _
             if (diag) {
                 const double i2 = l2.y, u = l2.z, v = l2.w;
                 const double4 l3 = L[3];
-                m00 = i2; m22 = (u * u + v * v) * i2;
-                A[0] = i2; A[4] = i2; A[8] = m22;
-                A[2] = A[6] = -u * i2;
-                A[5] = A[7] = -v * i2;
+                double pr2 = l3.z;                                      // (P2^T W r)[2]
+                if constexpr (kW) {                                     // M = P2^T W P2
+                    m00 = l3.z * i2; m11 = l3.w * i2; m22 = (l3.z * u * u + l3.w * v * v) * i2;
+                    A[0] = m00; A[4] = m11; A[8] = m22;
+                    A[2] = A[6] = -u * m00;
+                    A[5] = A[7] = -v * m11;
+                    pr2 = -(u * l3.x + v * l3.y);
+                } else {
+                    m00 = i2; m22 = (u * u + v * v) * i2;
+                    A[0] = i2; A[4] = i2; A[8] = m22;
+                    A[2] = A[6] = -u * i2;
+                    A[5] = A[7] = -v * i2;
+                }
                 const double e0 = pb[6], e1 = pb[7], e2 = pb[8];        // z = P2^T r - T e_j
                 z[0] = l3.x - (T[0][0] * e0 + T[0][1] * e1 + T[0][2] * e2);
                 z[1] = l3.y - (T[1][0] * e0 + T[1][1] * e1 + T[1][2] * e2);
-                z[2] = l3.z - (T[2][0] * e0 + T[2][1] * e1 + T[2][2] * e2);
+                z[2] = pr2 - (T[2][0] * e0 + T[2][1] * e1 + T[2][2] * e2);
                 valid = true;
             }
             for (int o2 = t0; o2 < t1; ++o2) {
@@ -276,11 +351,15 @@ __global__ void __launch_bounds__(kBaBlockThreads, 3) ba_blocks(const BaState* _
             total += wcount[w];
         }
         if (valid) {
-            double* r = rec + slot * kBaRec;
+            double* r = rec + slot * kRec;
 #pragma unroll
             for (int q = 0; q < 9; ++q) r[q] = A[q];
             r[9] = Xh[0]; r[10] = Xh[1]; r[11] = Xh[2];
-            if (diag) { r[12] = z[0]; r[13] = z[1]; r[14] = z[2]; r[15] = m00; r[16] = m22; }
+            if (diag) {
+                r[12] = z[0]; r[13] = z[1]; r[14] = z[2]; r[15] = m00;
+                if constexpr (kW) { r[16] = m11; r[17] = m22; }
+                else r[16] = m22;
+            }
         }
         __syncthreads();
         if (tid < 144) {
@@ -288,33 +367,33 @@ __global__ void __launch_bounds__(kBaBlockThreads, 3) ba_blocks(const BaState* _
             const int ia = ea * 3 + ea2, ib = eb < 3 ? 9 + eb : -1, ib2 = eb2 < 3 ? 9 + eb2 : -1;
             int i = 0;
             for (; i + 4 <= total; i += 4) {                 // four independent chains (fixed order: still reproducible)
-                const double* r = rec + i * kBaRec;
-                const double xa0 = ib >= 0 ? r[ib] : 1.0, xa1 = ib >= 0 ? r[kBaRec + ib] : 1.0;
-                const double xa2 = ib >= 0 ? r[2 * kBaRec + ib] : 1.0, xa3 = ib >= 0 ? r[3 * kBaRec + ib] : 1.0;
-                const double xc0 = ib2 >= 0 ? r[ib2] : 1.0, xc1 = ib2 >= 0 ? r[kBaRec + ib2] : 1.0;
-                const double xc2 = ib2 >= 0 ? r[2 * kBaRec + ib2] : 1.0, xc3 = ib2 >= 0 ? r[3 * kBaRec + ib2] : 1.0;
+                const double* r = rec + i * kRec;
+                const double xa0 = ib >= 0 ? r[ib] : 1.0, xa1 = ib >= 0 ? r[kRec + ib] : 1.0;
+                const double xa2 = ib >= 0 ? r[2 * kRec + ib] : 1.0, xa3 = ib >= 0 ? r[3 * kRec + ib] : 1.0;
+                const double xc0 = ib2 >= 0 ? r[ib2] : 1.0, xc1 = ib2 >= 0 ? r[kRec + ib2] : 1.0;
+                const double xc2 = ib2 >= 0 ? r[2 * kRec + ib2] : 1.0, xc3 = ib2 >= 0 ? r[3 * kRec + ib2] : 1.0;
                 acc = fma(r[ia] * xa0, xc0, acc);
-                acc1 = fma(r[kBaRec + ia] * xa1, xc1, acc1);
-                acc2 = fma(r[2 * kBaRec + ia] * xa2, xc2, acc2);
-                acc3 = fma(r[3 * kBaRec + ia] * xa3, xc3, acc3);
+                acc1 = fma(r[kRec + ia] * xa1, xc1, acc1);
+                acc2 = fma(r[2 * kRec + ia] * xa2, xc2, acc2);
+                acc3 = fma(r[3 * kRec + ia] * xa3, xc3, acc3);
                 if (dd) {
-                    const int im = ea < 2 ? 15 : 16;
+                    const int im = kW ? 15 + ea : (ea < 2 ? 15 : 16);     // M_aa of the diagonal damping sum
                     accd = fma(r[im] * xa0, xa0, accd);
-                    accd = fma(r[kBaRec + im] * xa1, xa1, accd);
-                    accd = fma(r[2 * kBaRec + im] * xa2, xa2, accd);
-                    accd = fma(r[3 * kBaRec + im] * xa3, xa3, accd);
+                    accd = fma(r[kRec + im] * xa1, xa1, accd);
+                    accd = fma(r[2 * kRec + im] * xa2, xa2, accd);
+                    accd = fma(r[3 * kRec + im] * xa3, xa3, accd);
                 }
             }
             for (; i < total; ++i) {
-                const double* r = rec + i * kBaRec;
+                const double* r = rec + i * kRec;
                 const double xb = ib >= 0 ? r[ib] : 1.0, xb2 = ib2 >= 0 ? r[ib2] : 1.0;
                 acc = fma(r[ia] * xb, xb2, acc);
-                if (dd) accd = fma((ea < 2 ? r[15] : r[16]) * xb, xb, accd);
+                if (dd) accd = fma((kW ? r[15 + ea] : (ea < 2 ? r[15] : r[16])) * xb, xb, accd);
             }
         } else if (diag && rz < 12) {
             const int za = rz >> 2, zb = rz & 3;
             for (int i = 0; i < total; ++i) {
-                const double* r = rec + i * kBaRec;
+                const double* r = rec + i * kRec;
                 acc = fma(r[12 + za], zb < 3 ? r[9 + zb] : 1.0, acc);
             }
         }
@@ -770,12 +849,13 @@ __global__ void ba_solve_none(BaState* __restrict__ st) {
 // ------------------------------------------------------------------------------------------------
 // step 4 (kBaPointLanes lanes per point): point steps by back-substitution, trial points, trial cost partials
 // ------------------------------------------------------------------------------------------------
+template <int kLoss>
 __global__ void __launch_bounds__(kBaPointThreads) ba_trial(const BaState* __restrict__ st, const double* __restrict__ cams,
                                                             const double* __restrict__ dC, const double* __restrict__ X,
                                                             double* __restrict__ Xtrial, const double2* __restrict__ uv,
                                                             const int* __restrict__ ocam, const int* __restrict__ pt_off, int nP,
                                                             const double* __restrict__ pblk, const double* __restrict__ lin,
-                                                            double* __restrict__ trial_part) {
+                                                            double* __restrict__ trial_part, double ic, double c2) {
     __shared__ double sh[kBaPointThreads / 32];
     if (st->done || st->accepted < 0) return;
     double cost = 0.0;
@@ -821,7 +901,12 @@ __global__ void __launch_bounds__(kBaPointThreads) ba_trial(const BaState* __res
             const double2 m = uv[o];
             BaObs t;
             ba_obs(Cn, n0, n1, n2, m.x, m.y, t);
-            cost += t.ok ? t.r0 * t.r0 + t.r1 * t.r1 : INFINITY;
+            if constexpr (kLoss != LOSS_LINEAR) {
+                double w0, w1;
+                cost += t.ok ? ba_robust<kLoss>(t, ic, c2, w0, w1) : INFINITY;
+            } else {
+                cost += t.ok ? t.r0 * t.r0 + t.r1 * t.r1 : INFINITY;
+            }
         }
     }
     const double s = ba_block_sum(cost, sh);

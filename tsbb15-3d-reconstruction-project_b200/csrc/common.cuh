@@ -54,6 +54,7 @@ enum : int { MODE_EPI_MAX = 0, MODE_SAMPSON = 1 };
 enum : int { TIE_FIRST = 0, TIE_REFERENCE = 1 };
 enum : int { SOLVER_QR = 0, SOLVER_JACOBI = 1 };
 enum : int { SCORE_FP32_GUARDED = 0, SCORE_FP64 = 1, SCORE_FP32_BOUND = 2 };
+enum : int { LOSS_LINEAR = 0, LOSS_SOFT_L1 = 1, LOSS_HUBER = 2, LOSS_CAUCHY = 3, LOSS_ARCTAN = 4 };
 
 // ---------------------------------------------------------------------------------------------
 // device-side records

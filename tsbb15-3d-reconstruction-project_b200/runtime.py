@@ -493,11 +493,28 @@ def fmatrix_residuals_gs(params, pl, pr, device=None, stream=0):
     return out
 
 
-def bundle_adjust(cams, pts, uv, cam_idx, pt_idx, n_fixed=1, max_iter=50, ftol=1e-4, device=None, stream=0) -> dict:
+BA_LOSSES = {"linear": cabi.LOSS_LINEAR, "soft_l1": cabi.LOSS_SOFT_L1, "huber": cabi.LOSS_HUBER, "cauchy": cabi.LOSS_CAUCHY,
+             "arctan": cabi.LOSS_ARCTAN}
+
+
+def bundle_adjust(cams, pts, uv, cam_idx, pt_idx, n_fixed=1, max_iter=50, ftol=1e-4, device=None, stream=0, loss="linear",
+                  f_scale=1.0) -> dict:
     """Bundle adjustment (the minimisation of tables.Tables.BundleAdjustment2, tables.py:260-333) in ONE library call.
     cams (V, 3, 4) camera matrices, pts (P, 3), uv (O, 2) observed C-normalised image points, cam_idx / pt_idx (O,) the
     view and point of every observation; the first n_fixed views are held fixed (the reference fixes view 0).
-    Returns dict(cams, pts, cost = 0.5 * sum r^2, iters, status: 2 converged, 3 no further descent, 4 max_iter)."""
+    loss / f_scale are those of scipy.optimize.least_squares (names and defaults): "linear", "soft_l1", "huber", "cauchy"
+    or "arctan"; every residual component f contributes f_scale^2 rho((f / f_scale)^2).  uv is C-normalised, so a scale
+    of s pixels is f_scale = s / K[0, 0].
+    Returns dict(cams, pts, cost = 0.5 * sum f_scale^2 rho (0.5 * sum r^2 for "linear"), iters, status: 2 converged,
+    3 no further descent, 4 max_iter)."""
+    if not isinstance(loss, str) or loss not in BA_LOSSES:
+        raise ValueError(f"loss must be one of {sorted(BA_LOSSES)} (callable losses are not supported), got {loss!r}")
+    try:
+        f_scale = float(f_scale)
+    except (TypeError, ValueError):
+        raise ValueError(f"f_scale must be a finite number > 0, got {f_scale!r}") from None
+    if not (np.isfinite(f_scale) and f_scale > 0.0):
+        raise ValueError(f"f_scale must be a finite number > 0, got {f_scale!r}")
     cams = np.array(cams, dtype=np.float64).reshape(-1, 3, 4)
     pts = np.array(pts, dtype=np.float64).reshape(-1, 3)
     uv = _f64(uv).reshape(-1, 2)
@@ -507,8 +524,8 @@ def bundle_adjust(cams, pts, uv, cam_idx, pt_idx, n_fixed=1, max_iter=50, ftol=1
         raise ValueError("uv, cam_idx and pt_idx must have one row per observation")
     cost = np.full(1, np.nan)
     it_st = np.zeros(2, dtype=np.int32)
-    _call("rg_bundle_adjust_host", device, stream, cams.shape[0], pts.shape[0], uv.shape[0], cams, pts, uv, ci, pi,
-          n_fixed, max_iter, ftol, cost, it_st[:1], it_st[1:])
+    _call("rg_bundle_adjust_host2", device, stream, cams.shape[0], pts.shape[0], uv.shape[0], cams, pts, uv, ci, pi,
+          n_fixed, max_iter, ftol, BA_LOSSES[loss], f_scale, cost, it_st[:1], it_st[1:])
     return {"cams": cams, "pts": pts, "cost": float(cost[0]), "iters": int(it_st[0]), "status": int(it_st[1])}
 
 

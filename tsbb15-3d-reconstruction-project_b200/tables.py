@@ -82,9 +82,11 @@ class Tables:
         pt_idx = np.array([o.point_3D_index for o in self.T_obs], dtype=np.int32)
         return uv, cam_idx, pt_idx
 
-    def BundleAdjustment2(self, max_iter=50, ftol=1e-4):
+    def BundleAdjustment2(self, max_iter=50, ftol=1e-4, loss="linear", f_scale=1.0):
         """tables.py:298-333: all camera matrices (first view fixed) and all points refined against every observation.
         ftol is the reference's (tables.py:317); here it bounds the relative cost decrease of an accepted LM step.
+        loss / f_scale: the robust loss options of the reference's least_squares call, with SciPy's names and defaults
+        (see runtime.bundle_adjust); observations are C-normalised, so a scale of s pixels is f_scale = s / K[0, 0].
         Returns the solver record (cost, iters, status) — the reference returns None."""
         Rktk = np.empty((len(self.T_views), 3, 4))
         xj = np.empty((len(self.T_points), 3))
@@ -93,7 +95,8 @@ class Tables:
         for i, o in enumerate(self.T_points):
             xj[i] = o.point
         uv, cam_idx, pt_idx = self.observationArrays()
-        res = _rt.bundle_adjust(Rktk, xj, uv, cam_idx, pt_idx, n_fixed=1, max_iter=max_iter, ftol=ftol)
+        res = _rt.bundle_adjust(Rktk, xj, uv, cam_idx, pt_idx, n_fixed=1, max_iter=max_iter, ftol=ftol, loss=loss,
+                               f_scale=f_scale)
         self.updateCameras3Dpoints2(res["cams"], res["pts"])
         return {k: res[k] for k in ("cost", "iters", "status")}
 
