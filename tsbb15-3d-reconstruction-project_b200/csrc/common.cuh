@@ -203,16 +203,19 @@ struct Ctx {
     // Pass pipelining (F calls of several passes): the caller's stream runs the scorers back to back; the solver ("head") of
     // pass k+1 and the fix-up / selection / mask kernels ("tail") of pass k-1 run on a second stream BESIDE the scorer of pass k
     // — they are latency bound (23 % issue active) and one of their blocks fits next to the scorer's four on every SM.  The
-    // per-pass workspaces exist two or three times (the bounded sweep keeps a pass alive across the next pass's prefix
-    // stage); ws_use() moves the named buffers into spare[ws_slot] and those of the wanted set out of spare[slot], so all the
-    // code keeps using c->F64, c->state, ... for "the set of the pass being queued".  spare[ws_slot] is always empty.
-    struct PassSet { Buffer pair_info, pair_frame, state, pts32, F64, hyp32, flags, flag_list, best, tie_stats, bnd; } spare[3];
+    // per-pass workspaces exist two or four times (the bounded sweep keeps a pass alive from two passes before its prefix
+    // stage to two passes after it, f_run_piped); ws_use() moves the named buffers into spare[ws_slot] and those of the
+    // wanted set out of spare[slot], so all the code keeps using c->F64, c->state, ... for "the set of the pass being
+    // queued".  spare[ws_slot] is always empty.
+    static constexpr int kPassSets = 4;
+    struct PassSet { Buffer pair_info, pair_frame, state, pts32, F64, hyp32, flags, flag_list, best, tie_stats, bnd; } spare[kPassSets];
     cudaStream_t tail_stream = nullptr;
-    cudaEvent_t head_done[3] = {nullptr, nullptr, nullptr};   // recorded on the side stream after the solver of the pass in set i
-    cudaEvent_t score_done[3] = {nullptr, nullptr, nullptr};  // recorded on the caller's stream after the scorer of the pass in set i
-    cudaEvent_t cand_done[3] = {nullptr, nullptr, nullptr};   // bounded sweep: side stream, candidates of the pass in set i chosen
-    cudaEvent_t sweep_done[3] = {nullptr, nullptr, nullptr};  // bounded sweep: caller's stream, last scorer of the pass in set i
-    cudaEvent_t tail_done = nullptr;                    // recorded on the side stream behind the last tail kernel of a run
+    cudaStream_t pass_stream = nullptr;            // bounded sweep: heads and tails, apart from the small kernels between scorers
+    cudaEvent_t head_done[kPassSets] = {};   // recorded on the side stream after the solver of the pass in set i
+    cudaEvent_t score_done[kPassSets] = {};  // recorded on the caller's stream after the (latest) scorer of the pass in set i
+    cudaEvent_t cand_done[kPassSets] = {};   // bounded sweep: side stream, after the latest group of small kernels of the pass
+    cudaEvent_t sweep_done[kPassSets] = {};  // bounded sweep: caller's stream, last scorer of the pass in set i
+    cudaEvent_t tail_done = nullptr;                    // recorded on the side stream (bounded: pass_stream) behind the last tail of a run
     cudaEvent_t pipe_gate = nullptr;                    // recorded on the caller's stream before the side stream starts a run
     int tail_carve_max = -1;                            // shared-memory carve-out preference of the tail kernels: -1 never set, 0 default, 1 max
     int ws_slot = 0;                                    // which set is the current one

@@ -124,7 +124,7 @@ int rg_shutdown(void* ctx) {
         for (Buffer* b : {&o.pair_info, &o.pair_frame, &o.state, &o.pts32, &o.F64, &o.hyp32, &o.flags, &o.flag_list, &o.best,
                           &o.tie_stats, &o.bnd})
             release(*b);
-    for (int i = 0; i < 3; ++i) {
+    for (int i = 0; i < Ctx::kPassSets; ++i) {
         if (c->head_done[i]) cudaEventDestroy(c->head_done[i]);
         if (c->score_done[i]) cudaEventDestroy(c->score_done[i]);
         if (c->cand_done[i]) cudaEventDestroy(c->cand_done[i]);
@@ -133,6 +133,7 @@ int rg_shutdown(void* ctx) {
     if (c->tail_done) cudaEventDestroy(c->tail_done);
     if (c->pipe_gate) cudaEventDestroy(c->pipe_gate);
     if (c->tail_stream) cudaStreamDestroy(c->tail_stream);
+    if (c->pass_stream) cudaStreamDestroy(c->pass_stream);
     release_pinned(c->h_stage[0]);
     release_pinned(c->h_stage[1]);
     release_pinned(c->h_stats);

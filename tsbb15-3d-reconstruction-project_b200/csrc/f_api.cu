@@ -172,7 +172,8 @@ static int pipe_setup(Ctx* c) {
         RG_CUDA(cudaDeviceGetStreamPriorityRange(&lo_p, &hi_p));
         RG_CUDA(cudaStreamCreateWithPriority(&c->tail_stream, cudaStreamNonBlocking, low ? lo_p : 0));
     }
-    for (int i = 0; i < 3; ++i) {
+    if (!c->pass_stream) RG_CUDA(cudaStreamCreateWithFlags(&c->pass_stream, cudaStreamNonBlocking));
+    for (int i = 0; i < Ctx::kPassSets; ++i) {
         if (!c->head_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->head_done[i], cudaEventDisableTiming));
         if (!c->score_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->score_done[i], cudaEventDisableTiming));
         if (!c->cand_done[i]) RG_CUDA(cudaEventCreateWithFlags(&c->cand_done[i], cudaEventDisableTiming));
@@ -356,11 +357,18 @@ static int f_bnd_cands(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) 
     return RG_OK;
 }
 
-// bounded sweep, after the candidates: candidate stage + its fix-up, extension (bnd_extend, stage B), check, fallback
-// stage.  Stage B and the fallback are queued at full grid with their item counts read from the device (bnd_live_plan;
-// the fallback normally has none).  The fallback's fix-up and merge belong to the tail.
+// bounded sweep, after the candidates: five steps that alternate between a scorer launch and a group of small kernels
+// (one CTA per pair, or one CTA in all), so that a pipelined run can put each group beside the next pass's scorer:
+//   BND_CAND_STAGE  candidate stage                                                     scorer
+//   BND_EXTEND      its fix-up, bnd_extend, bnd_live_plan of stage B                    small
+//   BND_STAGE_B     prefix stage B (bound-only, the hypotheses still alive)             scorer
+//   BND_CHECK       bnd_check, bnd_live_plan of the fallback                            small
+//   BND_FALLBACK    fallback stage (normally no items)                                  scorer
+// Stage B and the fallback are queued at full grid with their item counts read from the device (bnd_live_plan).  The
+// fallback's fix-up and merge belong to the tail.  The kProfSweep marks bracket each scorer launch on its own stream.
+enum : int { BND_CAND_STAGE = 0, BND_EXTEND, BND_STAGE_B, BND_CHECK, BND_FALLBACK, BND_STEPS };
 template <int MODE>
-static int f_bnd_sweep(Ctx* c, cudaStream_t st, PassCtl& k) {
+static int f_bnd_step(Ctx* c, cudaStream_t st, PassCtl& k, int step, bool beside_scorer) {
     if (!k.scored) return RG_OK;
     const FPlan& plan = k.plan;
     const PairInfo* pi = (const PairInfo*)c->pair_info.ptr;
@@ -369,39 +377,55 @@ static int f_bnd_sweep(Ctx* c, cudaStream_t st, PassCtl& k) {
     int bps = 1, bps_b = 1, rc = score_blocks_per_sm<EpiPolicy<MODE>>(&bps);
     if (rc || (rc = score_blocks_per_sm<EpiBoundPolicy>(&bps_b))) return rc;
     constexpr size_t smem = score_smem_bytes<EpiPolicy<MODE>>();
-    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep);
-    if (plan.n_items_c > 0) {
-        score_packed<EpiPolicy<MODE>><<<std::min(plan.n_items_c, c->sm_count * bps), kScoreThreads, smem, st>>>(
-            (const float4*)c->pts32.ptr, k.bw.hypc, pc, plan.P, plan.n_items_c, k.s.sfx_c, k.flc, k.s.c_work);
+    switch (step) {
+    case BND_CAND_STAGE:
+        prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep);
+        if (plan.n_items_c > 0) {
+            score_packed<EpiPolicy<MODE>><<<std::min(plan.n_items_c, c->sm_count * bps), kScoreThreads, smem, st>>>(
+                (const float4*)c->pts32.ptr, k.bw.hypc, pc, plan.P, plan.n_items_c, k.s.sfx_c, k.flc, k.s.c_work);
+            c->last_stats[7] += 1;
+        }
+        prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 1);
+        break;
+    case BND_EXTEND:
+        if (plan.n_items_c > 0 && (rc = f_fixup_launch<MODE>(c, st, k, beside_scorer, STAGE_CAND))) return rc;
+        bnd_extend<<<plan.P, 256, 0, st>>>(k.s.counts, k.s.sfx_c, k.bw.map, pi, pc, pb, (const Hyp32*)c->hyp32.ptr, k.bw.sel,
+                                           k.bw.hypb, k.bw.mapb, k.s.n_s, k.s.mark, bstats,
+                                           !plan.bound_prefix);
         c->last_stats[7] += 1;
-    }
-    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 1);
-    if (plan.n_items_c > 0 && (rc = f_fixup_launch<MODE>(c, st, k, false, STAGE_CAND))) return rc;
-    bnd_extend<<<plan.P, 256, 0, st>>>(k.s.counts, k.s.sfx_c, k.bw.map, pi, pc, pb, (const Hyp32*)c->hyp32.ptr, k.bw.sel,
-                                       k.bw.hypb, k.bw.mapb, k.s.n_s, k.s.mark, bstats,
-                                       !plan.bound_prefix);
-    c->last_stats[7] += 1;
-    if (plan.n_items_b > 0) {
-        bnd_live_plan<<<1, kSelectThreads, 0, st>>>(pb, k.s.n_s, plan.P, k.bw.bt, k.s.b_items);
-        prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 2);
-        score_packed<EpiBoundPolicy><<<std::min(plan.n_items_b, c->sm_count * bps_b), kScoreThreads,
-                                       score_smem_bytes<EpiBoundPolicy>(), st>>>(
-            (const float4*)c->pts32.ptr, k.bw.hypb, k.bw.bt, plan.P, plan.n_items_b, k.s.cnt_b, k.fl, k.s.b_work, k.s.b_items);
-        prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 3);
+        if (plan.n_items_b > 0) {
+            bnd_live_plan<<<1, kSelectThreads, 0, st>>>(pb, k.s.n_s, plan.P, k.bw.bt, k.s.b_items);
+            c->last_stats[7] += 1;
+        }
+        break;
+    case BND_STAGE_B:
+        if (plan.n_items_b > 0) {
+            prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 2);
+            score_packed<EpiBoundPolicy><<<std::min(plan.n_items_b, c->sm_count * bps_b), kScoreThreads,
+                                           score_smem_bytes<EpiBoundPolicy>(), st>>>(
+                (const float4*)c->pts32.ptr, k.bw.hypb, k.bw.bt, plan.P, plan.n_items_b, k.s.cnt_b, k.fl, k.s.b_work,
+                k.s.b_items);
+            prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 3);
+            c->last_stats[7] += 1;
+        }
+        break;
+    case BND_CHECK:
+        bnd_check<<<plan.P, 256, 0, st>>>(k.s.counts, k.s.sfx_c, k.bw.map, k.s.cnt_b, k.bw.mapb, k.s.n_s, pi, pc, pb, k.bw.sel,
+                                          k.s.mark, bstats, !plan.bound_prefix);
+        bnd_live_plan<<<1, kSelectThreads, 0, st>>>(pf, k.s.mark, plan.P, k.bw.fb, k.s.f_items);
         c->last_stats[7] += 2;
+        break;
+    case BND_FALLBACK:
+        prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 4);
+        if (plan.n_items_f > 0) {
+            score_packed<EpiPolicy<MODE>><<<std::min(plan.n_items_f, c->sm_count * bps), kScoreThreads, smem, st>>>(
+                (const float4*)c->pts32.ptr, (const Hyp32*)c->hyp32.ptr, k.bw.fb, plan.P, plan.n_items_f, k.s.sfx_f, k.flf,
+                k.s.f_work, k.s.f_items);
+            c->last_stats[7] += 1;
+        }
+        prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 5);
+        break;
     }
-    bnd_check<<<plan.P, 256, 0, st>>>(k.s.counts, k.s.sfx_c, k.bw.map, k.s.cnt_b, k.bw.mapb, k.s.n_s, pi, pc, pb, k.bw.sel,
-                                      k.s.mark, bstats, !plan.bound_prefix);
-    bnd_live_plan<<<1, kSelectThreads, 0, st>>>(pf, k.s.mark, plan.P, k.bw.fb, k.s.f_items);
-    c->last_stats[7] += 2;
-    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 4);
-    if (plan.n_items_f > 0) {
-        score_packed<EpiPolicy<MODE>><<<std::min(plan.n_items_f, c->sm_count * bps), kScoreThreads, smem, st>>>(
-            (const float4*)c->pts32.ptr, (const Hyp32*)c->hyp32.ptr, k.bw.fb, plan.P, plan.n_items_f, k.s.sfx_f, k.flf,
-            k.s.f_work, k.s.f_items);
-        c->last_stats[7] += 1;
-    }
-    prof_mark_at(c, st, k.prof_call, Ctx::kProfSweep + 5);
     RG_CUDA(cudaGetLastError());
     return RG_OK;
 }
@@ -515,8 +539,9 @@ static int f_pass_cands(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer)
                                       : f_bnd_cands<MODE_EPI_MAX>(c, ts, k, beside_scorer);
 }
 
-static int f_pass_sweep(Ctx* c, cudaStream_t st, PassCtl& k) {
-    return (k.a.mode == MODE_SAMPSON) ? f_bnd_sweep<MODE_SAMPSON>(c, st, k) : f_bnd_sweep<MODE_EPI_MAX>(c, st, k);
+static int f_pass_bnd_step(Ctx* c, cudaStream_t st, PassCtl& k, int step, bool beside_scorer) {
+    return (k.a.mode == MODE_SAMPSON) ? f_bnd_step<MODE_SAMPSON>(c, st, k, step, beside_scorer)
+                                      : f_bnd_step<MODE_EPI_MAX>(c, st, k, step, beside_scorer);
 }
 
 static int f_pass_tail(Ctx* c, cudaStream_t ts, PassCtl& k, bool beside_scorer) {
@@ -561,7 +586,9 @@ static int f_run_serial(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs) {
     for (PassCtl& k : jobs) {
         if (k.ready) RG_CUDA(cudaStreamWaitEvent(st, k.ready, 0));
         if ((rc = f_pass_head(c, st, k)) || (rc = f_pass_score(c, st, k))) return rc;
-        if (k.a.bounded && ((rc = f_pass_cands(c, st, k, false)) || (rc = f_pass_sweep(c, st, k)))) return rc;
+        if (k.a.bounded && (rc = f_pass_cands(c, st, k, false))) return rc;
+        for (int step = 0; k.a.bounded && step < BND_STEPS; ++step)
+            if ((rc = f_pass_bnd_step(c, st, k, step, false))) return rc;
         if ((rc = f_pass_tail(c, st, k, false)) || (rc = f_pass_downloads(c, st, k))) return rc;
     }
     return RG_OK;
@@ -576,18 +603,26 @@ static int f_run_serial(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs) {
 // of pass k+2 need the same workspace set, which the side stream's own order serialises.  head(k+1) is queued before tail(k)
 // (tail(k) has to wait for score(k), head(k+1) has not).
 //
-// The bounded sweep uses THREE workspace sets (pass k lives until its tail, which follows the prefix stage of pass k+1 and its
-// own candidate stage):
+// The bounded sweep runs a pass's scorers on the caller's stream, the small kernels between them on the side stream, each
+// group beside the next scorer of the caller's stream, and its head and tail on a third stream (pass_stream).  Queued in
+// step i:
 //
-//   caller's stream :  S1(0)          S1(1)  S3+FB(0)          S1(2)  S3+FB(1)          S1(3) ...  S3+FB(n-1)        join
-//   side stream     :  head(0) head(1)  cands(0) head(2)  cands(1) tail(0) head(3)  cands(2) tail(1) head(4) ...  tail(n-1)
+//   caller's stream :  S1(i)  B(i-2)                    S3(i-1)                                 FB(i-2)     S1(i+1) ...
+//   side stream     :         check(i-2), plan_f(i-2) | cands(i) | cfix(i-1), extend(i-1), plan_b(i-1)
+//   pass_stream     :         head(i+1)                                                         tail(i-2)
 //
-// S1 = prefix stage A, cands = its fix-up + bnd_select, S3+FB = candidate stage, its fix-up, bnd_extend, bnd_live_plan,
-// prefix stage B, bnd_check, bnd_live_plan and the fallback stage, tail = fallback fix-up, bnd_merge, selection, masks.
-// The caller's stream only waits between S3 and FB for the candidate stage's fix-up, bnd_extend, the two table kernels
-// and bnd_check (small one-CTA-per-pair launches; stage B itself is a short full-grid scorer of a few hundred hypotheses
-// per pair); everything else on the side stream runs beside a scorer.
-// head(k+3) reuses pass k's set and is queued behind tail(k) on the side stream.
+// S1 = prefix stage A, cands = its fix-up + bnd_select, S3 = candidate stage, cfix = its fix-up, extend = bnd_extend,
+// plan_b / plan_f = bnd_live_plan of stage B / of the fallback, B = prefix stage B, check = bnd_check, FB = fallback stage
+// (normally no items), tail = fallback fix-up, bnd_merge, selection, masks.  Each side group waits for the scorer before
+// it and runs beside the one after it; each scorer waits only for work that ran beside a long scorer: S1(i+1) for
+// head(i+1) (beside S3(i-1)), B(i-2) for extend (beside S1(i)), S3(i-1) for cands (beside S3 of the step before), FB(i-2)
+// for check (beside S3(i-1)).  The side groups are queued in the order the caller's stream needs them.  Heads and tails
+// (≈ 3.5 ms of the 4.7 ms of a config-5 pass) have a stream of their own, so that they never hold up a side group the
+// caller's stream waits for; the tail runs beside S1(i+1), and the head waits for stage B so that its solver, a full-GPU
+// grid, runs beside S3 instead of taking the SMs S1 frees before B and S3 can.  A pass lives from its head, two steps
+// ahead, to its tail, two steps behind: the bounded sweep uses FOUR workspace sets, and head(i+1) reuses the set of pass
+// i-3 behind its tail.  A pass's score_done event is recorded behind each of its scorers and cand_done behind each of its
+// side groups (each record is waited for before the next one is queued); sweep_done follows FB.
 //
 // Either way the caller's stream ends behind the last tail (join), and the current set is the last pass's (counts_ptr / F64 /
 // flags of rg_f_last_hypotheses_dev and the prepared points).
@@ -597,16 +632,18 @@ static int f_run_piped(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs) {
     int rc;
     if ((rc = pipe_setup(c)) || (rc = tail_carveout(c, true))) return rc;
     cudaStream_t side = c->tail_stream;
-    RG_CUDA(cudaEventRecord(c->pipe_gate, st));       // the side stream may not overtake what the caller queued before the call
+    cudaStream_t hs = bounded ? c->pass_stream : side;                  // heads and tails
+    RG_CUDA(cudaEventRecord(c->pipe_gate, st));       // the side streams may not overtake what the caller queued before the call
     RG_CUDA(cudaStreamWaitEvent(side, c->pipe_gate, 0));
-    for (int k = 0; k < n; ++k) jobs[k].slot = (c->ws_slot + 1 + k) % (bounded ? 3 : 2);
-    auto head = [&](int k) -> int {                   // side stream
+    if (bounded) RG_CUDA(cudaStreamWaitEvent(hs, c->pipe_gate, 0));
+    for (int k = 0; k < n; ++k) jobs[k].slot = (c->ws_slot + 1 + k) % (bounded ? 4 : 2);
+    auto head = [&](int k) -> int {                   // stream hs
         PassCtl& j = jobs[k];
         ws_use(c, j.slot);
-        if (j.ready) RG_CUDA(cudaStreamWaitEvent(side, j.ready, 0));
-        int r = f_pass_head(c, side, j);
+        if (j.ready) RG_CUDA(cudaStreamWaitEvent(hs, j.ready, 0));
+        int r = f_pass_head(c, hs, j);
         if (r) return r;
-        RG_CUDA(cudaEventRecord(c->head_done[j.slot], side));
+        RG_CUDA(cudaEventRecord(c->head_done[j.slot], hs));
         return RG_OK;
     };
     auto score = [&](int k) -> int {                  // caller's stream
@@ -618,12 +655,12 @@ static int f_run_piped(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs) {
         RG_CUDA(cudaEventRecord(c->score_done[j.slot], st));
         return RG_OK;
     };
-    auto tail = [&](int k, cudaEvent_t gate, bool beside) -> int {      // side stream, behind `gate` of the caller's stream
+    auto tail = [&](int k, cudaEvent_t gate, bool beside) -> int {      // stream hs, behind `gate` of the caller's stream
         PassCtl& j = jobs[k];
-        RG_CUDA(cudaStreamWaitEvent(side, gate, 0));
+        RG_CUDA(cudaStreamWaitEvent(hs, gate, 0));
         ws_use(c, j.slot);
-        int r = f_pass_tail(c, side, j, beside);
-        return r ? r : f_pass_downloads(c, side, j);
+        int r = f_pass_tail(c, hs, j, beside);
+        return r ? r : f_pass_downloads(c, hs, j);
     };
     if ((rc = head(0))) return rc;
     if (!bounded) {
@@ -633,30 +670,39 @@ static int f_run_piped(Ctx* c, cudaStream_t st, std::vector<PassCtl>& jobs) {
             if ((rc = tail(k, c->score_done[jobs[k].slot], k + 1 < n))) return rc;
         }
     } else {
-        auto sweep = [&](int k) -> int {              // caller's stream
+        auto scorer = [&](int k, int step) -> int {   // caller's stream, behind the pass's last side group
             PassCtl& j = jobs[k];
             RG_CUDA(cudaStreamWaitEvent(st, c->cand_done[j.slot], 0));
             ws_use(c, j.slot);
-            int r = f_pass_sweep(c, st, j);
+            int r = f_pass_bnd_step(c, st, j, step, false);
             if (r) return r;
-            RG_CUDA(cudaEventRecord(c->sweep_done[j.slot], st));
+            RG_CUDA(cudaEventRecord(step == BND_FALLBACK ? c->sweep_done[j.slot] : c->score_done[j.slot], st));
             return RG_OK;
         };
-        if (n > 1 && (rc = head(1))) return rc;
-        for (int k = 0; k < n; ++k) {
+        auto group = [&](int k, int step, bool beside) -> int {      // side stream, behind the pass's last scorer
             PassCtl& j = jobs[k];
-            if ((rc = score(k))) return rc;
-            if (k > 0 && (rc = sweep(k - 1))) return rc;
             RG_CUDA(cudaStreamWaitEvent(side, c->score_done[j.slot], 0));
             ws_use(c, j.slot);
-            if ((rc = f_pass_cands(c, side, j, k + 1 < n))) return rc;
+            int r = step < 0 ? f_pass_cands(c, side, j, beside) : f_pass_bnd_step(c, side, j, step, beside);
+            if (r) return r;
             RG_CUDA(cudaEventRecord(c->cand_done[j.slot], side));
-            if (k > 0 && (rc = tail(k - 1, c->sweep_done[jobs[k - 1].slot], true))) return rc;
-            if (k + 2 < n && (rc = head(k + 2))) return rc;
+            return RG_OK;
+        };
+        for (int i = 0; i < n + 2; ++i) {
+            const bool beside = i < n;                // a candidate stage or a prefix stage A is still to come
+            if (i < n && (rc = score(i))) return rc;
+            if (i >= 2 && ((rc = scorer(i - 2, BND_STAGE_B)) || (rc = group(i - 2, BND_CHECK, beside)))) return rc;
+            if (i + 1 < n) {                          // head(i+1) beside S3(i-1): behind stage B, not at the end of S1
+                if (i >= 2) RG_CUDA(cudaStreamWaitEvent(hs, c->score_done[jobs[i - 2].slot], 0));
+                if ((rc = head(i + 1))) return rc;
+            }
+            if (i < n && (rc = group(i, -1, beside))) return rc;
+            if (i >= 1 && i <= n && ((rc = scorer(i - 1, BND_CAND_STAGE)) || (rc = group(i - 1, BND_EXTEND, beside)))) return rc;
+            if (i >= 2 && ((rc = scorer(i - 2, BND_FALLBACK)) || (rc = tail(i - 2, c->sweep_done[jobs[i - 2].slot], beside))))
+                return rc;
         }
-        if ((rc = sweep(n - 1)) || (rc = tail(n - 1, c->sweep_done[jobs[n - 1].slot], false))) return rc;
     }
-    RG_CUDA(cudaEventRecord(c->tail_done, side));
+    RG_CUDA(cudaEventRecord(c->tail_done, hs));       // (bounded: the side stream's last group precedes the last tail)
     RG_CUDA(cudaStreamWaitEvent(st, c->tail_done, 0));
     return RG_OK;
 }
@@ -809,6 +855,7 @@ static int f_run_passes(Ctx* c, cudaStream_t st, bool bounded, std::vector<PassC
     if (rc) {                                         // leave nothing in flight behind an error return
         cudaStreamSynchronize(st);
         if (piped && c->tail_stream) cudaStreamSynchronize(c->tail_stream);
+        if (piped && c->pass_stream) cudaStreamSynchronize(c->pass_stream);
         for (const PassCtl& j : jobs) {
             if (j.ready) cudaEventSynchronize(j.ready);       // (the host entry point's uploads)
             if (j.out_stream) cudaStreamSynchronize(j.out_stream);
