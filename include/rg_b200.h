@@ -247,6 +247,21 @@ int rg_pnp_refine_dev(void* ctx, void* stream, int V, const double* X_dev, const
 int rg_pnp_refine_host(void* ctx, void* stream, int V, const double* X, const double* y, const int32_t* view_off,
                        const double* K, const unsigned char* mask, double* Rt, int max_iter, double ftol, int rounds,
                        double thr2, unsigned char* mask_out, double* cost, int32_t* iters, int32_t* status);
+/* The same with a robust loss (SciPy's least_squares `loss` / `f_scale`; the RG_LOSS_* values and rho of
+ * rg_bundle_adjust_host2 below).  Every scalar residual f of W_v (pi(R X_k + t) - y_k) gets z = (f / C)^2, C = f_scale > 0,
+ * and cost = 0.5 * sum C^2 rho(z) (SciPy's sol.cost).  f_scale is in the units of the residuals: pixels when K is given,
+ * C-normalised otherwise.  Linearisation by iteratively reweighted least squares (weights rho'(z)); the stopping rules
+ * read the robust cost.  The consensus of rounds > 1 / mask_out is the same hard test thr2 >= e.  An unknown loss, or an
+ * f_scale that is not finite and > 0 (or whose square is 0 or not finite), is an invalid argument (-2) and nothing is
+ * enqueued.  RG_LOSS_LINEAR gives results bit-identical to rg_pnp_refine_dev / _host. */
+int rg_pnp_refine_dev2(void* ctx, void* stream, int V, const double* X_dev, const double* y_dev, const int32_t* view_off_host,
+                       const double* K_host, const unsigned char* mask_dev, double* Rt_dev, int max_iter, double ftol, int loss,
+                       double f_scale, int rounds, double thr2, unsigned char* mask_out_dev, double* cost_dev,
+                       int32_t* iters_dev, int32_t* status_dev);
+int rg_pnp_refine_host2(void* ctx, void* stream, int V, const double* X, const double* y, const int32_t* view_off,
+                        const double* K, const unsigned char* mask, double* Rt, int max_iter, double ftol, int loss,
+                        double f_scale, int rounds, double thr2, unsigned char* mask_out, double* cost, int32_t* iters,
+                        int32_t* status);
 
 /* ---- two-view geometry either side of the RANSAC path (SURVEY.md section 8f, rows N1-N3), all FP64 -------------- */
 #define RG_TRI_OPTIMAL 0    /* lab3.triangulate_optimal (lab3.py:382-475): Hartley-Sturm, degree-6 root solve per point */
@@ -305,6 +320,20 @@ int rg_gold_standard_host(void* ctx, void* stream, int P, const double* pts64, c
 int rg_gold_standard_dev(void* ctx, void* stream, int P, const double* pts64_dev, const int32_t* pair_off_host,
                          const double* F0_dev, const unsigned char* mask_dev, int max_iter, double ftol, double* F_gold_dev,
                          double* cost_dev, int32_t* iters_dev, int32_t* status_dev, double* X_dev);
+/* The same with a robust loss (SciPy's least_squares `loss` / `f_scale`, as a SciPy user adds them to the reference's
+ * call fun.py:358; the RG_LOSS_* values and rho of rg_bundle_adjust_host2 below).  Each of the four residuals of a
+ * correspondence gets z = (f / C)^2, C = f_scale > 0 in PIXELS (pts64 is in pixels), and cost = 0.5 * sum C^2 rho(z)
+ * (SciPy's sol.cost).  Linearisation by iteratively reweighted least squares (weights rho'(z) between the factors of
+ * every Jacobian product; the Schur structure is unchanged).  With mask == NULL every correspondence takes part, which
+ * makes this a refinement without a hard inlier set.  An unknown loss, or an f_scale that is not finite and > 0 (or
+ * whose square is 0 or not finite), is an invalid argument (-2) and nothing is enqueued.  RG_LOSS_LINEAR gives results
+ * bit-identical to rg_gold_standard_dev / _host. */
+int rg_gold_standard_dev2(void* ctx, void* stream, int P, const double* pts64_dev, const int32_t* pair_off_host,
+                          const double* F0_dev, const unsigned char* mask_dev, int max_iter, double ftol, int loss, double f_scale,
+                          double* F_gold_dev, double* cost_dev, int32_t* iters_dev, int32_t* status_dev, double* X_dev);
+int rg_gold_standard_host2(void* ctx, void* stream, int P, const double* pts64, const int32_t* pair_off, const double* F0,
+                           const unsigned char* mask, int max_iter, double ftol, int loss, double f_scale, double* F_gold,
+                           double* cost, int32_t* iters, int32_t* status, double* X);
 /* lab3.fmatrix_residuals_gs(params, pl, pr) (lab3.py:230-266): params = [C1.ravel() (12), X.T.ravel() (3N)], pl / pr (2, N)
  * row-major; out (4N) = leftx, lefty, rightx, righty */
 int rg_fmatrix_residuals_gs_host(void* ctx, void* stream, int N, const double* params, const double* pl, const double* pr,

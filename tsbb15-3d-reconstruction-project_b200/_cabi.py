@@ -76,8 +76,12 @@ SIGNATURES = {
     "rg_camera_resectioning_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rg_gold_standard_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
     "rg_gold_standard_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _d, _vp, _vp, _vp, _vp, _vp]),
+    "rg_gold_standard_host2": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _d, _i, _d, _vp, _vp, _vp, _vp, _vp]),
+    "rg_gold_standard_dev2": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i, _d, _i, _d, _vp, _vp, _vp, _vp, _vp]),
     "rg_pnp_refine_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _i, _d, _vp, _vp, _vp, _vp]),
     "rg_pnp_refine_dev": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _i, _d, _vp, _vp, _vp, _vp]),
+    "rg_pnp_refine_host2": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _i, _d, _i, _d, _vp, _vp, _vp, _vp]),
+    "rg_pnp_refine_dev2": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _d, _i, _d, _i, _d, _vp, _vp, _vp, _vp]),
     "rg_fmatrix_residuals_gs_host": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp]),
     "rg_bundle_adjust_host": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _d, _vp, _vp, _vp]),
     "rg_bundle_adjust_dev": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _d, _vp, _vp, _vp]),

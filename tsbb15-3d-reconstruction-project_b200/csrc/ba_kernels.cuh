@@ -74,24 +74,6 @@ __device__ __forceinline__ void ba_obs(const double* __restrict__ C, const doubl
     g.ok = isfinite(g.r0) && isfinite(g.r1) && isfinite(g.iy);
 }
 
-// rho(z) and w = rho'(z) of SciPy's losses (scipy/optimize/_lsq/least_squares.py) at z = (f / C)^2
-template <int kLoss>
-__device__ __forceinline__ void ba_rho(const double z, double& rho, double& w) {
-    if constexpr (kLoss == LOSS_SOFT_L1) {
-        const double s = sqrt(1.0 + z);
-        rho = 2.0 * (s - 1.0); w = 1.0 / s;
-    } else if constexpr (kLoss == LOSS_HUBER) {
-        if (z <= 1.0) { rho = z; w = 1.0; }
-        else { const double s = sqrt(z); rho = 2.0 * s - 1.0; w = 1.0 / s; }
-    } else if constexpr (kLoss == LOSS_CAUCHY) {
-        rho = log1p(z); w = 1.0 / (1.0 + z);
-    } else if constexpr (kLoss == LOSS_ARCTAN) {
-        rho = atan(z); w = 1.0 / fma(z, z, 1.0);
-    } else {
-        rho = z; w = 1.0;
-    }
-}
-
 // C^2 (rho(z0) + rho(z1)) of one observation, with the weights; ic = 1 / C, c2 = C^2
 template <int kLoss>
 __device__ __forceinline__ double ba_robust(const BaObs& g, const double ic, const double c2, double& w0, double& w1) {

@@ -56,6 +56,25 @@ enum : int { SOLVER_QR = 0, SOLVER_JACOBI = 1 };
 enum : int { SCORE_FP32_GUARDED = 0, SCORE_FP64 = 1, SCORE_FP32_BOUND = 2 };
 enum : int { LOSS_LINEAR = 0, LOSS_SOFT_L1 = 1, LOSS_HUBER = 2, LOSS_CAUCHY = 3, LOSS_ARCTAN = 4 };
 
+// rho(z) and w = rho'(z) of SciPy's losses (scipy/optimize/_lsq/least_squares.py) at z = (f / C)^2; shared by the
+// Levenberg-Marquardt solvers (bundle adjustment, PnP pose refinement, gold-standard refinement)
+template <int kLoss>
+__device__ __forceinline__ void ba_rho(const double z, double& rho, double& w) {
+    if constexpr (kLoss == LOSS_SOFT_L1) {
+        const double s = sqrt(1.0 + z);
+        rho = 2.0 * (s - 1.0); w = 1.0 / s;
+    } else if constexpr (kLoss == LOSS_HUBER) {
+        if (z <= 1.0) { rho = z; w = 1.0; }
+        else { const double s = sqrt(z); rho = 2.0 * s - 1.0; w = 1.0 / s; }
+    } else if constexpr (kLoss == LOSS_CAUCHY) {
+        rho = log1p(z); w = 1.0 / (1.0 + z);
+    } else if constexpr (kLoss == LOSS_ARCTAN) {
+        rho = atan(z); w = 1.0 / fma(z, z, 1.0);
+    } else {
+        rho = z; w = 1.0;
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // device-side records
 // ---------------------------------------------------------------------------------------------

@@ -4,14 +4,42 @@
 
 namespace rg {
 
+// the kernels that depend on the loss (gs_rho / gs_blocks_w inside them)
+struct GsLossKernels {
+    decltype(&gs_fused<LOSS_LINEAR>) fused;
+    decltype(&gs_accumulate<LOSS_LINEAR>) accumulate;
+    decltype(&gs_trial<LOSS_LINEAR>) trial;
+};
+
+template <int L>
+static GsLossKernels gs_loss_kernels() { return {gs_fused<L>, gs_accumulate<L>, gs_trial<L>}; }
+
+static bool gs_loss_kernels(int loss, GsLossKernels& k) {
+    switch (loss) {
+        case LOSS_LINEAR: k = gs_loss_kernels<LOSS_LINEAR>(); return true;
+        case LOSS_SOFT_L1: k = gs_loss_kernels<LOSS_SOFT_L1>(); return true;
+        case LOSS_HUBER: k = gs_loss_kernels<LOSS_HUBER>(); return true;
+        case LOSS_CAUCHY: k = gs_loss_kernels<LOSS_CAUCHY>(); return true;
+        case LOSS_ARCTAN: k = gs_loss_kernels<LOSS_ARCTAN>(); return true;
+        default: return false;
+    }
+}
+
+// loss (LOSS_*) and f_scale = C (pixels, the units of pts64): every scalar residual f contributes C^2 rho((f / C)^2) to
+// twice the cost.
 static int gold_standard_dev(Ctx* c, cudaStream_t st, int P, const double* pts64, const int* pair_off, const double* F0,
-                             const unsigned char* mask, int max_iter, double ftol, double* F_gold, double* cost, int* iters,
-                             int* status, double* X_out, bool host_paced) {
+                             const unsigned char* mask, int max_iter, double ftol, int loss, double f_scale, double* F_gold,
+                             double* cost, int* iters, int* status, double* X_out, bool host_paced) {
     RG_CHECK_ARG(P >= 0 && pair_off != nullptr, "bad pair table");
     RG_CHECK_ARG(pair_off[0] == 0, "pair_off must start at 0");
     for (int p = 0; p < P; ++p) RG_CHECK_ARG(pair_off[p + 1] >= pair_off[p], "pair_off must be non-decreasing");
     RG_CHECK_ARG(max_iter >= 0 && max_iter <= 10000, "max_iter must be in [0, 10000]");
     RG_CHECK_ARG(ftol >= 0.0 && std::isfinite(ftol), "ftol must be finite and >= 0");
+    GsLossKernels kern;
+    RG_CHECK_ARG(gs_loss_kernels(loss, kern), "loss must be one of RG_LOSS_LINEAR .. RG_LOSS_ARCTAN");
+    const double ic = 1.0 / f_scale, c2 = f_scale * f_scale;
+    RG_CHECK_ARG(std::isfinite(f_scale) && f_scale > 0.0 && std::isfinite(ic) && std::isfinite(c2) && c2 > 0.0,
+                 "f_scale must be finite and > 0 (with a finite, non-zero square)");
     RG_CUDA(cudaSetDevice(c->device));
     c->last_stats[7] = 0;
     if (P == 0) return RG_OK;
@@ -57,7 +85,8 @@ static int gold_standard_dev(Ctx* c, cudaStream_t st, int P, const double* pts64
         RG_CUDA(cudaEventRecord(c->staging_free[0], st));
         if (maxN <= kGsFusedMaxPts && !c->opt_gs_multi) {
             // small pairs: the whole LM loop of a pair in one CTA, one launch (gs_fused)
-            gs_fused<<<P, kGsFusedThreads, 0, st>>>((const double4*)pts64, mask, doff, gp, Xcur, Xtrial, C1, ftol, max_iter);
+            kern.fused<<<P, kGsFusedThreads, 0, st>>>((const double4*)pts64, mask, doff, gp, Xcur, Xtrial, C1, ftol, max_iter, ic,
+                                                          c2);
             launches += 1;
             RG_CUDA(cudaGetLastError());
         } else {
@@ -80,9 +109,9 @@ static int gold_standard_dev(Ctx* c, cudaStream_t st, int P, const double* pts64
                     RG_CUDA(cudaEventSynchronize(c->ba_iter_ev[it & 1]));      // iteration it - 2 has finished
                     if (h_act[it - 2] == 0) break;
                 }
-                gs_accumulate<<<grid, kGsThreads, 0, st>>>((const double4*)pts64, mask, doff, gp, Xcur, Xtrial, sums);
+                kern.accumulate<<<grid, kGsThreads, 0, st>>>((const double4*)pts64, mask, doff, gp, Xcur, Xtrial, sums, ic, c2);
                 gs_solve<<<ceil_div(P, kGsSolveWarps), 32 * kGsSolveWarps, 0, st>>>(gp, sums, P);
-                gs_trial<<<grid, kGsThreads, 0, st>>>((const double4*)pts64, mask, doff, gp, Xcur, Xtrial);
+                kern.trial<<<grid, kGsThreads, 0, st>>>((const double4*)pts64, mask, doff, gp, Xcur, Xtrial, ic, c2);
                 gs_accept<<<ceil_div(P, 32), 32, 0, st>>>(gp, sums, P, ftol, max_iter, h_act ? active + it : nullptr);
                 launches += 4;
                 if (h_act) {
@@ -117,17 +146,24 @@ using namespace rg;
 
 extern "C" {
 
+int rg_gold_standard_dev2(void* ctx, void* stream, int P, const double* pts64_dev, const int32_t* pair_off_host,
+                          const double* F0_dev, const unsigned char* mask_dev, int max_iter, double ftol, int loss, double f_scale,
+                          double* F_gold_dev, double* cost_dev, int32_t* iters_dev, int32_t* status_dev, double* X_dev) {
+    RG_CHECK_ARG(ctx != nullptr, "ctx is null");
+    return gold_standard_dev((Ctx*)ctx, (cudaStream_t)stream, P, pts64_dev, pair_off_host, F0_dev, mask_dev, max_iter, ftol, loss,
+                             f_scale, F_gold_dev, cost_dev, iters_dev, status_dev, X_dev, false);
+}
+
 int rg_gold_standard_dev(void* ctx, void* stream, int P, const double* pts64_dev, const int32_t* pair_off_host,
                          const double* F0_dev, const unsigned char* mask_dev, int max_iter, double ftol, double* F_gold_dev,
                          double* cost_dev, int32_t* iters_dev, int32_t* status_dev, double* X_dev) {
-    RG_CHECK_ARG(ctx != nullptr, "ctx is null");
-    return gold_standard_dev((Ctx*)ctx, (cudaStream_t)stream, P, pts64_dev, pair_off_host, F0_dev, mask_dev, max_iter, ftol,
-                             F_gold_dev, cost_dev, iters_dev, status_dev, X_dev, false);
+    return rg_gold_standard_dev2(ctx, stream, P, pts64_dev, pair_off_host, F0_dev, mask_dev, max_iter, ftol, LOSS_LINEAR, 1.0,
+                                 F_gold_dev, cost_dev, iters_dev, status_dev, X_dev);
 }
 
-int rg_gold_standard_host(void* ctx, void* stream, int P, const double* pts64, const int32_t* pair_off, const double* F0,
-                          const unsigned char* mask, int max_iter, double ftol, double* F_gold, double* cost, int32_t* iters,
-                          int32_t* status, double* X) {
+int rg_gold_standard_host2(void* ctx, void* stream, int P, const double* pts64, const int32_t* pair_off, const double* F0,
+                           const unsigned char* mask, int max_iter, double ftol, int loss, double f_scale, double* F_gold,
+                           double* cost, int32_t* iters, int32_t* status, double* X) {
     RG_CHECK_ARG(ctx != nullptr, "ctx is null");
     RG_CHECK_ARG(P >= 0 && pair_off != nullptr, "bad pair table");
     Ctx* c = (Ctx*)ctx;
@@ -151,8 +187,8 @@ int rg_gold_standard_host(void* ctx, void* stream, int P, const double* pts64, c
     int* dit = (int*)(dX + 3 * std::max<size_t>(N, 1));
     int* dst = dit + p;
     rc = gold_standard_dev(c, st, P, (const double*)c->d_in_a.ptr, pair_off, (const double*)c->d_in_b.ptr,
-                           (mask && N) ? (const unsigned char*)c->d_in_c.ptr : nullptr, max_iter, ftol, dF, dcost, dit, dst, dX,
-                           true);
+                           (mask && N) ? (const unsigned char*)c->d_in_c.ptr : nullptr, max_iter, ftol, loss, f_scale, dF, dcost,
+                           dit, dst, dX, true);
     if (rc) return rc;
     RG_CUDA(cudaMemcpyAsync(F_gold, dF, sizeof(double) * 9 * p, cudaMemcpyDeviceToHost, st));
     if (cost) RG_CUDA(cudaMemcpyAsync(cost, dcost, sizeof(double) * p, cudaMemcpyDeviceToHost, st));
@@ -161,6 +197,13 @@ int rg_gold_standard_host(void* ctx, void* stream, int P, const double* pts64, c
     if (X && N) RG_CUDA(cudaMemcpyAsync(X, dX, sizeof(double) * 3 * N, cudaMemcpyDeviceToHost, st));
     RG_CUDA(cudaStreamSynchronize(st));
     return RG_OK;
+}
+
+int rg_gold_standard_host(void* ctx, void* stream, int P, const double* pts64, const int32_t* pair_off, const double* F0,
+                          const unsigned char* mask, int max_iter, double ftol, double* F_gold, double* cost, int32_t* iters,
+                          int32_t* status, double* X) {
+    return rg_gold_standard_host2(ctx, stream, P, pts64, pair_off, F0, mask, max_iter, ftol, LOSS_LINEAR, 1.0, F_gold, cost,
+                                  iters, status, X);
 }
 
 int rg_fmatrix_residuals_gs_host(void* ctx, void* stream, int N, const double* params, const double* pl, const double* pr,

@@ -9,6 +9,8 @@
 //   J_c^T J_c = (P2^T P2) (x) (Xh Xh^T)          J_c^T J_p = (P2^T Q) (x) Xh          D = Q^T Q + Pr^T Pr
 // so the reduced camera system is  S = sum_i (M_i - T_i D_i'^-1 T_i^T) (x) (Xh_i Xh_i^T) + lambda diag(A):
 // 60 distinct products per point instead of a 12x12 block, accumulated in registers, reduced per block, atomically added.
+// A robust loss (template parameter kLoss, f_scale = C in pixels) replaces every squared residual f^2 by C^2 rho((f / C)^2)
+// and weights the products by rho' (IRLS, see gs_blocks_w); the structure above is unchanged.
 #pragma once
 #include "geom_kernels.cuh"
 
@@ -99,6 +101,42 @@ __device__ __forceinline__ bool gs_blocks(const GsPoint& g, double lambda, doubl
     for (int c = 0; c < 3; ++c)
         gp[c] = -(g.Q[0][c] * g.rl[0] + g.Q[1][c] * g.rl[1] + g.Pr[0][c] * g.rr[0] + g.Pr[1][c] * g.rr[1]);
     return inv_sym3(D, Di);
+}
+
+// Robust loss (ic = 1 / C, c2 = C^2): C^2 (sum of rho((r / C)^2) over the four residuals of g) and the weights
+// w = rho'(z) (left x, left y, right x, right y).
+template <int kLoss>
+__device__ __forceinline__ double gs_rho(const GsPoint& g, const double ic, const double c2, double (&w)[4]) {
+    const double s[4] = {g.rl[0] * ic, g.rl[1] * ic, g.rr[0] * ic, g.rr[1] * ic};
+    double sum = 0.0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        double p;
+        ba_rho<kLoss>(s[k] * s[k], p, w[k]);
+        sum += p;
+    }
+    return c2 * sum;
+}
+
+// gs_blocks for a loss: the squared loss is gs_blocks itself.  A robust loss puts Wl = diag(w0, w1), Wr = diag(w2, w3)
+// between the two factors of every product (IRLS, as in ba_kernels.cuh): M = P2^T Wl P2, T = P2^T Wl Q,
+// D = Q^T Wl Q + Pr^T Wr Pr, g_p = -(Q^T Wl rl + Pr^T Wr rr), and the callers' P2^T rl becomes P2^T Wl rl.  It does so by
+// scaling each residual of g and its rows of P2, Q, Pr by sqrt(w) in place (w > 0 for every loss), so that the
+// unweighted gs_blocks and the callers' code, with their register footprint, stay as they are; take the cost (gs_rho)
+// before.
+template <int kLoss>
+__device__ __forceinline__ bool gs_blocks_w(GsPoint& g, const double (&w)[4], double lambda, double (&M)[6], double (&T)[3][3],
+                                            double (&Di)[6], double (&gp)[3]) {
+    if constexpr (kLoss != LOSS_LINEAR) {
+#pragma unroll
+        for (int k = 0; k < 2; ++k) {
+            const double sl = sqrt(w[k]), sr = sqrt(w[2 + k]);
+            g.rl[k] *= sl; g.rr[k] *= sr;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) { g.P2[k][c] *= sl; g.Q[k][c] *= sl; g.Pr[k][c] *= sr; }
+        }
+    }
+    return gs_blocks(g, lambda, M, T, Di, gp);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -196,12 +234,13 @@ __global__ void __launch_bounds__(64) gs_init(const double* __restrict__ F0, int
 
 // ------------------------------------------------------------------------------------------------
 // LM iteration, step 1: commit the previous trial if it was accepted, accumulate the reduced camera system
-// grid = (blocks per pair, P)
+// grid = (blocks per pair, P); kLoss, ic = 1 / C, c2 = C^2: the loss (gs_rho, gs_blocks_w)
 // ------------------------------------------------------------------------------------------------
+template <int kLoss>
 __global__ void __launch_bounds__(kGsThreads) gs_accumulate(const double4* __restrict__ pts, const unsigned char* __restrict__ mask,
                                                             const int* __restrict__ pair_off, GsPair* __restrict__ gpair,
                                                             double* __restrict__ Xcur, const double* __restrict__ Xtrial,
-                                                            double* __restrict__ sums) {
+                                                            double* __restrict__ sums, double ic, double c2) {
     __shared__ double red[kGsSums];
     const int p = blockIdx.y;
     GsPair& G = gpair[p];
@@ -227,8 +266,10 @@ __global__ void __launch_bounds__(kGsThreads) gs_accumulate(const double4* __res
         GsPoint g;
         gs_point(C1, pts[i], X0, X1, X2, g);
         if (!g.ok) continue;
+        double w[4], rc = 0.0;
+        if constexpr (kLoss != LOSS_LINEAR) rc = gs_rho<kLoss>(g, ic, c2, w);
         double M[6], T[3][3], Di[6], gp[3];
-        if (!gs_blocks(g, lambda, M, T, Di, gp)) continue;
+        if (!gs_blocks_w<kLoss>(g, w, lambda, M, T, Di, gp)) continue;
         // W = M - T Di T^T  (symmetric 3x3),  z = P2^T rl + T Di gp
         double TD[3][3];
 #pragma unroll
@@ -260,7 +301,8 @@ __global__ void __launch_bounds__(kGsThreads) gs_accumulate(const double4* __res
                 acc[60 + a * 4 + b] = fma(z[a], g.Xh[b], acc[60 + a * 4 + b]);
                 acc[72 + a * 4 + b] = fma(M[sym3(a, a)], XX[sym4(b, b)], acc[72 + a * 4 + b]);
             }
-        acc[84] += g.rl[0] * g.rl[0] + g.rl[1] * g.rl[1] + g.rr[0] * g.rr[0] + g.rr[1] * g.rr[1];
+        if constexpr (kLoss == LOSS_LINEAR) acc[84] += g.rl[0] * g.rl[0] + g.rl[1] * g.rl[1] + g.rr[0] * g.rr[0] + g.rr[1] * g.rr[1];
+        else acc[84] += rc;
     }
 #pragma unroll
     for (int k = 0; k < kGsSums; ++k) {
@@ -337,9 +379,11 @@ __global__ void __launch_bounds__(32 * kGsSolveWarps) gs_solve(GsPair* __restric
 }
 
 // step 3: point steps by back-substitution, trial parameters, trial cost
+template <int kLoss>
 __global__ void __launch_bounds__(kGsThreads) gs_trial(const double4* __restrict__ pts, const unsigned char* __restrict__ mask,
                                                        const int* __restrict__ pair_off, GsPair* __restrict__ gpair,
-                                                       const double* __restrict__ Xcur, double* __restrict__ Xtrial) {
+                                                       const double* __restrict__ Xcur, double* __restrict__ Xtrial, double ic,
+                                                       double c2) {
     __shared__ double red;
     const int p = blockIdx.y;
     GsPair& G = gpair[p];
@@ -360,8 +404,9 @@ __global__ void __launch_bounds__(kGsThreads) gs_trial(const double4* __restrict
             const double4 m = pts[i];
             GsPoint g;
             gs_point(C1, m, X0, X1, X2, g);
-            double M[6], T[3][3], Di[6], gp[3];
-            if (g.ok && gs_blocks(g, lambda, M, T, Di, gp)) {
+            double M[6], T[3][3], Di[6], gp[3], w[4];
+            if constexpr (kLoss != LOSS_LINEAR) gs_rho<kLoss>(g, ic, c2, w);
+            if (g.ok && gs_blocks_w<kLoss>(g, w, lambda, M, T, Di, gp)) {
                 // delta_p = D'^-1 (-g_p - B^T dc),  (B^T dc)[c] = sum_a T[a][c] (dc[a, :] . Xh)
                 double q[3];
 #pragma unroll
@@ -375,7 +420,10 @@ __global__ void __launch_bounds__(kGsThreads) gs_trial(const double4* __restrict
                 n2 += Di[2] * rp[0] + Di[4] * rp[1] + Di[5] * rp[2];
                 GsPoint t;
                 gs_point(Cn, m, n0, n1, n2, t);
-                cost += t.ok ? t.rl[0] * t.rl[0] + t.rl[1] * t.rl[1] + t.rr[0] * t.rr[0] + t.rr[1] * t.rr[1] : INFINITY;
+                if constexpr (kLoss == LOSS_LINEAR)
+                    cost += t.ok ? t.rl[0] * t.rl[0] + t.rl[1] * t.rl[1] + t.rr[0] * t.rr[0] + t.rr[1] * t.rr[1] : INFINITY;
+                else
+                    cost += t.ok ? gs_rho<kLoss>(t, ic, c2, w) : INFINITY;
             }
         }
         Xtrial[3 * (size_t)i] = n0; Xtrial[3 * (size_t)i + 1] = n1; Xtrial[3 * (size_t)i + 2] = n2;
@@ -453,10 +501,12 @@ __device__ __forceinline__ double gs_block_sum(double v, double* sh) {      // f
     return s;
 }
 
+template <int kLoss>
 __global__ void __launch_bounds__(kGsFusedThreads) gs_fused(const double4* __restrict__ pts, const unsigned char* __restrict__ mask,
                                                             const int* __restrict__ pair_off, GsPair* __restrict__ gpair,
                                                             double* __restrict__ Xa, double* __restrict__ Xb,
-                                                            double* __restrict__ C1out, double ftol, int max_iter) {
+                                                            double* __restrict__ C1out, double ftol, int max_iter, double ic,
+                                                            double c2) {
     __shared__ double rec[kGsFusedThreads * kGsRec];
     __shared__ double part[3][84];
     __shared__ double sums[kGsSums];
@@ -500,8 +550,9 @@ __global__ void __launch_bounds__(kGsFusedThreads) gs_fused(const double4* __res
             if (i < hi && (mask == nullptr || mask[i] != 0)) {
                 GsPoint g;
                 gs_point(C1, pts[i], Xc[3 * (size_t)i], Xc[3 * (size_t)i + 1], Xc[3 * (size_t)i + 2], g);
-                double M[6], T[3][3], Di[6], gp[3];
-                if (g.ok && gs_blocks(g, lambda, M, T, Di, gp)) {
+                double M[6], T[3][3], Di[6], gp[3], w[4], rc = 0.0;
+                if constexpr (kLoss != LOSS_LINEAR) rc = gs_rho<kLoss>(g, ic, c2, w);
+                if (g.ok && gs_blocks_w<kLoss>(g, w, lambda, M, T, Di, gp)) {
                     double TD[3][3];
 #pragma unroll
                     for (int a = 0; a < 3; ++a)
@@ -517,7 +568,8 @@ __global__ void __launch_bounds__(kGsFusedThreads) gs_fused(const double4* __res
                         r[12 + a] = M[sym3(a, a)];
                         r[6 + a] = g.Xh[a];
                     }
-                    cost += g.rl[0] * g.rl[0] + g.rl[1] * g.rl[1] + g.rr[0] * g.rr[0] + g.rr[1] * g.rr[1];
+                    if constexpr (kLoss == LOSS_LINEAR) cost += g.rl[0] * g.rl[0] + g.rl[1] * g.rl[1] + g.rr[0] * g.rr[0] + g.rr[1] * g.rr[1];
+                    else cost += rc;
                     used = true;
                 }
             }
@@ -565,8 +617,9 @@ __global__ void __launch_bounds__(kGsFusedThreads) gs_fused(const double4* __res
                     const double4 m = pts[i];
                     GsPoint g;
                     gs_point(C1, m, X0, X1, X2, g);
-                    double M[6], T[3][3], Di[6], gp[3];
-                    if (g.ok && gs_blocks(g, lambda, M, T, Di, gp)) {
+                    double M[6], T[3][3], Di[6], gp[3], w[4];
+                    if constexpr (kLoss != LOSS_LINEAR) gs_rho<kLoss>(g, ic, c2, w);
+                    if (g.ok && gs_blocks_w<kLoss>(g, w, lambda, M, T, Di, gp)) {
                         double q[3];
 #pragma unroll
                         for (int a = 0; a < 3; ++a)
@@ -579,7 +632,10 @@ __global__ void __launch_bounds__(kGsFusedThreads) gs_fused(const double4* __res
                         n2 += Di[2] * rp[0] + Di[4] * rp[1] + Di[5] * rp[2];
                         GsPoint t;
                         gs_point(Cn, m, n0, n1, n2, t);
-                        tcost += t.ok ? t.rl[0] * t.rl[0] + t.rl[1] * t.rl[1] + t.rr[0] * t.rr[0] + t.rr[1] * t.rr[1] : INFINITY;
+                        if constexpr (kLoss == LOSS_LINEAR)
+                            tcost += t.ok ? t.rl[0] * t.rl[0] + t.rl[1] * t.rl[1] + t.rr[0] * t.rr[0] + t.rr[1] * t.rr[1] : INFINITY;
+                        else
+                            tcost += t.ok ? gs_rho<kLoss>(t, ic, c2, w) : INFINITY;
                     }
                 }
                 Xt[3 * (size_t)i] = n0; Xt[3 * (size_t)i + 1] = n1; Xt[3 * (size_t)i + 2] = n2;

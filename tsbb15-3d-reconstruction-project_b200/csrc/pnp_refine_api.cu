@@ -3,16 +3,43 @@
 
 namespace rg {
 
+// the kernels that depend on the loss (pr_point inside them: the weights and the robust cost)
+struct PrLossKernels {
+    decltype(&pnp_refine_fused<LOSS_LINEAR>) fused;
+    decltype(&pnp_refine_pass<LOSS_LINEAR>) pass;
+};
+
+template <int L>
+static PrLossKernels pr_loss_kernels() { return {pnp_refine_fused<L>, pnp_refine_pass<L>}; }
+
+static bool pr_loss_kernels(int loss, PrLossKernels& k) {
+    switch (loss) {
+        case LOSS_LINEAR: k = pr_loss_kernels<LOSS_LINEAR>(); return true;
+        case LOSS_SOFT_L1: k = pr_loss_kernels<LOSS_SOFT_L1>(); return true;
+        case LOSS_HUBER: k = pr_loss_kernels<LOSS_HUBER>(); return true;
+        case LOSS_CAUCHY: k = pr_loss_kernels<LOSS_CAUCHY>(); return true;
+        case LOSS_ARCTAN: k = pr_loss_kernels<LOSS_ARCTAN>(); return true;
+        default: return false;
+    }
+}
+
 // V views in CSR form (view_off host); Rt (V x 12, device) refined in place.  K_host: V x 9 row-major on the HOST (or
-// NULL): validated here, only W = K[:2, :2] is uploaded.  host_paced: see gold_standard_dev.
+// NULL): validated here, only W = K[:2, :2] is uploaded.  loss (LOSS_*) and f_scale = C: every scalar residual f (pixels
+// with K) contributes C^2 rho((f / C)^2) to twice the cost.  host_paced: see gold_standard_dev.
 static int pnp_refine_dev(Ctx* c, cudaStream_t st, int V, const double* X, const double* y, const int* view_off,
-                          const double* K_host, const unsigned char* mask, double* Rt, int max_iter, double ftol, int rounds,
-                          double thr2, unsigned char* mask_out, double* cost, int* iters, int* status, bool host_paced) {
+                          const double* K_host, const unsigned char* mask, double* Rt, int max_iter, double ftol, int loss,
+                          double f_scale, int rounds, double thr2, unsigned char* mask_out, double* cost, int* iters,
+                          int* status, bool host_paced) {
     RG_CHECK_ARG(V >= 0 && view_off != nullptr, "bad view table");
     RG_CHECK_ARG(view_off[0] == 0, "view_off must start at 0");
     for (int v = 0; v < V; ++v) RG_CHECK_ARG(view_off[v + 1] >= view_off[v], "view_off must be non-decreasing");
     RG_CHECK_ARG(max_iter >= 0 && max_iter <= 10000, "max_iter must be in [0, 10000]");
     RG_CHECK_ARG(ftol >= 0.0 && std::isfinite(ftol), "ftol must be finite and >= 0");
+    PrLossKernels kern;
+    RG_CHECK_ARG(pr_loss_kernels(loss, kern), "loss must be one of RG_LOSS_LINEAR .. RG_LOSS_ARCTAN");
+    const double ic = 1.0 / f_scale, c2 = f_scale * f_scale;
+    RG_CHECK_ARG(std::isfinite(f_scale) && f_scale > 0.0 && std::isfinite(ic) && std::isfinite(c2) && c2 > 0.0,
+                 "f_scale must be finite and > 0 (with a finite, non-zero square)");
     RG_CHECK_ARG(rounds >= 1 && rounds <= 100, "rounds must be in [1, 100]");
     const bool rescore = rounds > 1 || mask_out != nullptr;
     RG_CHECK_ARG(!rescore || (thr2 >= 0.0 && std::isfinite(thr2)), "thr2 must be finite and >= 0 when rounds > 1 or mask_out is given");
@@ -66,11 +93,11 @@ static int pnp_refine_dev(Ctx* c, cudaStream_t st, int V, const double* X, const
         pnp_refine_init<<<ceil_div(V, 64), 64, 0, st>>>(Rt, V, gv);
         launches += 1;
         if (fused) {
-            pnp_refine_fused<<<V, kPrThreads, 0, st>>>(X, y, doff, W, sel, gv, max_iter, ftol);
+            kern.fused<<<V, kPrThreads, 0, st>>>(X, y, doff, W, sel, gv, max_iter, ftol, ic, c2);
             launches += 1;
         } else {
             const dim3 grid(nb, V);
-            pnp_refine_pass<<<grid, kPrThreads, 0, st>>>(X, y, doff, W, sel, gv, part);
+            kern.pass<<<grid, kPrThreads, 0, st>>>(X, y, doff, W, sel, gv, part, ic, c2);
             pnp_refine_step<<<V, kPrThreads, 0, st>>>(gv, part, nb, 1, max_iter, ftol, nullptr);
             launches += 2;
             // host_paced (the host-buffer entry point, which synchronises anyway): the enqueue stays at most two
@@ -81,7 +108,7 @@ static int pnp_refine_dev(Ctx* c, cudaStream_t st, int V, const double* X, const
                     RG_CUDA(cudaEventSynchronize(c->pr_iter_ev[it & 1]));      // iteration it - 2 has finished
                     if (h_act[it - 2] == 0) break;
                 }
-                pnp_refine_pass<<<grid, kPrThreads, 0, st>>>(X, y, doff, W, sel, gv, part);
+                kern.pass<<<grid, kPrThreads, 0, st>>>(X, y, doff, W, sel, gv, part, ic, c2);
                 pnp_refine_step<<<V, kPrThreads, 0, st>>>(gv, part, nb, 0, max_iter, ftol, h_act ? active + it : nullptr);
                 launches += 2;
                 if (h_act) {
@@ -109,18 +136,27 @@ using namespace rg;
 
 extern "C" {
 
+int rg_pnp_refine_dev2(void* ctx, void* stream, int V, const double* X_dev, const double* y_dev, const int32_t* view_off_host,
+                       const double* K_host, const unsigned char* mask_dev, double* Rt_dev, int max_iter, double ftol, int loss,
+                       double f_scale, int rounds, double thr2, unsigned char* mask_out_dev, double* cost_dev,
+                       int32_t* iters_dev, int32_t* status_dev) {
+    RG_CHECK_ARG(ctx != nullptr, "ctx is null");
+    return pnp_refine_dev((Ctx*)ctx, (cudaStream_t)stream, V, X_dev, y_dev, view_off_host, K_host, mask_dev, Rt_dev, max_iter,
+                          ftol, loss, f_scale, rounds, thr2, mask_out_dev, cost_dev, iters_dev, status_dev, false);
+}
+
 int rg_pnp_refine_dev(void* ctx, void* stream, int V, const double* X_dev, const double* y_dev, const int32_t* view_off_host,
                       const double* K_host, const unsigned char* mask_dev, double* Rt_dev, int max_iter, double ftol,
                       int rounds, double thr2, unsigned char* mask_out_dev, double* cost_dev, int32_t* iters_dev,
                       int32_t* status_dev) {
-    RG_CHECK_ARG(ctx != nullptr, "ctx is null");
-    return pnp_refine_dev((Ctx*)ctx, (cudaStream_t)stream, V, X_dev, y_dev, view_off_host, K_host, mask_dev, Rt_dev, max_iter,
-                          ftol, rounds, thr2, mask_out_dev, cost_dev, iters_dev, status_dev, false);
+    return rg_pnp_refine_dev2(ctx, stream, V, X_dev, y_dev, view_off_host, K_host, mask_dev, Rt_dev, max_iter, ftol, LOSS_LINEAR,
+                              1.0, rounds, thr2, mask_out_dev, cost_dev, iters_dev, status_dev);
 }
 
-int rg_pnp_refine_host(void* ctx, void* stream, int V, const double* X, const double* y, const int32_t* view_off,
-                       const double* K, const unsigned char* mask, double* Rt, int max_iter, double ftol, int rounds,
-                       double thr2, unsigned char* mask_out, double* cost, int32_t* iters, int32_t* status) {
+int rg_pnp_refine_host2(void* ctx, void* stream, int V, const double* X, const double* y, const int32_t* view_off,
+                        const double* K, const unsigned char* mask, double* Rt, int max_iter, double ftol, int loss,
+                        double f_scale, int rounds, double thr2, unsigned char* mask_out, double* cost, int32_t* iters,
+                        int32_t* status) {
     RG_CHECK_ARG(ctx != nullptr, "ctx is null");
     RG_CHECK_ARG(V >= 0 && view_off != nullptr, "bad view table");
     Ctx* c = (Ctx*)ctx;
@@ -149,8 +185,8 @@ int rg_pnp_refine_host(void* ctx, void* stream, int V, const double* X, const do
     }
     RG_CUDA(cudaMemcpyAsync(dRt, Rt, sizeof(double) * 12 * v, cudaMemcpyHostToDevice, st));
     rc = pnp_refine_dev(c, st, V, (const double*)c->d_in_a.ptr, (const double*)c->d_in_c.ptr, view_off, K,
-                        (mask && N) ? dmask : nullptr, dRt, max_iter, ftol, rounds, thr2, mask_out ? dmask_out : nullptr, dcost,
-                        dit, dst, true);
+                        (mask && N) ? dmask : nullptr, dRt, max_iter, ftol, loss, f_scale, rounds, thr2,
+                        mask_out ? dmask_out : nullptr, dcost, dit, dst, true);
     if (rc) return rc;
     RG_CUDA(cudaMemcpyAsync(Rt, dRt, sizeof(double) * 12 * v, cudaMemcpyDeviceToHost, st));
     if (cost) RG_CUDA(cudaMemcpyAsync(cost, dcost, sizeof(double) * v, cudaMemcpyDeviceToHost, st));
@@ -159,6 +195,13 @@ int rg_pnp_refine_host(void* ctx, void* stream, int V, const double* X, const do
     if (mask_out && N) RG_CUDA(cudaMemcpyAsync(mask_out, dmask_out, N, cudaMemcpyDeviceToHost, st));
     RG_CUDA(cudaStreamSynchronize(st));
     return RG_OK;
+}
+
+int rg_pnp_refine_host(void* ctx, void* stream, int V, const double* X, const double* y, const int32_t* view_off,
+                       const double* K, const unsigned char* mask, double* Rt, int max_iter, double ftol, int rounds,
+                       double thr2, unsigned char* mask_out, double* cost, int32_t* iters, int32_t* status) {
+    return rg_pnp_refine_host2(ctx, stream, V, X, y, view_off, K, mask, Rt, max_iter, ftol, LOSS_LINEAR, 1.0, rounds, thr2,
+                               mask_out, cost, iters, status);
 }
 
 }  // extern "C"

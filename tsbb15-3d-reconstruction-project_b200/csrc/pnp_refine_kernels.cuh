@@ -6,6 +6,8 @@
 //   C_v(R, t) = 1/2 sum_k |W_v (pi(R X_k + t) - y_k)|^2,   pi(p) = (p0 / p2, p1 / p2),   W_v = [[fx, s], [0, fy]] or I
 // over R <- exp([dw]_x) R (Rodrigues, FP64) and t <- t + dt.  J_k = W Pi_k [-[R X_k]_x | I]: the row a of W Pi gives the
 // row [q x a | a] of J with q = R X_k.  pi is sign-agnostic (synth.pnp_scene has every point at negative depth).
+// A robust loss (template parameter kLoss, f_scale = C) replaces |r|^2 by C^2 (rho((r0 / C)^2) + rho((r1 / C)^2)) and
+// weights each scalar residual's row of J by rho' in J^T J and J^T r (IRLS, see pr_point).
 //
 // One pass over the points per iteration: at the trial pose it gives the cost AND the sums of J^T J (21) and J^T r (6);
 // an accepted step keeps them as the current system, a rejected one re-solves the saved system with a larger lambda.
@@ -40,10 +42,13 @@ __device__ __forceinline__ constexpr int sym6(int i, int j) {      // packed upp
     return i * 6 - i * (i - 1) / 2 + (j - i);
 }
 
-// one correspondence: J rows ja, jb (2 x 6) and residual (r0, r1) added to acc
+// one correspondence: J rows ja, jb (2 x 6) and residual (r0, r1) added to acc.  A robust loss (ic = 1 / C, c2 = C^2)
+// weights each scalar residual by w = rho'((r / C)^2) between the two factors of J^T J and J^T r (IRLS, as in
+// ba_kernels.cuh) and adds C^2 rho to slot 27 in place of r^2, so that 0.5 * acc[27] is SciPy's robust cost.
+template <int kLoss>
 __device__ __forceinline__ void pr_point(const double* __restrict__ P, const double w0, const double w1, const double w2,
                                          const double X0, const double X1, const double X2, const double y0, const double y1,
-                                         double (&acc)[kPrSums]) {
+                                         const double ic, const double c2, double (&acc)[kPrSums]) {
     const double q0 = P[0] * X0 + P[1] * X1 + P[2] * X2;
     const double q1 = P[3] * X0 + P[4] * X1 + P[5] * X2;
     const double q2 = P[6] * X0 + P[7] * X1 + P[8] * X2;
@@ -56,13 +61,28 @@ __device__ __forceinline__ void pr_point(const double* __restrict__ P, const dou
     const double b1 = w2 * iz, b2 = -w2 * v * iz;
     const double ja[6] = {q1 * a2 - q2 * a1, q2 * a0 - q0 * a2, q0 * a1 - q1 * a0, a0, a1, a2};
     const double jb[6] = {q1 * b2 - q2 * b1, -q0 * b2, q0 * b1, 0.0, b1, b2};
+    if constexpr (kLoss == LOSS_LINEAR) {
 #pragma unroll
-    for (int i = 0; i < 6; ++i) {
+        for (int i = 0; i < 6; ++i) {
 #pragma unroll
-        for (int j = i; j < 6; ++j) acc[sym6(i, j)] = fma(ja[i], ja[j], fma(jb[i], jb[j], acc[sym6(i, j)]));
-        acc[21 + i] = fma(ja[i], r0, fma(jb[i], r1, acc[21 + i]));
+            for (int j = i; j < 6; ++j) acc[sym6(i, j)] = fma(ja[i], ja[j], fma(jb[i], jb[j], acc[sym6(i, j)]));
+            acc[21 + i] = fma(ja[i], r0, fma(jb[i], r1, acc[21 + i]));
+        }
+        acc[27] = fma(r0, r0, fma(r1, r1, acc[27]));
+    } else {
+        const double s0 = r0 * ic, s1 = r1 * ic;
+        double p0, p1, o0, o1;
+        ba_rho<kLoss>(s0 * s0, p0, o0);
+        ba_rho<kLoss>(s1 * s1, p1, o1);
+#pragma unroll
+        for (int i = 0; i < 6; ++i) {
+            const double wa = o0 * ja[i], wb = o1 * jb[i];
+#pragma unroll
+            for (int j = i; j < 6; ++j) acc[sym6(i, j)] = fma(wa, ja[j], fma(wb, jb[j], acc[sym6(i, j)]));
+            acc[21 + i] = fma(wa, r0, fma(wb, r1, acc[21 + i]));
+        }
+        acc[27] = fma(c2, p0 + p1, acc[27]);
     }
-    acc[27] = fma(r0, r0, fma(r1, r1, acc[27]));
     acc[28] += 1.0;
 }
 
@@ -73,15 +93,17 @@ __device__ __forceinline__ void pr_weight(const double* __restrict__ W3, int v, 
 }
 
 // sums of the points [lo, hi) handled by this thread (stride `step` from `first`)
+template <int kLoss>
 __device__ __forceinline__ void pr_accumulate(const double* __restrict__ X, const double* __restrict__ y,
                                               const unsigned char* __restrict__ mask, const double* P, double w0, double w1,
-                                              double w2, int first, int hi, int step, double (&acc)[kPrSums]) {
+                                              double w2, int first, int hi, int step, double ic, double c2,
+                                              double (&acc)[kPrSums]) {
 #pragma unroll
     for (int k = 0; k < kPrSums; ++k) acc[k] = 0.0;
     for (int i = first; i < hi; i += step) {
         if (mask != nullptr && mask[i] == 0) continue;
-        pr_point(P, w0, w1, w2, X[3 * (size_t)i], X[3 * (size_t)i + 1], X[3 * (size_t)i + 2], y[2 * (size_t)i],
-                 y[2 * (size_t)i + 1], acc);
+        pr_point<kLoss>(P, w0, w1, w2, X[3 * (size_t)i], X[3 * (size_t)i + 1], X[3 * (size_t)i + 2], y[2 * (size_t)i],
+                        y[2 * (size_t)i + 1], ic, c2, acc);
     }
 }
 
@@ -256,10 +278,13 @@ __global__ void __launch_bounds__(64) pnp_refine_init(const double* __restrict__
 }
 
 // The whole loop of ONE view in ONE CTA (views of up to kPrFusedMaxPts points; the Dino views have 37-204).  grid = V.
+// kLoss, ic = 1 / C, c2 = C^2: the loss of pr_point.
+template <int kLoss>
 __global__ void __launch_bounds__(kPrThreads) pnp_refine_fused(const double* __restrict__ X, const double* __restrict__ y,
                                                                const int* __restrict__ off, const double* __restrict__ W3,
                                                                const unsigned char* __restrict__ mask,
-                                                               PrView* __restrict__ st, int max_iter, double ftol) {
+                                                               PrView* __restrict__ st, int max_iter, double ftol, double ic,
+                                                               double c2) {
     __shared__ PrView G;
     __shared__ double red[kPrWarps][kPrStride];
     __shared__ double T[kPrStride];
@@ -272,12 +297,12 @@ __global__ void __launch_bounds__(kPrThreads) pnp_refine_fused(const double* __r
     double w0, w1, w2;
     pr_weight(W3, v, w0, w1, w2);
     double acc[kPrSums];
-    pr_accumulate(X, y, mask, G.Rt, w0, w1, w2, lo + threadIdx.x, hi, kPrThreads, acc);
+    pr_accumulate<kLoss>(X, y, mask, G.Rt, w0, w1, w2, lo + threadIdx.x, hi, kPrThreads, ic, c2, acc);
     pr_block_sum(acc, red, T);
     if (threadIdx.x == 0) s_go = pr_start(G, T, max_iter, ftol) ? 1 : 0;
     __syncthreads();
     while (s_go) {
-        pr_accumulate(X, y, mask, G.Rn, w0, w1, w2, lo + threadIdx.x, hi, kPrThreads, acc);
+        pr_accumulate<kLoss>(X, y, mask, G.Rn, w0, w1, w2, lo + threadIdx.x, hi, kPrThreads, ic, c2, acc);
         pr_block_sum(acc, red, T);
         if (threadIdx.x == 0) s_go = pr_decide(G, T, true, max_iter, ftol) ? 1 : 0;
         __syncthreads();
@@ -286,10 +311,12 @@ __global__ void __launch_bounds__(kPrThreads) pnp_refine_fused(const double* __r
 }
 
 // multi-CTA path, pass: per-block partial sums at the pose G.Rn of every running view.  grid = (nb, V).
+template <int kLoss>
 __global__ void __launch_bounds__(kPrThreads) pnp_refine_pass(const double* __restrict__ X, const double* __restrict__ y,
                                                               const int* __restrict__ off, const double* __restrict__ W3,
                                                               const unsigned char* __restrict__ mask,
-                                                              const PrView* __restrict__ st, double* __restrict__ part) {
+                                                              const PrView* __restrict__ st, double* __restrict__ part,
+                                                              double ic, double c2) {
     __shared__ double red[kPrWarps][kPrStride];
     __shared__ double P[12];
     const int v = blockIdx.y;
@@ -300,7 +327,8 @@ __global__ void __launch_bounds__(kPrThreads) pnp_refine_pass(const double* __re
     double w0, w1, w2;
     pr_weight(W3, v, w0, w1, w2);
     double acc[kPrSums];
-    pr_accumulate(X, y, mask, P, w0, w1, w2, lo + blockIdx.x * kPrThreads + threadIdx.x, hi, gridDim.x * kPrThreads, acc);
+    pr_accumulate<kLoss>(X, y, mask, P, w0, w1, w2, lo + blockIdx.x * kPrThreads + threadIdx.x, hi, gridDim.x * kPrThreads,
+                         ic, c2, acc);
     double* out = part + ((size_t)v * gridDim.x + blockIdx.x) * kPrStride;
     pr_block_sum(acc, red, out);
 }

@@ -12,7 +12,7 @@ import numpy as np
 
 from . import _cabi as cabi
 from ._cabi import FLAG_BOUNDED, FLAG_REUSE_POINTS, MODE_EPI_MAX, SCORE_FP32_GUARDED, SOLVER_QR, TIE_FIRST
-from .runtime import offsets, pnp_k_table  # noqa: F401  (offsets: part of this module's interface)
+from .runtime import loss_args, offsets, pnp_k_table  # noqa: F401  (offsets: part of this module's interface)
 
 
 def _torch():
@@ -150,12 +150,13 @@ class PnpRefineOutputs:
 
 
 def pnp_refine(d_X, d_y, view_off, out: PnpOutputs, d_mask=None, K=None, max_iter=50, ftol=1e-12, rounds=1, thr2=None,
-               mask_out=None, res: PnpRefineOutputs | None = None):
+               mask_out=None, res: PnpRefineOutputs | None = None, loss="linear", f_scale=1.0):
     """rg_pnp_refine_dev: refines ``out.Rt`` IN PLACE on the current stream (Levenberg-Marquardt on the reprojection
     error, see runtime.pnp_refine_batched).  ``pnp_ransac(...)`` then ``pnp_refine(..., d_mask=out.mask)`` is the chained
     form: no host synchronisation between the two.  K: HOST (3, 3) or (V, 3, 3) array (validated before anything is
-    enqueued).  mask_out (uint8 CUDA tensor, may be out.mask) receives the last consensus (needs thr2).  Returns ``res``
-    (allocated when None)."""
+    enqueued).  mask_out (uint8 CUDA tensor, may be out.mask) receives the last consensus (needs thr2).  loss / f_scale:
+    the robust loss of runtime.pnp_refine_batched (rg_pnp_refine_dev2).  Returns ``res`` (allocated when None)."""
+    loss_id, f_scale = loss_args(loss, f_scale)
     V = len(view_off) - 1
     if int(rounds) > 1 and thr2 is None:
         raise ValueError("rounds > 1 needs thr2 (the consensus threshold)")
@@ -173,8 +174,8 @@ def pnp_refine(d_X, d_y, view_off, out: PnpOutputs, d_mask=None, K=None, max_ite
     Kt = pnp_k_table(K, V)
     if res is None:
         res = PnpRefineOutputs(V, device=_dev_index(d_X))
-    _call("rg_pnp_refine_dev", _dev_index(d_X), V, d_X, d_y, view_off, Kt, d_mask, out.Rt, max_iter, ftol, rounds,
-          0.0 if thr2 is None else thr2, mask_out, res.cost, res.iters, res.status)
+    _call("rg_pnp_refine_dev2", _dev_index(d_X), V, d_X, d_y, view_off, Kt, d_mask, out.Rt, max_iter, ftol, loss_id, f_scale,
+          rounds, 0.0 if thr2 is None else thr2, mask_out, res.cost, res.iters, res.status)
     return res
 
 

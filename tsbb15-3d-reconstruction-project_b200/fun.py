@@ -128,43 +128,50 @@ def f_ransac(p1, p2, r=10000, thr=1.5, sample_idx=None, seed=None, sampler="refe
             "idx": sample_idx}
 
 
-def gold_standard(F_guess, p1, p2, inliers):
+def gold_standard(F_guess, p1, p2, inliers, loss="linear", f_scale=1.0):
     """Gold-standard refinement of fun.py:342-369: cameras from F, optimal triangulation of the inliers, sparse-free
-    LM over (C1, X) with C2 = [I|0], F from the refined cameras."""
+    LM over (C1, X) with C2 = [I|0], F from the refined cameras.  loss / f_scale (pixels) are passed to the
+    least_squares call, as a SciPy user adds them there."""
     from scipy.optimize import least_squares
+    _rt.loss_args(loss, f_scale)
     C1, C2 = lab3.fmatrix_cameras(F_guess)
     in1 = p1[:, inliers]
     in2 = p2[:, inliers]
     X = lab3.triangulate_optimal_batch(C1, C2, in1.T, in2.T).T          # fun.py:352 loop, one GPU call
     params = np.hstack((C1.ravel(), X.T.ravel()))
-    sol = least_squares(lab3.fmatrix_residuals_gs, params, xtol=2.22e-14, tr_solver='lsmr', args=(in1, in2)).x
+    kw = {} if loss == "linear" else {"loss": loss, "f_scale": float(f_scale)}
+    sol = least_squares(lab3.fmatrix_residuals_gs, params, xtol=2.22e-14, tr_solver='lsmr', args=(in1, in2), **kw).x
     C1 = sol[:12].reshape(3, 4)
     C2 = np.hstack([np.eye(3), np.zeros((3, 1))])
     return lab3.fmatrix_from_cameras(C1, C2)
 
 
-def gold_standard_device(F_guess, p1, p2, inliers, max_iter=50, ftol=1e-12, full_output=False):
+def gold_standard_device(F_guess, p1, p2, inliers, max_iter=50, ftol=1e-12, full_output=False, loss="linear", f_scale=1.0):
     """The same minimisation as ``gold_standard`` — cameras from F, optimal triangulation, cost of
     lab3.fmatrix_residuals_gs, F from the refined cameras (fun.py:342-369) — but solved on the GPU by Levenberg-Marquardt
     with a Schur complement instead of SciPy's finite-difference trust-region solver: milliseconds instead of minutes,
-    and it reaches the minimum of the cost where the reference's solver stops early on ftol (DESIGN.md 4.5)."""
+    and it reaches the minimum of the cost where the reference's solver stops early on ftol (DESIGN.md 4.5).
+    loss / f_scale: SciPy's robust loss options (f_scale in pixels), see runtime.gold_standard."""
     p1 = np.asarray(p1, dtype=np.float64)
     p2 = np.asarray(p2, dtype=np.float64)
     pts = _rt.pack_pairs(p1[:, inliers], p2[:, inliers])
-    res = _rt.gold_standard([pts], np.asarray(F_guess, dtype=np.float64).reshape(1, 3, 3), max_iter=max_iter, ftol=ftol)
+    res = _rt.gold_standard([pts], np.asarray(F_guess, dtype=np.float64).reshape(1, 3, 3), max_iter=max_iter, ftol=ftol,
+                            loss=loss, f_scale=f_scale)
     if full_output:
         return res["F"][0], {"cost": float(res["cost"][0]), "iters": int(res["iters"][0]), "status": int(res["status"][0])}
     return res["F"][0]
 
 
 def getFFromLabCode(p1, p2, r=10000, thr=1.5, sample_idx=None, seed=None, sampler="reference", tie="reference",
-                    refine=True, device=None):
+                    refine=True, device=None, loss="linear", f_scale=1.0):
     """Drop-in for fun.getFFromLabCode(p1, p2) (fun.py:291-369): RANSAC over ``r`` 8-point hypotheses followed by the
     gold-standard refinement on the consensus set.  Returns the (3, 3) F_gold (or the RANSAC F if ``refine=False``).
 
     refine=True      the reference's own stage: SciPy least_squares on the host (same call, same stopping behaviour);
     refine="device"  the same cost minimised on the GPU (``gold_standard_device``);
-    refine=False     the RANSAC winner."""
+    refine=False     the RANSAC winner.
+    loss, f_scale    robust loss of the refine stage that runs (SciPy's names; f_scale in pixels)."""
+    _rt.loss_args(loss, f_scale)
     p1 = np.asarray(p1, dtype=np.float64)
     p2 = np.asarray(p2, dtype=np.float64)
     res = f_ransac(p1, p2, r=r, thr=thr, sample_idx=sample_idx, seed=seed, sampler=sampler, tie=tie, device=device)
@@ -174,5 +181,5 @@ def getFFromLabCode(p1, p2, r=10000, thr=1.5, sample_idx=None, seed=None, sample
     if not refine:
         return res["F"]
     if refine == "device":
-        return gold_standard_device(res["F"], p1, p2, res["inliers"])
-    return gold_standard(res["F"], p1, p2, res["inliers"])
+        return gold_standard_device(res["F"], p1, p2, res["inliers"], loss=loss, f_scale=f_scale)
+    return gold_standard(res["F"], p1, p2, res["inliers"], loss=loss, f_scale=f_scale)

@@ -46,17 +46,18 @@ def pnp_minimize(_3d_pts, img_pts, m=None):
     return _rt.pnp_minimize(X, y)
 
 
-def pnp_refine(_3d_pts, img_pts, R, t, K=None, m=None, mask=None, max_iter=50, ftol=1e-12):
+def pnp_refine(_3d_pts, img_pts, R, t, K=None, m=None, mask=None, max_iter=50, ftol=1e-12, loss="linear", f_scale=1.0):
     """Geometric refinement of a pose (the final stage of OpenCV's solvePnP(SOLVEPNP_ITERATIVE, useExtrinsicGuess) that
     the reference's cv.solvePnPRansac runs, tables.py:141): Levenberg-Marquardt on 1/2 sum |W (pi(R X + t) - y)|^2 on
     the GPU, W = K[:2, :2] (cost in pixels) or I (C-normalised units).
 
     _3d_pts, img_pts, m : as pnp_minimize;  R (3, 3), t (3,) : start pose, e.g. from pnp_minimize or ransac_robust
+    loss, f_scale : SciPy's robust loss options (f_scale in pixels with K, C-normalised without)
     Returns dict(R, t, cost, iters, status) (see runtime.pnp_refine_batched)."""
     X, y = _split_inputs(_3d_pts, img_pts, m)
     if mask is not None and m is not None:
         mask = np.asarray(mask)[:m]
-    return _rt.pnp_refine(X, y, R, t, mask=mask, K=K, max_iter=max_iter, ftol=ftol)
+    return _rt.pnp_refine(X, y, R, t, mask=mask, K=K, max_iter=max_iter, ftol=ftol, loss=loss, f_scale=f_scale)
 
 
 def p3p(_3d_pts, img_pts, K):

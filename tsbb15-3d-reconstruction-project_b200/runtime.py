@@ -310,6 +310,24 @@ def pnp_minimize(X, y, device=None, stream=0):
     return R, t
 
 
+BA_LOSSES = {"linear": cabi.LOSS_LINEAR, "soft_l1": cabi.LOSS_SOFT_L1, "huber": cabi.LOSS_HUBER, "cauchy": cabi.LOSS_CAUCHY,
+             "arctan": cabi.LOSS_ARCTAN}
+
+
+def loss_args(loss, f_scale):
+    """(loss id, f_scale) for the *2 entry points of the Levenberg-Marquardt solvers; ValueError for a loss that is not
+    one of BA_LOSSES (callables included) or an f_scale that is not a finite number > 0."""
+    if not isinstance(loss, str) or loss not in BA_LOSSES:
+        raise ValueError(f"loss must be one of {sorted(BA_LOSSES)} (callable losses are not supported), got {loss!r}")
+    try:
+        f_scale = float(f_scale)
+    except (TypeError, ValueError):
+        raise ValueError(f"f_scale must be a finite number > 0, got {f_scale!r}") from None
+    if not (np.isfinite(f_scale) and f_scale > 0.0):
+        raise ValueError(f"f_scale must be a finite number > 0, got {f_scale!r}")
+    return BA_LOSSES[loss], f_scale
+
+
 def pnp_k_table(K, V) -> np.ndarray | None:
     """K as the (V, 9) host table of rg_pnp_refine_*: None stays None, one (3, 3) is shared by every view."""
     if K is None:
@@ -325,13 +343,16 @@ def pnp_k_table(K, V) -> np.ndarray | None:
 
 
 def pnp_refine_batched(X_list, y_list, R, t, masks=None, K=None, max_iter=50, ftol=1e-12, rounds=1, thr2=None,
-                       device=None, stream=0) -> dict:
+                       device=None, stream=0, loss="linear", f_scale=1.0) -> dict:
     """Levenberg-Marquardt refinement of V PnP poses in ONE library call (rg_pnp_refine_host): per view, the minimum of
     1/2 sum |W (pi(R X + t) - y)|^2 over the selected correspondences, W = K[:2, :2] (cost in pixels) or I.
     X_list[v] (N_v, 3), y_list[v] (N_v, 2) C-normalised; R (V, 3, 3), t (V, 3) start poses; masks[v] optional selection;
     K (3, 3) or (V, 3, 3).  rounds > 1: re-score the consensus thr2 >= e at the refined pose and refine again on it.
+    loss / f_scale: SciPy's least_squares options (see bundle_adjust); every scalar residual f contributes
+    f_scale^2 rho((f / f_scale)^2), f_scale in the units of the residuals (pixels with K, C-normalised without).
     Returns dict(R, t, cost, iters, status) of the last round, plus the list ``mask`` of last consensus sets when thr2 is
     given.  status: 1 start pose not finite, 2 converged, 3 lambda > 1e12, 4 max_iter, 5 fewer than 3 points."""
+    loss_id, f_scale = loss_args(loss, f_scale)
     V = len(X_list)
     if len(y_list) != V:
         raise ValueError("X_list and y_list must have the same length")
@@ -354,7 +375,7 @@ def pnp_refine_batched(X_list, y_list, R, t, masks=None, K=None, max_iter=50, ft
     iters = np.zeros(V, dtype=np.int32)
     status = np.zeros(V, dtype=np.int32)
     mask_out = np.zeros(max(int(view_off[-1]), 1), dtype=np.uint8) if thr2 is not None else None
-    _call("rg_pnp_refine_host", device, stream, V, X, y, view_off, Kt, mask, Rt, max_iter, ftol, rounds,
+    _call("rg_pnp_refine_host2", device, stream, V, X, y, view_off, Kt, mask, Rt, max_iter, ftol, loss_id, f_scale, rounds,
           0.0 if thr2 is None else thr2, mask_out, cost, iters, status)
     R, t = _poses(Rt)
     out = {"R": R, "t": t, "cost": cost, "iters": iters, "status": status, "view_off": view_off}
@@ -362,12 +383,13 @@ def pnp_refine_batched(X_list, y_list, R, t, masks=None, K=None, max_iter=50, ft
     return out
 
 
-def pnp_refine(X, y, R, t, mask=None, K=None, max_iter=50, ftol=1e-12, rounds=1, thr2=None, device=None, stream=0) -> dict:
+def pnp_refine(X, y, R, t, mask=None, K=None, max_iter=50, ftol=1e-12, rounds=1, thr2=None, device=None, stream=0,
+               loss="linear", f_scale=1.0) -> dict:
     """pnp_refine_batched for ONE view: X (N, 3), y (N, 2), R (3, 3), t (3,), mask (N,) optional, K (3, 3) optional.
     Returns dict(R, t, cost, iters, status[, mask])."""
     r = pnp_refine_batched([X], [y], _f64(R).reshape(1, 3, 3), _f64(t).reshape(1, 3),
                            masks=None if mask is None else [mask], K=K, max_iter=max_iter, ftol=ftol, rounds=rounds,
-                           thr2=thr2, device=device, stream=stream)
+                           thr2=thr2, device=device, stream=stream, loss=loss, f_scale=f_scale)
     out = {"R": r["R"][0], "t": r["t"][0], "cost": float(r["cost"][0]), "iters": int(r["iters"][0]),
            "status": int(r["status"][0])}
     if "mask" in r:
@@ -461,10 +483,14 @@ def two_view_init(pts_list, F, K, masks=None, device=None, stream=0) -> dict:
     return {"R": R, "t": t, "which": which, "X": _split(X, off)}
 
 
-def gold_standard(pts_list, F0, masks=None, max_iter=50, ftol=1e-12, want_points=False, device=None, stream=0) -> dict:
+def gold_standard(pts_list, F0, masks=None, max_iter=50, ftol=1e-12, want_points=False, device=None, stream=0,
+                  loss="linear", f_scale=1.0) -> dict:
     """Gold-standard refinement (second half of fun.getFFromLabCode, fun.py:342-369) of P pairs in ONE library call.
     pts_list[p]: (N_p, 4) pixel rows; F0: (P, 3, 3); masks[p] optional inlier masks (zero = skip).
-    Returns dict(F (P,3,3), cost (P,), iters (P,), status (P,), X list when want_points)."""
+    loss / f_scale: SciPy's least_squares options (see bundle_adjust), f_scale in pixels; with masks=None and a robust
+    loss every correspondence takes part and the loss bounds the pull of the outliers.
+    Returns dict(F (P,3,3), cost (P,) = 0.5 * sum f_scale^2 rho, iters (P,), status (P,), X list when want_points)."""
+    loss_id, f_scale = loss_args(loss, f_scale)
     P = len(pts_list)
     F0 = _f64(F0).reshape(-1, 3, 3)
     if F0.shape[0] != P:
@@ -476,7 +502,8 @@ def gold_standard(pts_list, F0, masks=None, max_iter=50, ftol=1e-12, want_points
     iters = np.zeros(P, dtype=np.int32)
     status = np.zeros(P, dtype=np.int32)
     X = np.full((int(off[-1]), 3), np.nan) if want_points else None
-    _call("rg_gold_standard_host", device, stream, P, pts, off, F0, mask, max_iter, ftol, F, cost, iters, status, X)
+    _call("rg_gold_standard_host2", device, stream, P, pts, off, F0, mask, max_iter, ftol, loss_id, f_scale, F, cost, iters,
+          status, X)
     out = {"F": F, "cost": cost, "iters": iters, "status": status}
     out.update(_split_wanted(X=(X, off)))
     return out
@@ -493,10 +520,6 @@ def fmatrix_residuals_gs(params, pl, pr, device=None, stream=0):
     return out
 
 
-BA_LOSSES = {"linear": cabi.LOSS_LINEAR, "soft_l1": cabi.LOSS_SOFT_L1, "huber": cabi.LOSS_HUBER, "cauchy": cabi.LOSS_CAUCHY,
-             "arctan": cabi.LOSS_ARCTAN}
-
-
 def bundle_adjust(cams, pts, uv, cam_idx, pt_idx, n_fixed=1, max_iter=50, ftol=1e-4, device=None, stream=0, loss="linear",
                   f_scale=1.0) -> dict:
     """Bundle adjustment (the minimisation of tables.Tables.BundleAdjustment2, tables.py:260-333) in ONE library call.
@@ -507,14 +530,7 @@ def bundle_adjust(cams, pts, uv, cam_idx, pt_idx, n_fixed=1, max_iter=50, ftol=1
     of s pixels is f_scale = s / K[0, 0].
     Returns dict(cams, pts, cost = 0.5 * sum f_scale^2 rho (0.5 * sum r^2 for "linear"), iters, status: 2 converged,
     3 no further descent, 4 max_iter)."""
-    if not isinstance(loss, str) or loss not in BA_LOSSES:
-        raise ValueError(f"loss must be one of {sorted(BA_LOSSES)} (callable losses are not supported), got {loss!r}")
-    try:
-        f_scale = float(f_scale)
-    except (TypeError, ValueError):
-        raise ValueError(f"f_scale must be a finite number > 0, got {f_scale!r}") from None
-    if not (np.isfinite(f_scale) and f_scale > 0.0):
-        raise ValueError(f"f_scale must be a finite number > 0, got {f_scale!r}")
+    loss_id, f_scale = loss_args(loss, f_scale)
     cams = np.array(cams, dtype=np.float64).reshape(-1, 3, 4)
     pts = np.array(pts, dtype=np.float64).reshape(-1, 3)
     uv = _f64(uv).reshape(-1, 2)
@@ -525,7 +541,7 @@ def bundle_adjust(cams, pts, uv, cam_idx, pt_idx, n_fixed=1, max_iter=50, ftol=1
     cost = np.full(1, np.nan)
     it_st = np.zeros(2, dtype=np.int32)
     _call("rg_bundle_adjust_host2", device, stream, cams.shape[0], pts.shape[0], uv.shape[0], cams, pts, uv, ci, pi,
-          n_fixed, max_iter, ftol, BA_LOSSES[loss], f_scale, cost, it_st[:1], it_st[1:])
+          n_fixed, max_iter, ftol, loss_id, f_scale, cost, it_st[:1], it_st[1:])
     return {"cams": cams, "pts": pts, "cost": float(cost[0]), "iters": int(it_st[0]), "status": int(it_st[1])}
 
 

@@ -132,7 +132,7 @@ class Tables:
         return np.where(hit >= 0, obs_idx[np.maximum(hit, 0)], -1)
 
     def addNewView(self, K, img_index, y1_hom, y2_hom, y1, y2, r=1024, reproj_px=8.0, n=6, seed=0, sample_idx=None,
-                   refine="algebraic"):
+                   refine="algebraic", loss="linear", f_scale=1.0):
         """Adds the view seen in image ``img_index``: pose from the 2D<->3D correspondences found through the last view
         (PnP-RANSAC), consensus observations appended to the tables.  Returns (A_y1, A_y2): the putative
         correspondences without a 3-D point yet, exactly as the reference does.
@@ -141,9 +141,14 @@ class Tables:
         iterations, 8 px reprojection error); reproj_px is converted to C-normalised units with K[0, 0].
         refine : "algebraic" (default) refits the pose algebraically on the consensus set (runtime.pnp_minimize);
         "lm" minimises the reprojection error in pixels with K on the consensus set (runtime.pnp_refine), the final
-        stage of OpenCV's solvePnPRansac; the consensus appended is RANSAC's, as solvePnPRansac returns it."""
+        stage of OpenCV's solvePnPRansac; the consensus appended is RANSAC's, as solvePnPRansac returns it.
+        loss, f_scale : robust loss of the "lm" refinement (SciPy's names, see runtime.pnp_refine_batched); f_scale is in
+        pixels.  A loss other than "linear" needs refine="lm"."""
         if refine not in ("algebraic", "lm"):
             raise ValueError("refine must be 'algebraic' or 'lm'")
+        _rt.loss_args(loss, f_scale)
+        if loss != "linear" and refine != "lm":
+            raise ValueError(f"loss={loss!r} needs refine='lm' (the algebraic refit has no loss)")
         y1_hom = np.asarray(y1_hom, dtype=np.float64)
         y2_hom = np.asarray(y2_hom, dtype=np.float64)
         y1 = np.asarray(y1, dtype=np.float64)
@@ -168,7 +173,8 @@ class Tables:
         R, t = res["R"], res["t"]
         if refine == "lm":
             # np.triu: K of an RQ factorisation can carry rounding dust below the diagonal
-            ref = _rt.pnp_refine(D_3Dpoints, yn, R, t, mask=res["mask"], K=np.triu(np.asarray(K, dtype=np.float64)))
+            ref = _rt.pnp_refine(D_3Dpoints, yn, R, t, mask=res["mask"], K=np.triu(np.asarray(K, dtype=np.float64)),
+                                 loss=loss, f_scale=f_scale)
             R, t = ref["R"], ref["t"]
         elif inl.size >= 6:                                 # refit on the consensus set (OpenCV refines its winner too)
             R, t = _rt.pnp_minimize(D_3Dpoints[inl], yn[inl])
